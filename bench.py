@@ -2,6 +2,7 @@
 """bench.py — move-and-slide capsule queries/sec (BASELINE.json metric), one process per GPU.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--only NAME] [--no-extras]
+                  [--dump-outputs DIR]
 
 Headline workload (config C3 of BASELINE.json / SURVEY.md §8d): 1,048,576 characters per GPU, one fixed step of
 the reference's KinematicMoveStopSystem body each (gravity -> decay -> velocity gate -> depenetration ->
@@ -26,6 +27,10 @@ A "step" = one pass of the hot path over the whole batch; state is carried from 
 Multi-GPU: units are sharded across ranks (contiguous ranges), mesh + trees are replicated, no data-path collective in
 the move-and-slide step (weak scaling); torch.distributed is plumbing for the barrier, the max-over-ranks and the
 broadcast of the 128-byte NCCL id.
+
+Every configuration times exactly K steps.  --dump-outputs DIR writes the character records of the headline path as
+they stand after its last timed step (rank 0's characters) as DIR/<field>.npy; the inputs are seeded, so two builds run
+with the same arguments can be compared output for output (see dump_outputs).
 """
 import argparse
 import importlib
@@ -41,6 +46,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark leaves nothing in it
 
 # Libraries (NCCL, torch) may print to stdout; the contract is ONE JSON line there.  Keep the real stdout aside
 # and send everything else to stderr.
@@ -80,6 +86,28 @@ SEED = 0xC0111DE3
 DT = 1.0 / 60.0
 GRAVITY = (0.0, -98.0, 0.0)
 FP32_PEAK_TINST = 148 * 128 * 1.965e9 / 1e12  # lanes x clock: issue ceiling with FMA off (1 flop / lane / clk)
+DUMP_LIMIT = 64_000_000  # --dump-outputs: bytes of all the .npy files together
+DUMP_SEED = 0xC0111DE6
+
+
+def dump_outputs(out_dir, records, skip=("_pad",)):
+    """--dump-outputs: every field of `records` as out_dir/<field>.npy.  Float fields keep their precision; integer and
+    flag fields become float64, which holds every 32-bit value exactly.  When all records would not fit in DUMP_LIMIT, a
+    fixed, seeded sample of them is written (the same records in every run of the same size); record_index.npy holds
+    which records were written, in ascending order."""
+    names = [f for f in records.dtype.names if f not in skip]
+
+    def as_float(a):
+        return a.astype(a.dtype if a.dtype.kind == "f" else np.float64)
+
+    per_record = 8 + sum(as_float(records[f][:1]).itemsize * int(np.prod(records.dtype[f].shape)) for f in names)
+    keep = min(len(records), (DUMP_LIMIT - 256 * (len(names) + 1)) // per_record)  # 256: room for each .npy header
+    idx = np.arange(len(records)) if keep == len(records) else \
+        np.sort(np.random.default_rng(DUMP_SEED).choice(len(records), keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "record_index.npy"), idx.astype(np.float64))
+    for f in names:
+        np.save(os.path.join(out_dir, f + ".npy"), as_float(records[f][idx]))
 
 
 def load_peaks():
@@ -371,8 +399,9 @@ def roofline_block(kernel, kernel_ms, algo_bytes, evals, per_query, traffic):
 
 
 # ------------------------------------------------------------------------------------------ move-and-slide (C3 / terrain)
-def measure_mas(ctx, args, mesh, n, steps, warmup, cpu_baseline=True, clocks=True, full_record_e2e=True):
-    """One move-and-slide configuration: device-resident value, roofline, e2e legs, optional CPU baseline."""
+def measure_mas(ctx, args, mesh, n, steps, warmup, cpu_baseline=True, clocks=True, full_record_e2e=True, dump_dir=None):
+    """One move-and-slide configuration: device-resident value, roofline, e2e legs, optional CPU baseline.  dump_dir: where
+    rank 0 writes its character records as the last timed step left them (dump_outputs)."""
     cq, torch = ctx.cq, ctx.torch
     agents = args.agents if mesh == "terrain" else 0.0
     parts, pos, vel = make_workload(cq, mesh, n, ctx.rank, agents, args.cells)
@@ -527,6 +556,8 @@ def measure_mas(ctx, args, mesh, n, steps, warmup, cpu_baseline=True, clocks=Tru
             cpu["gpu_step_bit_identical_to_this_run"] = bool(g1.tobytes() == sub.tobytes())
         ow.close()
     world.close()
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, final_np)
     return {
         "metric": "move_and_slide_queries_per_sec", "value": value, "unit": "queries/s", "n_gpus": ctx.ws,
         "steps": steps, "warmup": warmup, "ms_per_step": total_ms / steps, "higher_is_better": True,
@@ -907,7 +938,7 @@ def run_ours(args):
     only = args.only
     line = None
     if only in (None, "c3"):
-        line = measure_mas(ctx, args, args.mesh, args.chars, args.steps, args.warmup)
+        line = measure_mas(ctx, args, args.mesh, args.chars, args.steps, args.warmup, dump_dir=args.dump_outputs)
     extras = {}
 
     def extra(name, fn):
@@ -921,18 +952,18 @@ def run_ours(args):
             extras[name] = {"error": f"{type(e).__name__}: {e}", "trace": traceback.format_exc()[-1500:]}
         ctx.barrier()
 
-    ks, kw = max(3, min(args.steps, 10)), 3
+    ks, kw = args.steps, 3
     multi = ctx.ws > 1
     if only is not None or (args.mesh == "hulls" and args.agents == 0):
         extra("terrain", lambda: measure_mas(ctx, args, "terrain", args.chars, ks, kw, cpu_baseline=True, clocks=False,
                                              full_record_e2e=False))
-        extra("c4", lambda: measure_c4(ctx, args, args.queries or (1 << 23), max(3, ks // 2), kw, sharded=multi))
+        extra("c4", lambda: measure_c4(ctx, args, args.queries or (1 << 23), ks, kw, sharded=multi))
         _TERRAIN.clear()
         if not multi:
-            extra("render", lambda: measure_mas(ctx, args, "render", args.chars, max(3, ks // 2), kw, cpu_baseline=True,
+            extra("render", lambda: measure_mas(ctx, args, "render", args.chars, ks, kw, cpu_baseline=True,
                                                 clocks=False, full_record_e2e=False))
-            extra("c2", lambda: measure_c2(ctx, args, args.queries or 65536, max(3, ks // 2), kw))
-        extra("c5", lambda: measure_c5(ctx, args, args.queries or (1 << 24), max(3, ks // 2), kw, sharded=multi))
+            extra("c2", lambda: measure_c2(ctx, args, args.queries or 65536, ks, kw))
+        extra("c5", lambda: measure_c5(ctx, args, args.queries or (1 << 24), ks, kw, sharded=multi))
         if multi:
             extra("c3_strong", lambda: measure_c3_strong(ctx, args, CHARS_PER_GPU, ks, kw))
     if ctx.rank == 0:
@@ -970,7 +1001,13 @@ def main():
     ap.add_argument("--ref-sample", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--gather", action="store_true", help="(kept for compatibility: sharded c4 always gathers)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline path's character records as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or (args.only or args.workload) not in (None, "c3")):
+        ap.error("--dump-outputs writes the move-and-slide headline's records: use it with --impl ours and no other --only")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload and not args.only:
         args.only = args.workload

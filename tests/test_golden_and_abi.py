@@ -298,8 +298,9 @@ def test_sharded_characters_equal_single_rank_gloo(tmp_path):
     script = tmp_path / "worker.py"
     script.write_text(_GLOO_WORKER)
     env = dict(os.environ, MASTER_ADDR="127.0.0.1", OMP_NUM_THREADS="1")
-    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2",
-                          "--master-addr", "127.0.0.1", "--master-port", "29517", str(script), ROOT],
+    # --standalone: the rendezvous takes a free local port, so runs on a shared host do not collide
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nproc-per-node=2",
+                          str(script), ROOT],
                          capture_output=True, text=True, env=env, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "GLOO_OK" in out.stdout
