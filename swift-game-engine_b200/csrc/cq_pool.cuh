@@ -447,8 +447,23 @@ __device__ __forceinline__ void pool_take_jobs(const WorldView &W, const WarpPoo
 // where candidates are many (C2: distance evaluations per sweep 5352 -> 4108, 32.8 -> 28.1 ms) and loses 1% on C4; the
 // move-and-slide kernel LOSES 3-5% on the hulls and terrain scenes (few candidates per query, the extra compares and the
 // longer loop body cost more than the 1.5% of evaluations they save), so only the query kernels instantiate it.
+// Bisection steps a bound decides (exact-safe, DESIGN.md §5.1 "Decided bisection steps"): the capsule only translates
+// along a unit direction, so the distance is 1-Lipschitz in t up to the float error `margin`; once this trip's evaluation
+// at tc returned dist, a refineTOI midpoint m with |m - tc| + margin < |dist - radius| would evaluate to the same side
+// of the radius and is applied without evaluating it.  The midpoints are the same floats 0.5f * (lo + hi), so lo and hi
+// end bit-identical.  No prediction for capsules of radius <= 5 mm (a missed piercing of a nearly vertical triangle can
+// read up to 4.6 mm) or half height > 16 radii (near-parallel edge error), nor in reference-stats counting launches.
+// Only the plain-walk kernels (worlds below 4096 triangles) instantiate it: measured on one box (profiles/r3_ab_same_box.txt)
+// the hulls step gains 13.5% (evaluations per character-step 27.9 -> 17.5), but the staged-walk kernels lose more to the
+// longer loop than they save (terrain +4.4%, C4 +2.6% for 6% / 2.5% fewer evaluations; render and C2 gain 3%).
+__device__ __forceinline__ float bisect_margin(const QShared &s, float radius, float hh) {
+    const volatile float *f = s.from; // (re-read: the copies loaded for the centre would stay live across the distance function)
+    const float scale = fabsf(f[0]) + fabsf(f[1]) + fabsf(f[2]) + s.L + hh + radius;
+    return radius > 5e-3f && hh <= 16.0f * radius ? scale * 1.9073486e-6f /* 16 * 2^-23 */ : INFINITY;
+}
+
 template <bool COUNT, bool LOOKAHEAD>
-__device__ __forceinline__ void pool_eval(Job &job, const WarpPool &wp, Commit &cm, bool &retired, Counters &ctr) {
+__device__ __forceinline__ void pool_eval(Job &job, const WarpPool &wp, Commit &cm, bool &retired, Counters &ctr, bool predict) {
     const int ph = job.phase;
     const QShared &s = wp.qs[job.owner()];
     float &hi = job.t, &lo = job.lastSafeT; // (slots shared between the phases, see Job)
@@ -502,13 +517,27 @@ __device__ __forceinline__ void pool_eval(Job &job, const WarpPool &wp, Commit &
         if (dist <= job.radius) hi = tc;
         else lo = tc;
         job.it++;
+    }
+    if (job.phase == PH_BIS && !retired) { // (also right after the PH_ADV -> PH_BIS transition)
+        const float margin = bisect_margin(s, job.radius, job.hh), gap = fabsf(dist - job.radius);
+#pragma unroll 1
+        for (; predict && job.it < 10; job.it++) { // decided steps (a NaN dist never decides)
+            const float mid = 0.5f * (lo + hi);
+            if (!(fabsf(mid - tc) + margin < gap)) break;
+            if (dist <= job.radius) hi = mid;
+            else lo = mid;
+        }
         if (job.it == 10) {
             if (hopeless(hi)) retired = true;
             else job.phase = PH_FIN;
         } else if (lo > bestT) {
             retired = true;
         }
-    } else if (ph == PH_FIN) { // contact at tHit = hi, :1325-1346; acceptance filters of :1087-1097
+    }
+    // PH_FIN evaluates at hi: when that is this trip's point (the last bisection step evaluated had contact, or the
+    // hi - lo < 1e-5 entry with hi = t), the centre, and so dist / sp / tp, are bit-identical: finish in this trip.
+    if (job.phase == PH_FIN && !retired && (ph == PH_FIN || (predict && __float_as_uint(hi) == __float_as_uint(tc)))) {
+        // contact at tHit = hi, :1325-1346; acceptance filters of :1087-1097
         retired = true;
         f3 triNormal = normalize(cross(job.T.v1 - job.T.v0, job.T.v2 - job.T.v0));
         f3 n;
@@ -531,7 +560,7 @@ __device__ __forceinline__ void pool_eval(Job &job, const WarpPool &wp, Commit &
             cm.n = n;
             cm.triN = triN;
         }
-    } else { // PH_OVL: capsuleOverlapBVHAll leaf body, :1248-1271
+    } else if (ph == PH_OVL) { // capsuleOverlapBVHAll leaf body, :1248-1271
         retired = true;
         if (dist < job.radius) {
             f3 triNormal = normalize(cross(job.T.v1 - job.T.v0, job.T.v2 - job.T.v0));
@@ -780,7 +809,7 @@ __device__ __forceinline__ void pool_run(const WorldView &W, const WarpPool &wp,
         cm.kind = 0;
         bool retired = false;
 #if CQ_EVAL_REPS <= 1
-        if (job.phase != PH_NONE) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr);
+        if (job.phase != PH_NONE) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr, !STAGED && !(COUNT && W.refStats));
 #else
         // Up to CQ_EVAL_REPS evaluations per trip while at least CQ_EVAL_KEEP lanes still hold a live pair: pickup, commit
         // and the exit vote are then paid once per several evaluations.  Exact: a finished pair keeps its contribution
@@ -790,7 +819,7 @@ __device__ __forceinline__ void pool_run(const WorldView &W, const WarpPool &wp,
             const bool go = job.phase != PH_NONE && !retired;
             const uint32_t live = (uint32_t)__popc(__ballot_sync(0xffffffffu, go));
             if (live == 0u || (rep > 0 && live < (uint32_t)CQ_EVAL_KEEP)) break;
-            if (go) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr);
+            if (go) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr, !STAGED && !(COUNT && W.refStats));
         }
 #endif
         pool_commit<LOOKAHEAD || (STAGED && FE_IDLE >= 16) || CQ_COMMIT_REDUCE_MAS>(wp, job, cm, retired, lane, ovl);
