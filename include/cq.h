@@ -78,7 +78,7 @@ typedef struct cq_world_info {
     int32_t n_parts;
     int32_t device;
     float build_ms;              /* device time of upload+filter+Morton+sort+tree+fit */
-    float refit_ms;              /* device time of the last cq_world_update_transforms */
+    float refit_ms;              /* device time of the last cq_world_update_transforms (the async call leaves it unchanged) */
     int32_t order;               /* CQ_ORDER_* the world was created with */
     float ref_order_ms;          /* host time of the reference-order build (0 in canonical order) */
     int32_t n_ref_nodes;         /* nodes of the reference's own tree, both sets (0 in canonical order) */
@@ -142,6 +142,30 @@ int cq_world_get_info(const cq_world *w, cq_world_info *info);
  * bounds (no degenerate re-filter), refit the BVH.  models = n * 16 floats. */
 int cq_world_update_transforms(cq_world *w, const uint32_t *entity_ids,
                                const float *models, int32_t n);
+
+/* Stream-ordered twin of cq_world_update_transforms.  entity_ids / models are HOST arrays (n, n*16 floats, column-major
+ * like cq_mesh_part.model); they are copied before the call returns, so the caller may reuse them at once.  stream: a
+ * cudaStream_t cast to void*, NULL = the world's own stream.  Nothing is synchronised.
+ *
+ * Same semantics as the synchronous call: every id is checked before anything is queued (an unknown id returns
+ * CQ_ERR_NOT_FOUND and queues nothing); n == 0 is a no-op; n < 0, or a NULL array with n > 0, returns CQ_ERR_INVALID;
+ * every part with a matching entity_id takes the model, parts that contributed no triangle are skipped
+ * (CollisionQuery.swift:427), and an id named twice takes its last model.  A set is refitted in full when at least a
+ * quarter of its triangles moved (or CQ_REFIT_FULL is set in the environment), else only the moved leaves' ancestors;
+ * either way a fixed number of kernel launches per set (at most 8) plus one host-to-device copy, however many parts moved.
+ * refit_ms is left unchanged.
+ *
+ * Ordering contract (both calls):
+ *  - the refit starts only after every launch already queued on this world, on any stream, has finished reading the
+ *    trees: queries, crowd steps, agent separation and earlier refits alike;
+ *  - every call made on the world after this one returns sees the new trees, whatever its stream: the *_device twins,
+ *    the host-pointer batches, cq_crowd_step, agent separation, cq_world_read_soup and cq_world_read_counters.
+ *
+ * Back-pressure: the id -> part table is staged in one of 4 pinned slots of the world; a slot is reused once its copy has
+ * completed.  When all 4 are still in flight the call waits on the host for the oldest copy, so at most 4 table
+ * copies are queued at once.  A call that stages more parts than any call before it allocates larger staging buffers (pinned host and
+ * device memory); cq_world_destroy frees them. */
+int cq_world_update_transforms_async(cq_world *w, const uint32_t *entity_ids, const float *models, int32_t n, void *stream);
 
 /* Read back the world-space soup (testing / material lookup on the host).
  * which: 0 = static set, 1 = dynamic set.  Any out pointer may be NULL. */
@@ -257,7 +281,8 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  * enqueued on any number of streams (from one host thread at a time): the
  * world's scratch blocks are handed from stream to stream behind events, so up
  * to four launches overlap and further ones queue behind them.
- * cq_world_update_transforms and cq_world_destroy wait for everything in flight. */
+ * cq_world_update_transforms and cq_world_destroy wait for everything in flight; cq_world_update_transforms_async is
+ * ordered against them by events instead (see its ordering contract). */
 int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, void *stream);
 int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode,
                            cq_cast_hit *d_out, void *stream);

@@ -127,7 +127,8 @@ class Counters(C.Structure):
 
 
 EXPORTS = [
-    "cq_world_create", "cq_world_create_ex", "cq_world_options_default", "cq_world_destroy", "cq_world_get_info", "cq_world_update_transforms", "cq_world_read_soup",
+    "cq_world_create", "cq_world_create_ex", "cq_world_options_default", "cq_world_destroy", "cq_world_get_info", "cq_world_update_transforms",
+    "cq_world_update_transforms_async", "cq_world_read_soup",
     "cq_world_triangle_material", "cq_static_mesh_load", "cq_static_mesh_free", "cq_static_mesh_part_count",
     "cq_static_mesh_part_name", "cq_static_mesh_part_transform", "cq_static_mesh_hull_count",
     "cq_static_mesh_geometry", "cq_raycast_batch", "cq_capsule_cast_batch", "cq_capsule_overlap_batch",
@@ -194,6 +195,7 @@ def lib():
         L.cq_world_destroy.argtypes = [vp]
         L.cq_world_get_info.argtypes = [vp, C.POINTER(WorldInfo)]
         L.cq_world_update_transforms.argtypes = [vp, vp, vp, i32]
+        L.cq_world_update_transforms_async.argtypes = [vp, vp, vp, i32, vp]
         L.cq_world_read_soup.argtypes = [vp, i32, vp, vp, vp, vp, vp]
         L.cq_world_triangle_material.argtypes = [vp, i32, C.POINTER(Material)]
         L.cq_static_mesh_load.argtypes = [C.c_char_p, C.POINTER(vp)]
@@ -426,6 +428,15 @@ class CollisionQuery:
 
     updateStaticTransforms = update_transforms
     updateDynamicTransforms = update_transforms
+
+    def update_transforms_async(self, entity_ids, models, stream=None):
+        """cq_world_update_transforms_async: the same update queued on `stream` (a cudaStream_t handle such as
+        torch.cuda.Stream().cuda_stream; None = the world's own stream) without synchronising.  The arrays are copied
+        before the call returns; every later call on the world, on any stream, sees the new pose."""
+        ids = np.ascontiguousarray(entity_ids, np.uint32)
+        m = np.ascontiguousarray(models, np.float32).reshape(-1, 16)
+        assert m.shape[0] == ids.shape[0]
+        _check(lib().cq_world_update_transforms_async(self._h, _ptr(ids), _ptr(m), len(ids), C.c_void_p(stream) if stream else None))
 
     # raycast(origin:direction:maxDistance:mask:) (CollisionQuery.swift:85)
     def raycast(self, rays, with_flags=False):

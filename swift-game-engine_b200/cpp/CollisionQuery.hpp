@@ -70,6 +70,11 @@ class CollisionQuery {
     bool updateTransforms(const std::vector<uint32_t> &entities, const std::vector<float> &models16) {
         return cq_world_update_transforms(w_, entities.data(), models16.data(), (int32_t)entities.size()) == CQ_OK;
     }
+    // the same update queued on `stream` (a cudaStream_t; nullptr = the world's own stream) without waiting; the arrays are
+    // copied before the call returns, and every later call on the world sees the new pose (include/cq.h)
+    bool updateTransformsAsync(const std::vector<uint32_t> &entities, const std::vector<float> &models16, void *stream = nullptr) {
+        return cq_world_update_transforms_async(w_, entities.data(), models16.data(), (int32_t)entities.size(), stream) == CQ_OK;
+    }
 
     std::optional<RaycastHit> raycast(Float3 origin, Float3 direction, float maxDistance, uint32_t mask = CQ_LAYER_ALL) {
         cq_ray r = {{origin.x, origin.y, origin.z}, {direction.x, direction.y, direction.z}, maxDistance, mask};

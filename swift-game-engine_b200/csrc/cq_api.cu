@@ -73,10 +73,33 @@ int release_held(cq_world *w, cudaStream_t st) {
     return rc;
 }
 
+int await_trees(const cq_world *w, cudaStream_t st) {
+    if (w->treesPending && st != w->treesStream) CQ_CUDA(cudaStreamWaitEvent(st, w->evTrees, 0));
+    return CQ_OK;
+}
+
+// one event per stream that ever launched on the world, re-recorded by every launch on it
+static int note_reader(cq_world *w, cudaStream_t st) {
+    ReaderEvent *r = nullptr;
+    for (ReaderEvent &e : w->readers)
+        if (e.st == st) r = &e;
+    if (!r) {
+        ReaderEvent e;
+        e.st = st;
+        CQ_CUDA(cudaEventCreateWithFlags(&e.ev, cudaEventDisableTiming));
+        w->readers.push_back(e);
+        r = &w->readers.back();
+    }
+    CQ_CUDA(cudaEventRecord(r->ev, st));
+    r->pending = true;
+    return CQ_OK;
+}
+
 int finish_launch(cq_world *w, cudaStream_t st, const char *what) {
     const int rc = check_cuda(cudaGetLastError(), what);
     const int rr = release_held(w, st);
-    return rc != CQ_OK ? rc : rr;
+    const int rn = note_reader(w, st);
+    return rc != CQ_OK ? rc : rr != CQ_OK ? rr : rn;
 }
 
 static void destroy_scratch(ScratchBuf &b) {
@@ -128,6 +151,100 @@ static void make_view(cq_world *w) {
 } // namespace cq
 
 using namespace cq;
+
+static cudaStream_t pick_stream(cq_world *w, void *stream) { return stream ? (cudaStream_t)stream : w->stream; }
+
+// ---------------------------------------------------------------- transform updates
+// Queues the refit of the rows staged in movedRows on `st`: after every launch that has read the trees since the last
+// refit (any stream) and after the previous refit, then records evTrees, which every later launch on another stream waits
+// for (await_trees).  The table reaches the device in one copy from a pinned slot of a ring of CQ_STAGE_SLOTS; a slot is
+// reused once its copy has completed, so the caller's arrays are free when the call returns and the host blocks only when
+// CQ_STAGE_SLOTS earlier updates still have their copy in flight (it then waits for the oldest).  A table larger than any
+// before it grows the slot and the device table; the old buffers are retired, not freed (a free would wait for the device),
+// until the next synchronous update or cq_world_destroy.
+static void free_retired(cq_world *w) {
+    for (void *p : w->retiredDev) cudaFree(p);
+    for (void *p : w->retiredHost) cudaFreeHost(p);
+    w->retiredDev.clear(), w->retiredHost.clear();
+}
+
+static int queue_refit(cq_world *w, cudaStream_t st, cudaEvent_t t0) {
+    for (ReaderEvent &r : w->readers)
+        if (r.pending) {
+            if (r.st != st) CQ_CUDA(cudaStreamWaitEvent(st, r.ev, 0));
+            r.pending = false;
+        }
+    CQ_TRY(await_trees(w, st));
+    const size_t n0 = w->movedRows[0].size(), nRows = n0 + w->movedRows[1].size(), bytes = nRows * sizeof(MovedPart);
+    StageSlot &slot = w->stage[w->stageSeq++ % CQ_STAGE_SLOTS];
+    if (!slot.ev) CQ_CUDA(cudaEventCreateWithFlags(&slot.ev, cudaEventDisableTiming));
+    if (slot.recorded) CQ_CUDA(cudaEventSynchronize(slot.ev));
+    if (slot.cap < nRows) {
+        if (slot.host) w->retiredHost.push_back(slot.host);
+        slot.host = nullptr, slot.cap = 0;
+        const size_t cap = nRows + nRows / 4 + 16;
+        CQ_CUDA(cudaHostAlloc((void **)&slot.host, cap * sizeof(MovedPart), cudaHostAllocDefault));
+        slot.cap = cap;
+    }
+    if (bytes > w->dTable.cap) { // the previous refit may still read the old table
+        if (w->dTable.ptr) w->retiredDev.push_back(w->dTable.ptr);
+        w->dTable.ptr = nullptr, w->dTable.cap = 0;
+        CQ_TRY(ensure_scratch(w->dTable, bytes));
+    }
+    std::copy(w->movedRows[0].begin(), w->movedRows[0].end(), slot.host);
+    std::copy(w->movedRows[1].begin(), w->movedRows[1].end(), slot.host + n0);
+    CQ_CUDA(cudaMemcpyAsync(w->dTable.ptr, slot.host, bytes, cudaMemcpyHostToDevice, st));
+    CQ_CUDA(cudaEventRecord(slot.ev, st));
+    slot.recorded = true;
+    if (t0) CQ_CUDA(cudaEventRecord(t0, st));
+    const MovedPart *dTab = (const MovedPart *)w->dTable.ptr;
+    CQ_TRY(refit_set(w, w->set[0], dTab, w->movedRows[0], st));
+    CQ_TRY(refit_set(w, w->set[1], dTab + n0, w->movedRows[1], st));
+    CQ_CUDA(cudaEventRecord(w->evTrees, st));
+    w->treesStream = st;
+    w->treesPending = true;
+    return CQ_OK;
+}
+
+// Both transform-update calls: check every id before anything is queued (a failed call changes nothing), build the table
+// of moved parts, queue the refit on `st`.  t0 (may be null) is recorded after the table copy, before the refit kernels.
+static int update_transforms_on(cq_world *w, const uint32_t *ids, const float *models, int n, cudaStream_t st, const char *what,
+                                cudaEvent_t t0) {
+    for (int i = 0; i < n; i++)
+        if (w->partsOfEntity.find(ids[i]) == w->partsOfEntity.end()) {
+            set_error("%s: unknown entity id %u", what, ids[i]);
+            return CQ_ERR_NOT_FOUND;
+        }
+    // every part with the id takes the model; `guard let slice = slices[e]`: parts that contributed no triangle are
+    // skipped (CollisionQuery.swift:427); a part named twice keeps the last model
+    for (int i = 0; i < n; i++)
+        for (int p : w->partsOfEntity.find(ids[i])->second) {
+            const PartInfo &pi = w->parts[p];
+            if (pi.triHi <= pi.triLo) continue;
+            std::vector<MovedPart> &rows = w->movedRows[pi.set];
+            int32_t &row = w->movedSlot[p];
+            if (row < 0) {
+                row = (int32_t)rows.size();
+                MovedPart r{};
+                r.part = p, r.vertLo = pi.vertLo, r.triLo = pi.triLo, r.nVerts = pi.vertHi - pi.vertLo, r.nTris = pi.triHi - pi.triLo;
+                rows.push_back(r);
+            }
+            memcpy(rows[row].model, models + 16 * (size_t)i, sizeof(float) * 16);
+        }
+    for (int s = 0; s < 2; s++) {
+        int32_t v = 0, t = 0;
+        for (MovedPart &r : w->movedRows[s]) {
+            w->movedSlot[r.part] = -1;
+            r.vertBase = v, r.triBase = t;
+            v += r.nVerts, t += r.nTris;
+        }
+    }
+    int rc = CQ_OK;
+    if (!w->movedRows[0].empty() || !w->movedRows[1].empty()) rc = queue_refit(w, st, t0);
+    else if (t0) rc = check_cuda(cudaEventRecord(t0, st), "update timing");
+    w->movedRows[0].clear(), w->movedRows[1].clear();
+    return rc;
+}
 
 // ---------------------------------------------------------------- host-pointer (synchronous) entry points
 // Three-stage pipeline over chunks of the batch: a dedicated H2D stream streams the inputs in back to back,
@@ -288,6 +405,7 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
     }
     if ((rc = check_cuda(cudaEventCreate(&w->evA), "event")) != CQ_OK) return fail(rc);
     if ((rc = check_cuda(cudaEventCreate(&w->evB), "event")) != CQ_OK) return fail(rc);
+    if ((rc = check_cuda(cudaEventCreateWithFlags(&w->evTrees, cudaEventDisableTiming), "event")) != CQ_OK) return fail(rc);
 
     // host-side assembly of the two sets' input arrays (partitionEntities, CollisionQuery.swift:886-900): cq_assemble.h
     SetPlan input[2];
@@ -343,7 +461,9 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
         pi.layer = mp.layer;
         memcpy(&models[(size_t)p * 16], mp.model, sizeof(float) * 16);
         materials[p] = make_float4(mp.mu_s, mp.mu_k, mp.flatten_ground ? 1.0f : 0.0f, 0.0f);
+        w->partsOfEntity[mp.entity_id].push_back(p);
     }
+    w->movedSlot.assign(n_parts, -1);
 
     if ((rc = check_cuda(cudaMalloc((void **)&w->dModels, sizeof(float) * 16 * (size_t)std::max(n_parts, 1)), "models")) != CQ_OK)
         return fail(rc);
@@ -408,6 +528,14 @@ void cq_world_destroy(cq_world *w) {
     destroy_scratch(w->agentScratch);
     sep_graphs_destroy(w);
     destroy_scratch(w->sepScratch);
+    destroy_scratch(w->dTable);
+    free_retired(w);
+    for (StageSlot &s : w->stage) {
+        if (s.host) cudaFreeHost(s.host);
+        if (s.ev) cudaEventDestroy(s.ev);
+    }
+    for (ReaderEvent &e : w->readers) cudaEventDestroy(e.ev);
+    if (w->evTrees) cudaEventDestroy(w->evTrees);
     if (w->evA) cudaEventDestroy(w->evA);
     if (w->evB) cudaEventDestroy(w->evB);
     if (w->stream) cudaStreamDestroy(w->stream);
@@ -444,43 +572,22 @@ int cq_world_get_info(const cq_world *w, cq_world_info *info) {
 int cq_world_update_transforms(cq_world *w, const uint32_t *entity_ids, const float *models, int32_t n) {
     if (!w || n < 0 || (n > 0 && (!entity_ids || !models))) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
-    // A refit mutates the world: every query still in flight on any stream (the *_device calls are asynchronous)
-    // must have finished reading the old boxes first.
+    // the documented contract of the synchronous call: everything in flight on any stream has finished first
     CQ_CUDA(cudaDeviceSynchronize());
-    std::vector<int> changed[2];
-    for (int i = 0; i < n; i++) { // validate every id before anything is queued: a failed call changes nothing
-        bool known = false;
-        for (size_t p = 0; p < w->parts.size() && !known; p++) known = w->parts[p].entityId == entity_ids[i];
-        if (!known) {
-            set_error("cq_world_update_transforms: unknown entity id %u", entity_ids[i]);
-            return CQ_ERR_NOT_FOUND;
-        }
-    }
-    for (int i = 0; i < n; i++) {
-        bool found = false;
-        for (size_t p = 0; p < w->parts.size(); p++) {
-            if (w->parts[p].entityId != entity_ids[i]) continue;
-            found = true;
-            // `guard let slice = slices[e]`: entities that contributed no triangle are skipped (CollisionQuery.swift:427)
-            if (w->parts[p].triHi <= w->parts[p].triLo) continue;
-            CQ_CUDA(cudaMemcpyAsync(w->dModels + 16 * p, models + 16 * (size_t)i, sizeof(float) * 16, cudaMemcpyHostToDevice, w->stream));
-            changed[w->parts[p].set].push_back((int)p);
-        }
-        if (!found) {
-            set_error("cq_world_update_transforms: unknown entity id %u", entity_ids[i]);
-            return CQ_ERR_NOT_FOUND;
-        }
-    }
-    cudaEventRecord(w->evA, w->stream);
-    for (int s = 0; s < 2; s++) {
-        if (changed[s].empty()) continue;
-        int rc = refit_set(w, w->set[s], changed[s]);
-        if (rc != CQ_OK) return rc;
-    }
+    free_retired(w);
+    CQ_TRY(update_transforms_on(w, entity_ids, models, n, w->stream, "cq_world_update_transforms", w->evA));
     cudaEventRecord(w->evB, w->stream);
-    CQ_CUDA(cudaStreamSynchronize(w->stream)); // the models array is the caller's; also makes refit_ms readable
+    CQ_CUDA(cudaStreamSynchronize(w->stream)); // makes refit_ms readable; later launches need not wait for this refit
+    w->treesPending = false;
     cudaEventElapsedTime(&w->refitMs, w->evA, w->evB);
     return CQ_OK;
+}
+
+int cq_world_update_transforms_async(cq_world *w, const uint32_t *entity_ids, const float *models, int32_t n, void *stream) {
+    if (!w || n < 0 || (n > 0 && (!entity_ids || !models))) return CQ_ERR_INVALID;
+    if (n == 0) return CQ_OK;
+    CQ_CUDA(cudaSetDevice(w->device));
+    return update_transforms_on(w, entity_ids, models, n, pick_stream(w, stream), "cq_world_update_transforms_async", nullptr);
 }
 
 int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, uint32_t *indices, float *tri_aabbs,
@@ -488,6 +595,7 @@ int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, u
     if (!w || which < 0 || which > 1) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
     const DeviceSet &S = w->set[which];
+    CQ_TRY(await_trees(w, w->stream));
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     std::vector<float4> pos(S.nVerts);
     std::vector<uint32_t> idx((size_t)S.nTris * 3);
@@ -552,6 +660,7 @@ int cq_world_read_counters(cq_world *w, cq_counters *out, int32_t reset) {
     if (!w || !out) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
     unsigned long long h[4];
+    CQ_TRY(await_trees(w, w->stream));
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     CQ_CUDA(cudaMemcpy(h, w->dCounters, sizeof(h), cudaMemcpyDeviceToHost));
     CQ_TRY(check_status(w, "cq_world_read_counters"));
@@ -568,7 +677,6 @@ int cq_world_read_counters(cq_world *w, cq_counters *out, int32_t reset) {
 }
 
 // ---------------------------------------------------------------- device-pointer entry points
-static cudaStream_t pick_stream(cq_world *w, void *stream) { return stream ? (cudaStream_t)stream : w->stream; }
 
 int cq_raycast_device_ex(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, uint8_t *d_flags, void *stream) {
     if (!w || n < 0 || (n > 0 && (!d_rays || !d_out))) return CQ_ERR_INVALID;

@@ -4,7 +4,7 @@
 //   TriangleMeshSet.rebuild           CollisionQuery.swift:331-417  -> k_transform, k_filter_flags, k_compact
 //   StaticTriMesh.BVH.build (top-down median split, :577-670) -> LBVH: k_centroid_bounds, k_morton,
 //        radix sort (rs_*), k_karras (Karras 2012 radix tree), k_fit (bottom-up boxes)
-//   TriangleMeshSet.updateTransforms  :419-462 + BVH.refit :528-575 -> k_transform_range + k_gather + k_fit
+//   TriangleMeshSet.updateTransforms  :419-462 + BVH.refit :528-575 -> k_update_parts + dirty-subtree refit or k_fit
 // The tree differs from the reference's (allowed: capsule candidate sets are tree-independent,
 // SURVEY.md §A.4); triangle NUMBERING and world-space vertices are bit-identical to the reference's.
 #include <algorithm>
@@ -645,23 +645,61 @@ __global__ void k_header(int n, const float4 *__restrict__ boxLo, const float4 *
     *hdr = h;
 }
 
-// ---------------------------------------------------------------- dirty-subtree refit (BVH.refit, CollisionQuery.swift:528-575)
-// The reference recomputes the leaves of the updated triangles and then only their ancestors, deepest first.  Here: one
-// thread per updated triangle rewrites its slot of the sorted SoA and its leaf box and MARKS its ancestors — `expect[p]`
-// counts the dirty children of p (1 or 2); the thread that finds p already marked stops, so every dirty edge is counted
-// once.  A second launch climbs: the last of a node's expected arrivals recomputes it from its children's boxes (the
-// clean child's box is still valid), re-collapses the 4-wide node when the depth is even, resets the counters and goes on.
+// ---------------------------------------------------------------- transform update + dirty-subtree refit
+// (TriangleMeshSet.updateTransforms :419-462, BVH.refit :528-575)
+// A transform update stages a table of the moved parts (MovedPart, cq_internal.h); every kernel below runs over that
+// table in ONE launch per set, whatever the number of parts: a thread finds its row by binary search over the rows'
+// running totals.  k_update_parts writes the parts' model rows and re-transforms their vertices.
+// The reference then recomputes the leaves of the updated triangles and only their ancestors, deepest first.  Here, when
+// fewer than a quarter of a set's triangles moved, three launches per tree:
+//   mark  — one thread per moved triangle rewrites its slot of the sorted SoA and its leaf box, and MARKS its ancestors:
+//           `expect[p]` counts the dirty children of p (1 or 2); the thread that finds p already marked stops, so every
+//           dirty edge is counted once;
+//   climb — the last of a node's expected arrivals recomputes it from its children's boxes (the clean child's box is
+//           still valid), re-collapses the 4-wide node when the depth is even, and goes on.  `expect` is final once the
+//           mark launch has ended and nothing in the climb writes it, so an arrival can never see a counter a sibling
+//           arrival has already reset;
+//   clear — resets `visit` / `expect` along the same paths for the next refit.
 // Same min / max arithmetic as the full fit, so the boxes are identical; cost O(updated triangles x depth).
 __global__ void k_invert_sorted(const uint32_t *__restrict__ sortedTri, int n, uint32_t *__restrict__ slotOfTri) {
     int s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s < n) slotOfTri[sortedTri[s]] = (uint32_t)s;
 }
 
-__global__ void k_refit_mark(int triLo, int triHi, const uint32_t *__restrict__ slotOfTri, int n,
-                             const float4 *__restrict__ world, const uint32_t *__restrict__ idx, float4 *tv0, float4 *tv1,
+// the row of the table that holds unit i (a vertex when tris == false, else a triangle): the last row whose base <= i
+__device__ __forceinline__ const MovedPart &moved_row(const MovedPart *__restrict__ tab, int nRows, int i, bool tris) {
+    int lo = 0, hi = nRows - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if ((tris ? tab[mid].triBase : tab[mid].vertBase) <= i) lo = mid;
+        else hi = mid - 1;
+    }
+    return tab[lo];
+}
+__device__ __forceinline__ int moved_triangle(const MovedPart *__restrict__ tab, int nRows, int i) {
+    const MovedPart &r = moved_row(tab, nRows, i, true);
+    return r.triLo + (i - r.triBase);
+}
+
+// one thread per vertex of the moved parts; the arithmetic of k_transform, so the positions are bit-identical
+__global__ void k_update_parts(const MovedPart *__restrict__ tab, int nRows, int nVerts, const float4 *__restrict__ local,
+                               float4 *__restrict__ world, float *__restrict__ models) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nVerts) return;
+    const MovedPart &r = moved_row(tab, nRows, i, false);
+    const int k = i - r.vertBase;
+    if (k == 0)
+        for (int c = 0; c < 16; c++) models[16 * r.part + c] = r.model[c];
+    const int v = r.vertLo + k;
+    world[v] = transform_point(r.model, local[v]);
+}
+
+__global__ void k_refit_mark(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
+                             int n, const float4 *__restrict__ world, const uint32_t *__restrict__ idx, float4 *tv0, float4 *tv1,
                              float4 *tv2, const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *expect) {
-    const int t = triLo + blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= triHi) return;
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved) return;
+    const int t = moved_triangle(tab, nRows, i);
     const int slot = (int)slotOfTri[t];
     const float4 a = world[idx[3 * t]], b = world[idx[3 * t + 1]], c = world[idx[3 * t + 2]];
     float4 o0 = tv0[slot], o1 = tv1[slot], o2 = tv2[slot]; // the w words (layer, triangle id, rank) stay
@@ -676,15 +714,14 @@ __global__ void k_refit_mark(int triLo, int triHi, const uint32_t *__restrict__ 
         if (atomicAdd(&expect[p], 1) != 0) break; // p was already marked through its other child
 }
 
-__global__ void k_refit_climb(int triLo, int triHi, const uint32_t *__restrict__ slotOfTri, int n, Node *nodes,
-                              const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *visit, int32_t *expect,
-                              const uint8_t *__restrict__ parity, Node4 *nodes4) {
-    const int t = triLo + blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= triHi || n == 1) return;
-    __threadfence();
-    int p = parent[(n - 1) + (int)slotOfTri[t]];
+__global__ void k_refit_climb(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
+                              int n, Node *nodes, const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *visit,
+                              const int32_t *__restrict__ expect, const uint8_t *__restrict__ parity, Node4 *nodes4) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved || n == 1) return;
+    int p = parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, nRows, i)]];
     while (p >= 0) {
-        if (atomicAdd(&visit[p], 1) + 1 < *(volatile int32_t *)&expect[p]) return; // a dirty sibling subtree is not done yet
+        if (atomicAdd(&visit[p], 1) + 1 < expect[p]) return; // a dirty sibling subtree is not done yet
         __threadfence();
         Node nd = nodes[p];
         const int lb = __float_as_int(nd.n2.w), rb = __float_as_int(nd.n3.w);
@@ -696,7 +733,6 @@ __global__ void k_refit_climb(int triLo, int triHi, const uint32_t *__restrict__
         nodes[p] = nd;
         boxLo[p] = make_float4(fminf(l0.x, l1.x), fminf(l0.y, l1.y), fminf(l0.z, l1.z), 0.0f);
         boxHi[p] = make_float4(fmaxf(h0.x, h1.x), fmaxf(h0.y, h1.y), fmaxf(h0.z, h1.z), 0.0f);
-        visit[p] = 0, expect[p] = 0; // clean for the next refit
         __threadfence();
         // 4-wide nodes: an even-depth node absorbs its internal (odd-depth) children, which are final by now
         if (!parity[p]) collapse4_node(p, nodes, nodes4);
@@ -705,18 +741,31 @@ __global__ void k_refit_climb(int triLo, int triHi, const uint32_t *__restrict__
     }
 }
 
-// the same two steps on the reference's tree (reference order): leaves hold <= 4 triangles; a leaf is refitted by the
-// thread of its FIRST triangle in triOrder that belongs to the updated range (ties: the lowest position wins the CAS)
+// Every marked node lies on the path of a moved triangle, so walking those paths clears them all.  A thread stops at the
+// first node another thread has cleared: that thread goes on above it.
+__global__ void k_refit_clear(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
+                              int n, const int32_t *__restrict__ parent, int32_t *visit, int32_t *expect) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved || n == 1) return;
+    for (int p = parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, nRows, i)]]; p >= 0; p = parent[p]) {
+        visit[p] = 0;
+        if (atomicExch(&expect[p], 0) == 0) break;
+    }
+}
+
+// the same three steps on the reference's tree (reference order): leaves hold <= 4 triangles; a leaf is refitted by the
+// moved triangle that claims it first in the mark launch (leafMark = its triangle id + 1), which also climbs for it
 __device__ __forceinline__ void ref_store_child_box(Node *nd, int which, f3 lo, f3 hi);
-__global__ void k_ref_refit_mark(int triLo, int triHi, const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafRange,
-                                 const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent,
-                                 const uint32_t *__restrict__ refSlot, const float4 *__restrict__ tv0,
-                                 const float4 *__restrict__ tv1, const float4 *__restrict__ tv2, Node *nodes, int32_t *leafMark,
-                                 int32_t *expect, SetHeader *hdr) {
-    const int t = triLo + blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= triHi) return;
+__global__ void k_ref_refit_mark(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
+                                 const int32_t *__restrict__ leafRange, const int32_t *__restrict__ leafParent,
+                                 const int32_t *__restrict__ nodeParent, const uint32_t *__restrict__ refSlot,
+                                 const float4 *__restrict__ tv0, const float4 *__restrict__ tv1, const float4 *__restrict__ tv2,
+                                 Node *nodes, int32_t *leafMark, int32_t *expect, SetHeader *hdr) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved) return;
+    const int t = moved_triangle(tab, nRows, i);
     const int l = leafOfTri[t];
-    if (atomicExch(&leafMark[l], 1) != 0) return; // another triangle of the same leaf got here first
+    if (atomicCAS(&leafMark[l], 0, t + 1) != 0) return; // another triangle of the same leaf got here first
     const int range = leafRange[l], start = range >> 2, count = (range & 3) + 1;
     f3 lo = {0, 0, 0}, hi = {0, 0, 0};
     for (int k = 0; k < count; k++) {
@@ -737,19 +786,19 @@ __global__ void k_ref_refit_mark(int triLo, int triHi, const int32_t *__restrict
         if (atomicAdd(&expect[pw >> 1], 1) != 0) break;
 }
 
-__global__ void k_ref_refit_climb(int triLo, int triHi, const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafParent,
-                                  const int32_t *__restrict__ nodeParent, Node *nodes, int32_t *leafMark, int32_t *visit,
-                                  int32_t *expect, SetHeader *hdr) {
-    const int t = triLo + blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= triHi) return;
+__global__ void k_ref_refit_climb(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
+                                  const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent, Node *nodes,
+                                  const int32_t *__restrict__ leafMark, int32_t *visit, const int32_t *__restrict__ expect,
+                                  SetHeader *hdr) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved) return;
+    const int t = moved_triangle(tab, nRows, i);
     const int l = leafOfTri[t];
-    if (atomicExch(&leafMark[l], 0) != 1) return; // one climber per marked leaf; the mark is cleared on the way
-    __threadfence();
+    if (leafMark[l] != t + 1) return; // one climber per marked leaf: the triangle that claimed it
     int pw = leafParent[l];
     while (pw >= 0) {
         const int p = pw >> 1;
-        if (atomicAdd(&visit[p], 1) + 1 < *(volatile int32_t *)&expect[p]) return;
-        visit[p] = 0, expect[p] = 0;
+        if (atomicAdd(&visit[p], 1) + 1 < expect[p]) return;
         __threadfence();
         const float4 *q = reinterpret_cast<const float4 *>(nodes + p);
         const float4 l0 = __ldcg(q), h0 = __ldcg(q + 1), l1 = __ldcg(q + 2), h1 = __ldcg(q + 3);
@@ -762,6 +811,19 @@ __global__ void k_ref_refit_climb(int triLo, int triHi, const int32_t *__restric
         }
         ref_store_child_box(nodes + (pw >> 1), pw & 1, lo, hi);
         __threadfence();
+    }
+}
+
+__global__ void k_ref_refit_clear(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
+                                  const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent, int32_t *leafMark,
+                                  int32_t *visit, int32_t *expect) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= nMoved) return;
+    const int l = leafOfTri[moved_triangle(tab, nRows, i)];
+    leafMark[l] = 0;
+    for (int pw = leafParent[l]; pw >= 0; pw = nodeParent[pw >> 1]) {
+        visit[pw >> 1] = 0;
+        if (atomicExch(&expect[pw >> 1], 0) == 0) break;
     }
 }
 
@@ -860,8 +922,7 @@ static bool use_classic_sort() {
     return e && !strcmp(e, "classic");
 }
 
-static int build_tree(cq_world *w, DeviceSet &S, const uint32_t *sortedKeys /* may be null on refit */) {
-    cudaStream_t st = w->stream;
+static int build_tree(cq_world *w, DeviceSet &S, const uint32_t *sortedKeys /* may be null on refit */, cudaStream_t st) {
     int n = S.nTris;
     if (n > 0) {
         const int triOffset = &S == &w->set[1] ? w->set[0].nTris : 0;
@@ -1069,14 +1130,14 @@ int build_set(cq_world *w, DeviceSet &S, const SetPlan &in,
         w->launches += 4;
         rc = use_classic_sort() ? radix_sort_pairs_classic(w, dKeys, S.sortedTri, dKeysTmp, dValsTmp, n, dHist)
                                 : radix_sort_pairs_onesweep(w, dKeys, S.sortedTri, dKeysTmp, dValsTmp, n, dHist, histWords);
-        if (rc == CQ_OK) rc = build_tree(w, S, dKeys);
+        if (rc == CQ_OK) rc = build_tree(w, S, dKeys, st);
         if (rc == CQ_OK) { // for the dirty-subtree refit: where every triangle sits, and clean marking counters
             k_invert_sorted<<<cdiv(n, 256), 256, 0, st>>>(S.sortedTri, n, S.slotOfTri);
             w->launches++;
             rc = check_cuda(cudaMemsetAsync(S.expect, 0, sizeof(int32_t) * (size_t)n, st), "expect");
         }
     } else {
-        rc = build_tree(w, S, nullptr);
+        rc = build_tree(w, S, nullptr, st);
     }
     cudaEventRecord(e1, st);
     cudaError_t e = cudaStreamSynchronize(st);
@@ -1343,10 +1404,10 @@ __global__ void k_ref_fit(int nLeaves, const int32_t *__restrict__ leafRange, co
     }
 }
 
-static int ref_fit(cq_world *w, DeviceSet &S) {
+static int ref_fit(cq_world *w, DeviceSet &S, cudaStream_t st) {
     if (!S.refArena || S.nRefLeaves <= 0) return CQ_OK;
-    k_ref_fit<<<cdiv(S.nRefLeaves, 256), 256, 0, w->stream>>>(S.nRefLeaves, S.refLeafRange, S.refLeafParent, S.refNodeParent,
-                                                             S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refVisit, S.refHdr);
+    k_ref_fit<<<cdiv(S.nRefLeaves, 256), 256, 0, st>>>(S.nRefLeaves, S.refLeafRange, S.refLeafParent, S.refNodeParent,
+                                                     S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refVisit, S.refHdr);
     w->launches++;
     return check_cuda(cudaGetLastError(), "k_ref_fit");
 }
@@ -1459,7 +1520,7 @@ int attach_ref_order(cq_world *w) {
         CQ_CUDA(cudaMemsetAsync(S.refLeafMark, 0, sizeof(int32_t) * (size_t)std::max(nLeaf, 1), st));
         CQ_CUDA(cudaMemcpyAsync(S.refLeafOfTri, leafOfTri.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
         CQ_CUDA(cudaMemcpyAsync(S.refHdr, &h, sizeof(h), cudaMemcpyHostToDevice, st));
-        CQ_TRY(ref_fit(w, S));
+        CQ_TRY(ref_fit(w, S, st));
         CQ_CUDA(cudaStreamSynchronize(st)); // the host vectors above are the copies' sources
     }
     if (nS + nD > 0) {
@@ -1481,46 +1542,38 @@ int attach_ref_order(cq_world *w) {
     return CQ_OK;
 }
 
-// TriangleMeshSet.updateTransforms + BVH.refit: re-transform the changed parts' vertices, then
+// TriangleMeshSet.updateTransforms + BVH.refit: re-transform the moved parts' vertices (k_update_parts), then
 //   * few triangles moved (less than a quarter of the set): the dirty-subtree refit above — the updated triangles' slots,
 //     their leaves and only the ancestors of those, in the LBVH, its 4-wide collapse and (reference order) the reference's
-//     own tree, like BVH.refit (CollisionQuery.swift:528-575);
-//   * otherwise: regather the whole sorted SoA and recompute every box bottom-up (same topology).
-// Both give the same boxes (min / max are exact).  Asynchronous on the world stream.
-int refit_set(cq_world *w, DeviceSet &S, const std::vector<int> &partIdx) {
-    cudaStream_t st = w->stream;
-    long long moved = 0;
-    for (int pi : partIdx) {
-        const PartInfo &p = w->parts[pi];
-        int nv = p.vertHi - p.vertLo;
-        moved += p.triHi - p.triLo;
-        if (nv <= 0) continue;
-        k_transform<<<cdiv(nv, 256), 256, 0, st>>>(S.localPos, S.worldPos, w->dModels, p.vertLo, p.vertHi);
-        w->launches++;
-    }
+//     own tree, like BVH.refit (CollisionQuery.swift:528-575): 1 + 3 + 3 + 1 launches;
+//   * otherwise: regather the whole sorted SoA and recompute every box bottom-up (same topology): 1 + 4 + 1 launches.
+// Both give the same boxes (min / max are exact).  Stream-ordered on `st`, no host synchronisation.
+int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const std::vector<MovedPart> &rows, cudaStream_t st) {
+    const int nRows = (int)rows.size();
+    if (nRows == 0) return CQ_OK;
+    const int nVerts = rows.back().vertBase + rows.back().nVerts, moved = rows.back().triBase + rows.back().nTris;
+    k_update_parts<<<cdiv(nVerts, 256), 256, 0, st>>>(dTab, nRows, nVerts, S.localPos, S.worldPos, w->dModels);
+    w->launches++;
     static const bool forceFull = getenv("CQ_REFIT_FULL") != nullptr; // A/B and the test that both paths agree
-    if (forceFull || moved * 4 >= (long long)S.nTris) {
-        CQ_TRY(build_tree(w, S, nullptr));
-        return ref_fit(w, S); // reference order: the reference's own tree keeps its topology too (BVH.refit)
+    if (forceFull || (long long)moved * 4 >= (long long)S.nTris) {
+        CQ_TRY(build_tree(w, S, nullptr, st));
+        return ref_fit(w, S, st); // reference order: the reference's own tree keeps its topology too (BVH.refit)
     }
-    const int n = S.nTris;
-    for (int pi : partIdx) {
-        const PartInfo &p = w->parts[pi];
-        const int cnt = p.triHi - p.triLo;
-        if (cnt <= 0) continue;
-        k_refit_mark<<<cdiv(cnt, 256), 256, 0, st>>>(p.triLo, p.triHi, S.slotOfTri, n, S.worldPos, S.indices, S.tv0, S.tv1, S.tv2,
-                                                      S.parent, S.boxLo, S.boxHi, S.expect);
-        k_refit_climb<<<cdiv(cnt, 256), 256, 0, st>>>(p.triLo, p.triHi, S.slotOfTri, n, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit,
-                                                       S.expect, S.depthParity, S.nodes4);
-        w->launches += 2;
-        if (S.refArena && S.nRefLeaves > 0) {
-            k_ref_refit_mark<<<cdiv(cnt, 256), 256, 0, st>>>(p.triLo, p.triHi, S.refLeafOfTri, S.refLeafRange, S.refLeafParent,
-                                                              S.refNodeParent, S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes,
-                                                              S.refLeafMark, S.refExpect, S.refHdr);
-            k_ref_refit_climb<<<cdiv(cnt, 256), 256, 0, st>>>(p.triLo, p.triHi, S.refLeafOfTri, S.refLeafParent, S.refNodeParent,
-                                                               S.refNodes, S.refLeafMark, S.refVisit, S.refExpect, S.refHdr);
-            w->launches += 2;
-        }
+    const int n = S.nTris, blocks = cdiv(moved, 256);
+    k_refit_mark<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.worldPos, S.indices, S.tv0, S.tv1, S.tv2, S.parent,
+                                         S.boxLo, S.boxHi, S.expect);
+    k_refit_climb<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit, S.expect,
+                                          S.depthParity, S.nodes4);
+    k_refit_clear<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.parent, S.visit, S.expect);
+    w->launches += 3;
+    if (S.refArena && S.nRefLeaves > 0) {
+        k_ref_refit_mark<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafRange, S.refLeafParent, S.refNodeParent,
+                                                 S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refLeafMark, S.refExpect, S.refHdr);
+        k_ref_refit_climb<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafParent, S.refNodeParent, S.refNodes,
+                                                  S.refLeafMark, S.refVisit, S.refExpect, S.refHdr);
+        k_ref_refit_clear<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafParent, S.refNodeParent,
+                                                  S.refLeafMark, S.refVisit, S.refExpect);
+        w->launches += 3;
     }
     k_header<<<1, 32, 0, st>>>(n, S.boxLo, S.boxHi, S.hdr);
     w->launches++;

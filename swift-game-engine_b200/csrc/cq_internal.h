@@ -5,6 +5,7 @@
 
 #include <algorithm>
 #include <string>
+#include <unordered_map>
 #include <vector>
 
 #include "../../include/cq.h"
@@ -74,9 +75,37 @@ struct ScratchBuf {
     bool recorded = false;
 };
 
+// One row of the part table a transform update stages (cq_api.cu: update_transforms_on): a moved part of one set, its
+// vertex and triangle ranges, and the running totals of both over the set's earlier rows (the refit kernels find a
+// thread's row by binary search over them).  The table holds the static set's rows, then the dynamic set's.
+struct MovedPart {
+    int32_t part;             // index into the parts array (row of dModels)
+    int32_t vertLo, triLo;    // first vertex / filtered triangle of the part in its set
+    int32_t nVerts, nTris;
+    int32_t vertBase, triBase; // sum of nVerts / nTris over the set's earlier rows
+    int32_t _pad;
+    float model[16];          // the new model matrix, column-major
+};
+
+// Host side of one staged table: pinned memory, reused once the copy that read it has completed (event).
+struct StageSlot {
+    MovedPart *host = nullptr;
+    size_t cap = 0; // rows
+    cudaEvent_t ev = nullptr;
+    bool recorded = false;
+};
+
+// Completion of the last launch on `st` that read the world's trees (finish_launch); `pending` until a refit waited on it.
+struct ReaderEvent {
+    cudaStream_t st = nullptr;
+    cudaEvent_t ev = nullptr;
+    bool pending = false;
+};
+
 } // namespace cq
 
 #define CQ_PIPE_EVENTS 64
+#define CQ_STAGE_SLOTS 4 // transform updates whose table copy may be in flight at once; a fifth waits for the oldest
 
 struct cq_world {
     int device = 0;
@@ -117,6 +146,19 @@ struct cq_world {
     int occSep[2][2] = {};       // resident CTAs per SM of k_sep_turns / k_sep_post ([counting build])
     void *sepGraphs = nullptr;   // instantiated round-loop graphs of cq_agent_separation (cq_sep.cu: SepGraphCache)
     std::vector<cq::ScratchBuf *> held; // scratch blocks acquired by the launch being enqueued (release_held)
+    // transform updates (cq_api.cu: update_transforms_on)
+    std::unordered_map<uint32_t, std::vector<int>> partsOfEntity; // entity id -> parts with that id, in part order
+    std::vector<int32_t> movedSlot;         // per part: its row in movedRows[set] during staging, else -1
+    std::vector<cq::MovedPart> movedRows[2]; // the table being staged, per set
+    cq::StageSlot stage[CQ_STAGE_SLOTS];
+    uint32_t stageSeq = 0;
+    cq::ScratchBuf dTable; // device copy of the staged table (read by the refit kernels of one update at a time)
+    std::vector<void *> retiredDev, retiredHost; // outgrown table buffers a queued update may still use (cq_api.cu: free_retired)
+    // Ordering of stream-ordered refits against every other launch on the world (await_trees / note_reader):
+    std::vector<cq::ReaderEvent> readers; // per stream: the last launch that read the trees
+    cudaEvent_t evTrees = nullptr;        // recorded after the last kernel of the latest asynchronous refit
+    cudaStream_t treesStream = nullptr;   // ... on this stream
+    bool treesPending = false;            // an asynchronous refit was queued and no synchronous call has waited for it since
 };
 
 namespace cq {
@@ -143,7 +185,11 @@ int check_status(cq_world *w, const char *what);
 // release_held(w, st) once everything that touches its blocks is enqueued (records the completion events).
 int scratch_acquire(cq_world *w, ScratchBuf &b, cudaStream_t st);
 int release_held(cq_world *w, cudaStream_t st);
-// end of every launcher: pick up the launch error of the kernel just enqueued, then release the held scratch blocks
+// First call of every launcher: a launch on `st` must see the trees the latest asynchronous refit writes, so `st` waits
+// for that refit when it was queued on another stream.
+int await_trees(const cq_world *w, cudaStream_t st);
+// end of every launcher: pick up the launch error of the kernel just enqueued, release the held scratch blocks, and
+// record that `st` has read the trees (the next asynchronous refit waits for it)
 int finish_launch(cq_world *w, cudaStream_t st, const char *what);
 #define CQ_WORK_RING 256
 // zeroed work counter for the next persistent-kernel launch on `st` (nullptr on CUDA error)
@@ -158,7 +204,9 @@ int build_set(cq_world *w, DeviceSet &S, const SetPlan &in /* upload plan of the
               std::vector<int> &partTriStart /* in: first input triangle of each part of the set (+ end); out: after the filter */,
               int *badTriangle /* out: smallest input triangle with an out-of-range index (CQ_ERR_INVALID), else -1 */,
               const int32_t *matIn = nullptr /* host, per INPUT triangle: row of the material table, or nullptr (row = part) */);
-int refit_set(cq_world *w, DeviceSet &S, const std::vector<int> &partIdx);
+// Refit one set after its parts moved: dTab = the set's rows of the staged table on the device (rows = the same rows on
+// the host, for the totals).  Stream-ordered on `st`; a fixed number of launches however many parts moved.
+int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const std::vector<MovedPart> &rows, cudaStream_t st);
 // reference order: rebuild the reference's tree on the host from the set's triangle boxes, upload rank + tree (cq_reftree.h)
 int attach_ref_order(cq_world *w);
 void free_set(DeviceSet &S);

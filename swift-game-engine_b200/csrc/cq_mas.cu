@@ -837,6 +837,7 @@ __global__ void __launch_bounds__(MAS_THREADS, MAS_MIN_BLOCKS) k_move_and_slide(
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
                           const float g[3], uint32_t flags, const cq_platform *platforms, int nPlatforms, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
+    CQ_TRY(await_trees(w, st));
     if (nPlatforms < 0 || nPlatforms > MAS_MAX_PLATFORMS || (nPlatforms > 0 && !platforms)) {
         set_error("cq_move_and_slide: 0..%d platforms supported, got %d", MAS_MAX_PLATFORMS, nPlatforms);
         return CQ_ERR_INVALID;

@@ -764,6 +764,7 @@ static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 #define CQ_OCC_SLOT 1
 int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
+    CQ_TRY(await_trees(w, st));
     int *blocksPerSm = w->occ[CQ_OCC_SLOT]; int &numSms = w->numSms;
     const bool ref = w->order == CQ_ORDER_REFERENCE; // the reference's own walk over the reference's own tree
     const int ci = (w->counting ? 1 : 0) + (ref ? 2 : 0);
@@ -795,6 +796,7 @@ int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, 
 #define CQ_OCC_SLOT 2
 int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cast_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
+    CQ_TRY(await_trees(w, st));
     int *blocksPerSm = w->occ[CQ_OCC_SLOT]; int &numSms = w->numSms;
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     using Kernel = void (*)(WorldView, const cq_capsule_cast *, int, int, cq_cast_hit *, uint8_t *, int, uint2 *, int *,
@@ -828,6 +830,7 @@ template <bool ALL>
 static int launch_overlap_pool(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                                uint8_t *d_overflow, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
+    CQ_TRY(await_trees(w, st));
     int &numSms = w->numSms;
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     int &blocksPerSm = w->occ[CQ_OCC_SLOT][ci];

@@ -763,6 +763,7 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
                             const float *d_massWeight, int iterations, float sepMargin, float heightMargin, int useQuery,
                             cudaStream_t st) {
     if (n <= 1) return CQ_OK; // `guard agents.count > 1` (SYS:2178)
+    CQ_TRY(await_trees(w, st));
     iterations = std::max(1, iterations);
     const size_t sortWords = sort_scratch_words(n);
     // float4 x5 (pos vel orig posSave velSave), int4 x2 (rows), int2 x2 (cellRaw cell0), int x3 (cnt queueA queueB),

@@ -183,6 +183,15 @@ public final class CollisionQuery {
         lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
     }
 
+    /// Stream-ordered update (cq_world_update_transforms_async): entity ids + column-major model matrices (16 floats each),
+    /// queued on `stream` (a cudaStream_t; nil = the world's own stream) without waiting.  The arrays are copied before
+    /// the call returns; every later call on the world sees the new pose.
+    public func updateTransformsAsync(ids: [UInt32], models: [Float], stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        let rc = cq_world_update_transforms_async(handle, ids, models, Int32(ids.count), stream)
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
     /// Entities with Transform + StaticMesh (collides), ascending id (the reference iterates a Dictionary, i.e. in
     /// per-process random order — World.swift:99-118; the library fixes the order so triangle numbering is stable).
     /// Geometry is returned as plain Swift arrays; `withArrays` lends their storage to the C structs for one call.
