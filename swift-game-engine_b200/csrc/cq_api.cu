@@ -37,6 +37,30 @@ int ensure_scratch(ScratchBuf &b, size_t bytes) {
     return r;
 }
 
+int resident_blocks(cq_world *w, const void *kernel, int threads, size_t dynSmem) {
+    const auto it = w->residentBlocks.find(kernel);
+    if (it != w->residentBlocks.end()) return it->second;
+    if (dynSmem > 0 &&
+        check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynSmem), "smem attr") != CQ_OK)
+        return 0;
+    int b = 0;
+    if (check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, threads, dynSmem), "occupancy") != CQ_OK) return 0;
+    return w->residentBlocks[kernel] = w->numSms * std::max(b, 1);
+}
+
+int pipeline_chunks(int n, float hint, float computeBoundAbove, bool singleChunk) {
+    static const int CH = [] { // units per chunk (CQ_CHUNK overrides, for tuning)
+        const char *e = getenv("CQ_CHUNK");
+        int v = e ? atoi(e) : 0;
+        return v >= 1024 ? v : (1 << 17);
+    }();
+    int nChunks = (n + CH - 1) / CH;
+    if (hint > computeBoundAbove && nChunks > 2) nChunks = 2;
+    if (nChunks > CQ_PIPE_EVENTS) nChunks = CQ_PIPE_EVENTS;
+    if (singleChunk) nChunks = 1;
+    return nChunks;
+}
+
 int check_status(cq_world *w, const char *what) {
     if (!w->hStatus) return CQ_OK;
     const unsigned int v = *(volatile unsigned int *)w->hStatus;
@@ -274,15 +298,8 @@ static int run_batch(cq_world *w, const In *in, size_t inStride, Out *out, size_
                      uint8_t *flagsHost = nullptr) {
     if (n <= 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
-    static const int CH = [] { // units per chunk of the copy/compute pipeline (CQ_CHUNK overrides, for tuning)
-        const char *e = getenv("CQ_CHUNK");
-        int v = e ? atoi(e) : 0;
-        return v >= 1024 ? v : (1 << 17);
-    }();
-    int nChunks = (n + CH - 1) / CH;
-    if (computeBoundHint && *computeBoundHint > 3.0f && nChunks > 2) nChunks = 2;
-    if (nChunks > CQ_PIPE_EVENTS) nChunks = CQ_PIPE_EVENTS;
-    if (singleChunk) nChunks = 1; // the units interact (agents): every one must be resident before the kernel starts
+    // singleChunk: the units interact (agents), every one must be resident before the kernel starts
+    const int nChunks = pipeline_chunks(n, computeBoundHint ? *computeBoundHint : 0.0f, 3.0f, singleChunk);
     const auto t0 = std::chrono::steady_clock::now();
     int chunk = (n + nChunks - 1) / nChunks;
     int r;
@@ -383,10 +400,12 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
         set_error("cq_world_create: unknown order %d", opt.order);
         return CQ_ERR_INVALID;
     }
-    int dev = 0;
+    int dev = 0, sms = 0;
     CQ_CUDA(cudaGetDevice(&dev));
+    CQ_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     cq_world *w = new cq_world();
     w->device = dev;
+    w->numSms = sms;
     w->order = opt.order;
     int rc = CQ_OK;
     auto fail = [&](int r) {

@@ -20,7 +20,7 @@ struct cq_crowd {
     cq_character_state *dStates = nullptr;
     double *dVelIn = nullptr;      // n * 3
     cq_crowd_pose *dPose = nullptr; // n
-    float hint = 0.0f;              // wall / PCIe ratio of the previous step (chunking heuristic of run_batch)
+    float hint = 0.0f;              // wall / PCIe ratio of the previous step (chunking heuristic, pipeline_chunks)
 };
 
 namespace cq {
@@ -113,20 +113,13 @@ int cq_crowd_step(cq_crowd *c, const double *velocity_in_xyz, const cq_controlle
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
     CQ_CUDA(cudaStreamSynchronize(w->stream));
-    static const int CH = [] { // units per chunk, as in run_batch (CQ_CHUNK overrides)
-        const char *e = getenv("CQ_CHUNK");
-        int v = e ? atoi(e) : 0;
-        return v >= 1024 ? v : (1 << 17);
-    }();
-    int nChunks = (n + CH - 1) / CH;
     static const float HINT = [] { // wall / PCIe-time ratio above which the step counts as compute bound (CQ_CROWD_HINT overrides)
         const char *e = getenv("CQ_CROWD_HINT");
         const float v = e ? (float)atof(e) : 0.0f;
         return v > 0.0f ? v : 3.0f;
     }();
-    if (c->hint > HINT && nChunks > 2) nChunks = 2; // compute bound last time: every chunk kernel pays its own tail
-    if (nChunks > CQ_PIPE_EVENTS) nChunks = CQ_PIPE_EVENTS;
-    if (flags & CQ_MAS_AGENTS) nChunks = 1; // the characters interact: all velocities must be in place before the kernel starts
+    // CQ_MAS_AGENTS: the characters interact, all velocities must be in place before the kernel starts
+    const int nChunks = pipeline_chunks(n, c->hint, HINT, (flags & CQ_MAS_AGENTS) != 0);
     const auto t0 = std::chrono::steady_clock::now();
     const int chunk = (n + nChunks - 1) / nChunks;
     int k = 0;

@@ -131,8 +131,8 @@ struct cq_world {
     std::vector<cq_material> hMaterials;
     std::vector<int32_t> hTriMat[2]; // host copy of DeviceSet::triMat (cq_world_triangle_material)
     unsigned long long *dCounters = nullptr; // 4 x u64: nodes, cands, evals, queries
-    int occ[6][4] = {}; // (raycast: [counting + 2 * reference-order walker]) // resident CTAs per SM of each persistent kernel ([counting + 2 * staged-walk variant])
-    int numSms = 0;
+    int numSms = 0; // SMs of `device`
+    std::unordered_map<const void *, int> residentBlocks; // persistent kernel -> one resident wave of its CTAs (resident_blocks)
     uint64_t launches = 0;
     cq::ScratchBuf nodeScratch[4], orderScratch[4];
     uint32_t orderSeq = 0;
@@ -143,7 +143,6 @@ struct cq_world {
     cq::ScratchBuf in, out, aux, aux2;
     cq::ScratchBuf agentScratch; // agent snapshot + grid of the move-and-slide call in flight (CQ_MAS_AGENTS)
     cq::ScratchBuf sepScratch;   // cq_agent_separation working set
-    int occSep[2][2] = {};       // resident CTAs per SM of k_sep_turns / k_sep_post ([counting build])
     void *sepGraphs = nullptr;   // instantiated round-loop graphs of cq_agent_separation (cq_sep.cu: SepGraphCache)
     std::vector<cq::ScratchBuf *> held; // scratch blocks acquired by the launch being enqueued (release_held)
     // transform updates (cq_api.cu: update_transforms_on)
@@ -177,6 +176,14 @@ int check_cuda(cudaError_t e, const char *what);
     } while (0)
 
 int ensure_scratch(ScratchBuf &b, size_t bytes);
+// CTAs of `kernel` (`threads` per CTA, `dynSmem` bytes of dynamic shared memory) that fit on the device at once: SMs x
+// resident CTAs per SM (at least one per SM), cached per world.  dynSmem > 0 also raises the kernel's dynamic shared-memory
+// limit to dynSmem.  0 on CUDA error.
+int resident_blocks(cq_world *w, const void *kernel, int threads, size_t dynSmem);
+// Chunk count of the copy/compute pipeline of a host-pointer call over n units (CQ_CHUNK sets the units per chunk): two
+// chunks only when the previous call's wall / PCIe-time ratio `hint` was above `computeBoundAbove`, because every chunk
+// kernel pays its own tail; at most CQ_PIPE_EVENTS; one when `singleChunk` (the units interact).
+int pipeline_chunks(int n, float hint, float computeBoundAbove, bool singleChunk);
 // after a synchronisation: has any kernel raised the world's status word since the last check?
 int check_status(cq_world *w, const char *what);
 // The world's scratch blocks (node stacks, unit order, agent grid, separation state) are shared by successive launches.

@@ -196,10 +196,6 @@ enum { NX_LOAD = 0, NX_DEPEN, NX_SLIDE, NX_SNAP, NX_FALL, NX_GATE, NX_OFFSET, NX
 #ifndef CQ_MAS_FE_IDLE
 #define CQ_MAS_FE_IDLE 16 /* idle lanes that open the front end (cq_pool.cuh: pool_run); >= 16 also selects the readiness rule */
 #endif
-#ifndef CQ_SINGLE_POST
-#define CQ_SINGLE_POST 1 /* every sweep of the controller is posted from ONE inlined pool_post_cast: 7 KB less code in the front end
-                            (measured, same box: hulls 432 -> 440 M/s, terrain 282 -> 285 M/s); 0 = one copy per posting state */
-#endif
 enum {
     F_WAS_G = 1, F_WAS_GN = 2, F_HAVE_LAST = 4, F_HAVE_CENTER = 8, F_GROUNDED = 16, F_GROUNDED_NEAR = 32,
     F_CAN_SNAP = 64, F_NEAR_GROUND = 128, F_PROBE_HIT = 256, F_DID_RESOLVE = 512
@@ -483,11 +479,9 @@ __device__ __forceinline__ bool mas_advance(CharCtx &c, const QResult &q, QShare
     const cq_controller_params &P = A.p;
     const f3 down = {0.0f, -1.0f, 0.0f};
     int next = NX_LOAD;
-#if CQ_SINGLE_POST
     f3 postFrom = {0.0f, 0.0f, 0.0f}, postDelta = {0.0f, 0.0f, 0.0f};
     int postMode = CQ_MODE_ALL, postWait = W_NONE;
     float postMinY = 0.0f;
-#endif
     // ---------------- consume
     switch (c.wait) {
     case W_DEPEN: { // DepenetrationResolver.resolve loop body after the overlap query (SYS:756-799)
@@ -697,47 +691,26 @@ __device__ __forceinline__ bool mas_advance(CharCtx &c, const QResult &q, QShare
             if (c.slideIt >= P.max_slide_iterations || c.slideLen < 1e-6f) { // SYS:1674-1676
                 next = NX_SNAP;
             } else {
-#if CQ_SINGLE_POST
                 postFrom = ld3(c.pos), postDelta = remaining, postMode = CQ_MODE_BLOCKING, postMinY = 0.0f, postWait = W_SLIDE;
                 next = NX_POST;
-#else
-                pool_post_cast<COUNT>(W, wp, lane, s, ld3(c.pos), remaining, P.radius, P.half_height, P.collision_mask,
-                                    CQ_MODE_BLOCKING, 0.0f, ctr);
-                c.wait = W_SLIDE;
-                return true;
-#endif
             }
         }
         if (next == NX_SNAP) {
             if (!(P.snap_distance > 0.0f)) { // SYS:845
                 next = NX_FALL;
             } else {
-#if CQ_SINGLE_POST
                 postFrom = ld3(c.pos), postDelta = down * P.snap_distance, postMode = CQ_MODE_GROUND, postMinY = P.min_ground_dot;
                 postWait = W_SNAP;
                 next = NX_POST;
-#else
-                pool_post_cast<COUNT>(W, wp, lane, s, ld3(c.pos), down * P.snap_distance, P.radius, P.half_height,
-                                    P.collision_mask, CQ_MODE_GROUND, P.min_ground_dot, ctr);
-                c.wait = W_SNAP;
-                return true;
-#endif
             }
         }
         if (next == NX_FALL) {
             if (!(P.fall_probe_distance > 0.0f)) { // SYS:855
                 next = NX_GATE;
             } else {
-#if CQ_SINGLE_POST
                 postFrom = ld3(c.pos), postDelta = down * P.fall_probe_distance, postMode = CQ_MODE_GROUND;
                 postMinY = P.min_ground_dot, postWait = W_FALL;
                 next = NX_POST;
-#else
-                pool_post_cast<COUNT>(W, wp, lane, s, ld3(c.pos), down * P.fall_probe_distance, P.radius, P.half_height,
-                                    P.collision_mask, CQ_MODE_GROUND, P.min_ground_dot, ctr);
-                c.wait = W_FALL;
-                return true;
-#endif
             }
         }
         if (next == NX_GATE) { // validity gates after the centre + fall casts (SYS:868-925)
@@ -779,25 +752,18 @@ __device__ __forceinline__ bool mas_advance(CharCtx &c, const QResult &q, QShare
             int oi = c.offsetIt;
             float ox = oi == 0 ? offset : (oi == 1 ? -offset : 0.0f);
             float oz = oi == 2 ? offset : (oi == 3 ? -offset : 0.0f);
-#if CQ_SINGLE_POST
             postFrom = ld3(c.pos) + mk3(ox, 0.0f, oz), postDelta = down * P.snap_distance, postMode = CQ_MODE_GROUND;
             postMinY = P.min_ground_dot, postWait = W_OFFSET;
             next = NX_POST;
-#else
-            pool_post_cast<COUNT>(W, wp, lane, s, ld3(c.pos) + mk3(ox, 0.0f, oz), down * P.snap_distance, P.radius, P.half_height,
-                                P.collision_mask, CQ_MODE_GROUND, P.min_ground_dot, ctr);
-            c.wait = W_OFFSET;
-            return true;
-#endif
         }
-#if CQ_SINGLE_POST
-        if (next == NX_POST) { // the one place a sweep is posted from: pool_post_cast is ~150 instructions per inlined copy
+        // the one place a sweep is posted from: pool_post_cast is ~150 instructions per inlined copy, and one site instead of
+        // four keeps 7 KB of code out of the front end (DESIGN.md §5.1)
+        if (next == NX_POST) {
             pool_post_cast<COUNT>(W, wp, lane, s, postFrom, postDelta, P.radius, P.half_height, P.collision_mask, postMode, postMinY,
                                   ctr);
             c.wait = postWait;
             return true;
         }
-#endif
         if (next == NX_FINISH) {
             mas_finish(c, W, A, states + c.charIndex, COUNT, ctr.evals);
             next = NX_LOAD;
@@ -832,8 +798,6 @@ __global__ void __launch_bounds__(MAS_THREADS, MAS_MIN_BLOCKS) k_move_and_slide(
     pool_flush_counters(ctr, gctr, COUNT);
 }
 
-#define CQ_OCC_SLOT 0
-#define CQ_OCC_SLOT_AGENTS 5
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
                           const float g[3], uint32_t flags, const cq_platform *platforms, int nPlatforms, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
@@ -851,8 +815,6 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
     A.nPlatforms = nPlatforms;
     for (int k = 0; k < nPlatforms; k++) A.platforms[k] = platforms[k];
     const bool agents = (flags & CQ_MAS_AGENTS) != 0;
-    int *blocksPerSm = w->occ[agents ? CQ_OCC_SLOT_AGENTS : CQ_OCC_SLOT];
-    int &numSms = w->numSms;
     const int staged = w->view.stagedLeaves ? 1 : 0;
     const int ci = (w->counting ? 1 : 0) + 2 * staged;
     using Kernel = void (*)(WorldView, cq_character_state *, int, const MasArgs, int, uint2 *, int *, const uint32_t *,
@@ -862,20 +824,13 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
                                          {k_move_and_slide<false, true, false>, k_move_and_slide<true, true, false>,
                                           k_move_and_slide<false, true, true>, k_move_and_slide<true, true, true>}};
     const Kernel kernel = kernels[agents ? 1 : 0][ci];
-    if (!blocksPerSm[ci]) {
-        cudaDeviceProp prop;
-        CQ_CUDA(cudaGetDeviceProperties(&prop, w->device));
-        numSms = prop.multiProcessorCount;
-        int b = 0;
-        CQ_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MAS_SMEM_BYTES));
-        CQ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, MAS_THREADS, MAS_SMEM_BYTES));
-        blocksPerSm[ci] = b > 0 ? b : 1;
-    }
-    // persistent lanes: one resident wave of CTAs (148 SMs x resident CTAs per SM), lanes stride over characters
-    int blocks = std::min((n + MAS_THREADS - 1) / MAS_THREADS, numSms * blocksPerSm[ci]);
+    const int resident = resident_blocks(w, (const void *)kernel, MAS_THREADS, MAS_SMEM_BYTES);
+    if (!resident) return CQ_ERR_CUDA;
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;
-    blocks = std::min((n + 3) / 4, numSms * blocksPerSm[ci]); // small batches: still fill the machine (>= 4 units per CTA)
+    // persistent lanes: one resident wave of CTAs, lanes stride over characters; small batches still fill the machine
+    // (>= 4 units per CTA)
+    const int blocks = std::min((n + 3) / 4, resident);
     const int opw = pool_owners_per_warp(n, (long long)blocks * MAS_WARPS);
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * MAS_WARPS, st);
     if (!ns) return CQ_ERR_CUDA;

@@ -32,20 +32,11 @@ namespace cq {
 enum { PH_NONE = 0, PH_ADV = 1, PH_BIS = 2, PH_FIN = 3, PH_OVL = 4 };
 #define CQ_KIND_OVERLAP 3 /* query mode: two-deepest overlap (move-and-slide depenetration) */
 #define CQ_QCAP 256       /* pair-ring entries per warp */
-#ifndef CQ_EVAL_REPS
-#define CQ_EVAL_REPS 1    /* distance evaluations per main-loop trip (see pool_run) */
-#endif
 #ifndef CQ_WALK_FILL /* walk rounds run until the pair ring holds this many pairs.  Swept on one box after the slim pair state
                         (profiles/r2_ab_same_box.txt, call 20; 96 everywhere before): the move-and-slide kernels gain 0.3-0.8% with a
                         fuller ring (a round always leaves room for 128 more, so 160 means "up to 128"), the query kernels
                         2.8% on C2 with a shorter one (fresher bestT for the culling of the next walk rounds; C4 unchanged) */
 #define CQ_WALK_FILL (LOOKAHEAD ? 64 : 160)
-#endif
-#ifndef CQ_PICKUP_DROP
-#define CQ_PICKUP_DROP 1 /* 0: sweeps keep every candidate of the whole sweep's box (no bestT-based drops in walk / pickup; A/B) */
-#endif
-#ifndef CQ_EVAL_KEEP
-#define CQ_EVAL_KEEP 0    /* with CQ_EVAL_REPS > 1: keep evaluating only while this many lanes hold a live pair */
 #endif
 #define CQ_NSCAP 2048     /* node-stack entries per warp (global memory; 32 concurrent walks) */
 // Stack budget.  A walk round with 32 poppers grows the stack by at most 32 x (4 - 1) = 96 entries; posting roots adds at
@@ -281,7 +272,7 @@ __device__ __forceinline__ void pool_walk_round(const WorldView &W, const WarpPo
         const int owner = e.x >> 2, set = (e.x >> 1) & 1;
         QShared &s = wp.qs[owner];
         f3 qlo = mk3(s.qlo[0], s.qlo[1], s.qlo[2]), qhi = mk3(s.qhi[0], s.qhi[1], s.qhi[2]);
-        if (LOOKAHEAD && CQ_PICKUP_DROP && !(COUNT && W.refStats)) {
+        if (LOOKAHEAD && !(COUNT && W.refStats)) {
             float bestT, margin;
             if (sweep_reach(s, bestT, margin)) sweep_reach_box(s, bestT, margin, qlo, qhi);
         }
@@ -365,7 +356,7 @@ __device__ __forceinline__ void pool_walk_round(const WorldView &W, const WarpPo
             f3 v0 = xyz(a), v1 = xyz(b), v2 = xyz(c);
             f3 tlo = vmin(v0, vmin(v1, v2)), thi = vmax(v0, vmax(v1, v2));
             if (box_disjoint(tlo, thi, qlo, qhi)) continue; // :1060-1065
-            if (LOOKAHEAD && CQ_PICKUP_DROP && !(COUNT && W.refStats)) {
+            if (LOOKAHEAD && !(COUNT && W.refStats)) {
                 float bestT, margin;
                 if (sweep_reach(s, bestT, margin) && sweep_cannot_matter(s, bestT, margin, tlo, thi, __float_as_int(c.w))) continue;
             }
@@ -390,10 +381,8 @@ __device__ __forceinline__ void pool_walk_round(const WorldView &W, const WarpPo
 // OVLDROP (the staged-walk move-and-slide kernel and the query kernels): an overlap candidate is dropped when the kernel's
 // bookkeeping says it cannot matter (OverlapTop2::cannot_matter: reference order, eight overlaps on record, this triangle
 // visited after all of them; OverlapTopK::cannot_matter: the same once the overflow of capsuleOverlapAll is established).
-template <bool COUNT, bool LOOKAHEAD_, bool OVLDROP_, class OvlCommit>
+template <bool COUNT, bool LOOKAHEAD, bool OVLDROP, class OvlCommit>
 __device__ __forceinline__ void pool_take_jobs(const WorldView &W, const WarpPool &wp, Job &job, int lane, const OvlCommit &ovl) {
-    constexpr bool LOOKAHEAD = LOOKAHEAD_ && CQ_PICKUP_DROP;
-    constexpr bool OVLDROP = OVLDROP_ && CQ_PICKUP_DROP;
 #pragma unroll 1
     for (int rep = 0; rep < (LOOKAHEAD ? 4 : 1); rep++) { // (an overlap drop is rare: its lane simply idles one trip)
         uint32_t idle = __ballot_sync(0xffffffffu, job.phase == PH_NONE);
@@ -650,10 +639,6 @@ static __device__ __noinline__ void pool_post_first_hits(const uint32_t *__restr
     s.pending = CQ_MAX_OVERLAP_HITS;
 }
 
-#ifndef CQ_COMMIT_REDUCE_MAS
-#define CQ_COMMIT_REDUCE_MAS 0 /* 1: every move-and-slide kernel settles sweep hits with warp reductions (A/B) */
-#endif
-
 // Commit step: the lanes that finished a pair this trip hand their contribution to the owner's record; pending counters drop.
 // Contributions to DIFFERENT owners touch different records and commute; contributions to the same owner are order-free
 // reductions (smallest (toi, rank); deepest two / smallest ranks; counts).  So the lanes are grouped by owner (one MATCH) and
@@ -808,21 +793,8 @@ __device__ __forceinline__ void pool_run(const WorldView &W, const WarpPool &wp,
         Commit cm;
         cm.kind = 0;
         bool retired = false;
-#if CQ_EVAL_REPS <= 1
         if (job.phase != PH_NONE) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr, !STAGED && !(COUNT && W.refStats));
-#else
-        // Up to CQ_EVAL_REPS evaluations per trip while at least CQ_EVAL_KEEP lanes still hold a live pair: pickup, commit
-        // and the exit vote are then paid once per several evaluations.  Exact: a finished pair keeps its contribution
-        // in `cm` until the commit below, and a stale bestT only delays a prune (the commit compares again).
-#pragma unroll 1
-        for (int rep = 0; rep < CQ_EVAL_REPS; rep++) {
-            const bool go = job.phase != PH_NONE && !retired;
-            const uint32_t live = (uint32_t)__popc(__ballot_sync(0xffffffffu, go));
-            if (live == 0u || (rep > 0 && live < (uint32_t)CQ_EVAL_KEEP)) break;
-            if (go) pool_eval<COUNT, LOOKAHEAD>(job, wp, cm, retired, ctr, !STAGED && !(COUNT && W.refStats));
-        }
-#endif
-        pool_commit<LOOKAHEAD || (STAGED && FE_IDLE >= 16) || CQ_COMMIT_REDUCE_MAS>(wp, job, cm, retired, lane, ovl);
+        pool_commit<LOOKAHEAD || (STAGED && FE_IDLE >= 16)>(wp, job, cm, retired, lane, ovl);
         if (__all_sync(0xffffffffu, !alive && job.phase == PH_NONE) && *wp.ntop == 0u && *wp.tail == *wp.head) break;
     }
 }

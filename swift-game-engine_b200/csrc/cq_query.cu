@@ -8,19 +8,6 @@ namespace cq {
 
 #define Q_THREADS 128
 
-template <bool COUNT> __device__ __forceinline__ void flush_counters(const Counters &c, unsigned long long *g) {
-    if (!COUNT) return;
-    // warp-reduce, one atomic per warp per counter
-    uint32_t v[4] = {c.nodes, c.cands, c.evals, c.queries};
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-        unsigned long long s = v[k];
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-        if ((threadIdx.x & 31) == 0 && s) atomicAdd(g + k, s);
-    }
-}
-
 __device__ __forceinline__ void store3(float *o, f3 v) {
     o[0] = v.x;
     o[1] = v.y;
@@ -29,131 +16,7 @@ __device__ __forceinline__ void store3(float *o, f3 v) {
 __device__ __forceinline__ f3 load3(const float *p) { return {p[0], p[1], p[2]}; }
 
 // ---------------------------------------------------------------- raycast (CollisionQuery.swift:768-785, 916-978)
-// Flat per-lane state machine over persistent lanes: every trip of the loop each lane performs exactly ONE step
-// of its ray — a node step (fetch a 64-byte node, test both child boxes, push/descend) or a triangle step
-// (Moller-Trumbore on the next triangle of the current leaf range) — and a lane whose ray is finished writes the
-// hit and fetches the next ray in the same trip.  The nested while-while version ran 3.5 of 32 lanes (ncu).
-// Result = the triangle with the smallest t over ALL triangles (ties -> smallest index); boxes only skip work and
-// the box test is conservative (see ray_box).
-template <bool COUNT>
-__global__ void __launch_bounds__(Q_THREADS) k_raycast(WorldView W, const cq_ray *__restrict__ rays, int n,
-                                                       cq_ray_hit *__restrict__ out, uint8_t *__restrict__ flagsOut,
-                                                       int *workCounter, const uint32_t *__restrict__ order,
-                                                       unsigned long long *gctr) {
-    Counters ctr = {0, 0, 0, 0};
-    uint32_t tie = 0;
-    int stack[CQ_STACK];
-    int sp = 0, set = 2, leafPos = 0, leafEnd = 0, cur = -1;
-    int bestTri = -1;
-    float closestT = 0.0f;
-    f3 o = {0, 0, 0}, d = {0, 0, 0}, inv = {0, 0, 0}, bestN = {0, 0, 0};
-    uint32_t mask = 0;
-    bool alive = true;
-    while (true) {
-        if (alive && leafPos >= leafEnd && sp == 0) {
-            if (set < 2) { // next triangle set of this ray (static, then dynamic), or finish the ray
-                const SetHeader h = *(set ? W.set[1].hdr : W.set[0].hdr);
-                if (h.rootRef != CQ_REF_EMPTY) {
-                    if (COUNT) {
-                        ctr.queries++;
-                        ctr.nodes++;
-                    }
-                    if (ray_box(o, inv, mk3(h.lo[0], h.lo[1], h.lo[2]), mk3(h.hi[0], h.hi[1], h.hi[2]), closestT))
-                        stack[sp++] = h.rootRef < 0 ? ~((~h.rootRef) | (set << 30)) : (h.rootRef | (set << 30)); // bit 30 = set
-                }
-                set++;
-            } else {
-                if (cur >= 0) {
-                    cq_ray_hit hres;
-                    if (bestTri >= 0) {
-                        hres.distance = closestT;
-                        store3(hres.position, o + d * closestT); // :962
-                        store3(hres.normal, bestN);
-                        hres.triangle_index = bestTri;
-                    } else {
-                        hres.distance = 0.0f;
-                        store3(hres.position, mk3(0, 0, 0));
-                        store3(hres.normal, mk3(0, 0, 0));
-                        hres.triangle_index = -1;
-                    }
-                    out[cur] = hres;
-                    if (flagsOut) flagsOut[cur] = (uint8_t)tie;
-                }
-                cur = atomicAdd(workCounter, 1);
-                if (cur >= n) {
-                    cur = -1;
-                    alive = false;
-                } else {
-                    if (order) cur = (int)order[cur];
-                    cq_ray r = rays[cur];
-                    o = load3(r.origin), d = load3(r.direction);
-                    closestT = r.max_distance;
-                    mask = r.mask;
-                    bestTri = -1, tie = 0;
-                    // CollisionQuery.swift:1606-1608: 1/d, or greatestFiniteMagnitude when d == 0
-                    inv = mk3(d.x != 0.0f ? 1.0f / d.x : FLT_MAX, d.y != 0.0f ? 1.0f / d.y : FLT_MAX,
-                              d.z != 0.0f ? 1.0f / d.z : FLT_MAX);
-                    set = 0;
-                }
-            }
-        } else if (alive && leafPos < leafEnd) { // triangle step
-            const int s1 = (leafPos >> 30) & 1, slot = leafPos & 0x3fffffff;
-            leafPos++;
-            const SetView &S = W.set[s1];
-            uint32_t layer;
-            int triId, part;
-            Tri T = load_tri(S, slot, layer, triId, part);
-            if ((layer & mask) != 0u) {
-                if (COUNT) ctr.cands++;
-                float t;
-                if (ray_triangle(o, d, T, t)) {
-                    int gid = triId + S.triOffset;
-                    if (bestTri >= 0 && t == closestT) tie = CQ_HIT_TIE;
-                    if (t < closestT) tie = 0;
-                    if (t < closestT || (bestTri >= 0 && t == closestT && gid < bestTri)) {
-                        closestT = t;
-                        bestTri = gid;
-                        f3 nrm = normalize(cross(T.v1 - T.v0, T.v2 - T.v0)); // :960-961
-                        bestN = dot(nrm, d) > 0.0f ? -nrm : nrm;
-                    }
-                }
-            }
-        } else if (alive) { // node step
-            int ref = stack[--sp];
-            if (ref < 0) {
-                int enc = ~ref;
-                const int s1 = (enc >> 30) & 1;
-                enc &= 0x3fffffff;
-                leafPos = (enc >> 2) | (s1 << 30);
-                leafEnd = leafPos + (enc & 3) + 1;
-            } else {
-                const int s1 = (ref >> 30) & 1;
-                const Node *nd = W.set[s1].nodes + (ref & 0x3fffffff);
-                float4 n0 = __ldg(&nd->n0), n1 = __ldg(&nd->n1), n2 = __ldg(&nd->n2), n3 = __ldg(&nd->n3);
-                if (COUNT) ctr.nodes += 2;
-                bool h0 = ray_box(o, inv, xyz(n0), xyz(n1), closestT);
-                bool h1 = ray_box(o, inv, xyz(n2), xyz(n3), closestT);
-                int r0 = __float_as_int(n0.w), r1 = __float_as_int(n1.w);
-                // tag the set into bit 30 (internal refs are < 2^26; leaf encodings are stored complemented)
-                r0 = r0 < 0 ? ~((~r0) | (s1 << 30)) : (r0 | (s1 << 30));
-                r1 = r1 < 0 ? ~((~r1) | (s1 << 30)) : (r1 | (s1 << 30));
-                if (h1) stack[sp++] = r1;
-                if (h0) stack[sp++] = r0;
-            }
-        }
-        if (__all_sync(0xffffffffu, !alive)) break;
-    }
-    flush_counters<COUNT>(ctr, gctr);
-}
-
-// ---------------------------------------------------------------- raycast in REFERENCE order
-// The reference's walk itself (CollisionQuery.swift:916-978) over the reference's own tree (cq_reftree.h, uploaded by
-// attach_ref_order): per set, closestT starts at maxDistance; pop a node, cull it when rayAABB (:1603-1631, restated
-// below with the same operations) misses or starts beyond closestT, test a leaf's triangles in triOrder with strict
-// `t < closestT`, push left then right.  The slab test of a child is evaluated when its parent is visited (a miss
-// never depends on closestT) and its tmin travels with the stack entry, so the `tmin > closestT` test happens at pop
-// time with the value closestT has THEN — the same nodes are culled as in the reference, including the grazing hits its
-// non-conservative slab test loses.  Static and dynamic sets are walked independently and merged with `<=` (:902-907).
+// rayAABB (:1603-1631) with the same operations: the slab test of the reference's own walk
 __device__ __forceinline__ bool ref_ray_aabb(f3 o, f3 inv, f3 lo, f3 hi, float &tminOut) {
     float tmin = (lo.x - o.x) * inv.x, tmax = (hi.x - o.x) * inv.x;
     if (tmin > tmax) {
@@ -178,142 +41,27 @@ __device__ __forceinline__ bool ref_ray_aabb(f3 o, f3 inv, f3 lo, f3 hi, float &
     return true;
 }
 
-template <bool COUNT>
-__global__ void __launch_bounds__(Q_THREADS) k_raycast_ref(WorldView W, const cq_ray *__restrict__ rays, int n,
-                                                           cq_ray_hit *__restrict__ out, uint8_t *__restrict__ flagsOut,
-                                                           int *workCounter, const uint32_t *__restrict__ order,
-                                                           unsigned long long *gctr) {
-    Counters ctr = {0, 0, 0, 0};
-    int stackRef[CQ_STACK];
-    float stackT[CQ_STACK];
-    int sp = 0, set = 2, leafPos = 0, leafEnd = 0, cur = -1;
-    int bestTri = -1, setTri = -1;
-    float closestT = 0.0f, bestT = 0.0f, maxDist = 0.0f;
-    f3 o = {0, 0, 0}, d = {0, 0, 0}, inv = {0, 0, 0}, bestN = {0, 0, 0}, setN = {0, 0, 0};
-    uint32_t mask = 0, tie = 0, setTie = 0;
-    bool alive = true;
-    while (true) {
-        if (alive && leafPos >= leafEnd && sp == 0) {
-            // a set's walk is over: merge its hit (static wins `<=`, :902-907), then the next set or the next ray
-            if (setTri >= 0 && (bestTri < 0 || !(bestT <= closestT))) bestT = closestT, bestTri = setTri, bestN = setN, tie = setTie;
-            setTri = -1, setTie = 0;
-            if (set < 2) {
-                const SetHeader h = *(set ? W.set[1].refHdr : W.set[0].refHdr);
-                closestT = maxDist;
-                if (h.rootRef != CQ_REF_EMPTY) {
-                    if (COUNT) {
-                        ctr.queries++;
-                        ctr.nodes++;
-                    }
-                    float tmin;
-                    if (ref_ray_aabb(o, inv, mk3(h.lo[0], h.lo[1], h.lo[2]), mk3(h.hi[0], h.hi[1], h.hi[2]), tmin)) {
-                        stackRef[sp] = h.rootRef < 0 ? ~((~h.rootRef) | (set << 30)) : (h.rootRef | (set << 30));
-                        stackT[sp++] = tmin;
-                    }
-                }
-                set++;
-            } else {
-                if (cur >= 0) {
-                    cq_ray_hit hres;
-                    if (bestTri >= 0) {
-                        hres.distance = bestT;
-                        store3(hres.position, o + d * bestT); // :962
-                        store3(hres.normal, bestN);
-                        hres.triangle_index = bestTri;
-                    } else {
-                        hres.distance = 0.0f;
-                        store3(hres.position, mk3(0, 0, 0));
-                        store3(hres.normal, mk3(0, 0, 0));
-                        hres.triangle_index = -1;
-                    }
-                    out[cur] = hres;
-                    if (flagsOut) flagsOut[cur] = (uint8_t)tie;
-                }
-                cur = atomicAdd(workCounter, 1);
-                if (cur >= n) {
-                    cur = -1;
-                    alive = false;
-                } else {
-                    if (order) cur = (int)order[cur];
-                    cq_ray r = rays[cur];
-                    o = load3(r.origin), d = load3(r.direction);
-                    maxDist = r.max_distance;
-                    mask = r.mask;
-                    bestTri = -1, setTri = -1, tie = 0;
-                    inv = mk3(d.x != 0.0f ? 1.0f / d.x : FLT_MAX, d.y != 0.0f ? 1.0f / d.y : FLT_MAX,
-                              d.z != 0.0f ? 1.0f / d.z : FLT_MAX); // :1606-1608
-                    set = 0;
-                }
-            }
-        } else if (alive && leafPos < leafEnd) { // triangle step, ascending triOrder positions (:938-940)
-            const int s1 = (leafPos >> 30) & 1, pos = leafPos & 0x3fffffff;
-            leafPos++;
-            const SetView &S = W.set[s1];
-            const int slot = (int)__ldg(S.refSlot + pos);
-            uint32_t layer;
-            int triId, part;
-            Tri T = load_tri(S, slot, layer, triId, part);
-            if ((layer & mask) != 0u) {
-                if (COUNT) ctr.cands++;
-                float t;
-                if (ray_triangle(o, d, T, t)) {
-                    if (t < closestT) { // strict: the first visited keeps an exact tie (:944)
-                        closestT = t;
-                        setTri = triId + S.triOffset;
-                        setTie = 0;
-                        f3 nrm = normalize(cross(T.v1 - T.v0, T.v2 - T.v0));
-                        setN = dot(nrm, d) > 0.0f ? -nrm : nrm;
-                    } else if (t == closestT && setTri >= 0) {
-                        setTie = CQ_HIT_TIE;
-                    }
-                }
-            }
-        } else if (alive) { // node step
-            --sp;
-            const int ref = stackRef[sp];
-            const float tminNode = stackT[sp];
-            if (!(tminNode > closestT)) { // :933, with the closestT of NOW
-                if (ref < 0) {
-                    int enc = ~ref;
-                    const int s1 = (enc >> 30) & 1;
-                    enc &= 0x3fffffff;
-                    leafPos = (enc >> 2) | (s1 << 30);
-                    leafEnd = leafPos + (enc & 3) + 1;
-                } else {
-                    const int s1 = (ref >> 30) & 1;
-                    const Node *nd = W.set[s1].refNodes + (ref & 0x3fffffff);
-                    float4 n0 = __ldg(&nd->n0), n1 = __ldg(&nd->n1), n2 = __ldg(&nd->n2), n3 = __ldg(&nd->n3);
-                    if (COUNT) ctr.nodes += 2;
-                    float t0, t1;
-                    const bool h0 = ref_ray_aabb(o, inv, xyz(n0), xyz(n1), t0); // left
-                    const bool h1 = ref_ray_aabb(o, inv, xyz(n2), xyz(n3), t1); // right
-                    int r0 = __float_as_int(n0.w), r1 = __float_as_int(n1.w);
-                    r0 = r0 < 0 ? ~((~r0) | (s1 << 30)) : (r0 | (s1 << 30));
-                    r1 = r1 < 0 ? ~((~r1) | (s1 << 30)) : (r1 | (s1 << 30));
-                    if (h0) stackRef[sp] = r0, stackT[sp++] = t0; // push left, then right: the right child is popped first (:965-966)
-                    if (h1) stackRef[sp] = r1, stackT[sp++] = t1;
-                }
-            }
-        }
-        if (__all_sync(0xffffffffu, !alive)) break;
-    }
-    flush_counters<COUNT>(ctr, gctr);
-}
-
-// ---------------------------------------------------------------- raycast, phase-voted (both order rules)
-// ncu on the one-step-per-trip kernels above (profiles/r2_c5_raycast_v12_summary.txt): 7.2 of 32 lanes active per warp
-// instruction, 65% of the stall samples long-scoreboard.  A ray of C5 takes ~8 node steps, ~1.4 triangle steps and one
-// finish + fetch; with one step of whatever kind per trip every trip pays for all three bodies while each is populated
-// by a third of the lanes or fewer.  Here the three bodies are PHASES of the warp:
+// One kernel, both order rules (REF):
+//   canonical  the triangle with the smallest t over ALL triangles (ties -> smallest index); boxes only skip work and the
+//              box test is conservative (see ray_box).
+//   reference  the reference's walk itself (CollisionQuery.swift:916-978) over the reference's own tree (cq_reftree.h,
+//              uploaded by attach_ref_order): per set, closestT starts at maxDistance; pop a node, cull it when rayAABB
+//              (ref_ray_aabb) misses or starts beyond closestT, test a leaf's triangles in triOrder with strict
+//              `t < closestT`, push left then right.  The slab test of a child is evaluated when its parent is visited (a
+//              miss never depends on closestT) and its tmin travels with the stack entry, so the `tmin > closestT` test
+//              happens at pop time with the value closestT has THEN — the same nodes are culled as in the reference,
+//              including the grazing hits its non-conservative slab test loses.  Static and dynamic sets are walked
+//              independently and merged with `<=` (:902-907).
+// Phase voting.  ncu on the earlier one-step-per-trip kernels (profiles/r2_c5_raycast_v12_summary.txt): 7.2 of 32 lanes
+// active per warp instruction, 65% of the stall samples long-scoreboard.  A ray of C5 takes ~8 node steps, ~1.4 triangle
+// steps and one finish + fetch; with one step of whatever kind per trip every trip pays for all three bodies while each
+// is populated by a third of the lanes or fewer.  Here the three bodies are PHASES of the warp:
 //   refill    finished lanes write their hit and fetch the next ray — only when at least RAY_REFILL_MIN lanes are idle
 //             (or nobody has anything else to do), so the long, latency-heavy body runs for many lanes at once;
 //   nodes     lanes with a non-empty stack pop / test / push, and the phase REPEATS while at least RAY_NODE_MIN lanes
 //             still want a node step: the dependent node fetches of most of the warp are in flight together;
 //   triangles lanes holding a leaf range test their next triangle, repeated while RAY_TRI_MIN lanes have one.
 // Every phase runs at least once per round when any lane wants it, so progress never depends on the thresholds.
-// The per-ray logic is exactly that of k_raycast (canonical: nearest over all triangles, conservative padded slabs,
-// ties to the smaller index) and k_raycast_ref (the reference's walk over the reference's tree, its own slab test,
-// tmin re-tested at pop time, sets walked independently and merged with `<=`).
 #ifndef RAY_REFILL_MIN
 #define RAY_REFILL_MIN 8
 #endif
@@ -534,7 +282,7 @@ __global__ void __launch_bounds__(Q_THREADS) k_raycast_phased(WorldView W, const
             if (__popc(tMask) < RAY_TRI_MIN) break;
         }
     }
-    flush_counters<COUNT>(ctr, gctr);
+    pool_flush_counters(ctr, gctr, COUNT);
 }
 
 // ---------------------------------------------------------------- capsule cast (CollisionQuery.swift:787-828, 980-1117)
@@ -542,9 +290,6 @@ __global__ void __launch_bounds__(Q_THREADS) k_raycast_phased(WorldView W, const
 // walks the LBVH for it and pushes its candidate triangles into the warp's ring; all 32 lanes execute
 // the (sweep, triangle) pairs, one distance evaluation per trip.
 #define CAST_WARPS (Q_THREADS / 32)
-#ifndef CQ_UNIT_BATCH
-#define CQ_UNIT_BATCH 1 /* > 1: sweeps claimed per atomic by k_capsule_cast, with an L2 prefetch of their records (round-2 A/B) */
-#endif
 #ifndef CAST_MIN_BLOCKS
 #define CAST_MIN_BLOCKS 5 /* 96 registers: +9% on C4 against 4 CTAs/SM (107 registers); 6 CTAs/SM (80) gains nothing */
 #endif
@@ -562,9 +307,6 @@ __global__ void __launch_bounds__(Q_THREADS, CAST_MIN_BLOCKS) k_capsule_cast(Wor
     pool_bind(wp, qsAll, words, nodeScratch, warp, CAST_WARPS, W.rank, W.status);
     Counters ctr = {0, 0, 0, 0};
     int cur = -1;
-#if CQ_UNIT_BATCH > 1
-    int batchNext = 0, batchEnd = 0; // [batchNext, batchEnd): positions in the processing order this owner has claimed
-#endif
     pool_run<COUNT, STAGED, 8, true>(W, wp, lane, ownersPerWarp, ctr, [&](QShared &mine, Counters &ct) {
         if (cur >= 0) { // write the finished hit
             cq_cast_hit h;
@@ -584,38 +326,18 @@ __global__ void __launch_bounds__(Q_THREADS, CAST_MIN_BLOCKS) k_capsule_cast(Wor
             out[cur] = h;
             if (flagsOut) flagsOut[cur] = (mine.mode & CQ_QF_TIE) ? CQ_HIT_TIE : 0;
         }
-#if CQ_UNIT_BATCH > 1
-        // claim CQ_UNIT_BATCH sweeps per atomic and start their query records towards L2 right away: the chain
-        // atomic -> order[] -> query record is three dependent long-latency accesses, paid once per sweep on a single lane
-        // (C4: 8% of the kernel's stall samples sit in this fetch + posting, 64-78% of them long-scoreboard waits)
-        if (batchNext == batchEnd) {
-            batchNext = atomicAdd(workCounter, CQ_UNIT_BATCH);
-            batchEnd = min(batchNext + CQ_UNIT_BATCH, n);
-            if (batchNext >= n) {
-                batchNext = batchEnd = 0;
-                cur = -1;
-                return false;
-            }
-            for (int k = batchNext + 1; k < batchEnd; k++) {
-                const int id = order ? (int)order[k] : k;
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(qs + id));
-            }
-        }
-        cur = batchNext++;
-#else
         cur = atomicAdd(workCounter, 1); // dynamic fetch of the next sweep
         if (cur >= n) {
             cur = -1;
             return false;
         }
-#endif
         if (order) cur = (int)order[cur]; // Morton-coherent processing order (big worlds)
         cq_capsule_cast c = qs[cur];
         pool_post_cast<COUNT>(W, wp, lane, mine, load3(c.from), load3(c.delta), c.radius, c.half_height, c.mask, mode,
                               c.min_normal_y, ct);
         return true;
     }, OverlapTop2{W.rank != nullptr});
-    flush_counters<COUNT>(ctr, gctr);
+    pool_flush_counters(ctr, gctr, COUNT);
 }
 
 __device__ __forceinline__ void write_overlap(cq_overlap_hit &h, const OverlapRec &r) {
@@ -754,36 +476,24 @@ __global__ void __launch_bounds__(Q_THREADS, 4) k_capsule_overlap_pool(WorldView
         pool_post_overlap<COUNT>(W, wp, lane, mine, curFrom, curR, curHH, c.mask, ct);
         return true;
     }, OverlapTopK{tops + warp * 32, ALL && W.rank != nullptr});
-    flush_counters<COUNT>(ctr, gctr);
+    pool_flush_counters(ctr, gctr, COUNT);
 }
 
 // ---------------------------------------------------------------- launchers
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 
-#undef CQ_OCC_SLOT
-#define CQ_OCC_SLOT 1
 int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
     CQ_TRY(await_trees(w, st));
-    int *blocksPerSm = w->occ[CQ_OCC_SLOT]; int &numSms = w->numSms;
     const bool ref = w->order == CQ_ORDER_REFERENCE; // the reference's own walk over the reference's own tree
     const int ci = (w->counting ? 1 : 0) + (ref ? 2 : 0);
     using Kernel = void (*)(WorldView, const cq_ray *, int, cq_ray_hit *, uint8_t *, int *, const uint32_t *, unsigned long long *);
-    static const bool stepwise = getenv("CQ_RAY_STEPWISE") != nullptr; // the older one-step-per-trip kernels (A/B)
-    static const Kernel phased[4] = {k_raycast_phased<false, false>, k_raycast_phased<true, false>, k_raycast_phased<false, true>,
-                                     k_raycast_phased<true, true>};
-    static const Kernel kernels_old[4] = {k_raycast<false>, k_raycast<true>, k_raycast_ref<false>, k_raycast_ref<true>};
-    const Kernel *kernels = stepwise ? kernels_old : phased;
+    static const Kernel kernels[4] = {k_raycast_phased<false, false>, k_raycast_phased<true, false>, k_raycast_phased<false, true>,
+                                      k_raycast_phased<true, true>};
     const Kernel kernel = kernels[ci];
-    if (!blocksPerSm[ci]) {
-        cudaDeviceProp prop;
-        CQ_CUDA(cudaGetDeviceProperties(&prop, w->device));
-        numSms = prop.multiProcessorCount;
-        int b = 0;
-        CQ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, Q_THREADS, 0));
-        blocksPerSm[ci] = b > 0 ? b : 1;
-    }
-    int blocks = std::min(cdiv(n, Q_THREADS), numSms * blocksPerSm[ci]); // one resident wave of persistent lanes
+    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
+    if (!resident) return CQ_ERR_CUDA;
+    int blocks = std::min(cdiv(n, Q_THREADS), resident); // one resident wave of persistent lanes
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;
     const uint32_t *order = make_unit_order(w, d_rays, sizeof(cq_ray), false, n, st);
@@ -792,27 +502,18 @@ int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, 
     return finish_launch(w, st, ref ? "k_raycast_ref" : "k_raycast");
 }
 
-#undef CQ_OCC_SLOT
-#define CQ_OCC_SLOT 2
 int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cast_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
     CQ_TRY(await_trees(w, st));
-    int *blocksPerSm = w->occ[CQ_OCC_SLOT]; int &numSms = w->numSms;
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     using Kernel = void (*)(WorldView, const cq_capsule_cast *, int, int, cq_cast_hit *, uint8_t *, int, uint2 *, int *,
                             const uint32_t *, unsigned long long *);
     static const Kernel kernels[4] = {k_capsule_cast<false, false>, k_capsule_cast<true, false>, k_capsule_cast<false, true>,
                                       k_capsule_cast<true, true>};
     const Kernel kernel = kernels[ci];
-    if (!blocksPerSm[ci]) {
-        cudaDeviceProp prop;
-        CQ_CUDA(cudaGetDeviceProperties(&prop, w->device));
-        numSms = prop.multiProcessorCount;
-        int b = 0;
-        CQ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, Q_THREADS, 0));
-        blocksPerSm[ci] = b > 0 ? b : 1;
-    }
-    int blocks = std::min(cdiv(n, 4), numSms * blocksPerSm[ci]); // one resident wave of persistent lanes
+    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
+    if (!resident) return CQ_ERR_CUDA;
+    int blocks = std::min(cdiv(n, 4), resident); // one resident wave of persistent lanes
     const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;
@@ -824,30 +525,20 @@ int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cas
     return finish_launch(w, st, "k_capsule_cast");
 }
 
-#undef CQ_OCC_SLOT
-#define CQ_OCC_SLOT (3 + (ALL ? 1 : 0))
 template <bool ALL>
 static int launch_overlap_pool(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                                uint8_t *d_overflow, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
     CQ_TRY(await_trees(w, st));
-    int &numSms = w->numSms;
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
-    int &blocksPerSm = w->occ[CQ_OCC_SLOT][ci];
     using Kernel = void (*)(WorldView, const cq_capsule *, int, int, cq_overlap_hit *, int32_t *, uint8_t *, int, uint2 *, int *,
                             unsigned long long *);
     static const Kernel kernels[4] = {k_capsule_overlap_pool<false, ALL, false>, k_capsule_overlap_pool<true, ALL, false>,
                                       k_capsule_overlap_pool<false, ALL, true>, k_capsule_overlap_pool<true, ALL, true>};
     const Kernel kernel = kernels[ci];
-    if (!blocksPerSm) {
-        cudaDeviceProp prop;
-        CQ_CUDA(cudaGetDeviceProperties(&prop, w->device));
-        numSms = prop.multiProcessorCount;
-        int b = 0;
-        CQ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, Q_THREADS, 0));
-        blocksPerSm = b > 0 ? b : 1;
-    }
-    int blocks = std::min(cdiv(n, 4), numSms * blocksPerSm);
+    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
+    if (!resident) return CQ_ERR_CUDA;
+    int blocks = std::min(cdiv(n, 4), resident);
     const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;

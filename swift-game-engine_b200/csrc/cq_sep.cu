@@ -631,20 +631,6 @@ __global__ void __launch_bounds__(SEP_THREADS, 4) k_sep_post(WorldView W, const 
 }
 
 // ---------------------------------------------------------------- host driver
-static int sep_grid_blocks(cq_world *w, const void *kernel, size_t smem, int &cache) {
-    if (!cache) {
-        cudaDeviceProp prop;
-        if (check_cuda(cudaGetDeviceProperties(&prop, w->device), "props") != CQ_OK) return 0;
-        w->numSms = prop.multiProcessorCount;
-        int b = 0;
-        if (check_cuda(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "smem attr") != CQ_OK)
-            return 0;
-        if (check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, kernel, SEP_THREADS, smem), "occupancy") != CQ_OK) return 0;
-        cache = b > 0 ? b : 1;
-    }
-    return w->numSms * cache;
-}
-
 // The rounds of one sweep as ONE graph launch: a WHILE node whose body is two rounds (turns -> release -> round end, with
 // the queues in either role); k_sep_round_end_dev sets the loop condition, so the host neither launches rounds nor reads
 // progress back while the schedule runs (round 1 read it back every 8 rounds).  Instantiated graphs are kept per world,
@@ -788,8 +774,8 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     const void *turnKernel = ci ? (const void *)k_sep_turns<true> : (const void *)k_sep_turns<false>;
     const void *postKernel = ci ? (const void *)k_sep_post<true> : (const void *)k_sep_post<false>;
     const size_t turnSmem = SEP_SMEM_BYTES(SepCtx), postSmem = SEP_SMEM_BYTES(PostCtx);
-    const int turnBlocksMax = sep_grid_blocks(w, turnKernel, turnSmem, w->occSep[0][ci]);
-    const int postBlocksMax = sep_grid_blocks(w, postKernel, postSmem, w->occSep[1][ci]);
+    const int turnBlocksMax = resident_blocks(w, turnKernel, SEP_THREADS, turnSmem);
+    const int postBlocksMax = resident_blocks(w, postKernel, SEP_THREADS, postSmem);
     if (!turnBlocksMax || !postBlocksMax) return CQ_ERR_CUDA;
     const int turnBlocks = std::min(cdiv(n, 4), turnBlocksMax), postBlocks = std::min(cdiv(n, 4), postBlocksMax);
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)std::max(turnBlocks, postBlocks) * SEP_WARPS, st);

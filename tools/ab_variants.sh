@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B of alternative builds of libcq.so on the device-resident bench line, one box, back to back.
 #   build the variants here (no GPU needed), e.g.
-#     make -C swift-game-engine_b200/csrc clean; make -C swift-game-engine_b200/csrc -j8 EXTRA="-DCQ_EVAL_REPS=2"
+#     make -C swift-game-engine_b200/csrc clean; make -C swift-game-engine_b200/csrc -j8 EXTRA="-DCQ_WALK_FILL=96"
 #     cp swift-game-engine_b200/csrc/libcq.so swift-game-engine_b200/csrc/libcq_r2.so      (*.so travels with gpurun)
 #   then on the GPU box:   bash tools/ab_variants.sh "hulls terrain" libcq.so libcq_r2.so ...
 # Every run is `bench.py --mesh M --no-cpu-baseline` with CQ_LIB pointing at the build; prints value and ms/step per run.
