@@ -155,7 +155,8 @@ int cq_world_update_transforms(cq_world *w, const uint32_t *entity_ids,
  * either way a fixed number of kernel launches per set (at most 8) plus one host-to-device copy, however many parts moved.
  * refit_ms is left unchanged.
  *
- * Ordering contract (both calls):
+ * Ordering contract (all three update calls: this one, cq_world_update_transforms and
+ * cq_world_update_transforms_device; uncaptured):
  *  - the refit starts only after every launch already queued on this world, on any stream, has finished reading the
  *    trees: queries, crowd steps, agent separation and earlier refits alike;
  *  - every call made on the world after this one returns sees the new trees, whatever its stream: the *_device twins,
@@ -167,6 +168,30 @@ int cq_world_update_transforms(cq_world *w, const uint32_t *entity_ids,
  * device memory); cq_world_destroy frees them. */
 int cq_world_update_transforms_async(cq_world *w, const uint32_t *entity_ids, const float *models, int32_t n, void *stream);
 
+/* Device-resident twin: d_entity_ids (n ids) and d_models (n*16 floats, column-major like cq_mesh_part.model) are DEVICE
+ * pointers, read by the kernels the call queues on `stream` (NULL = the world's stream), so the caller keeps them
+ * unchanged until the stream has passed the call.  The call does not synchronise, allocate or touch host memory: the ids
+ * are resolved and the table of moved parts is built on the device, from an index the world uploads at creation.
+ *
+ * Same semantics as the other two calls (every part with a matching entity_id takes the model, parts without triangles
+ * are skipped, an id named twice takes the model of its last position, a set is refitted in full when at least a quarter
+ * of its triangles moved or CQ_REFIT_FULL is set, refit_ms is left unchanged) and the same ordering contract.  Errors are
+ * all-or-nothing and decided on the device: when any id is unknown the update changes nothing (no model row, vertex or
+ * box is written), and *d_status (a device int32, may be NULL) receives the number of unknown ids, 0 on success, in
+ * stream order.  NULL world, n < 0, or a NULL array with n > 0 return CQ_ERR_INVALID before any CUDA call; n == 0 returns
+ * CQ_OK and queues nothing.
+ *
+ * Launches: a fixed number per call whatever n is and whatever moved: 2 (resolve the ids, build the table) plus, for
+ * each set that has triangles, 13 (the part update, the 5 kernels of the full refit and the 7 of the dirty one, of which
+ * the path not chosen exits at once): at most 28.  Fewer in canonical order (no reference tree: 4 fewer per set) and for
+ * a set of one triangle (1 fewer).  The kernels of both paths stride over their work with grids of at most one resident
+ * wave, so the unchosen path and an untouched set cost a few empty CTAs per SM, whatever the set's size.
+ *
+ * Stream capture: the call, and every *_device query twin below, may be recorded into a CUDA graph (see the capture
+ * contract below the *_device twins). */
+int cq_world_update_transforms_device(cq_world *w, const uint32_t *d_entity_ids, const float *d_models, int32_t n,
+                                      int32_t *d_status, void *stream);
+
 /* Read back the world-space soup (testing / material lookup on the host).
  * which: 0 = static set, 1 = dynamic set.  Any out pointer may be NULL. */
 int cq_world_read_soup(const cq_world *w, int32_t which,
@@ -175,6 +200,10 @@ int cq_world_read_soup(const cq_world *w, int32_t which,
                        float *tri_aabbs /* n_triangles*6: min xyz, max xyz */,
                        uint32_t *tri_layers /* n_triangles */,
                        int32_t *tri_parts /* n_triangles: index into the parts array */);
+
+/* The model matrix of every part (n_parts * 16 floats, column-major, in the order of the parts array given to
+ * cq_world_create), as the last completed update left it.  Waits for queued updates like cq_world_read_soup. */
+int cq_world_read_models(const cq_world *w, float *models_out);
 
 typedef struct cq_material {
     float mu_s, mu_k;
@@ -282,7 +311,24 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  * world's scratch blocks are handed from stream to stream behind events, so up
  * to four launches overlap and further ones queue behind them.
  * cq_world_update_transforms and cq_world_destroy wait for everything in flight; cq_world_update_transforms_async is
- * ordered against them by events instead (see its ordering contract). */
+ * ordered against them by events instead (see its ordering contract).
+ *
+ * CUDA-graph capture: while `stream` is being captured (cudaStreamBeginCapture, torch.cuda.graph, ...), the *_device
+ * query twins, cq_move_and_slide_device(_ex) and cq_world_update_transforms_device enqueue kernels, memsets and copies
+ * only: they neither wait on nor record nor create world events.  So:
+ *  - a graph is ordered only by the stream it is launched on; the caller orders its replays against other work on the
+ *    world, as for a synchronous call (e.g. synchronise before an uncaptured call on another stream);
+ *  - kernel_launches counts the launches once, at capture; replays are not counted;
+ *  - scalar arguments (n, mode, params, platforms, flags, the environment's CQ_REFIT_FULL) are recorded with the graph;
+ *    device buffers are read at replay, so new models written into the same buffer move the parts of each replay;
+ *  - a call that would grow scratch, allocate, synchronise or create an event while capturing returns CQ_ERR_INVALID
+ *    ("make one uncaptured call of this size first") and leaves the capture valid; so does CQ_MAS_AGENTS when its grid
+ *    needs more scratch than an uncaptured call gave it;
+ *  - scratch blocks a graph recorded stay allocated when a later uncaptured call outgrows them (the call takes new
+ *    blocks), so graphs stay valid until cq_world_destroy, which frees them: replay no graph after destroying its world;
+ *  - cq_agent_separation_device (it synchronises per sweep), cq_crowd_step and the host-pointer calls (checked on the
+ *    world's stream, or on `stream` where they take one) refuse a capture the same way.
+ * Uncaptured calls behave as described everywhere else in this header. */
 int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, void *stream);
 int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode,
                            cq_cast_hit *d_out, void *stream);

@@ -128,7 +128,7 @@ class Counters(C.Structure):
 
 EXPORTS = [
     "cq_world_create", "cq_world_create_ex", "cq_world_options_default", "cq_world_destroy", "cq_world_get_info", "cq_world_update_transforms",
-    "cq_world_update_transforms_async", "cq_world_read_soup",
+    "cq_world_update_transforms_async", "cq_world_update_transforms_device", "cq_world_read_soup", "cq_world_read_models",
     "cq_world_triangle_material", "cq_static_mesh_load", "cq_static_mesh_free", "cq_static_mesh_part_count",
     "cq_static_mesh_part_name", "cq_static_mesh_part_transform", "cq_static_mesh_hull_count",
     "cq_static_mesh_geometry", "cq_raycast_batch", "cq_capsule_cast_batch", "cq_capsule_overlap_batch",
@@ -196,7 +196,9 @@ def lib():
         L.cq_world_get_info.argtypes = [vp, C.POINTER(WorldInfo)]
         L.cq_world_update_transforms.argtypes = [vp, vp, vp, i32]
         L.cq_world_update_transforms_async.argtypes = [vp, vp, vp, i32, vp]
+        L.cq_world_update_transforms_device.argtypes = [vp, vp, vp, i32, vp, vp]
         L.cq_world_read_soup.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+        L.cq_world_read_models.argtypes = [vp, vp]
         L.cq_world_triangle_material.argtypes = [vp, i32, C.POINTER(Material)]
         L.cq_static_mesh_load.argtypes = [C.c_char_p, C.POINTER(vp)]
         L.cq_static_mesh_free.argtypes = [vp]
@@ -414,6 +416,12 @@ class CollisionQuery:
         _check(lib().cq_world_read_soup(self._h, which, _ptr(pos), _ptr(idx), _ptr(aabb), _ptr(lay), _ptr(par)))
         return {"positions": pos, "indices": idx, "aabbs": aabb, "layers": lay, "parts": par}
 
+    def read_models(self):
+        """cq_world_read_models: every part's current model matrix, (n_parts, 16) column-major, in parts order."""
+        out = np.zeros((self.info()["n_parts"], 16), np.float32)
+        _check(lib().cq_world_read_models(self._h, _ptr(out)))
+        return out
+
     def triangle_material(self, triangle_index):
         m = Material()
         _check(lib().cq_world_triangle_material(self._h, int(triangle_index), C.byref(m)))
@@ -437,6 +445,15 @@ class CollisionQuery:
         m = np.ascontiguousarray(models, np.float32).reshape(-1, 16)
         assert m.shape[0] == ids.shape[0]
         _check(lib().cq_world_update_transforms_async(self._h, _ptr(ids), _ptr(m), len(ids), C.c_void_p(stream) if stream else None))
+
+    def update_transforms_device(self, d_ids_ptr, d_models_ptr, n, d_status_ptr=None, stream=None):
+        """cq_world_update_transforms_device: the same update from DEVICE arrays (n uint32 ids, n*16 float32 models),
+        queued on `stream` without synchronising and without touching host memory, so it can be captured in a CUDA
+        graph.  The kernels read the arrays in stream order: keep them unchanged until the stream has passed the call.
+        Unknown ids make the update change nothing; d_status_ptr (a device int32, optional) receives their count."""
+        _check(lib().cq_world_update_transforms_device(self._h, C.c_void_p(d_ids_ptr), C.c_void_p(d_models_ptr), int(n),
+                                                       C.c_void_p(d_status_ptr) if d_status_ptr else None,
+                                                       C.c_void_p(stream) if stream else None))
 
     # raycast(origin:direction:maxDistance:mask:) (CollisionQuery.swift:85)
     def raycast(self, rays, with_flags=False):

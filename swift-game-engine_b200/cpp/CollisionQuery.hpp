@@ -75,6 +75,11 @@ class CollisionQuery {
     bool updateTransformsAsync(const std::vector<uint32_t> &entities, const std::vector<float> &models16, void *stream = nullptr) {
         return cq_world_update_transforms_async(w_, entities.data(), models16.data(), (int32_t)entities.size(), stream) == CQ_OK;
     }
+    // device arrays (n ids, n*16 floats); dStatus (device int32, may be null) receives the number of unknown ids
+    bool updateTransformsDevice(const uint32_t *dEntities, const float *dModels16, int32_t n, int32_t *dStatus = nullptr,
+                                void *stream = nullptr) {
+        return cq_world_update_transforms_device(w_, dEntities, dModels16, n, dStatus, stream) == CQ_OK;
+    }
 
     std::optional<RaycastHit> raycast(Float3 origin, Float3 direction, float maxDistance, uint32_t mask = CQ_LAYER_ALL) {
         cq_ray r = {{origin.x, origin.y, origin.z}, {direction.x, direction.y, direction.z}, maxDistance, mask};

@@ -37,6 +37,14 @@ int ensure_scratch(ScratchBuf &b, size_t bytes) {
     return r;
 }
 
+int grow_scratch(cq_world *w, ScratchBuf &b, size_t bytes) {
+    if (bytes > b.cap && b.captured) {
+        w->graphScratch.push_back(b.ptr);
+        b.ptr = nullptr, b.cap = 0, b.captured = false;
+    }
+    return ensure_scratch(b, bytes);
+}
+
 int resident_blocks(cq_world *w, const void *kernel, int threads, size_t dynSmem) {
     const auto it = w->residentBlocks.find(kernel);
     if (it != w->residentBlocks.end()) return it->second;
@@ -78,7 +86,29 @@ int *next_work_counter(cq_world *w, cudaStream_t st) {
     return p;
 }
 
+bool stream_capturing(cudaStream_t st) {
+    cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+    if (cudaStreamGetCaptureInfo(st, &cs) != cudaSuccess) return false;
+    return cs != cudaStreamCaptureStatusNone;
+}
+
+int refuse_capture(cudaStream_t st, const char *what) {
+    if (!stream_capturing(st)) return CQ_OK;
+    set_error("%s cannot be captured in a CUDA graph (it synchronises or stages host memory); call it outside the capture", what);
+    return CQ_ERR_INVALID;
+}
+
+int refuse_growth(cq_world *w, const char *what) {
+    set_error("%s: the call needs more scratch than any uncaptured call gave it, and growing it cannot be captured; "
+              "make one uncaptured call of this size first", what);
+    w->captureRefused = true;
+    return CQ_ERR_INVALID;
+}
+
+// Under capture the world's events are left alone: a graph is ordered only by the stream it is launched on, and an
+// event recorded into a capture would fail every later uncaptured wait on it.
 int scratch_acquire(cq_world *w, ScratchBuf &b, cudaStream_t st) {
+    if (w->capturing) return CQ_OK;
     if (!b.ev) CQ_CUDA(cudaEventCreateWithFlags(&b.ev, cudaEventDisableTiming));
     if (b.recorded && b.last != st) CQ_CUDA(cudaStreamWaitEvent(st, b.ev, 0));
     if (std::find(w->held.begin(), w->held.end(), &b) == w->held.end()) w->held.push_back(&b);
@@ -98,12 +128,14 @@ int release_held(cq_world *w, cudaStream_t st) {
 }
 
 int await_trees(const cq_world *w, cudaStream_t st) {
+    if (w->capturing) return CQ_OK;
     if (w->treesPending && st != w->treesStream) CQ_CUDA(cudaStreamWaitEvent(st, w->evTrees, 0));
     return CQ_OK;
 }
 
 // one event per stream that ever launched on the world, re-recorded by every launch on it
 static int note_reader(cq_world *w, cudaStream_t st) {
+    if (w->capturing) return CQ_OK;
     ReaderEvent *r = nullptr;
     for (ReaderEvent &e : w->readers)
         if (e.st == st) r = &e;
@@ -135,13 +167,18 @@ static void destroy_scratch(ScratchBuf &b) {
 void *pool_node_scratch(cq_world *w, size_t warps, cudaStream_t st) {
     size_t bytes = warps * (size_t)2048 /* CQ_NSCAP */ * sizeof(uint2);
     if (bytes > w->nodeScratch[0].cap) {
+        if (w->capturing) {
+            refuse_growth(w, "node scratch");
+            return nullptr;
+        }
         // grow all four regions at once (a cudaMalloc inside a timed step costs milliseconds); growing frees the
         // old blocks, so make sure no launch still uses them
         if (check_cuda(cudaDeviceSynchronize(), "node scratch sync") != CQ_OK) return nullptr;
         for (int k = 0; k < 4; k++)
-            if (ensure_scratch(w->nodeScratch[k], bytes) != CQ_OK) return nullptr;
+            if (grow_scratch(w, w->nodeScratch[k], bytes) != CQ_OK) return nullptr;
     }
     ScratchBuf &b = w->nodeScratch[w->nodeSeq++ & 3];
+    if (w->capturing) b.captured = true;
     if (scratch_acquire(w, b, st) != CQ_OK) return nullptr;
     return b.ptr;
 }
@@ -178,6 +215,18 @@ using namespace cq;
 
 static cudaStream_t pick_stream(cq_world *w, void *stream) { return stream ? (cudaStream_t)stream : w->stream; }
 
+// One device call being enqueued on `st`: while a stream capture records `st`, the world's helpers neither wait on nor
+// record nor create world events, and refuse to grow scratch (refuse_growth); the call then returns CQ_ERR_INVALID.
+struct CaptureScope {
+    cq_world *w;
+    CaptureScope(cq_world *world, cudaStream_t st) : w(world) {
+        w->capturing = stream_capturing(st);
+        w->captureRefused = false;
+    }
+    ~CaptureScope() { w->capturing = false, w->captureRefused = false; }
+    int result(int rc) const { return w->captureRefused ? CQ_ERR_INVALID : rc; }
+};
+
 // ---------------------------------------------------------------- transform updates
 // Queues the refit of the rows staged in movedRows on `st`: after every launch that has read the trees since the last
 // refit (any stream) and after the previous refit, then records evTrees, which every later launch on another stream waits
@@ -192,14 +241,29 @@ static void free_retired(cq_world *w) {
     w->retiredDev.clear(), w->retiredHost.clear();
 }
 
-static int queue_refit(cq_world *w, cudaStream_t st, cudaEvent_t t0) {
+// every launch that has read the trees (any stream), and the previous refit, before the refit queued next on `st`
+static int refit_after_readers(cq_world *w, cudaStream_t st) {
+    if (w->capturing) return CQ_OK;
     for (ReaderEvent &r : w->readers)
         if (r.pending) {
             if (r.st != st) CQ_CUDA(cudaStreamWaitEvent(st, r.ev, 0));
             r.pending = false;
         }
-    CQ_TRY(await_trees(w, st));
-    const size_t n0 = w->movedRows[0].size(), nRows = n0 + w->movedRows[1].size(), bytes = nRows * sizeof(MovedPart);
+    return await_trees(w, st);
+}
+
+// later launches on other streams wait for the refit just queued on `st` (await_trees)
+static int refit_done(cq_world *w, cudaStream_t st) {
+    CQ_CUDA(cudaEventRecord(w->evTrees, st));
+    w->treesStream = st;
+    w->treesPending = true;
+    return CQ_OK;
+}
+
+static int queue_refit(cq_world *w, cudaStream_t st, cudaEvent_t t0) {
+    CQ_TRY(refit_after_readers(w, st));
+    // one copy: a RefitHeader row with both sets' counts, then the rows
+    const size_t n0 = w->movedRows[0].size(), nRows = 1 + n0 + w->movedRows[1].size(), bytes = nRows * sizeof(MovedPart);
     StageSlot &slot = w->stage[w->stageSeq++ % CQ_STAGE_SLOTS];
     if (!slot.ev) CQ_CUDA(cudaEventCreateWithFlags(&slot.ev, cudaEventDisableTiming));
     if (slot.recorded) CQ_CUDA(cudaEventSynchronize(slot.ev));
@@ -215,19 +279,72 @@ static int queue_refit(cq_world *w, cudaStream_t st, cudaEvent_t t0) {
         w->dTable.ptr = nullptr, w->dTable.cap = 0;
         CQ_TRY(ensure_scratch(w->dTable, bytes));
     }
-    std::copy(w->movedRows[0].begin(), w->movedRows[0].end(), slot.host);
-    std::copy(w->movedRows[1].begin(), w->movedRows[1].end(), slot.host + n0);
+    RefitHeader h{};
+    for (int s = 0; s < 2; s++) {
+        const std::vector<MovedPart> &rows = w->movedRows[s];
+        RefitCounts &c = h.set[s];
+        c.nRows = (int32_t)rows.size();
+        c.nVerts = rows.empty() ? 0 : rows.back().vertBase + rows.back().nVerts;
+        c.nMoved = rows.empty() ? 0 : rows.back().triBase + rows.back().nTris;
+        c.path = refit_path(w->set[s], c.nMoved);
+    }
+    memcpy((void *)slot.host, &h, sizeof(h));
+    std::copy(w->movedRows[0].begin(), w->movedRows[0].end(), slot.host + 1);
+    std::copy(w->movedRows[1].begin(), w->movedRows[1].end(), slot.host + 1 + n0);
     CQ_CUDA(cudaMemcpyAsync(w->dTable.ptr, slot.host, bytes, cudaMemcpyHostToDevice, st));
     CQ_CUDA(cudaEventRecord(slot.ev, st));
     slot.recorded = true;
     if (t0) CQ_CUDA(cudaEventRecord(t0, st));
-    const MovedPart *dTab = (const MovedPart *)w->dTable.ptr;
-    CQ_TRY(refit_set(w, w->set[0], dTab, w->movedRows[0], st));
-    CQ_TRY(refit_set(w, w->set[1], dTab + n0, w->movedRows[1], st));
-    CQ_CUDA(cudaEventRecord(w->evTrees, st));
-    w->treesStream = st;
-    w->treesPending = true;
-    return CQ_OK;
+    const RefitHeader *dHdr = (const RefitHeader *)w->dTable.ptr;
+    const MovedPart *dTab = (const MovedPart *)w->dTable.ptr + 1;
+    CQ_TRY(refit_set(w, w->set[0], dTab, &dHdr->set[0], &w->movedRows[0], st));
+    CQ_TRY(refit_set(w, w->set[1], dTab + n0, &dHdr->set[1], &w->movedRows[1], st));
+    return refit_done(w, st);
+}
+
+// The device path's index, built from partsOfEntity once the parts' triangle ranges are known, and its working state,
+// in one allocation: sorted unique ids, CSR offsets, one EntityEntry per part with triangles, a last-writer word per part,
+// the RefitHeader and a table of one row per part with triangles (static set's rows first).  Per part at most
+// 4 + 4 + 24 + 8 + 96 = 136 bytes, plus 100 bytes.
+static int upload_entity_index(cq_world *w) {
+    std::vector<uint32_t> ids;
+    ids.reserve(w->partsOfEntity.size());
+    for (const auto &kv : w->partsOfEntity) ids.push_back(kv.first);
+    std::sort(ids.begin(), ids.end());
+    std::vector<int32_t> off(1, 0);
+    std::vector<EntityEntry> entries;
+    int rows[2] = {0, 0};
+    for (uint32_t id : ids) {
+        for (int p : w->partsOfEntity[id]) {
+            const PartInfo &pi = w->parts[p];
+            if (pi.triHi <= pi.triLo) continue; // CollisionQuery.swift:427: parts without triangles are skipped
+            entries.push_back({p, pi.set, pi.vertLo, pi.triLo, pi.vertHi - pi.vertLo, pi.triHi - pi.triLo});
+            rows[pi.set]++;
+        }
+        off.push_back((int32_t)entries.size());
+    }
+    const size_t nIds = ids.size(), nParts = w->parts.size(), nEntries = entries.size();
+    size_t at = 0;
+    auto take = [&](size_t bytes) { // 256-byte aligned offsets
+        const size_t o = at;
+        at = (at + std::max(bytes, (size_t)1) + 255) & ~(size_t)255;
+        return o;
+    };
+    const size_t oIds = take(4 * nIds), oOff = take(4 * (nIds + 1)), oEnt = take(sizeof(EntityEntry) * nEntries),
+                 oLast = take(8 * nParts), oHdr = take(sizeof(RefitHeader)), oTab = take(sizeof(MovedPart) * nEntries);
+    CQ_CUDA(cudaMalloc(&w->devArena, at));
+    char *b = (char *)w->devArena;
+    w->dEntityIds = (uint32_t *)(b + oIds), w->dEntityOff = (int32_t *)(b + oOff), w->dEntries = (EntityEntry *)(b + oEnt);
+    w->dLastWriter = (unsigned long long *)(b + oLast), w->dDevHdr = (RefitHeader *)(b + oHdr), w->dDevTable = (MovedPart *)(b + oTab);
+    w->nEntities = (int)nIds, w->devRows0 = rows[0];
+    const RefitHeader h{};
+    cudaStream_t st = w->stream;
+    if (nIds) CQ_CUDA(cudaMemcpyAsync(w->dEntityIds, ids.data(), 4 * nIds, cudaMemcpyHostToDevice, st));
+    CQ_CUDA(cudaMemcpyAsync(w->dEntityOff, off.data(), 4 * (nIds + 1), cudaMemcpyHostToDevice, st));
+    if (nEntries) CQ_CUDA(cudaMemcpyAsync(w->dEntries, entries.data(), sizeof(EntityEntry) * nEntries, cudaMemcpyHostToDevice, st));
+    if (nParts) CQ_CUDA(cudaMemsetAsync(w->dLastWriter, 0, 8 * nParts, st));
+    CQ_CUDA(cudaMemcpyAsync(w->dDevHdr, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+    return check_cuda(cudaStreamSynchronize(st), "entity index"); // the host vectors are the copies' sources
 }
 
 // Both transform-update calls: check every id before anything is queued (a failed call changes nothing), build the table
@@ -530,6 +647,7 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
                 return fail(rc);
         }
     if (w->order == CQ_ORDER_REFERENCE && (rc = attach_ref_order(w)) != CQ_OK) return fail(rc);
+    if ((rc = upload_entity_index(w)) != CQ_OK) return fail(rc);
     make_view(w);
     *out = w;
     return CQ_OK;
@@ -548,6 +666,8 @@ void cq_world_destroy(cq_world *w) {
     sep_graphs_destroy(w);
     destroy_scratch(w->sepScratch);
     destroy_scratch(w->dTable);
+    cudaFree(w->devArena);
+    for (void *p : w->graphScratch) cudaFree(p);
     free_retired(w);
     for (StageSlot &s : w->stage) {
         if (s.host) cudaFreeHost(s.host);
@@ -591,6 +711,7 @@ int cq_world_get_info(const cq_world *w, cq_world_info *info) {
 int cq_world_update_transforms(cq_world *w, const uint32_t *entity_ids, const float *models, int32_t n) {
     if (!w || n < 0 || (n > 0 && (!entity_ids || !models))) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_update_transforms");
     // the documented contract of the synchronous call: everything in flight on any stream has finished first
     CQ_CUDA(cudaDeviceSynchronize());
     free_retired(w);
@@ -606,13 +727,30 @@ int cq_world_update_transforms_async(cq_world *w, const uint32_t *entity_ids, co
     if (!w || n < 0 || (n > 0 && (!entity_ids || !models))) return CQ_ERR_INVALID;
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(pick_stream(w, stream), "cq_world_update_transforms_async");
     return update_transforms_on(w, entity_ids, models, n, pick_stream(w, stream), "cq_world_update_transforms_async", nullptr);
+}
+
+int cq_world_update_transforms_device(cq_world *w, const uint32_t *d_entity_ids, const float *d_models, int32_t n,
+                                      int32_t *d_status, void *stream) {
+    if (!w || n < 0 || (n > 0 && (!d_entity_ids || !d_models))) return CQ_ERR_INVALID;
+    if (n == 0) return CQ_OK;
+    CQ_CUDA(cudaSetDevice(w->device));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    CQ_TRY(refit_after_readers(w, st)); // no-op under capture
+    CQ_TRY(build_moved_device(w, d_entity_ids, d_models, n, d_status, st));
+    for (int s = 0; s < 2; s++)
+        CQ_TRY(refit_set(w, w->set[s], w->dDevTable + (s ? w->devRows0 : 0), &w->dDevHdr->set[s], nullptr, st));
+    if (w->capturing) return CQ_OK;
+    return refit_done(w, st);
 }
 
 int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, uint32_t *indices, float *tri_aabbs,
                        uint32_t *tri_layers, int32_t *tri_parts) {
     if (!w || which < 0 || which > 1) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_read_soup");
     const DeviceSet &S = w->set[which];
     CQ_TRY(await_trees(w, w->stream));
     CQ_CUDA(cudaStreamSynchronize(w->stream));
@@ -643,6 +781,17 @@ int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, u
         CQ_CUDA(cudaMemcpy(tri_layers, S.triLayer, sizeof(uint32_t) * (size_t)S.nTris, cudaMemcpyDeviceToHost));
     if (tri_parts && S.nTris)
         CQ_CUDA(cudaMemcpy(tri_parts, S.triPart, sizeof(int32_t) * (size_t)S.nTris, cudaMemcpyDeviceToHost));
+    return CQ_OK;
+}
+
+int cq_world_read_models(const cq_world *w, float *models_out) {
+    if (!w || (!w->parts.empty() && !models_out)) return CQ_ERR_INVALID;
+    if (w->parts.empty()) return CQ_OK;
+    CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_read_models");
+    CQ_TRY(await_trees(w, w->stream));
+    CQ_CUDA(cudaStreamSynchronize(w->stream));
+    CQ_CUDA(cudaMemcpy(models_out, w->dModels, sizeof(float) * 16 * w->parts.size(), cudaMemcpyDeviceToHost));
     return CQ_OK;
 }
 
@@ -678,6 +827,7 @@ int cq_world_set_counting(cq_world *w, int32_t mode) {
 int cq_world_read_counters(cq_world *w, cq_counters *out, int32_t reset) {
     if (!w || !out) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_read_counters");
     unsigned long long h[4];
     CQ_TRY(await_trees(w, w->stream));
     CQ_CUDA(cudaStreamSynchronize(w->stream));
@@ -699,7 +849,9 @@ int cq_world_read_counters(cq_world *w, cq_counters *out, int32_t reset) {
 
 int cq_raycast_device_ex(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, uint8_t *d_flags, void *stream) {
     if (!w || n < 0 || (n > 0 && (!d_rays || !d_out))) return CQ_ERR_INVALID;
-    return launch_raycast(w, d_rays, n, d_out, d_flags, pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_raycast(w, d_rays, n, d_out, d_flags, st));
 }
 int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, void *stream) {
     return cq_raycast_device_ex(w, d_rays, n, d_out, nullptr, stream);
@@ -707,7 +859,9 @@ int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *
 int cq_capsule_cast_device_ex(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode, cq_cast_hit *d_out,
                               uint8_t *d_flags, void *stream) {
     if (!w || n < 0 || mode < 0 || mode > 2 || (n > 0 && (!d_q || !d_out))) return CQ_ERR_INVALID;
-    return launch_cast(w, d_q, n, mode, d_out, d_flags, pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_cast(w, d_q, n, mode, d_out, d_flags, st));
 }
 int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode, cq_cast_hit *d_out, void *stream) {
     return cq_capsule_cast_device_ex(w, d_q, n, mode, d_out, nullptr, stream);
@@ -715,7 +869,9 @@ int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, i
 int cq_capsule_overlap_device_ex(cq_world *w, const cq_capsule *d_q, int32_t n, cq_overlap_hit *d_out, uint8_t *d_flags,
                                  void *stream) {
     if (!w || n < 0 || (n > 0 && (!d_q || !d_out))) return CQ_ERR_INVALID;
-    return launch_overlap(w, d_q, n, d_out, d_flags, pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_overlap(w, d_q, n, d_out, d_flags, st));
 }
 int cq_capsule_overlap_device(cq_world *w, const cq_capsule *d_q, int32_t n, cq_overlap_hit *d_out, void *stream) {
     return cq_capsule_overlap_device_ex(w, d_q, n, d_out, nullptr, stream);
@@ -728,13 +884,17 @@ int cq_capsule_overlap_all_device(cq_world *w, const cq_capsule *d_q, int32_t n,
         set_error("max_hits %d > %d", max_hits, CQ_MAX_OVERLAP_HITS);
         return CQ_ERR_INVALID;
     }
-    return launch_overlap_all(w, d_q, n, max_hits, d_out, d_counts, d_overflow, pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_overlap_all(w, d_q, n, max_hits, d_out, d_counts, d_overflow, st));
 }
 int cq_move_and_slide_device_ex(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
                                 float dt, const float gravity[3], uint32_t flags, const cq_platform *platforms,
                                 int32_t n_platforms, void *stream) {
     if (!w || n < 0 || !params || !gravity || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
-    return launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, n_platforms, pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, n_platforms, st));
 }
 int cq_move_and_slide_device(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params, float dt,
                              const float gravity[3], uint32_t flags, void *stream) {
@@ -743,6 +903,7 @@ int cq_move_and_slide_device(cq_world *w, cq_character_state *d_inout, int32_t n
 
 int cq_raycast_batch_ex(cq_world *w, const cq_ray *rays, int32_t n, cq_ray_hit *out, uint8_t *flags) {
     if (!w || n < 0 || (n > 0 && (!rays || !out))) return CQ_ERR_INVALID;
+    CQ_NO_CAPTURE(w->stream, "cq_raycast_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     return run_batch(w, rays, sizeof(cq_ray), out, sizeof(cq_ray_hit), n,
                      [&](void *di, void *dout, int cnt, int lo, cudaStream_t st) {
@@ -757,6 +918,7 @@ int cq_raycast_batch(cq_world *w, const cq_ray *rays, int32_t n, cq_ray_hit *out
 
 int cq_capsule_cast_batch_ex(cq_world *w, const cq_capsule_cast *q, int32_t n, int32_t mode, cq_cast_hit *out, uint8_t *flags) {
     if (!w || n < 0 || mode < 0 || mode > 2 || (n > 0 && (!q || !out))) return CQ_ERR_INVALID;
+    CQ_NO_CAPTURE(w->stream, "cq_capsule_cast_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     return run_batch(w, q, sizeof(cq_capsule_cast), out, sizeof(cq_cast_hit), n,
                      [&](void *di, void *dout, int cnt, int lo, cudaStream_t st) {
@@ -771,6 +933,7 @@ int cq_capsule_cast_batch(cq_world *w, const cq_capsule_cast *q, int32_t n, int3
 
 int cq_capsule_overlap_batch_ex(cq_world *w, const cq_capsule *q, int32_t n, cq_overlap_hit *out, uint8_t *flags) {
     if (!w || n < 0 || (n > 0 && (!q || !out))) return CQ_ERR_INVALID;
+    CQ_NO_CAPTURE(w->stream, "cq_capsule_overlap_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     return run_batch(w, q, sizeof(cq_capsule), out, sizeof(cq_overlap_hit), n,
                      [&](void *di, void *dout, int cnt, int lo, cudaStream_t st) {
@@ -793,6 +956,7 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
     }
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_capsule_overlap_all_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     cudaStream_t st = w->stream;
     int r;
@@ -819,6 +983,7 @@ int cq_move_and_slide_batch(cq_world *w, cq_character_state *inout, int32_t n, c
 int cq_move_and_slide_batch_ex(cq_world *w, cq_character_state *inout, int32_t n, const cq_controller_params *params, float dt,
                                const float gravity[3], uint32_t flags, const cq_platform *platforms, int32_t n_platforms) {
     if (!w || n < 0 || !params || !gravity || (n > 0 && !inout)) return CQ_ERR_INVALID;
+    CQ_NO_CAPTURE(w->stream, "cq_move_and_slide_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     return run_batch(w, inout, sizeof(cq_character_state), inout, sizeof(cq_character_state), n,
                      [&](void *di, void *, int cnt, int, cudaStream_t st) {
@@ -833,6 +998,7 @@ int cq_agent_separation_device(cq_world *w, cq_character_state *d_inout, int32_t
                                int32_t use_query, void *stream) {
     if (!w || n < 0 || !params || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(pick_stream(w, stream), "cq_agent_separation_device");
     return launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin, height_margin, use_query,
                                    pick_stream(w, stream));
 }
@@ -843,6 +1009,7 @@ int cq_agent_separation_batch(cq_world *w, cq_character_state *inout, int32_t n,
     if (!w || n < 0 || !params || (n > 0 && !inout)) return CQ_ERR_INVALID;
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_agent_separation_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     int r;
     if ((r = ensure_scratch(w->in, sizeof(cq_character_state) * (size_t)n)) != CQ_OK) return r;

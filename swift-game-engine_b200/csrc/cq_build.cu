@@ -468,21 +468,31 @@ __global__ void __launch_bounds__(RS_THREADS) k_os_pass(const uint32_t *__restri
 // NB: k_rs_hist walks the tile thread-strided while k_rs_scatter walks it warp-chunked; both count the
 // same multiset per tile, which is all the histogram needs.
 
+// A refit kernel the device path launches for both refits runs only when the set's counts chose its path; the build
+// passes no counts (nullptr) and always runs.
+__device__ __forceinline__ bool skip_path(const RefitCounts *counts, int path) { return counts && counts->path != path; }
+
+// Refit kernels stride over their work: the build and the host-staged refit launch exact grids (one pass each), the
+// device path launches grids capped at one resident wave, whatever the set's size.
+#define CQ_GRID_STRIDE(i, count) for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < (count); i += gridDim.x * blockDim.x)
+
 // ---------------------------------------------------------------- gather into the sorted float4 SoA
 __global__ void k_gather_sorted(const uint32_t *__restrict__ sortedTri, int nTris, const float4 *__restrict__ world,
                                 const uint32_t *__restrict__ idx, const uint32_t *__restrict__ layer,
                                 const int32_t *__restrict__ rank /* global index -> visiting rank, or null */, int triOffset,
-                                float4 *__restrict__ tv0, float4 *__restrict__ tv1, float4 *__restrict__ tv2) {
-    int s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= nTris) return;
-    uint32_t t = sortedTri[s];
-    float4 a = world[idx[3 * t]], b = world[idx[3 * t + 1]], c = world[idx[3 * t + 2]];
-    a.w = __uint_as_float(layer[t]);
-    b.w = __int_as_float((int)t);
-    c.w = __int_as_float(rank ? rank[triOffset + (int)t] : triOffset + (int)t); // canonical order: rank = global index
-    tv0[s] = a;
-    tv1[s] = b;
-    tv2[s] = c;
+                                float4 *__restrict__ tv0, float4 *__restrict__ tv1, float4 *__restrict__ tv2,
+                                const RefitCounts *__restrict__ counts = nullptr) {
+    if (skip_path(counts, CQ_PATH_FULL)) return;
+    CQ_GRID_STRIDE(s, nTris) {
+        uint32_t t = sortedTri[s];
+        float4 a = world[idx[3 * t]], b = world[idx[3 * t + 1]], c = world[idx[3 * t + 2]];
+        a.w = __uint_as_float(layer[t]);
+        b.w = __int_as_float((int)t);
+        c.w = __int_as_float(rank ? rank[triOffset + (int)t] : triOffset + (int)t); // canonical order: rank = global index
+        tv0[s] = a;
+        tv1[s] = b;
+        tv2[s] = c;
+    }
 }
 
 // ---------------------------------------------------------------- Karras 2012 radix tree
@@ -534,12 +544,12 @@ __global__ void k_karras(const uint32_t *__restrict__ keys, int n, Node *__restr
     nodes[i].n3.w = __int_as_float(rightBox);
 }
 
-// bottom-up boxes: one thread per leaf slot climbs while it is the second to arrive
-__global__ void k_fit(int n, const float4 *__restrict__ tv0, const float4 *__restrict__ tv1,
-                      const float4 *__restrict__ tv2, Node *__restrict__ nodes, const int32_t *__restrict__ parent,
-                      float4 *__restrict__ boxLo, float4 *__restrict__ boxHi, int32_t *__restrict__ visit) {
-    int s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n) return;
+// bottom-up boxes: one thread per leaf slot climbs while it is the second to arrive, and leaves the arrival counter at
+// zero (the dirty-subtree refit, and the next fit of the device path, start from zero counters)
+__device__ __forceinline__ void fit_leaf(int s, int n, const float4 *__restrict__ tv0, const float4 *__restrict__ tv1,
+                                         const float4 *__restrict__ tv2, Node *__restrict__ nodes,
+                                         const int32_t *__restrict__ parent, float4 *__restrict__ boxLo,
+                                         float4 *__restrict__ boxHi, int32_t *__restrict__ visit) {
     f3 a = xyz(tv0[s]), b = xyz(tv1[s]), c = xyz(tv2[s]);
     f3 lo = vmin(a, vmin(b, c)), hi = vmax(a, vmax(b, c));
     int me = (n - 1) + s;
@@ -550,6 +560,7 @@ __global__ void k_fit(int n, const float4 *__restrict__ tv0, const float4 *__res
     int p = parent[me];
     while (p >= 0) {
         if (atomicAdd(&visit[p], 1) == 0) return; // first arrival: the sibling subtree is not done yet
+        visit[p] = 0;
         __threadfence();
         Node nd = nodes[p];
         int lb = __float_as_int(nd.n2.w), rb = __float_as_int(nd.n3.w);
@@ -566,6 +577,13 @@ __global__ void k_fit(int n, const float4 *__restrict__ tv0, const float4 *__res
         p = parent[p];
     }
 }
+__global__ void k_fit(int n, const float4 *__restrict__ tv0, const float4 *__restrict__ tv1,
+                      const float4 *__restrict__ tv2, Node *__restrict__ nodes, const int32_t *__restrict__ parent,
+                      float4 *__restrict__ boxLo, float4 *__restrict__ boxHi, int32_t *__restrict__ visit,
+                      const RefitCounts *__restrict__ counts) {
+    if (skip_path(counts, CQ_PATH_FULL)) return;
+    CQ_GRID_STRIDE(s, n) fit_leaf(s, n, tv0, tv1, tv2, nodes, parent, boxLo, boxHi, visit);
+}
 
 // depth parity of every internal node (root = depth 0): only even-depth nodes become 4-wide nodes
 __global__ void k_depth_parity(int nInternal, const int32_t *__restrict__ parent, uint8_t *__restrict__ parity) {
@@ -579,10 +597,10 @@ __global__ void k_depth_parity(int nInternal, const int32_t *__restrict__ parent
 // collapse: wide node i = binary node i (even depth) with its internal children replaced by THEIR children
 __device__ __forceinline__ void collapse4_node(int i, const Node *nodes, Node4 *nodes4);
 __global__ void k_collapse4(int nInternal, const Node *__restrict__ nodes, const uint8_t *__restrict__ parity,
-                            Node4 *__restrict__ nodes4) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nInternal || parity[i]) return;
-    collapse4_node(i, nodes, nodes4);
+                            Node4 *__restrict__ nodes4, const RefitCounts *__restrict__ counts) {
+    if (skip_path(counts, CQ_PATH_FULL)) return;
+    CQ_GRID_STRIDE(i, nInternal)
+    if (!parity[i]) collapse4_node(i, nodes, nodes4);
 }
 __device__ __forceinline__ void collapse4_node(int i, const Node *nodes, Node4 *nodes4) {
     Node nb = nodes[i];
@@ -627,8 +645,9 @@ __device__ __forceinline__ void collapse4_node(int i, const Node *nodes, Node4 *
     nodes4[i] = w;
 }
 
-__global__ void k_header(int n, const float4 *__restrict__ boxLo, const float4 *__restrict__ boxHi, SetHeader *hdr) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+__global__ void k_header(int n, const float4 *__restrict__ boxLo, const float4 *__restrict__ boxHi, SetHeader *hdr,
+                         const RefitCounts *__restrict__ counts, int path) {
+    if (threadIdx.x != 0 || blockIdx.x != 0 || skip_path(counts, path)) return;
     SetHeader h;
     h.nTris = n;
     if (n == 0) {
@@ -681,24 +700,26 @@ __device__ __forceinline__ int moved_triangle(const MovedPart *__restrict__ tab,
     return r.triLo + (i - r.triBase);
 }
 
+// The kernels below read their counts from the set's RefitCounts and stride over them (CQ_GRID_STRIDE).
+
 // one thread per vertex of the moved parts; the arithmetic of k_transform, so the positions are bit-identical
-__global__ void k_update_parts(const MovedPart *__restrict__ tab, int nRows, int nVerts, const float4 *__restrict__ local,
-                               float4 *__restrict__ world, float *__restrict__ models) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nVerts) return;
-    const MovedPart &r = moved_row(tab, nRows, i, false);
-    const int k = i - r.vertBase;
-    if (k == 0)
-        for (int c = 0; c < 16; c++) models[16 * r.part + c] = r.model[c];
-    const int v = r.vertLo + k;
-    world[v] = transform_point(r.model, local[v]);
+__global__ void k_update_parts(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                               const float4 *__restrict__ local, float4 *__restrict__ world, float *__restrict__ models) {
+    const RefitCounts c = *counts;
+    CQ_GRID_STRIDE(i, c.nVerts) {
+        const MovedPart &r = moved_row(tab, c.nRows, i, false);
+        const int k = i - r.vertBase;
+        if (k == 0)
+            for (int q = 0; q < 16; q++) models[16 * r.part + q] = r.model[q];
+        const int v = r.vertLo + k;
+        world[v] = transform_point(r.model, local[v]);
+    }
 }
 
-__global__ void k_refit_mark(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
-                             int n, const float4 *__restrict__ world, const uint32_t *__restrict__ idx, float4 *tv0, float4 *tv1,
-                             float4 *tv2, const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *expect) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved) return;
+__device__ __forceinline__ void refit_mark_one(const MovedPart *__restrict__ tab, int nRows, int i,
+                                               const uint32_t *__restrict__ slotOfTri, int n, const float4 *__restrict__ world,
+                                               const uint32_t *__restrict__ idx, float4 *tv0, float4 *tv1, float4 *tv2,
+                                               const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *expect) {
     const int t = moved_triangle(tab, nRows, i);
     const int slot = (int)slotOfTri[t];
     const float4 a = world[idx[3 * t]], b = world[idx[3 * t + 1]], c = world[idx[3 * t + 2]];
@@ -713,13 +734,19 @@ __global__ void k_refit_mark(const MovedPart *__restrict__ tab, int nRows, int n
     for (int p = parent[node]; p >= 0; p = parent[p])
         if (atomicAdd(&expect[p], 1) != 0) break; // p was already marked through its other child
 }
+__global__ void k_refit_mark(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                             const uint32_t *__restrict__ slotOfTri, int n, const float4 *__restrict__ world,
+                             const uint32_t *__restrict__ idx, float4 *tv0, float4 *tv1, float4 *tv2,
+                             const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *expect) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY) return;
+    CQ_GRID_STRIDE(i, c.nMoved)
+    refit_mark_one(tab, c.nRows, i, slotOfTri, n, world, idx, tv0, tv1, tv2, parent, boxLo, boxHi, expect);
+}
 
-__global__ void k_refit_climb(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
-                              int n, Node *nodes, const int32_t *__restrict__ parent, float4 *boxLo, float4 *boxHi, int32_t *visit,
-                              const int32_t *__restrict__ expect, const uint8_t *__restrict__ parity, Node4 *nodes4) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved || n == 1) return;
-    int p = parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, nRows, i)]];
+__device__ __forceinline__ void refit_climb_one(int p, Node *nodes, const int32_t *__restrict__ parent, float4 *boxLo,
+                                                float4 *boxHi, int32_t *visit, const int32_t *__restrict__ expect,
+                                                const uint8_t *__restrict__ parity, Node4 *nodes4) {
     while (p >= 0) {
         if (atomicAdd(&visit[p], 1) + 1 < expect[p]) return; // a dirty sibling subtree is not done yet
         __threadfence();
@@ -740,14 +767,26 @@ __global__ void k_refit_climb(const MovedPart *__restrict__ tab, int nRows, int 
         p = parent[p];
     }
 }
+__global__ void k_refit_climb(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                              const uint32_t *__restrict__ slotOfTri, int n, Node *nodes, const int32_t *__restrict__ parent,
+                              float4 *boxLo, float4 *boxHi, int32_t *visit, const int32_t *__restrict__ expect,
+                              const uint8_t *__restrict__ parity, Node4 *nodes4) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY || n == 1) return;
+    CQ_GRID_STRIDE(i, c.nMoved)
+    refit_climb_one(parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, c.nRows, i)]], nodes, parent, boxLo, boxHi, visit, expect,
+                    parity, nodes4);
+}
 
 // Every marked node lies on the path of a moved triangle, so walking those paths clears them all.  A thread stops at the
 // first node another thread has cleared: that thread goes on above it.
-__global__ void k_refit_clear(const MovedPart *__restrict__ tab, int nRows, int nMoved, const uint32_t *__restrict__ slotOfTri,
-                              int n, const int32_t *__restrict__ parent, int32_t *visit, int32_t *expect) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved || n == 1) return;
-    for (int p = parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, nRows, i)]]; p >= 0; p = parent[p]) {
+__global__ void k_refit_clear(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                              const uint32_t *__restrict__ slotOfTri, int n, const int32_t *__restrict__ parent, int32_t *visit,
+                              int32_t *expect) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY || n == 1) return;
+    CQ_GRID_STRIDE(i, c.nMoved)
+    for (int p = parent[(n - 1) + (int)slotOfTri[moved_triangle(tab, c.nRows, i)]]; p >= 0; p = parent[p]) {
         visit[p] = 0;
         if (atomicExch(&expect[p], 0) == 0) break;
     }
@@ -756,14 +795,11 @@ __global__ void k_refit_clear(const MovedPart *__restrict__ tab, int nRows, int 
 // the same three steps on the reference's tree (reference order): leaves hold <= 4 triangles; a leaf is refitted by the
 // moved triangle that claims it first in the mark launch (leafMark = its triangle id + 1), which also climbs for it
 __device__ __forceinline__ void ref_store_child_box(Node *nd, int which, f3 lo, f3 hi);
-__global__ void k_ref_refit_mark(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
-                                 const int32_t *__restrict__ leafRange, const int32_t *__restrict__ leafParent,
-                                 const int32_t *__restrict__ nodeParent, const uint32_t *__restrict__ refSlot,
-                                 const float4 *__restrict__ tv0, const float4 *__restrict__ tv1, const float4 *__restrict__ tv2,
-                                 Node *nodes, int32_t *leafMark, int32_t *expect, SetHeader *hdr) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved) return;
-    const int t = moved_triangle(tab, nRows, i);
+__device__ __forceinline__ void ref_refit_mark_one(int t, const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafRange,
+                                                   const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent,
+                                                   const uint32_t *__restrict__ refSlot, const float4 *__restrict__ tv0,
+                                                   const float4 *__restrict__ tv1, const float4 *__restrict__ tv2, Node *nodes,
+                                                   int32_t *leafMark, int32_t *expect, SetHeader *hdr) {
     const int l = leafOfTri[t];
     if (atomicCAS(&leafMark[l], 0, t + 1) != 0) return; // another triangle of the same leaf got here first
     const int range = leafRange[l], start = range >> 2, count = (range & 3) + 1;
@@ -785,14 +821,22 @@ __global__ void k_ref_refit_mark(const MovedPart *__restrict__ tab, int nRows, i
     for (; pw >= 0; pw = nodeParent[pw >> 1])
         if (atomicAdd(&expect[pw >> 1], 1) != 0) break;
 }
+__global__ void k_ref_refit_mark(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                                 const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafRange,
+                                 const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent,
+                                 const uint32_t *__restrict__ refSlot, const float4 *__restrict__ tv0, const float4 *__restrict__ tv1,
+                                 const float4 *__restrict__ tv2, Node *nodes, int32_t *leafMark, int32_t *expect, SetHeader *hdr) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY) return;
+    CQ_GRID_STRIDE(i, c.nMoved)
+    ref_refit_mark_one(moved_triangle(tab, c.nRows, i), leafOfTri, leafRange, leafParent, nodeParent, refSlot, tv0, tv1, tv2, nodes,
+                       leafMark, expect, hdr);
+}
 
-__global__ void k_ref_refit_climb(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
-                                  const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent, Node *nodes,
-                                  const int32_t *__restrict__ leafMark, int32_t *visit, const int32_t *__restrict__ expect,
-                                  SetHeader *hdr) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved) return;
-    const int t = moved_triangle(tab, nRows, i);
+__device__ __forceinline__ void ref_refit_climb_one(int t, const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafParent,
+                                                    const int32_t *__restrict__ nodeParent, Node *nodes,
+                                                    const int32_t *__restrict__ leafMark, int32_t *visit,
+                                                    const int32_t *__restrict__ expect, SetHeader *hdr) {
     const int l = leafOfTri[t];
     if (leafMark[l] != t + 1) return; // one climber per marked leaf: the triangle that claimed it
     int pw = leafParent[l];
@@ -813,17 +857,28 @@ __global__ void k_ref_refit_climb(const MovedPart *__restrict__ tab, int nRows, 
         __threadfence();
     }
 }
+__global__ void k_ref_refit_climb(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                                  const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafParent,
+                                  const int32_t *__restrict__ nodeParent, Node *nodes, const int32_t *__restrict__ leafMark,
+                                  int32_t *visit, const int32_t *__restrict__ expect, SetHeader *hdr) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY) return;
+    CQ_GRID_STRIDE(i, c.nMoved)
+    ref_refit_climb_one(moved_triangle(tab, c.nRows, i), leafOfTri, leafParent, nodeParent, nodes, leafMark, visit, expect, hdr);
+}
 
-__global__ void k_ref_refit_clear(const MovedPart *__restrict__ tab, int nRows, int nMoved, const int32_t *__restrict__ leafOfTri,
-                                  const int32_t *__restrict__ leafParent, const int32_t *__restrict__ nodeParent, int32_t *leafMark,
-                                  int32_t *visit, int32_t *expect) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= nMoved) return;
-    const int l = leafOfTri[moved_triangle(tab, nRows, i)];
-    leafMark[l] = 0;
-    for (int pw = leafParent[l]; pw >= 0; pw = nodeParent[pw >> 1]) {
-        visit[pw >> 1] = 0;
-        if (atomicExch(&expect[pw >> 1], 0) == 0) break;
+__global__ void k_ref_refit_clear(const MovedPart *__restrict__ tab, const RefitCounts *__restrict__ counts,
+                                  const int32_t *__restrict__ leafOfTri, const int32_t *__restrict__ leafParent,
+                                  const int32_t *__restrict__ nodeParent, int32_t *leafMark, int32_t *visit, int32_t *expect) {
+    const RefitCounts c = *counts;
+    if (c.path != CQ_PATH_DIRTY) return;
+    CQ_GRID_STRIDE(i, c.nMoved) {
+        const int l = leafOfTri[moved_triangle(tab, c.nRows, i)];
+        leafMark[l] = 0;
+        for (int pw = leafParent[l]; pw >= 0; pw = nodeParent[pw >> 1]) {
+            visit[pw >> 1] = 0;
+            if (atomicExch(&expect[pw >> 1], 0) == 0) break;
+        }
     }
 }
 
@@ -922,34 +977,38 @@ static bool use_classic_sort() {
     return e && !strcmp(e, "classic");
 }
 
-static int build_tree(cq_world *w, DeviceSet &S, const uint32_t *sortedKeys /* may be null on refit */, cudaStream_t st) {
+// counts == nullptr: the build (and a refit of no table); else the full refit of one update, skipped on the device when the
+// set's counts chose another path.  k_fit leaves `visit` at zero, which every refit keeps, so only the build clears it.
+// maxBlocks > 0 caps the grids of the strided kernels (the device path); 0 = exact grids.
+static int build_tree(cq_world *w, DeviceSet &S, const uint32_t *sortedKeys /* may be null on refit */, cudaStream_t st,
+                      const RefitCounts *counts = nullptr, int maxBlocks = 0) {
     int n = S.nTris;
+    auto grid = [&](int m) { return maxBlocks > 0 ? std::min(cdiv(m, 256), maxBlocks) : cdiv(m, 256); };
     if (n > 0) {
         const int triOffset = &S == &w->set[1] ? w->set[0].nTris : 0;
-        k_gather_sorted<<<cdiv(n, 256), 256, 0, st>>>(S.sortedTri, n, S.worldPos, S.indices, S.triLayer,
+        k_gather_sorted<<<grid(n), 256, 0, st>>>(S.sortedTri, n, S.worldPos, S.indices, S.triLayer,
                                                       w->order == CQ_ORDER_REFERENCE ? w->dRank : nullptr, triOffset, S.tv0, S.tv1,
-                                                      S.tv2);
+                                                      S.tv2, counts);
         w->launches++;
         if (n > 1) {
             if (sortedKeys) {
                 k_karras<<<cdiv(n - 1, 256), 256, 0, st>>>(sortedKeys, n, S.nodes, S.parent, S.rangeLo, S.rangeHi);
                 w->launches++;
             }
-            CQ_CUDA(cudaMemsetAsync(S.visit, 0, sizeof(int32_t) * (size_t)(n - 1), st));
+            if (!counts) CQ_CUDA(cudaMemsetAsync(S.visit, 0, sizeof(int32_t) * (size_t)(n - 1), st));
         }
-        k_fit<<<cdiv(n, 256), 256, 0, st>>>(n, S.tv0, S.tv1, S.tv2, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit);
+        k_fit<<<grid(n), 256, 0, st>>>(n, S.tv0, S.tv1, S.tv2, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit, counts);
         w->launches++;
-        if (n > 1) CQ_CUDA(cudaMemsetAsync(S.visit, 0, sizeof(int32_t) * (size_t)(n - 1), st)); // clean for a dirty-subtree refit
         if (n > 1) {
             if (sortedKeys) { // topology is new: depth parities
                 k_depth_parity<<<cdiv(n - 1, 256), 256, 0, st>>>(n - 1, S.parent, S.depthParity);
                 w->launches++;
             }
-            k_collapse4<<<cdiv(n - 1, 256), 256, 0, st>>>(n - 1, S.nodes, S.depthParity, S.nodes4);
+            k_collapse4<<<grid(n - 1), 256, 0, st>>>(n - 1, S.nodes, S.depthParity, S.nodes4, counts);
             w->launches++;
         }
     }
-    k_header<<<1, 32, 0, st>>>(n, S.boxLo, S.boxHi, S.hdr);
+    k_header<<<1, 32, 0, st>>>(n, S.boxLo, S.boxHi, S.hdr, counts, CQ_PATH_FULL);
     w->launches++;
     return check_cuda(cudaGetLastError(), "build_tree");
 }
@@ -1180,10 +1239,15 @@ const uint32_t *make_unit_order(cq_world *w, const void *dUnits, size_t stride, 
     const size_t words = (size_t)4 * n + sortWords + 64;
     ScratchBuf &b = w->orderScratch[w->orderSeq++ & 3];
     if (words * 4 > b.cap) {
+        if (w->capturing) {
+            refuse_growth(w, "unit order scratch");
+            return nullptr;
+        }
         if (check_cuda(cudaDeviceSynchronize(), "order scratch sync") != CQ_OK) return nullptr;
         for (int k = 0; k < 4; k++)
-            if (ensure_scratch(w->orderScratch[k], words * 4) != CQ_OK) return nullptr;
+            if (grow_scratch(w, w->orderScratch[k], words * 4) != CQ_OK) return nullptr;
     }
+    if (w->capturing) b.captured = true;
     if (scratch_acquire(w, b, st) != CQ_OK) return nullptr;
     uint32_t *keys = (uint32_t *)b.ptr, *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n, *scratch = valsTmp + n;
     k_order_keys<<<cdiv(n, 256), 256, 0, st>>>((const unsigned char *)dUnits, stride, positionIsDouble ? 1 : 0, n, w->set[0].hdr,
@@ -1331,9 +1395,11 @@ int make_agent_grid(cq_world *w, const cq_character_state *dStates, int n, float
     // bounds, params
     const size_t bytes = (size_t)n * 112 + ((size_t)4 * n + sortWords + 64) * 4;
     if (bytes > w->agentScratch.cap) {
+        if (w->capturing) return refuse_growth(w, "CQ_MAS_AGENTS grid scratch");
         CQ_CUDA(cudaDeviceSynchronize());
-        CQ_TRY(ensure_scratch(w->agentScratch, bytes));
+        CQ_TRY(grow_scratch(w, w->agentScratch, bytes));
     }
+    if (w->capturing) w->agentScratch.captured = true;
     CQ_TRY(scratch_acquire(w, w->agentScratch, st));
     float4 *pos = (float4 *)w->agentScratch.ptr, *vel = pos + n, *posS = vel + n, *velS = posS + n;
     int4 *rows = (int4 *)(velS + n);
@@ -1368,12 +1434,10 @@ __device__ __forceinline__ void ref_store_child_box(Node *nd, int which, f3 lo, 
     h[0] = hi.x, h[1] = hi.y, h[2] = hi.z;
 }
 
-__global__ void k_ref_fit(int nLeaves, const int32_t *__restrict__ leafRange, const int32_t *__restrict__ leafParent,
-                          const int32_t *__restrict__ nodeParent, const uint32_t *__restrict__ refSlot,
-                          const float4 *__restrict__ tv0, const float4 *__restrict__ tv1, const float4 *__restrict__ tv2,
-                          Node *nodes, int32_t *visit, SetHeader *hdr) {
-    const int l = blockIdx.x * blockDim.x + threadIdx.x;
-    if (l >= nLeaves) return;
+__device__ __forceinline__ void ref_fit_leaf(int l, const int32_t *__restrict__ leafRange, const int32_t *__restrict__ leafParent,
+                                             const int32_t *__restrict__ nodeParent, const uint32_t *__restrict__ refSlot,
+                                             const float4 *__restrict__ tv0, const float4 *__restrict__ tv1,
+                                             const float4 *__restrict__ tv2, Node *nodes, int32_t *visit, SetHeader *hdr) {
     const int range = leafRange[l], start = range >> 2, count = (range & 3) + 1;
     f3 lo = {0, 0, 0}, hi = {0, 0, 0};
     for (int k = 0; k < count; k++) {
@@ -1403,11 +1467,19 @@ __global__ void k_ref_fit(int nLeaves, const int32_t *__restrict__ leafRange, co
         pw = nodeParent[p];
     }
 }
+__global__ void k_ref_fit(int nLeaves, const int32_t *__restrict__ leafRange, const int32_t *__restrict__ leafParent,
+                          const int32_t *__restrict__ nodeParent, const uint32_t *__restrict__ refSlot,
+                          const float4 *__restrict__ tv0, const float4 *__restrict__ tv1, const float4 *__restrict__ tv2,
+                          Node *nodes, int32_t *visit, SetHeader *hdr, const RefitCounts *__restrict__ counts) {
+    if (skip_path(counts, CQ_PATH_FULL)) return;
+    CQ_GRID_STRIDE(l, nLeaves) ref_fit_leaf(l, leafRange, leafParent, nodeParent, refSlot, tv0, tv1, tv2, nodes, visit, hdr);
+}
 
-static int ref_fit(cq_world *w, DeviceSet &S, cudaStream_t st) {
+static int ref_fit(cq_world *w, DeviceSet &S, cudaStream_t st, const RefitCounts *counts = nullptr, int maxBlocks = 0) {
     if (!S.refArena || S.nRefLeaves <= 0) return CQ_OK;
-    k_ref_fit<<<cdiv(S.nRefLeaves, 256), 256, 0, st>>>(S.nRefLeaves, S.refLeafRange, S.refLeafParent, S.refNodeParent,
-                                                     S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refVisit, S.refHdr);
+    const int grid = maxBlocks > 0 ? std::min(cdiv(S.nRefLeaves, 256), maxBlocks) : cdiv(S.nRefLeaves, 256);
+    k_ref_fit<<<grid, 256, 0, st>>>(S.nRefLeaves, S.refLeafRange, S.refLeafParent, S.refNodeParent,
+                                                     S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refVisit, S.refHdr, counts);
     w->launches++;
     return check_cuda(cudaGetLastError(), "k_ref_fit");
 }
@@ -1548,36 +1620,201 @@ int attach_ref_order(cq_world *w) {
 //     own tree, like BVH.refit (CollisionQuery.swift:528-575): 1 + 3 + 3 + 1 launches;
 //   * otherwise: regather the whole sorted SoA and recompute every box bottom-up (same topology): 1 + 4 + 1 launches.
 // Both give the same boxes (min / max are exact).  Stream-ordered on `st`, no host synchronisation.
-int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const std::vector<MovedPart> &rows, cudaStream_t st) {
-    const int nRows = (int)rows.size();
-    if (nRows == 0) return CQ_OK;
-    const int nVerts = rows.back().vertBase + rows.back().nVerts, moved = rows.back().triBase + rows.back().nTris;
-    k_update_parts<<<cdiv(nVerts, 256), 256, 0, st>>>(dTab, nRows, nVerts, S.localPos, S.worldPos, w->dModels);
-    w->launches++;
+// The device path (rows == nullptr) launches 1 + 5 + 7 of them, whatever moved (fewer for a set of one triangle or in
+// canonical order); the path its counts did not choose exits at once.
+int refit_path(const DeviceSet &S, int moved) {
     static const bool forceFull = getenv("CQ_REFIT_FULL") != nullptr; // A/B and the test that both paths agree
-    if (forceFull || (long long)moved * 4 >= (long long)S.nTris) {
-        CQ_TRY(build_tree(w, S, nullptr, st));
-        return ref_fit(w, S, st); // reference order: the reference's own tree keeps its topology too (BVH.refit)
+    if (moved <= 0) return CQ_PATH_NONE;
+    return forceFull || (long long)moved * 4 >= (long long)S.nTris ? CQ_PATH_FULL : CQ_PATH_DIRTY;
+}
+
+int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const RefitCounts *counts, const std::vector<MovedPart> *rows,
+              cudaStream_t st) {
+    const int n = S.nTris;
+    int vertGrid, triGrid, path, fullCap = 0;
+    if (rows) { // host-staged: the host knows the counts, so it launches the chosen path only, with exact grids
+        if (rows->empty()) return CQ_OK;
+        const MovedPart &last = rows->back();
+        const int nVerts = last.vertBase + last.nVerts, moved = last.triBase + last.nTris;
+        vertGrid = cdiv(nVerts, 256), triGrid = cdiv(moved, 256), path = refit_path(S, moved);
+    } else { // device path: bounds only (a dirty refit moves less than a quarter of the set), one resident wave at most
+        if (n == 0) return CQ_OK; // no part with triangles lies in an empty set
+        const int wave = w->numSms * 8;
+        vertGrid = std::min(cdiv(S.nVerts, 256), wave), triGrid = std::min(cdiv(cdiv(n, 4), 256), wave), path = -1;
+        fullCap = wave; // the full fit's kernels stride over the whole set: an unchosen full path costs one wave, not n / 256 CTAs
     }
-    const int n = S.nTris, blocks = cdiv(moved, 256);
-    k_refit_mark<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.worldPos, S.indices, S.tv0, S.tv1, S.tv2, S.parent,
-                                         S.boxLo, S.boxHi, S.expect);
-    k_refit_climb<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit, S.expect,
-                                          S.depthParity, S.nodes4);
-    k_refit_clear<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.slotOfTri, n, S.parent, S.visit, S.expect);
+    k_update_parts<<<vertGrid, 256, 0, st>>>(dTab, counts, S.localPos, S.worldPos, w->dModels);
+    w->launches++;
+    if (path != CQ_PATH_DIRTY) { // FULL, or both (-1)
+        CQ_TRY(build_tree(w, S, nullptr, st, counts, fullCap));
+        CQ_TRY(ref_fit(w, S, st, counts, fullCap)); // reference order: the reference's own tree keeps its topology too (BVH.refit)
+        if (path == CQ_PATH_FULL) return CQ_OK;
+    }
+    k_refit_mark<<<triGrid, 256, 0, st>>>(dTab, counts, S.slotOfTri, n, S.worldPos, S.indices, S.tv0, S.tv1, S.tv2, S.parent, S.boxLo,
+                                          S.boxHi, S.expect);
+    k_refit_climb<<<triGrid, 256, 0, st>>>(dTab, counts, S.slotOfTri, n, S.nodes, S.parent, S.boxLo, S.boxHi, S.visit, S.expect,
+                                           S.depthParity, S.nodes4);
+    k_refit_clear<<<triGrid, 256, 0, st>>>(dTab, counts, S.slotOfTri, n, S.parent, S.visit, S.expect);
     w->launches += 3;
     if (S.refArena && S.nRefLeaves > 0) {
-        k_ref_refit_mark<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafRange, S.refLeafParent, S.refNodeParent,
-                                                 S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refLeafMark, S.refExpect, S.refHdr);
-        k_ref_refit_climb<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafParent, S.refNodeParent, S.refNodes,
-                                                  S.refLeafMark, S.refVisit, S.refExpect, S.refHdr);
-        k_ref_refit_clear<<<blocks, 256, 0, st>>>(dTab, nRows, moved, S.refLeafOfTri, S.refLeafParent, S.refNodeParent,
-                                                  S.refLeafMark, S.refVisit, S.refExpect);
+        k_ref_refit_mark<<<triGrid, 256, 0, st>>>(dTab, counts, S.refLeafOfTri, S.refLeafRange, S.refLeafParent, S.refNodeParent,
+                                                  S.refSlot, S.tv0, S.tv1, S.tv2, S.refNodes, S.refLeafMark, S.refExpect, S.refHdr);
+        k_ref_refit_climb<<<triGrid, 256, 0, st>>>(dTab, counts, S.refLeafOfTri, S.refLeafParent, S.refNodeParent, S.refNodes,
+                                                   S.refLeafMark, S.refVisit, S.refExpect, S.refHdr);
+        k_ref_refit_clear<<<triGrid, 256, 0, st>>>(dTab, counts, S.refLeafOfTri, S.refLeafParent, S.refNodeParent, S.refLeafMark,
+                                                   S.refVisit, S.refExpect);
         w->launches += 3;
     }
-    k_header<<<1, 32, 0, st>>>(n, S.boxLo, S.boxHi, S.hdr);
+    k_header<<<1, 32, 0, st>>>(n, S.boxLo, S.boxHi, S.hdr, counts, CQ_PATH_DIRTY);
     w->launches++;
     return check_cuda(cudaGetLastError(), "dirty refit");
+}
+
+// ---------------------------------------------------------------- device path: ids -> table of moved parts
+// (cq_world_update_transforms_device) The ids and models are device arrays, so the lookup and the table build run here.
+// k_resolve_ids: one thread per input looks its id up in the sorted unique ids (binary search), counts it when unknown,
+// and claims every part of the entity with atomicMax((generation << 32) | input index), so the LAST mention of a part
+// wins, like the host path's "a part named twice keeps the last model".  The generation advances once per update, so
+// words of earlier updates never match and nothing has to be cleared between updates (or between graph replays).
+__device__ __forceinline__ int find_entity(const uint32_t *__restrict__ ids, int nIds, uint32_t id) {
+    int lo = 0, hi = nIds - 1;
+    while (lo <= hi) {
+        const int mid = (lo + hi) >> 1;
+        const uint32_t v = ids[mid];
+        if (v == id) return mid;
+        if (v < id) lo = mid + 1;
+        else hi = mid - 1;
+    }
+    return -1;
+}
+
+__global__ void k_resolve_ids(const uint32_t *__restrict__ in, int n, const uint32_t *__restrict__ ids, int nIds,
+                              const int32_t *__restrict__ off, const EntityEntry *__restrict__ entries,
+                              unsigned long long *lastWriter, RefitHeader *hdr) {
+    const unsigned long long gen = (unsigned long long)(hdr->generation + 1u) << 32;
+    CQ_GRID_STRIDE(i, n) {
+        const int e = find_entity(ids, nIds, in[i]);
+        if (e < 0) {
+            atomicAdd(&hdr->unknown, 1);
+            continue;
+        }
+        for (int k = off[e]; k < off[e + 1]; k++) atomicMax(&lastWriter[entries[k].part], gen | (unsigned)i);
+    }
+}
+
+// Block-wide exclusive scan of V ints per thread (blockDim.x = BUILD_THREADS); tot = the block's sums.
+#define BUILD_THREADS 1024
+template <int V> __device__ __forceinline__ void block_scan(int (&v)[V], int (&tot)[V], int (*warpSum)[V]) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl[V];
+#pragma unroll
+    for (int k = 0; k < V; k++) {
+        incl[k] = v[k];
+        for (int d = 1; d < 32; d <<= 1) {
+            const int o = __shfl_up_sync(0xffffffffu, incl[k], d);
+            if (lane >= d) incl[k] += o;
+        }
+        if (lane == 31) warpSum[warp][k] = incl[k];
+    }
+    __syncthreads();
+    if (warp == 0) {
+#pragma unroll
+        for (int k = 0; k < V; k++) {
+            int x = warpSum[lane][k];
+            for (int d = 1; d < 32; d <<= 1) {
+                const int o = __shfl_up_sync(0xffffffffu, x, d);
+                if (lane >= d) x += o;
+            }
+            warpSum[lane][k] = x; // inclusive over warps
+        }
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < V; k++) {
+        v[k] = incl[k] - v[k] + (warp ? warpSum[warp - 1][k] : 0);
+        tot[k] = warpSum[31][k];
+    }
+    __syncthreads(); // warpSum is reused by the next chunk
+}
+
+// k_build_moved: one block walks the inputs in chunks.  An input emits a row for each part it claimed last (its word holds
+// this generation and its index); rows are placed by a block scan of (rows, vertices, triangles) per set, which gives
+// each row its vertBase / triBase running totals, and the row copies its model from the input.  Cost grows with the
+// inputs and their parts, never with the world's part count.  Rows come in last-mention order, not the host path's
+// first-mention order: nothing depends on it, because the boxes are min / max of the same positions, which is exact in
+// any order.  Then thread 0 writes the sets' counts and paths (CQ_PATH_NONE for both when an id was unknown: the update
+// changes nothing), the caller's status word, and advances the generation.  When the 32-bit generation would wrap, the
+// block clears every last-writer word first (once per 2^32 updates).
+__global__ void __launch_bounds__(BUILD_THREADS) k_build_moved(const uint32_t *__restrict__ in, const float *__restrict__ models, int n,
+                                                               const uint32_t *__restrict__ ids, int nIds, const int32_t *__restrict__ off,
+                                                               const EntityEntry *__restrict__ entries,
+                                                               unsigned long long *lastWriter, int nParts, RefitHeader *hdr,
+                                                               MovedPart *tab0, MovedPart *tab1, int nTris0, int nTris1,
+                                                               int forceFull, int32_t *status) {
+    __shared__ int warpSum[32][6];
+    __shared__ int base[6]; // per set: rows, vertices, triangles emitted by earlier chunks
+    const uint32_t g = hdr->generation + 1u;
+    const unsigned long long gen = (unsigned long long)g << 32;
+    const int unknown = hdr->unknown;
+    if (threadIdx.x < 6) base[threadIdx.x] = 0;
+    __syncthreads();
+    if (unknown == 0)
+        for (int c0 = 0; c0 < n; c0 += BUILD_THREADS) {
+            const int i = c0 + threadIdx.x;
+            const int e = i < n ? find_entity(ids, nIds, in[i]) : -1;
+            int v[6] = {0, 0, 0, 0, 0, 0}, tot[6];
+            if (e >= 0)
+                for (int k = off[e]; k < off[e + 1]; k++) {
+                    const EntityEntry &x = entries[k];
+                    if (lastWriter[x.part] != (gen | (unsigned)i)) continue; // a later input names this part too
+                    v[3 * x.set]++, v[3 * x.set + 1] += x.nVerts, v[3 * x.set + 2] += x.nTris;
+                }
+            block_scan<6>(v, tot, warpSum);
+            if (e >= 0)
+                for (int k = off[e]; k < off[e + 1]; k++) {
+                    const EntityEntry &x = entries[k];
+                    if (lastWriter[x.part] != (gen | (unsigned)i)) continue;
+                    const int s = 3 * x.set;
+                    MovedPart &r = (x.set ? tab1 : tab0)[base[s] + v[s]];
+                    r.part = x.part, r.vertLo = x.vertLo, r.triLo = x.triLo, r.nVerts = x.nVerts, r.nTris = x.nTris;
+                    r.vertBase = base[s + 1] + v[s + 1], r.triBase = base[s + 2] + v[s + 2], r._pad = 0;
+                    for (int q = 0; q < 16; q++) r.model[q] = models[16 * (size_t)i + q];
+                    v[s]++, v[s + 1] += x.nVerts, v[s + 2] += x.nTris;
+                }
+            __syncthreads();
+            if (threadIdx.x < 6) base[threadIdx.x] += tot[threadIdx.x];
+            __syncthreads();
+        }
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < 2; s++) {
+            RefitCounts c;
+            c.nRows = base[3 * s], c.nVerts = base[3 * s + 1], c.nMoved = base[3 * s + 2];
+            c.path = c.nMoved <= 0 ? CQ_PATH_NONE
+                     : forceFull || (long long)c.nMoved * 4 >= (long long)(s ? nTris1 : nTris0) ? CQ_PATH_FULL : CQ_PATH_DIRTY;
+            hdr->set[s] = c;
+        }
+        if (status) *status = unknown;
+        hdr->unknown = 0;
+    }
+    if (g == 0xffffffffu) {
+        __syncthreads(); // every comparison above is done
+        for (int p = threadIdx.x; p < nParts; p += blockDim.x) lastWriter[p] = 0;
+        if (threadIdx.x == 0) hdr->generation = 0;
+    } else if (threadIdx.x == 0) {
+        hdr->generation = g;
+    }
+}
+
+int build_moved_device(cq_world *w, const uint32_t *dIds, const float *dModels, int n, int32_t *dStatus, cudaStream_t st) {
+    static const bool forceFull = getenv("CQ_REFIT_FULL") != nullptr;
+    const int grid = std::min(cdiv(n, 256), w->numSms * 8);
+    k_resolve_ids<<<grid, 256, 0, st>>>(dIds, n, w->dEntityIds, w->nEntities, w->dEntityOff, w->dEntries, w->dLastWriter, w->dDevHdr);
+    k_build_moved<<<1, BUILD_THREADS, 0, st>>>(dIds, dModels, n, w->dEntityIds, w->nEntities, w->dEntityOff, w->dEntries,
+                                               w->dLastWriter, (int)w->parts.size(), w->dDevHdr, w->dDevTable,
+                                               w->dDevTable + w->devRows0, w->set[0].nTris, w->set[1].nTris, forceFull ? 1 : 0,
+                                               dStatus);
+    w->launches += 2;
+    return check_cuda(cudaGetLastError(), "transform table");
 }
 
 } // namespace cq

@@ -112,6 +112,7 @@ int cq_crowd_step(cq_crowd *c, const double *velocity_in_xyz, const cq_controlle
     const int n = c->n;
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_crowd_step");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     static const float HINT = [] { // wall / PCIe-time ratio above which the step counts as compute bound (CQ_CROWD_HINT overrides)
         const char *e = getenv("CQ_CROWD_HINT");

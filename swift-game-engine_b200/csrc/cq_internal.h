@@ -73,6 +73,7 @@ struct ScratchBuf {
     cudaEvent_t ev = nullptr;
     cudaStream_t last = nullptr;
     bool recorded = false;
+    bool captured = false; // a stream capture recorded this block's address: on growth it is kept, not freed (grow_scratch)
 };
 
 // One row of the part table a transform update stages (cq_api.cu: update_transforms_on): a moved part of one set, its
@@ -85,6 +86,34 @@ struct MovedPart {
     int32_t vertBase, triBase; // sum of nVerts / nTris over the set's earlier rows
     int32_t _pad;
     float model[16];          // the new model matrix, column-major
+};
+
+// What the refit kernels of one update do to one set.  They read these counts on the device: the host-staged path copies
+// them with its table, the device path (cq_world_update_transforms_device) has k_build_moved write them, so the same
+// kernels serve both.  path: which of the two refits runs (the kernels of the other one exit at once).
+#define CQ_PATH_NONE 0  // no part of the set moved
+#define CQ_PATH_DIRTY 1 // the dirty-subtree refit
+#define CQ_PATH_FULL 2  // regather + full fit
+struct RefitCounts {
+    int32_t nRows;  // rows of the set in the table
+    int32_t nVerts; // sum of their nVerts
+    int32_t nMoved; // sum of their nTris
+    int32_t path;
+};
+// The header in front of a table of moved parts: both sets' counts.  generation / unknown are the device path's state
+// (k_resolve_ids / k_build_moved); the host-staged path leaves them zero.
+struct RefitHeader {
+    RefitCounts set[2];
+    uint32_t generation; // of the last device-path update: its last-writer words hold (generation << 32) | input index
+    int32_t unknown;     // unknown ids counted by k_resolve_ids for the update being built (reset by k_build_moved)
+    int32_t _pad[14];
+};
+static_assert(sizeof(RefitHeader) == sizeof(MovedPart), "the header takes one row of the staged table");
+
+// Device entity index (cq_world_update_transforms_device): the sorted unique entity ids, CSR offsets into the entries of
+// their parts that have triangles, and one entry per such part.
+struct EntityEntry {
+    int32_t part, set, vertLo, triLo, nVerts, nTris;
 };
 
 // Host side of one staged table: pinned memory, reused once the copy that read it has completed (event).
@@ -151,7 +180,21 @@ struct cq_world {
     std::vector<cq::MovedPart> movedRows[2]; // the table being staged, per set
     cq::StageSlot stage[CQ_STAGE_SLOTS];
     uint32_t stageSeq = 0;
-    cq::ScratchBuf dTable; // device copy of the staged table (read by the refit kernels of one update at a time)
+    cq::ScratchBuf dTable; // device copy of the staged table: a RefitHeader row, then the rows (one update at a time)
+    // device path (cq_world_update_transforms_device), one allocation made at creation so that the call never allocates
+    void *devArena = nullptr;
+    uint32_t *dEntityIds = nullptr;         // nEntities sorted unique ids
+    int32_t *dEntityOff = nullptr;          // nEntities + 1 offsets into dEntries
+    cq::EntityEntry *dEntries = nullptr;    // parts with triangles, grouped by entity, in part order
+    unsigned long long *dLastWriter = nullptr; // per part: (generation << 32) | index of the input that claimed it last
+    cq::RefitHeader *dDevHdr = nullptr;     // counts, generation and unknown-id count of the device path
+    cq::MovedPart *dDevTable = nullptr;     // static set's rows at [0, devRows0), dynamic set's after
+    int nEntities = 0, devRows0 = 0;
+    // a device call is being recorded into a stream capture (CaptureScope, cq_api.cu): no world event is waited on,
+    // recorded or created, and scratch must not grow (captureRefused then makes the call return CQ_ERR_INVALID)
+    bool capturing = false;
+    bool captureRefused = false;
+    std::vector<void *> graphScratch; // outgrown scratch blocks that captured graphs may still use: freed by cq_world_destroy
     std::vector<void *> retiredDev, retiredHost; // outgrown table buffers a queued update may still use (cq_api.cu: free_retired)
     // Ordering of stream-ordered refits against every other launch on the world (await_trees / note_reader):
     std::vector<cq::ReaderEvent> readers; // per stream: the last launch that read the trees
@@ -176,6 +219,9 @@ int check_cuda(cudaError_t e, const char *what);
     } while (0)
 
 int ensure_scratch(ScratchBuf &b, size_t bytes);
+// ensure_scratch for the blocks a captured call may use (node, unit-order and agent scratch): a block whose address a
+// graph recorded (ScratchBuf::captured) is moved to w->graphScratch instead of being freed, so replays stay valid
+int grow_scratch(cq_world *w, ScratchBuf &b, size_t bytes);
 // CTAs of `kernel` (`threads` per CTA, `dynSmem` bytes of dynamic shared memory) that fit on the device at once: SMs x
 // resident CTAs per SM (at least one per SM), cached per world.  dynSmem > 0 also raises the kernel's dynamic shared-memory
 // limit to dynSmem.  0 on CUDA error.
@@ -211,9 +257,27 @@ int build_set(cq_world *w, DeviceSet &S, const SetPlan &in /* upload plan of the
               std::vector<int> &partTriStart /* in: first input triangle of each part of the set (+ end); out: after the filter */,
               int *badTriangle /* out: smallest input triangle with an out-of-range index (CQ_ERR_INVALID), else -1 */,
               const int32_t *matIn = nullptr /* host, per INPUT triangle: row of the material table, or nullptr (row = part) */);
-// Refit one set after its parts moved: dTab = the set's rows of the staged table on the device (rows = the same rows on
-// the host, for the totals).  Stream-ordered on `st`; a fixed number of launches however many parts moved.
-int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const std::vector<MovedPart> &rows, cudaStream_t st);
+// Refit one set after its parts moved: dTab = the set's rows of the table on the device, counts = the set's RefitCounts
+// on the device (every kernel reads its counts and path there).  rows = the same rows on the host (host-staged path):
+// only the chosen path is launched, with exact grids.  rows == nullptr (device path): the host knows no counts, so both
+// paths are launched with grids sized from the set's own vertex / triangle counts and the unchosen one exits at once.
+// Stream-ordered on `st`; a fixed number of launches however many parts moved.
+int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const RefitCounts *counts, const std::vector<MovedPart> *rows,
+              cudaStream_t st);
+// the path the host-staged update takes for a set of which `moved` triangles moved (CQ_PATH_*)
+int refit_path(const DeviceSet &S, int moved);
+// Device path of cq_world_update_transforms_device: resolve the ids and build the table + counts on `st` (2 launches).
+int build_moved_device(cq_world *w, const uint32_t *dIds, const float *dModels, int n, int32_t *dStatus, cudaStream_t st);
+// a stream capture is recording `st` (cudaStreamGetCaptureInfo)
+bool stream_capturing(cudaStream_t st);
+// Calls that synchronise, allocate, create events or stage host memory: CQ_ERR_INVALID while `st` is capturing (the
+// capture stays valid), else CQ_OK.
+int refuse_capture(cudaStream_t st, const char *what);
+#define CQ_NO_CAPTURE(st, what) CQ_TRY(cq::refuse_capture((st), (what)))
+// Under capture: the call needs more scratch than any uncaptured call gave it, which would take a synchronisation and an
+// allocation.  Sets the error and w->captureRefused, returns CQ_ERR_INVALID.  captureRefused is only ever true between a
+// CaptureScope's construction and its destruction (cq_api.cu), so uncaptured calls never see it set.
+int refuse_growth(cq_world *w, const char *what);
 // reference order: rebuild the reference's tree on the host from the set's triangle boxes, upload rank + tree (cq_reftree.h)
 int attach_ref_order(cq_world *w);
 void free_set(DeviceSet &S);

@@ -835,6 +835,9 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * MAS_WARPS, st);
     if (!ns) return CQ_ERR_CUDA;
     const uint32_t *order = make_unit_order(w, d_inout, sizeof(cq_character_state), true, n, st);
+    // refused under capture: the kernels are not enqueued; the work-counter memset (and, for CQ_MAS_AGENTS, the unit
+    // order's keys and sort) already are, and only write scratch
+    if (w->captureRefused) return CQ_ERR_INVALID;
     if (flags & CQ_MAS_AGENTS) {
         CQ_TRY(make_agent_grid(w, d_inout, n, p.radius, dt, g, flags, st, A.agents));
         k_agent_first_hit<<<(n + 255) / 256, 256, 0, st>>>(d_inout, n, A);

@@ -497,6 +497,7 @@ int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, 
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;
     const uint32_t *order = make_unit_order(w, d_rays, sizeof(cq_ray), false, n, st);
+    if (w->captureRefused) return CQ_ERR_INVALID; // the query kernel is not enqueued (the work counter memset already is)
     kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_rays, n, d_out, d_flags, work, order, w->dCounters);
     w->launches++;
     return finish_launch(w, st, ref ? "k_raycast_ref" : "k_raycast");
@@ -520,6 +521,7 @@ int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cas
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
     if (!ns) return CQ_ERR_CUDA;
     const uint32_t *order = make_unit_order(w, d_q, sizeof(cq_capsule_cast), false, n, st);
+    if (w->captureRefused) return CQ_ERR_INVALID; // the query kernel is not enqueued (the work counter memset already is)
     kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, mode, d_out, d_flags, opw, ns, work, order, w->dCounters);
     w->launches++;
     return finish_launch(w, st, "k_capsule_cast");
@@ -543,7 +545,7 @@ static int launch_overlap_pool(cq_world *w, const cq_capsule *d_q, int n, int ma
     int *work = next_work_counter(w, st);
     if (!work) return CQ_ERR_CUDA;
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
-    if (!ns) return CQ_ERR_CUDA;
+    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
     kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, opw, ns, work, w->dCounters);
     w->launches++;
     return finish_launch(w, st, "k_capsule_overlap_pool");

@@ -192,6 +192,17 @@ public final class CollisionQuery {
         return rc == CQ_OK
     }
 
+    /// cq_world_update_transforms_device: the same update from device arrays (`count` ids, `count`*16 floats), queued on
+    /// `stream` without synchronising or touching host memory, so it can be recorded into a CUDA graph.  `status` (a
+    /// device Int32, may be nil) receives the number of unknown ids; with any unknown id the update changes nothing.
+    public func updateTransformsDevice(ids: UnsafePointer<UInt32>, models: UnsafePointer<Float>, count: Int32,
+                                       status: UnsafeMutablePointer<Int32>? = nil,
+                                       stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        let rc = cq_world_update_transforms_device(handle, ids, models, count, status, stream)
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
     /// Entities with Transform + StaticMesh (collides), ascending id (the reference iterates a Dictionary, i.e. in
     /// per-process random order — World.swift:99-118; the library fixes the order so triangle numbering is stable).
     /// Geometry is returned as plain Swift arrays; `withArrays` lends their storage to the C structs for one call.
