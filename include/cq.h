@@ -314,8 +314,9 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  * ordered against them by events instead (see its ordering contract).
  *
  * CUDA-graph capture: while `stream` is being captured (cudaStreamBeginCapture, torch.cuda.graph, ...), the *_device
- * query twins, cq_move_and_slide_device(_ex) and cq_world_update_transforms_device enqueue kernels, memsets and copies
- * only: they neither wait on nor record nor create world events.  So:
+ * query twins, cq_move_and_slide_device(_ex), cq_world_update_transforms_device and cq_agent_separation_device_async
+ * enqueue kernels, memsets, copies and (agent separation) conditional WHILE nodes only: they neither wait on nor record
+ * nor create world events.  So:
  *  - a graph is ordered only by the stream it is launched on; the caller orders its replays against other work on the
  *    world, as for a synchronous call (e.g. synchronise before an uncaptured call on another stream);
  *  - kernel_launches counts the launches once, at capture; replays are not counted;
@@ -326,8 +327,9 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  *    needs more scratch than an uncaptured call gave it;
  *  - scratch blocks a graph recorded stay allocated when a later uncaptured call outgrows them (the call takes new
  *    blocks), so graphs stay valid until cq_world_destroy, which frees them: replay no graph after destroying its world;
- *  - cq_agent_separation_device (it synchronises per sweep), cq_crowd_step and the host-pointer calls (checked on the
- *    world's stream, or on `stream` where they take one) refuse a capture the same way.
+ *  - cq_agent_separation_device and cq_agent_separation_batch (they synchronise to report the outcome), cq_crowd_step
+ *    and the host-pointer calls (checked on the world's stream, or on `stream` where they take one) refuse a capture the
+ *    same way.
  * Uncaptured calls behave as described everywhere else in this header. */
 int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, void *stream);
 int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode,
@@ -466,13 +468,41 @@ cq_character_state *cq_crowd_device_states(cq_crowd *c);
  * velocity are written back through Float as the reference does.  The sequential semantics are reproduced exactly (the
  * turns are scheduled along their conflict DAG).  mass_weight: AgentCollisionComponent.massWeight per character
  * (<= 0 = immovable), NULL = 1.0.  separation_margin 0.2, height_margin 0.1 are the reference defaults.  n < 2 is a
- * no-op.  The _device variant is stream-ordered but synchronises the stream internally (the schedule is host-driven). */
+ * no-op.  The _device variant is stream-ordered but synchronises the stream once at its end to report the outcome; on
+ * an error neither call changes any record.  Errors: CQ_ERR_INVALID "the crowd spans more than 2^31 grid cells" and
+ * "agents drifted more than 15 cells within one sweep", CQ_ERR_CUDA "the turn schedule stalled". */
 int cq_agent_separation_batch(cq_world *w, cq_character_state *inout, int32_t n, const cq_controller_params *params,
                               const float *mass_weight, int32_t iterations, float separation_margin, float height_margin,
                               int32_t use_query);
 int cq_agent_separation_device(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
                                const float *d_mass_weight, int32_t iterations, float separation_margin, float height_margin,
                                int32_t use_query, void *stream);
+
+/* Outcome of an agent separation, as cq_agent_separation_device_async writes it to *d_status. */
+#define CQ_SEP_STATUS_OK 0
+#define CQ_SEP_STATUS_GRID 1    /* the crowd spans more than 2^31 grid cells (synchronous calls: CQ_ERR_INVALID) */
+#define CQ_SEP_STATUS_DRIFT 2   /* agents drifted more than 15 cells within one sweep (synchronous calls: CQ_ERR_INVALID) */
+#define CQ_SEP_STATUS_STALLED 3 /* the turn schedule made no progress (synchronous calls: CQ_ERR_CUDA) */
+
+/* Stream-ordered twin of cq_agent_separation_device: the same sweeps with the same results, byte for byte, queued on
+ * `stream` (NULL = the world's stream).  The call never synchronises and never reads device memory back, so it may be
+ * recorded into a CUDA graph (see the capture contract above).  Uncaptured, each attempt is a launch of an instantiated
+ * graph the world caches.  Every outcome is decided on the device: each sweep queues
+ * its attempts for the safety radii R = 1, 3, 7, 15 up front, and an attempt runs only when the sweep is not finished
+ * and nothing failed; an agent that drifted more than R cells restores the sweep's inputs on the device for the next.
+ *
+ * Errors are all-or-nothing: on any non-zero status the records are left byte for byte unchanged.  *d_status (a device
+ * int32, may be NULL) receives CQ_SEP_STATUS_* in stream order.  NULL world, NULL params, n < 0, or a NULL d_inout with
+ * n > 0 return CQ_ERR_INVALID before any CUDA call; n < 2 returns CQ_OK and queues nothing (d_status is not written).
+ * Ordering against transform updates is that of every other launcher (see the update calls' ordering contract).
+ *
+ * Launches: a fixed number for given n and iterations, whatever drifted or failed: 3 + 23 * max(1, iterations) (per
+ * sweep: 11 to rebuild the grid, 3 per attempt).  The rounds each attempt's device-side loop runs (3 kernels per round,
+ * as many rounds as the conflict DAG is deep) are not known when the call returns and are not counted;
+ * cq_agent_separation_device and cq_agent_separation_batch add them after their synchronisation. */
+int cq_agent_separation_device_async(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
+                                     const float *d_mass_weight, int32_t iterations, float separation_margin,
+                                     float height_margin, int32_t use_query, int32_t *d_status, void *stream);
 
 /* ---- the GPUs of one box -----------------------------------------------------
  * The path shards by independent units (characters, sweeps, rays): mesh and trees are replicated on every GPU (the build

@@ -112,6 +112,8 @@ def surface_materials(rows):
 ORDER_REFERENCE, ORDER_CANONICAL = 0, 1  # include/cq.h: which of several exactly equal candidates a query names
 COUNT_OFF, COUNT_REFERENCE, COUNT_PATH = 0, 1, 2  # include/cq.h: cq_world_set_counting modes
 HIT_TIE, HIT_OVERFLOW = 1, 2
+# include/cq.h: what cq_agent_separation_device_async writes to its status word
+SEP_STATUS_OK, SEP_STATUS_GRID, SEP_STATUS_DRIFT, SEP_STATUS_STALLED = 0, 1, 2, 3
 
 
 class Material(C.Structure):
@@ -137,6 +139,7 @@ EXPORTS = [
     "cq_capsule_overlap_all_device", "cq_controller_params_default", "cq_character_state_init",
     "cq_move_and_slide_batch", "cq_move_and_slide_device", "cq_move_and_slide_batch_ex",
     "cq_move_and_slide_device_ex", "cq_agent_separation_batch", "cq_agent_separation_device",
+    "cq_agent_separation_device_async",
     "cq_world_set_counting", "cq_world_read_counters",
     "cq_crowd_create", "cq_crowd_destroy", "cq_crowd_size", "cq_crowd_step", "cq_crowd_read", "cq_crowd_write",
     "cq_crowd_device_states",
@@ -225,6 +228,7 @@ def lib():
         L.cq_move_and_slide_device_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32, vp]
         L.cq_agent_separation_batch.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32]
         L.cq_agent_separation_device.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp]
+        L.cq_agent_separation_device_async.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp, vp]
         L.cq_crowd_create.argtypes = [vp, vp, i32, C.POINTER(vp)]
         L.cq_crowd_destroy.argtypes = [vp]
         L.cq_crowd_size.argtypes = [vp]
@@ -528,6 +532,18 @@ class CollisionQuery:
                                                 C.c_void_p(d_mass_weight_ptr) if d_mass_weight_ptr else None, iterations,
                                                 separation_margin, height_margin, 1 if use_query else 0,
                                                 C.c_void_p(stream) if stream else None))
+
+    def agent_separation_device_async(self, d_states_ptr, n, params, d_mass_weight_ptr=None, iterations=2,
+                                      separation_margin=0.2, height_margin=0.1, use_query=True, d_status_ptr=None, stream=None):
+        """cq_agent_separation_device_async: the same separation queued on `stream` without synchronising or reading
+        anything back, so it can be captured in a CUDA graph.  The outcome (SEP_STATUS_*) goes to d_status_ptr (a device
+        int32, optional) in stream order; on a non-zero status the records are left unchanged."""
+        params = np.ascontiguousarray(params, PARAMS)
+        _check(lib().cq_agent_separation_device_async(self._h, C.c_void_p(d_states_ptr), int(n), _ptr(params),
+                                                      C.c_void_p(d_mass_weight_ptr) if d_mass_weight_ptr else None,
+                                                      iterations, separation_margin, height_margin, 1 if use_query else 0,
+                                                      C.c_void_p(d_status_ptr) if d_status_ptr else None,
+                                                      C.c_void_p(stream) if stream else None))
 
     def move_and_slide_device(self, d_states_ptr, n, params, dt=1.0 / 60.0, gravity=(0.0, -98.0, 0.0),
                               flags=MAS_APPLY_GRAVITY, stream=None):

@@ -80,6 +80,15 @@ class CollisionQuery {
                                 void *stream = nullptr) {
         return cq_world_update_transforms_device(w_, dEntities, dModels16, n, dStatus, stream) == CQ_OK;
     }
+    // agent separation of resident records, queued on `stream` without synchronising (capturable in a CUDA graph);
+    // *dStatus (device int32, optional) receives CQ_SEP_STATUS_* in stream order
+    bool agentSeparationDeviceAsync(cq_character_state *dInout, int32_t n, const cq_controller_params &p,
+                                    const float *dMassWeight = nullptr, int32_t iterations = 2, float separationMargin = 0.2f,
+                                    float heightMargin = 0.1f, bool useQuery = true, int32_t *dStatus = nullptr,
+                                    void *stream = nullptr) {
+        return cq_agent_separation_device_async(w_, dInout, n, &p, dMassWeight, iterations, separationMargin, heightMargin,
+                                                useQuery ? 1 : 0, dStatus, stream) == CQ_OK;
+    }
 
     std::optional<RaycastHit> raycast(Float3 origin, Float3 direction, float maxDistance, uint32_t mask = CQ_LAYER_ALL) {
         cq_ray r = {{origin.x, origin.y, origin.z}, {direction.x, direction.y, direction.z}, maxDistance, mask};

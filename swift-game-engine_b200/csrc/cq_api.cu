@@ -998,9 +998,23 @@ int cq_agent_separation_device(cq_world *w, cq_character_state *d_inout, int32_t
                                int32_t use_query, void *stream) {
     if (!w || n < 0 || !params || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
     CQ_CUDA(cudaSetDevice(w->device));
-    CQ_NO_CAPTURE(pick_stream(w, stream), "cq_agent_separation_device");
-    return launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin, height_margin, use_query,
-                                   pick_stream(w, stream));
+    const cudaStream_t st = pick_stream(w, stream);
+    CQ_NO_CAPTURE(st, "cq_agent_separation_device");
+    CQ_TRY(launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin, height_margin,
+                                   use_query, nullptr, st));
+    return wait_agent_separation(w, n, *params, separation_margin, st);
+}
+
+int cq_agent_separation_device_async(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
+                                     const float *d_mass_weight, int32_t iterations, float separation_margin,
+                                     float height_margin, int32_t use_query, int32_t *d_status, void *stream) {
+    if (!w || n < 0 || !params || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
+    if (n < 2) return CQ_OK;
+    CQ_CUDA(cudaSetDevice(w->device));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin,
+                                              height_margin, use_query, d_status, st));
 }
 
 int cq_agent_separation_batch(cq_world *w, cq_character_state *inout, int32_t n, const cq_controller_params *params,
@@ -1019,8 +1033,9 @@ int cq_agent_separation_batch(cq_world *w, cq_character_state *inout, int32_t n,
     CQ_CUDA(cudaMemcpyAsync(d, inout, sizeof(cq_character_state) * (size_t)n, cudaMemcpyHostToDevice, st));
     if (mass_weight) CQ_CUDA(cudaMemcpyAsync(w->aux.ptr, mass_weight, sizeof(float) * (size_t)n, cudaMemcpyHostToDevice, st));
     r = launch_agent_separation(w, d, n, *params, mass_weight ? (const float *)w->aux.ptr : nullptr, iterations,
-                                separation_margin, height_margin, use_query, st);
+                                separation_margin, height_margin, use_query, nullptr, st);
     if (r != CQ_OK) return r;
+    if ((r = wait_agent_separation(w, n, *params, separation_margin, st)) != CQ_OK) return r;
     CQ_CUDA(cudaMemcpyAsync(inout, d, sizeof(cq_character_state) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CQ_CUDA(cudaStreamSynchronize(st));
     return CQ_OK;

@@ -305,7 +305,10 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
                           const float g[3], uint32_t flags, const cq_platform *platforms, int nPlatforms, cudaStream_t st);
 // cq_sep.cu
 void sep_graphs_destroy(cq_world *w);
+// Queues the whole separation on `st` without waiting for the device; the outcome goes to d_status (may be nullptr).
 int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p,
                             const float *d_massWeight, int iterations, float sepMargin, float heightMargin, int useQuery,
-                            cudaStream_t st);
+                            int32_t *d_status, cudaStream_t st);
+// The synchronous calls: waits for the separation just queued on `st` and turns its outcome into an error code.
+int wait_agent_separation(cq_world *w, int n, const cq_controller_params &p, float sepMargin, cudaStream_t st);
 } // namespace cq

@@ -12,7 +12,9 @@
 //     finished), k_sep_release decrements the counters of the higher-indexed agents within D cells of each finished
 //     one and queues those that reach zero.  The schedule is a topological order of the conflict DAG, hence the result
 //     is bit-identical to the sequential loop.  With random entity order the DAG is O(log n) deep.
-//   * if any agent drifted more than R cells the sweep is repeated from a saved copy with a larger R.
+//   * if any agent drifted more than R cells the sweep is repeated from a saved copy with a larger R.  Every sweep queues
+//     its four attempts (R = 1, 3, 7, 15) up front and the device decides which of them run (k_sep_attempt_begin /
+//     k_sep_attempt_end), so a call never waits for the device and can be captured in a CUDA graph.
 // The world casts inside a turn (SYS:1994-2033) and the per-agent slide + ground snap afterwards (SYS:2043-2117) run on
 // the warp-cooperative pair pool (cq_pool.cuh), like every other capsule query of the library.
 #include "cq_pool.cuh"
@@ -32,6 +34,15 @@ struct SepGridParams {
     int minX, minZ, dimX, dimZ;
     int err; // 1 = the crowd spans more cells than a 32-bit key can number
     int _pad[3];
+};
+
+// What the device decided so far in one call (one per call, in the scratch block; zeroed when the call starts).
+struct SepState {
+    int status; // CQ_SEP_STATUS_*: set once; every later attempt and the post-process then skip
+    int done;   // the current sweep had an attempt without drift
+    int skip;   // the current attempt does not run (the sweep is done, or the call failed)
+    int rounds; // rounds run by every attempt of the call (the synchronous calls count their launches)
+    int stalledAt; // turns processed when the schedule stalled (the synchronous calls' error message)
 };
 
 struct SepArgs {
@@ -163,9 +174,9 @@ __global__ void k_sep_rows(const uint32_t *__restrict__ keys, const int2 *__rest
 // blockers(h) = lower-indexed agents whose rebuild cell is within D cells (Chebyshev) of h's
 __global__ void k_sep_count_blockers(const uint32_t *__restrict__ keys, const uint32_t *__restrict__ sidx,
                                      const int2 *__restrict__ cell0, const SepGridParams *__restrict__ gp, int n, int D,
-                                     int *cnt, int *queue, int *qcount) {
+                                     int *cnt, int *queue, int *qcount, const SepState *S) {
     int h = blockIdx.x * blockDim.x + threadIdx.x;
-    if (h >= n) return;
+    if (h >= n || S->skip) return;
     const int dimX = gp->dimX, dimZ = gp->dimZ;
     const int2 c = cell0[h];
     const int x0 = max(c.x - D, 0), x1 = min(c.x + D, dimX - 1);
@@ -200,15 +211,10 @@ __global__ void k_sep_release(const int *__restrict__ queue, const int *__restri
     }
 }
 
-__global__ void k_sep_round_end(int *qcount, int *flags, int *work) { // the consumed queue becomes the next round's output
-    flags[1] += *qcount;
-    *qcount = 0;
-    *work = 0;
-}
-
-// The same inside the CUDA-graph WHILE node that runs the rounds of a sweep on the device (sep_rounds_graph below).  The
-// body of the loop holds two rounds (the queues swap roles); its last node decides whether the body runs again: turns
-// remain, no agent drifted out of the safety radius, and the pass retired at least one turn.
+// The end of a round, inside the CUDA-graph WHILE node that runs the rounds of an attempt on the device (sep_add_attempt
+// below): the consumed queue becomes the next round's output.  The body of the loop holds two rounds (the queues swap
+// roles); its last node decides whether the body runs again: turns remain, no agent drifted out of the safety radius,
+// and the pass retired at least one turn.
 // flags: [0] drift violation, [1] processed turns, [2] processed at the end of the previous pass, [3] stalled, [4] rounds
 __global__ void k_sep_round_end_dev(int *qcount, int *flags, int *work, int n, int last, cudaGraphConditionalHandle loop) {
     flags[1] += *qcount;
@@ -222,6 +228,52 @@ __global__ void k_sep_round_end_dev(int *qcount, int *flags, int *work, int n, i
         flags[2] = processed;
         cudaGraphSetConditional(loop, go ? 1u : 0u);
     }
+}
+
+// The head of one attempt (safety radius R) of a sweep.  It is queued whatever happened before it, and skips the attempt
+// when the sweep is already done or the call failed (a crowd too wide for the grid is caught here, before any round runs
+// on the 1x1 fallback grid); otherwise it resets the attempt's counters.  Either way it sets the loop condition of the
+// attempt's rounds, whose WHILE node tests it before the first pass.
+__global__ void k_sep_attempt_begin(const SepGridParams *gp, int *flags, int *qcount, SepState *S, int first,
+                                    cudaGraphConditionalHandle loop) {
+    if (first) S->done = 0;
+    if (!S->status && gp->err) S->status = CQ_SEP_STATUS_GRID;
+    const int skip = S->done || S->status;
+    S->skip = skip;
+    if (!skip) {
+        for (int k = 0; k < 8; k++) flags[k] = 0;
+        qcount[0] = qcount[1] = qcount[2] = 0; // both queue counters + the work counter
+    }
+    cudaGraphSetConditional(loop, skip ? 0u : 1u);
+}
+
+// The outcome of an attempt that ran (flags as k_sep_round_end_dev left them): an agent drifted more than R cells, so
+// the sweep's inputs are restored for the next attempt (after the last one the call fails); the schedule stalled; or the
+// sweep is done.  Grid-stride over the agents for the restore.
+__global__ void k_sep_attempt_end(const int *flags, SepState *S, int last, float4 *pos, float4 *vel,
+                                  const float4 *__restrict__ posSave, const float4 *__restrict__ velSave, int n) {
+    if (S->skip) return;
+    const bool drift = flags[0] != 0;
+    if (drift)
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+            pos[i] = posSave[i];
+            vel[i] = velSave[i];
+        }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        S->rounds += flags[4];
+        if (drift) {
+            if (last) S->status = CQ_SEP_STATUS_DRIFT;
+        } else if (flags[3]) {
+            S->status = CQ_SEP_STATUS_STALLED;
+            S->stalledAt = flags[1];
+        } else {
+            S->done = 1;
+        }
+    }
+}
+
+__global__ void k_sep_status(const SepState *S, int32_t *out) {
+    if (out) *out = S->status;
 }
 
 // ---------------------------------------------------------------- turns (AgentSeparationResolver.resolve, SYS:1946-2041)
@@ -513,6 +565,7 @@ struct PostArgs {
     int useQuery, n;
     const float4 *pos, *vel, *orig;
     cq_character_state *states;
+    const int *status; // SepState::status: a failed call writes no record
 };
 
 template <bool COUNT>
@@ -611,6 +664,7 @@ __device__ __forceinline__ bool post_advance(PostCtx &c, const QResult &q, QShar
 template <bool COUNT>
 __global__ void __launch_bounds__(SEP_THREADS, 4) k_sep_post(WorldView W, const __grid_constant__ PostArgs A, uint2 *nodeScratch,
                                                              int *workCounter, unsigned long long *gctr) {
+    if (*A.status) return;
     extern __shared__ __align__(16) unsigned char sepSmem[];
     PostCtx *ctxs = reinterpret_cast<PostCtx *>(sepSmem);
     QShared *qsAll = reinterpret_cast<QShared *>(sepSmem + sizeof(PostCtx) * SEP_THREADS);
@@ -631,10 +685,12 @@ __global__ void __launch_bounds__(SEP_THREADS, 4) k_sep_post(WorldView W, const 
 }
 
 // ---------------------------------------------------------------- host driver
-// The rounds of one sweep as ONE graph launch: a WHILE node whose body is two rounds (turns -> release -> round end, with
-// the queues in either role); k_sep_round_end_dev sets the loop condition, so the host neither launches rounds nor reads
-// progress back while the schedule runs (round 1 read it back every 8 rounds).  Instantiated graphs are kept per world,
-// keyed by every launch parameter (the node-scratch block rotates over four buffers, hence a few entries).
+// One attempt of a sweep as graph nodes: begin -> count blockers -> WHILE{2 x (turns -> release -> round end)} -> end.
+// k_sep_round_end_dev sets the loop condition, so the host neither launches rounds nor reads progress back while the
+// schedule runs, and k_sep_attempt_begin / k_sep_attempt_end decide on the device whether the attempt runs and what its
+// outcome is.  Uncaptured, each attempt is its own instantiated graph, kept per world and keyed by every launch
+// parameter (R, and the node-scratch block, which rotates over four buffers: a few entries per crowd size).  Under a
+// stream capture the same nodes are added to the capture graph itself (sep_attempt).
 struct SepGraph {
     std::vector<unsigned char> key;
     cudaGraph_t graph = nullptr;
@@ -657,7 +713,7 @@ void sep_graphs_destroy(cq_world *w) {
     w->sepGraphs = nullptr;
 }
 
-struct SepRoundsLaunch {
+struct SepAttempt {
     const void *turnKernel;
     int turnBlocks, releaseBlocks;
     size_t turnSmem;
@@ -670,11 +726,82 @@ struct SepRoundsLaunch {
     const uint32_t *keys, *vals;
     const int2 *cell0;
     const SepGridParams *gp;
-    int n, D;
+    int n, D, first, last;
     int *cnt, *flags;
+    SepState *state;
+    float4 *pos, *vel;
+    const float4 *posSave, *velSave;
 };
 
-static int sep_rounds_graph(cq_world *w, SepRoundsLaunch &L, cudaGraphExec_t *out) {
+static int add_kernel(cudaGraph_t g, cudaGraphNode_t *node, const cudaGraphNode_t *deps, size_t nDeps, const void *func,
+                      int blocks, int threads, size_t smem, void **args) {
+    cudaKernelNodeParams kp = {};
+    kp.func = (void *)func;
+    kp.gridDim = dim3(blocks), kp.blockDim = dim3(threads);
+    kp.sharedMemBytes = (unsigned)smem;
+    kp.kernelParams = args;
+    CQ_CUDA(cudaGraphAddKernelNode(node, g, deps, nDeps, &kp));
+    return CQ_OK;
+}
+
+// adds the attempt's nodes to `g` after `deps`; *end = its last node
+static int sep_add_attempt(cudaGraph_t g, const cudaGraphNode_t *deps, size_t nDeps, SepAttempt &L, cudaGraphNode_t *end) {
+    cudaGraphConditionalHandle loop;
+    CQ_CUDA(cudaGraphConditionalHandleCreate(&loop, g, 0, cudaGraphCondAssignDefault));
+    cudaGraphNode_t node;
+    void *beginArgs[] = {(void *)&L.gp, (void *)&L.flags, (void *)&L.qcount, (void *)&L.state, (void *)&L.first, (void *)&loop};
+    CQ_TRY(add_kernel(g, &node, deps, nDeps, (const void *)k_sep_attempt_begin, 1, 1, 0, beginArgs));
+    void *countArgs[] = {(void *)&L.keys, (void *)&L.vals, (void *)&L.cell0, (void *)&L.gp, (void *)&L.n, (void *)&L.D,
+                         (void *)&L.cnt, (void *)&L.queue[0], (void *)&L.qcount, (void *)&L.state};
+    CQ_TRY(add_kernel(g, &node, &node, 1, (const void *)k_sep_count_blockers, cdiv(L.n, 256), 256, 0, countArgs));
+    cudaGraphNodeParams cp = {cudaGraphNodeTypeConditional};
+    cp.conditional.handle = loop;
+    cp.conditional.type = cudaGraphCondTypeWhile;
+    cp.conditional.size = 1;
+    CQ_CUDA(cudaGraphAddNode(&node, g, &node, 1, &cp));
+    const cudaGraphNode_t whileNode = node;
+    cudaGraph_t body = cp.conditional.phGraph_out[0];
+    cudaGraphNode_t prev = nullptr;
+    for (int half = 0; half < 2; half++) {
+        int *q = L.queue[half], *qn = L.queue[half ^ 1];
+        int *qc = L.qcount + half, *qcn = L.qcount + (half ^ 1);
+        SepArgs A = L.A;
+        A.queue = q, A.qcount = qc;
+        void *turnArgs[] = {(void *)&L.view, (void *)&A, (void *)&L.ns, (void *)&L.work, (void *)&L.counters};
+        CQ_TRY(add_kernel(body, &node, prev ? &prev : nullptr, prev ? 1 : 0, L.turnKernel, L.turnBlocks, SEP_THREADS,
+                          L.turnSmem, turnArgs));
+        prev = node;
+        void *relArgs[] = {(void *)&q, (void *)&qc, (void *)&L.keys, (void *)&L.vals, (void *)&L.cell0, (void *)&L.gp,
+                           (void *)&L.n, (void *)&L.D, (void *)&L.cnt, (void *)&qn, (void *)&qcn};
+        CQ_TRY(add_kernel(body, &node, &prev, 1, (const void *)k_sep_release, L.releaseBlocks, 256, 0, relArgs));
+        prev = node;
+        int last = half;
+        void *endArgs[] = {(void *)&qc, (void *)&L.flags, (void *)&L.work, (void *)&L.n, (void *)&last, (void *)&loop};
+        CQ_TRY(add_kernel(body, &node, &prev, 1, (const void *)k_sep_round_end_dev, 1, 1, 0, endArgs));
+        prev = node;
+    }
+    void *endArgs[] = {(void *)&L.flags, (void *)&L.state, (void *)&L.last, (void *)&L.pos, (void *)&L.vel,
+                       (void *)&L.posSave, (void *)&L.velSave, (void *)&L.n};
+    return add_kernel(g, end, &whileNode, 1, (const void *)k_sep_attempt_end, L.releaseBlocks, 256, 0, endArgs);
+}
+
+// Queues one attempt on `st`: into the capture graph while `st` is captured (cudaStreamGetCaptureInfo gives the graph and
+// the current dependencies, cudaStreamUpdateCaptureDependencies makes later work wait for the attempt's last node), else
+// as a launch of its cached instantiated graph.  3 kernel launches are counted; the rounds are not known here.
+static int sep_attempt(cq_world *w, SepAttempt &L, cudaStream_t st) {
+    w->launches += 3;
+    if (w->capturing) {
+        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+        cudaGraph_t g = nullptr;
+        const cudaGraphNode_t *d = nullptr;
+        size_t nd = 0;
+        CQ_CUDA(cudaStreamGetCaptureInfo(st, &cs, nullptr, &g, &d, &nd));
+        const std::vector<cudaGraphNode_t> deps(d, d + nd);
+        cudaGraphNode_t end;
+        CQ_TRY(sep_add_attempt(g, deps.data(), deps.size(), L, &end));
+        CQ_CUDA(cudaStreamUpdateCaptureDependencies(st, &end, 1, cudaStreamSetCaptureDependencies));
+        return CQ_OK;
+    }
     if (!w->sepGraphs) w->sepGraphs = new SepGraphCache();
     SepGraphCache &cache = *(SepGraphCache *)w->sepGraphs;
     L.A.queue = nullptr, L.A.qcount = nullptr;
@@ -683,10 +810,10 @@ static int sep_rounds_graph(cq_world *w, SepRoundsLaunch &L, cudaGraphExec_t *ou
     for (SepGraph &g : cache.items)
         if (g.key == key) {
             g.used = ++cache.tick;
-            *out = g.exec;
+            CQ_CUDA(cudaGraphLaunch(g.exec, st));
             return CQ_OK;
         }
-    if (cache.items.size() >= 8) { // evict the least recently used
+    if (cache.items.size() >= 32) { // evict the least recently used
         size_t lru = 0;
         for (size_t i = 1; i < cache.items.size(); i++)
             if (cache.items[i].used < cache.items[lru].used) lru = i;
@@ -697,57 +824,32 @@ static int sep_rounds_graph(cq_world *w, SepRoundsLaunch &L, cudaGraphExec_t *ou
     SepGraph g;
     g.key = key;
     CQ_CUDA(cudaGraphCreate(&g.graph, 0));
-    cudaGraphConditionalHandle loop;
-    CQ_CUDA(cudaGraphConditionalHandleCreate(&loop, g.graph, 1, cudaGraphCondAssignDefault));
-    cudaGraphNodeParams cp = {cudaGraphNodeTypeConditional};
-    cp.conditional.handle = loop;
-    cp.conditional.type = cudaGraphCondTypeWhile;
-    cp.conditional.size = 1;
-    cudaGraphNode_t whileNode;
-    CQ_CUDA(cudaGraphAddNode(&whileNode, g.graph, nullptr, 0, &cp));
-    cudaGraph_t body = cp.conditional.phGraph_out[0];
-    cudaGraphNode_t prev = nullptr;
-    for (int half = 0; half < 2; half++) {
-        int *q = L.queue[half], *qn = L.queue[half ^ 1];
-        int *qc = L.qcount + half, *qcn = L.qcount + (half ^ 1);
-        SepArgs A = L.A;
-        A.queue = q, A.qcount = qc;
-        cudaGraphNode_t node;
-        cudaKernelNodeParams kp = {};
-        void *turnArgs[] = {(void *)&L.view, (void *)&A, (void *)&L.ns, (void *)&L.work, (void *)&L.counters};
-        kp.func = (void *)L.turnKernel;
-        kp.gridDim = dim3(L.turnBlocks), kp.blockDim = dim3(SEP_THREADS);
-        kp.sharedMemBytes = (unsigned)L.turnSmem;
-        kp.kernelParams = turnArgs;
-        CQ_CUDA(cudaGraphAddKernelNode(&node, body, prev ? &prev : nullptr, prev ? 1 : 0, &kp));
-        prev = node;
-        void *relArgs[] = {(void *)&q, (void *)&qc, (void *)&L.keys, (void *)&L.vals, (void *)&L.cell0, (void *)&L.gp,
-                           (void *)&L.n, (void *)&L.D, (void *)&L.cnt, (void *)&qn, (void *)&qcn};
-        kp = cudaKernelNodeParams{};
-        kp.func = (void *)k_sep_release;
-        kp.gridDim = dim3(L.releaseBlocks), kp.blockDim = dim3(256);
-        kp.kernelParams = relArgs;
-        CQ_CUDA(cudaGraphAddKernelNode(&node, body, &prev, 1, &kp));
-        prev = node;
-        int last = half;
-        void *endArgs[] = {(void *)&qc, (void *)&L.flags, (void *)&L.work, (void *)&L.n, (void *)&last, (void *)&loop};
-        kp = cudaKernelNodeParams{};
-        kp.func = (void *)k_sep_round_end_dev;
-        kp.gridDim = dim3(1), kp.blockDim = dim3(1);
-        kp.kernelParams = endArgs;
-        CQ_CUDA(cudaGraphAddKernelNode(&node, body, &prev, 1, &kp));
-        prev = node;
+    cudaGraphNode_t end;
+    int rc = sep_add_attempt(g.graph, nullptr, 0, L, &end);
+    if (rc == CQ_OK) rc = check_cuda(cudaGraphInstantiate(&g.exec, g.graph, 0), "sep graph instantiate");
+    if (rc != CQ_OK) {
+        cudaGraphDestroy(g.graph);
+        return rc;
     }
-    CQ_CUDA(cudaGraphInstantiate(&g.exec, g.graph, 0));
     g.used = ++cache.tick;
     cache.items.push_back(g);
-    *out = g.exec;
+    CQ_CUDA(cudaGraphLaunch(g.exec, st));
     return CQ_OK;
+}
+
+static float sep_cell_size(const cq_controller_params &p, float sepMargin) {
+    return std::max(p.radius * 2 + sepMargin, 0.001f); // SYS:2180 (every agent has the controller radius)
+}
+
+// Where the scratch block of a call for n agents keeps its small words: bounds[4] flags[8] qcount[2] work[1], the grid
+// parameters at +16, the SepState at +24.
+static int *sep_small(void *scratch, int n) {
+    return (int *)((uint32_t *)((char *)scratch + (size_t)n * (7 * 16 + 2 * 8 + 3 * 4 + 4 * 4)) + sort_scratch_words(n));
 }
 
 int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p,
                             const float *d_massWeight, int iterations, float sepMargin, float heightMargin, int useQuery,
-                            cudaStream_t st) {
+                            int32_t *d_status, cudaStream_t st) {
     if (n <= 1) return CQ_OK; // `guard agents.count > 1` (SYS:2178)
     CQ_TRY(await_trees(w, st));
     iterations = std::max(1, iterations);
@@ -756,9 +858,11 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     // u32 x4 (sort), scratch
     const size_t bytes = (size_t)n * (7 * 16 + 2 * 8 + 3 * 4 + 4 * 4) + sortWords * 4 + 256;
     if (bytes > w->sepScratch.cap) {
+        if (w->capturing) return refuse_growth(w, "agent separation scratch");
         CQ_CUDA(cudaDeviceSynchronize());
-        CQ_TRY(ensure_scratch(w->sepScratch, bytes));
+        CQ_TRY(grow_scratch(w, w->sepScratch, bytes));
     }
+    if (w->capturing) w->sepScratch.captured = true;
     CQ_TRY(scratch_acquire(w, w->sepScratch, st));
     float4 *pos = (float4 *)w->sepScratch.ptr, *vel = pos + n, *orig = vel + n, *posSave = orig + n, *velSave = posSave + n;
     int4 *rows = (int4 *)(velSave + n);
@@ -766,9 +870,10 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     int *cnt = (int *)(cell0 + n), *queueA = cnt + n, *queueB = queueA + n;
     uint32_t *keys = (uint32_t *)(queueB + n), *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n;
     uint32_t *scratch = valsTmp + n;
-    int *small = (int *)(scratch + sortWords); // bounds[4] flags[8] qcount[2] work[1] + grid params
+    int *small = sep_small(w->sepScratch.ptr, n);
     int *bounds = small, *flags = small + 4, *qcount = small + 12, *work = small + 14;
     SepGridParams *gp = (SepGridParams *)(small + 16);
+    SepState *state = (SepState *)(small + 24);
 
     const int ci = w->counting ? 1 : 0;
     const void *turnKernel = ci ? (const void *)k_sep_turns<true> : (const void *)k_sep_turns<false>;
@@ -779,22 +884,25 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     if (!turnBlocksMax || !postBlocksMax) return CQ_ERR_CUDA;
     const int turnBlocks = std::min(cdiv(n, 4), turnBlocksMax), postBlocks = std::min(cdiv(n, 4), postBlocksMax);
     uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)std::max(turnBlocks, postBlocks) * SEP_WARPS, st);
-    if (!ns) return CQ_ERR_CUDA;
+    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
 
-    const float cellSize = std::max(p.radius * 2 + sepMargin, 0.001f); // SYS:2180 (every agent has the controller radius)
+    const float cellSize = sep_cell_size(p, sepMargin);
+    CQ_CUDA(cudaMemsetAsync(state, 0, sizeof(SepState), st));
     k_sep_collect<<<cdiv(n, 256), 256, 0, st>>>(d_inout, d_massWeight, n, pos, vel, orig);
     w->launches++;
 
-    SepArgs A;
-    memset(&A, 0, sizeof(A));
-    A.p = p;
-    A.sepMargin = sepMargin, A.heightMargin = heightMargin, A.cellSize = cellSize;
-    A.useQuery = useQuery, A.n = n;
-    A.pos = pos, A.vel = vel, A.cell0 = cell0, A.keys = keys, A.sidx = vals, A.rows = rows, A.gp = gp, A.flags = flags;
-
-    // CQ_SEP_HOST_ROUNDS=1: launch the rounds from the host, progress read back every 8 rounds (the round-1 schedule; A/B)
-    const char *hr = getenv("CQ_SEP_HOST_ROUNDS");
-    const bool hostRounds = hr && hr[0] == '1';
+    SepAttempt L;
+    memset(&L, 0, sizeof(L));
+    L.A.p = p;
+    L.A.sepMargin = sepMargin, L.A.heightMargin = heightMargin, L.A.cellSize = cellSize;
+    L.A.useQuery = useQuery, L.A.n = n;
+    L.A.pos = pos, L.A.vel = vel, L.A.cell0 = cell0, L.A.keys = keys, L.A.sidx = vals, L.A.rows = rows, L.A.gp = gp;
+    L.A.flags = flags;
+    L.turnKernel = turnKernel, L.turnBlocks = turnBlocks, L.releaseBlocks = std::min(cdiv(n, 64), 148 * 8);
+    L.turnSmem = turnSmem, L.view = w->view, L.ns = ns, L.work = work, L.counters = w->dCounters;
+    L.queue[0] = queueA, L.queue[1] = queueB, L.qcount = qcount;
+    L.keys = keys, L.vals = vals, L.cell0 = cell0, L.gp = gp, L.n = n, L.cnt = cnt, L.flags = flags, L.state = state;
+    L.pos = pos, L.vel = vel, L.posSave = posSave, L.velSave = velSave;
     for (int it = 0; it < iterations; it++) {
         // grid.rebuild(agents) (SYS:1931-1937): cells of the CURRENT positions; a stable sort keeps each cell's list in
         // ascending agent index = the reference's append order
@@ -808,74 +916,10 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
         w->launches++;
         CQ_CUDA(cudaMemcpyAsync(posSave, pos, sizeof(float4) * n, cudaMemcpyDeviceToDevice, st));
         CQ_CUDA(cudaMemcpyAsync(velSave, vel, sizeof(float4) * n, cudaMemcpyDeviceToDevice, st));
-        bool done = false;
-        for (int R = 1; R <= 15 && !done; R = 2 * R + 1) {
-            const int D = 2 * (R + 1);
-            A.R = R;
-            CQ_CUDA(cudaMemsetAsync(flags, 0, sizeof(int) * 8, st));
-            CQ_CUDA(cudaMemsetAsync(qcount, 0, sizeof(int) * 3, st)); // both queue counters + the work counter
-            k_sep_count_blockers<<<cdiv(n, 256), 256, 0, st>>>(keys, vals, cell0, gp, n, D, cnt, queueA, qcount);
-            w->launches++;
-            if (!hostRounds) { // the rounds run as a device-side loop
-                SepRoundsLaunch L;
-                memset(&L, 0, sizeof(L));
-                L.turnKernel = turnKernel, L.turnBlocks = turnBlocks, L.releaseBlocks = std::min(cdiv(n, 64), 148 * 8);
-                L.turnSmem = turnSmem, L.view = w->view, L.A = A, L.ns = ns, L.work = work, L.counters = w->dCounters;
-                L.queue[0] = queueA, L.queue[1] = queueB, L.qcount = qcount;
-                L.keys = keys, L.vals = vals, L.cell0 = cell0, L.gp = gp, L.n = n, L.D = D, L.cnt = cnt, L.flags = flags;
-                cudaGraphExec_t exec = nullptr;
-                CQ_TRY(sep_rounds_graph(w, L, &exec));
-                CQ_CUDA(cudaGraphLaunch(exec, st));
-            }
-            int processed = 0, lastProcessed = -1, round = 0;
-            while (hostRounds && processed < n) {
-                for (int k = 0; k < 8; k++, round++) {
-                    int *q = (round & 1) ? queueB : queueA, *qn = (round & 1) ? queueA : queueB;
-                    int *qc = qcount + (round & 1), *qcn = qcount + ((round & 1) ^ 1);
-                    A.queue = q, A.qcount = qc;
-                    void *args[] = {(void *)&w->view, (void *)&A, (void *)&ns, (void *)&work, (void *)&w->dCounters};
-                    CQ_CUDA(cudaLaunchKernel(turnKernel, dim3(turnBlocks), dim3(SEP_THREADS), args, turnSmem, st));
-                    k_sep_release<<<std::min(cdiv(n, 64), 148 * 8), 256, 0, st>>>(q, qc, keys, vals, cell0, gp, n, D, cnt, qn, qcn);
-                    k_sep_round_end<<<1, 1, 0, st>>>(qc, flags, work);
-                    w->launches += 3;
-                }
-                int host[2];
-                CQ_CUDA(cudaMemcpyAsync(host, flags, sizeof(host), cudaMemcpyDeviceToHost, st));
-                CQ_CUDA(cudaStreamSynchronize(st));
-                processed = host[1];
-                if (host[0]) break; // an agent drifted more than R cells: this schedule cannot be trusted
-                if (processed == lastProcessed) {
-                    set_error("cq_agent_separation: the turn schedule stalled at %d of %d agents", processed, n);
-                    return CQ_ERR_CUDA;
-                }
-                lastProcessed = processed;
-            }
-            int hostFlags[5] = {0, 0, 0, 0, 0}, gridErr = 0;
-            CQ_CUDA(cudaMemcpyAsync(hostFlags, flags, sizeof(hostFlags), cudaMemcpyDeviceToHost, st));
-            CQ_CUDA(cudaMemcpyAsync(&gridErr, &gp->err, sizeof(int), cudaMemcpyDeviceToHost, st));
-            CQ_CUDA(cudaStreamSynchronize(st));
-            const int hostFlag = hostFlags[0];
-            if (!hostRounds) {
-                w->launches += 3 * (uint64_t)hostFlags[4];
-                if (!hostFlag && !gridErr && hostFlags[3]) {
-                    set_error("cq_agent_separation: the turn schedule stalled at %d of %d agents", hostFlags[1], n);
-                    return CQ_ERR_CUDA;
-                }
-            }
-            if (gridErr) {
-                set_error("cq_agent_separation: the crowd spans more than 2^31 grid cells of %.3f m", cellSize);
-                return CQ_ERR_INVALID;
-            }
-            if (!hostFlag) {
-                done = true;
-            } else { // restore the sweep's inputs and retry with a wider safety radius
-                CQ_CUDA(cudaMemcpyAsync(pos, posSave, sizeof(float4) * n, cudaMemcpyDeviceToDevice, st));
-                CQ_CUDA(cudaMemcpyAsync(vel, velSave, sizeof(float4) * n, cudaMemcpyDeviceToDevice, st));
-            }
-        }
-        if (!done) {
-            set_error("cq_agent_separation: agents drifted more than 15 cells within one sweep");
-            return CQ_ERR_INVALID;
+        for (int R = 1; R <= 15; R = 2 * R + 1) { // a sweep whose agents drift more than R cells is rerun with a wider R
+            L.A.R = R, L.D = 2 * (R + 1);
+            L.first = R == 1, L.last = R == 15;
+            CQ_TRY(sep_attempt(w, L, st));
         }
     }
 
@@ -883,12 +927,34 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     memset(&PA, 0, sizeof(PA));
     PA.p = p;
     PA.useQuery = useQuery, PA.n = n;
-    PA.pos = pos, PA.vel = vel, PA.orig = orig, PA.states = d_inout;
+    PA.pos = pos, PA.vel = vel, PA.orig = orig, PA.states = d_inout, PA.status = &state->status;
     CQ_CUDA(cudaMemsetAsync(work, 0, sizeof(int), st));
     void *args[] = {(void *)&w->view, (void *)&PA, (void *)&ns, (void *)&work, (void *)&w->dCounters};
     CQ_CUDA(cudaLaunchKernel(postKernel, dim3(postBlocks), dim3(SEP_THREADS), args, postSmem, st));
-    w->launches++;
+    k_sep_status<<<1, 1, 0, st>>>(state, d_status);
+    w->launches += 2;
     return finish_launch(w, st, "agent separation");
+}
+
+int wait_agent_separation(cq_world *w, int n, const cq_controller_params &p, float sepMargin, cudaStream_t st) {
+    if (n <= 1) return CQ_OK;
+    const int *small = sep_small(w->sepScratch.ptr, n);
+    SepState S;
+    CQ_CUDA(cudaMemcpyAsync(&S, small + 24, sizeof(S), cudaMemcpyDeviceToHost, st));
+    CQ_CUDA(cudaStreamSynchronize(st));
+    w->launches += 3 * (uint64_t)S.rounds;
+    switch (S.status) {
+    case CQ_SEP_STATUS_OK: return CQ_OK;
+    case CQ_SEP_STATUS_GRID:
+        set_error("cq_agent_separation: the crowd spans more than 2^31 grid cells of %.3f m", sep_cell_size(p, sepMargin));
+        return CQ_ERR_INVALID;
+    case CQ_SEP_STATUS_DRIFT:
+        set_error("cq_agent_separation: agents drifted more than 15 cells within one sweep");
+        return CQ_ERR_INVALID;
+    default:
+        set_error("cq_agent_separation: the turn schedule stalled at %d of %d agents", S.stalledAt, n);
+        return CQ_ERR_CUDA;
+    }
 }
 
 } // namespace cq

@@ -203,6 +203,21 @@ public final class CollisionQuery {
         return rc == CQ_OK
     }
 
+    /// Agent separation of resident records (`states`: a device pointer), queued on `stream` without synchronising, so
+    /// it can be captured in a CUDA graph.  `status` (a device Int32) receives CQ_SEP_STATUS_* in stream order; on a
+    /// non-zero status the records are left unchanged.
+    public func agentSeparationDeviceAsync(states: UnsafeMutablePointer<cq_character_state>, count: Int32,
+                                           params: cq_controller_params, massWeights: UnsafePointer<Float>? = nil,
+                                           iterations: Int32 = 2, separationMargin: Float = 0.2, heightMargin: Float = 0.1,
+                                           useQuery: Bool = true, status: UnsafeMutablePointer<Int32>? = nil,
+                                           stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        var p = params
+        let rc = cq_agent_separation_device_async(handle, states, count, &p, massWeights, iterations, separationMargin,
+                                                  heightMargin, useQuery ? 1 : 0, status, stream)
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
     /// Entities with Transform + StaticMesh (collides), ascending id (the reference iterates a Dictionary, i.e. in
     /// per-process random order — World.swift:99-118; the library fixes the order so triangle numbering is stable).
     /// Geometry is returned as plain Swift arrays; `withArrays` lends their storage to the C structs for one call.
