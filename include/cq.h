@@ -42,7 +42,12 @@ extern "C" {
 #define CQ_ERR_NCCL (-6)      /* NCCL missing or failed (multi-GPU groups only) */
 
 #define CQ_LAYER_ALL 0xFFFFFFFFu /* CollisionLayer.all, Components.swift:47-50 */
-#define CQ_MAX_OVERLAP_HITS 8    /* capsuleOverlapAll default maxHits, CollisionQuery.swift:151 */
+/* capsuleOverlapAll's default maxHits (CollisionQuery.swift:151) and the maxHits of move-and-slide's depenetration
+ * (Systems.swift:751-767).  It is not a limit of cq_capsule_overlap_all_*: max_hits up to 8 runs a kernel that keeps
+ * the hits in shared memory, larger values run the wide path (see cq_capsule_overlap_all_batch). */
+#define CQ_MAX_OVERLAP_HITS 8
+/* Device scratch bound of cq_capsule_overlap_all_batch: it runs in query chunks whose records fit 256 MiB. */
+#define CQ_OVERLAP_ALL_CHUNK_BYTES ((size_t)256 << 20)
 #define CQ_MANIFOLD_MAX 4        /* ContactManifoldCache.maxCount, Systems.swift:1160 */
 
 typedef struct cq_world cq_world;
@@ -300,7 +305,14 @@ int cq_capsule_overlap_batch(cq_world *w, const cq_capsule *q, int32_t n, cq_ove
 /* out = n * max_hits records; counts[i] = hits written for query i; overflow[i] (may be NULL) = 1 when more than
  * max_hits triangles overlapped.  CQ_ORDER_REFERENCE: the first max_hits triangles the reference visits, in its
  * visiting order (:1272-1274; its callers sort by depth themselves, Systems.swift:759).  CQ_ORDER_CANONICAL: the
- * max_hits deepest, deepest first (ties: smaller triangle index).  1 <= max_hits <= 8. */
+ * max_hits deepest, deepest first (ties: smaller triangle index).  Slots past counts[i] hold nil records.
+ * Any max_hits is accepted; values below 1 become 1 (max(1, maxHits), CollisionQuery.swift:157).  The call fails with
+ * CQ_ERR_INVALID, before any CUDA call, only when n * max_hits * sizeof(cq_overlap_hit) overflows size_t.
+ * max_hits <= CQ_MAX_OVERLAP_HITS: one kernel launch.  Larger max_hits: the wide path, always three launches (the pair
+ * pool keeps each query's winners as a heap in the query's own output slots, one thread per query sorts them, one thread
+ * per slot writes the records); it needs no scratch beyond the smaller path's, so its device call is captured like it.
+ * This host-pointer call runs in query chunks so that its record scratch stays within CQ_OVERLAP_ALL_CHUNK_BYTES (one
+ * query whose records exceed that is a chunk of its own): one set of launches per chunk, identical results. */
 int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, int32_t max_hits,
                                  cq_overlap_hit *out, int32_t *counts, uint8_t *overflow);
 

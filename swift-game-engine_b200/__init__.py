@@ -112,6 +112,7 @@ def surface_materials(rows):
 ORDER_REFERENCE, ORDER_CANONICAL = 0, 1  # include/cq.h: which of several exactly equal candidates a query names
 COUNT_OFF, COUNT_REFERENCE, COUNT_PATH = 0, 1, 2  # include/cq.h: cq_world_set_counting modes
 HIT_TIE, HIT_OVERFLOW = 1, 2
+OVERLAP_ALL_CHUNK_BYTES = 256 << 20  # CQ_OVERLAP_ALL_CHUNK_BYTES: record scratch bound of the host-pointer overlap-all call
 # include/cq.h: what cq_agent_separation_device_async writes to its status word
 SEP_STATUS_OK, SEP_STATUS_GRID, SEP_STATUS_DRIFT, SEP_STATUS_STALLED = 0, 1, 2, 3
 
@@ -551,6 +552,14 @@ class CollisionQuery:
         g = np.asarray(gravity, np.float32)
         _check(lib().cq_move_and_slide_device(self._h, C.c_void_p(d_states_ptr), n, _ptr(params), C.c_float(dt),
                                               _ptr(g), flags, C.c_void_p(stream) if stream else None))
+
+    def capsule_overlap_all_device(self, d_q_ptr, n, max_hits, d_out_ptr, d_counts_ptr, d_overflow_ptr=None, stream=None):
+        """cq_capsule_overlap_all_device: n CAPSULE records in, n * max_hits OVERLAP_HIT records, n int32 counts and
+        (optional) n overflow bytes out, all device pointers, enqueued on `stream` without synchronising."""
+        _check(lib().cq_capsule_overlap_all_device(self._h, C.c_void_p(d_q_ptr), int(n), int(max_hits), C.c_void_p(d_out_ptr),
+                                                   C.c_void_p(d_counts_ptr),
+                                                   C.c_void_p(d_overflow_ptr) if d_overflow_ptr else None,
+                                                   C.c_void_p(stream) if stream else None))
 
     def capsule_cast_device(self, d_q_ptr, n, mode, d_out_ptr, stream=None):
         _check(lib().cq_capsule_cast_device(self._h, C.c_void_p(d_q_ptr), n, mode, C.c_void_p(d_out_ptr),

@@ -117,13 +117,12 @@ class CollisionQuery {
     }
     std::vector<CapsuleOverlapHit> capsuleOverlapAll(Float3 from, float radius, float halfHeight, int maxHits = 8,
                                                      uint32_t mask = CQ_LAYER_ALL) {
-        if (maxHits < 1) maxHits = 1; // max(1, maxHits), CollisionQuery.swift:157
-        if (maxHits > CQ_MAX_OVERLAP_HITS) maxHits = CQ_MAX_OVERLAP_HITS;
+        if (maxHits < 1) maxHits = 1; // max(1, maxHits), CollisionQuery.swift:157; any larger value is honoured
         cq_capsule c = {{from.x, from.y, from.z}, radius, halfHeight, mask};
-        cq_overlap_hit h[CQ_MAX_OVERLAP_HITS];
+        std::vector<cq_overlap_hit> h((size_t)maxHits);
         int32_t count = 0;
         std::vector<CapsuleOverlapHit> out;
-        if (cq_capsule_overlap_all_batch(w_, &c, 1, maxHits, h, &count, nullptr) != CQ_OK) return out;
+        if (cq_capsule_overlap_all_batch(w_, &c, 1, maxHits, h.data(), &count, nullptr) != CQ_OK) return out;
         for (int i = 0; i < count; i++) out.push_back(ov(h[i]));
         return out;
     }

@@ -876,14 +876,19 @@ int cq_capsule_overlap_device_ex(cq_world *w, const cq_capsule *d_q, int32_t n, 
 int cq_capsule_overlap_device(cq_world *w, const cq_capsule *d_q, int32_t n, cq_overlap_hit *d_out, void *stream) {
     return cq_capsule_overlap_device_ex(w, d_q, n, d_out, nullptr, stream);
 }
+// n * max_hits records must be addressable before any CUDA call is made for them
+static int check_overlap_all_size(int32_t n, int32_t max_hits) {
+    if (n > 0 && (size_t)max_hits > SIZE_MAX / sizeof(cq_overlap_hit) / (size_t)n) {
+        set_error("capsule overlap-all: %d queries x max_hits %d records overflow size_t", n, max_hits);
+        return CQ_ERR_INVALID;
+    }
+    return CQ_OK;
+}
 int cq_capsule_overlap_all_device(cq_world *w, const cq_capsule *d_q, int32_t n, int32_t max_hits, cq_overlap_hit *d_out,
                                   int32_t *d_counts, uint8_t *d_overflow, void *stream) {
     if (!w || n < 0 || (n > 0 && (!d_q || !d_out || !d_counts))) return CQ_ERR_INVALID;
     if (max_hits < 1) max_hits = 1; // max(1, maxHits), CollisionQuery.swift:157
-    if (max_hits > CQ_MAX_OVERLAP_HITS) {
-        set_error("max_hits %d > %d", max_hits, CQ_MAX_OVERLAP_HITS);
-        return CQ_ERR_INVALID;
-    }
+    CQ_TRY(check_overlap_all_size(n, max_hits));
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
     return cap.result(launch_overlap_all(w, d_q, n, max_hits, d_out, d_counts, d_overflow, st));
@@ -950,25 +955,28 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
                                  int32_t *counts, uint8_t *overflow) {
     if (!w || n < 0 || (n > 0 && (!q || !out || !counts))) return CQ_ERR_INVALID;
     if (max_hits < 1) max_hits = 1;
-    if (max_hits > CQ_MAX_OVERLAP_HITS) {
-        set_error("max_hits %d > %d", max_hits, CQ_MAX_OVERLAP_HITS);
-        return CQ_ERR_INVALID;
-    }
+    CQ_TRY(check_overlap_all_size(n, max_hits));
     if (n == 0) return CQ_OK;
     CQ_CUDA(cudaSetDevice(w->device));
     CQ_NO_CAPTURE(w->stream, "cq_capsule_overlap_all_batch");
     CQ_CUDA(cudaStreamSynchronize(w->stream));
     cudaStream_t st = w->stream;
+    // queries per chunk: the records of one chunk fit CQ_OVERLAP_ALL_CHUNK_BYTES (a query larger than that is a chunk)
+    const size_t perQuery = sizeof(cq_overlap_hit) * (size_t)max_hits;
+    const int chunk = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, CQ_OVERLAP_ALL_CHUNK_BYTES / perQuery));
     int r;
     if ((r = ensure_scratch(w->in, sizeof(cq_capsule) * (size_t)n)) != CQ_OK) return r;
-    if ((r = ensure_scratch(w->out, sizeof(cq_overlap_hit) * (size_t)n * max_hits)) != CQ_OK) return r;
+    if ((r = ensure_scratch(w->out, perQuery * (size_t)chunk)) != CQ_OK) return r;
     if ((r = ensure_scratch(w->aux, sizeof(int32_t) * (size_t)n)) != CQ_OK) return r;
     if ((r = ensure_scratch(w->aux2, (size_t)n)) != CQ_OK) return r;
     CQ_CUDA(cudaMemcpyAsync(w->in.ptr, q, sizeof(cq_capsule) * (size_t)n, cudaMemcpyHostToDevice, st));
-    r = launch_overlap_all(w, (const cq_capsule *)w->in.ptr, n, max_hits, (cq_overlap_hit *)w->out.ptr, (int32_t *)w->aux.ptr,
-                           (uint8_t *)w->aux2.ptr, st);
-    if (r != CQ_OK) return r;
-    CQ_CUDA(cudaMemcpyAsync(out, w->out.ptr, sizeof(cq_overlap_hit) * (size_t)n * max_hits, cudaMemcpyDeviceToHost, st));
+    for (int lo = 0; lo < n; lo += chunk) { // (stream order: a chunk's records are copied out before the next overwrites them)
+        const int cnt = std::min(chunk, n - lo);
+        r = launch_overlap_all(w, (const cq_capsule *)w->in.ptr + lo, cnt, max_hits, (cq_overlap_hit *)w->out.ptr,
+                               (int32_t *)w->aux.ptr + lo, (uint8_t *)w->aux2.ptr + lo, st);
+        if (r != CQ_OK) return r;
+        CQ_CUDA(cudaMemcpyAsync(out + (size_t)lo * max_hits, w->out.ptr, perQuery * (size_t)cnt, cudaMemcpyDeviceToHost, st));
+    }
     CQ_CUDA(cudaMemcpyAsync(counts, w->aux.ptr, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
     if (overflow) CQ_CUDA(cudaMemcpyAsync(overflow, w->aux2.ptr, (size_t)n, cudaMemcpyDeviceToHost, st));
     CQ_CUDA(cudaStreamSynchronize(st));

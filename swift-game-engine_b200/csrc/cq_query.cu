@@ -1,5 +1,5 @@
 // cq_query.cu — batched query kernels: raycast, capsule cast (3 modes), capsule overlap (deepest),
-// capsule overlap-all (8 deepest).  One thread per query; the BVH walk and the narrow phase live in
+// capsule overlap-all (max_hits hits).  One thread per query; the BVH walk and the narrow phase live in
 // cq_world.cuh / cq_math.cuh.  Replaces the per-call CPU entry points of CollisionQuery.swift:85-159.
 #include "cq_pool.cuh"
 #include "cq_internal.h"
@@ -479,6 +479,183 @@ __global__ void __launch_bounds__(Q_THREADS, 4) k_capsule_overlap_pool(WorldView
     pool_flush_counters(ctr, gctr, COUNT);
 }
 
+// ---------------------------------------------------------------- capsule overlap-all, wide path (max_hits > CQ_OVL_WIDE_ABOVE)
+// OvlTop keeps 8 winners per owner in shared memory and the owner emits them serially; neither scales to a large maxHits.
+// The wide path keeps each query's winners in its own output slots and emits them in two more launches:
+//   k_capsule_overlap_wide  the pair pool; an owner's kept list is a binary heap in global memory, one OvlEntry at the head
+//                           of each of the query's cq_overlap_hit slots, with the WORST kept entry at the root, so that a
+//                           commit costs O(log maxHits).  Per owner, shared memory holds only OvlHead.  At completion the
+//                           owner writes counts / overflow and nothing else;
+//   k_overlap_wide_sort     one thread per query: heapsort of the kept entries in place (best first);
+//   k_overlap_wide_emit     one thread per slot: entry k -> full record k (the arithmetic of overlap_record), nil past count.
+// Both orders keep the same entries as OverlapTopK: the smallest visiting ranks (reference order), or the deepest with
+// exact ties to the smaller rank (canonical order); ranks are unique, so the kept set and its sorted order are too.
+#ifndef CQ_OVL_WIDE_ABOVE
+#define CQ_OVL_WIDE_ABOVE CQ_MAX_OVERLAP_HITS /* max_hits above this runs the wide path (0: every call, for A/B builds) */
+#endif
+
+struct OvlEntry { // 16 B at the head of a 44 B output slot until the emit pass overwrites it
+    float depth;
+    int rank, gid;
+    uint32_t enc;
+};
+struct OvlHead { // per owner: the heap's size, overlaps committed, the query, and the root (worst kept) entry's key
+    int count, total, cur, worstRank;
+    float worstDepth;
+};
+
+// a sits nearer the root than b: larger rank (reference order), or shallower with exact ties to the larger rank
+__device__ __forceinline__ bool ovl_worse(bool byRank, float da, int ra, float db, int rb) {
+    return byRank ? ra > rb : (da < db || (da == db && ra > rb));
+}
+__device__ __forceinline__ OvlEntry *ovl_slot(cq_overlap_hit *out, size_t base, unsigned i) {
+    return reinterpret_cast<OvlEntry *>(out + base + i);
+}
+__device__ __forceinline__ void ovl_put(cq_overlap_hit *out, size_t base, unsigned i, const OvlEntry &e) {
+    OvlEntry *p = ovl_slot(out, base, i); // (4-byte aligned only: four word stores)
+    p->depth = e.depth, p->rank = e.rank, p->gid = e.gid, p->enc = e.enc;
+}
+__device__ __forceinline__ OvlEntry ovl_get(const cq_overlap_hit *out, size_t base, unsigned i) {
+    const OvlEntry *p = ovl_slot(const_cast<cq_overlap_hit *>(out), base, i);
+    return OvlEntry{p->depth, p->rank, p->gid, p->enc};
+}
+// sift e down from the root of the heap out[base .. base + n); returns the new root
+__device__ __forceinline__ OvlEntry ovl_sift_down(cq_overlap_hit *out, size_t base, unsigned n, const OvlEntry &e, bool byRank) {
+    unsigned i = 0;
+    OvlEntry root = e;
+#pragma unroll 1
+    for (;;) {
+        const unsigned l = 2u * i + 1u; // (i < n / 2 < 2^30: no wrap)
+        if (l >= n) break;
+        unsigned c = l;
+        OvlEntry C = ovl_get(out, base, l);
+        if (l + 1u < n) {
+            const OvlEntry R = ovl_get(out, base, l + 1u);
+            if (ovl_worse(byRank, R.depth, R.rank, C.depth, C.rank)) c = l + 1u, C = R;
+        }
+        if (!ovl_worse(byRank, C.depth, C.rank, e.depth, e.rank)) break;
+        ovl_put(out, base, i, C);
+        if (i == 0) root = C;
+        i = c;
+    }
+    ovl_put(out, base, i, e);
+    return root;
+}
+
+// Commit of one overlap, run by the executor lane in the owner's pool_commit round.  Out of line for the same reason as
+// overlap_top2_commit: it sits in the steady-state loop.
+static __device__ __noinline__ void overlap_heap_commit(OvlHead &h, cq_overlap_hit *out, int cap, bool byRank, float depth, int gid,
+                                                        int rk, uint32_t enc) {
+    h.total++;
+    const OvlEntry e{depth, rk, gid, enc};
+    const size_t base = (size_t)h.cur * cap;
+    if (h.count < cap) { // not full: sift up
+        unsigned i = (unsigned)h.count;
+#pragma unroll 1
+        while (i > 0) {
+            const unsigned p = (i - 1u) >> 1;
+            const OvlEntry P = ovl_get(out, base, p);
+            if (!ovl_worse(byRank, e.depth, e.rank, P.depth, P.rank)) break;
+            ovl_put(out, base, i, P);
+            i = p;
+        }
+        ovl_put(out, base, i, e);
+        h.count++;
+        if (i == 0) h.worstDepth = depth, h.worstRank = rk;
+    } else if (ovl_worse(byRank, h.worstDepth, h.worstRank, depth, rk)) { // full: replaces the worst kept entry
+        const OvlEntry root = ovl_sift_down(out, base, (unsigned)cap, e, byRank);
+        h.worstDepth = root.depth, h.worstRank = root.rank;
+    }
+}
+
+struct OverlapHeapK {
+    OvlHead *heads; // the warp's 32 owners
+    cq_overlap_hit *out;
+    int cap;
+    bool byRank;
+    // OverlapTopK::cannot_matter: more than maxHits overlaps on record and this triangle visited after every kept one
+    __device__ __forceinline__ bool cannot_matter(QShared &, int rk, uint32_t enc) const {
+        if (!byRank) return false;
+        const OvlHead &h = heads[enc >> 27];
+        return h.total > cap && rk > h.worstRank;
+    }
+    __device__ __forceinline__ void operator()(QShared &, float depth, int gid, int rk, uint32_t enc, f3) const {
+        overlap_heap_commit(heads[enc >> 27], out, cap, byRank, depth, gid, rk, enc);
+    }
+};
+
+template <bool COUNT, bool STAGED>
+__global__ void __launch_bounds__(Q_THREADS, 4) k_capsule_overlap_wide(WorldView W, const cq_capsule *__restrict__ qs, int n,
+                                                                       int maxHits, cq_overlap_hit *out, int32_t *__restrict__ counts,
+                                                                       uint8_t *__restrict__ overflow, int ownersPerWarp,
+                                                                       uint2 *nodeScratch, int *workCounter,
+                                                                       unsigned long long *gctr) {
+    __shared__ QShared qsAll[Q_THREADS];
+    __shared__ OvlHead heads[Q_THREADS];
+    __shared__ uint32_t words[CQ_POOL_WORDS * CAST_WARPS];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    WarpPool wp;
+    pool_bind(wp, qsAll, words, nodeScratch, warp, CAST_WARPS, W.rank, W.status);
+    OvlHead &head = heads[threadIdx.x];
+    Counters ctr = {0, 0, 0, 0};
+    int cur = -1;
+    pool_run<COUNT, STAGED, 8, true>(W, wp, lane, ownersPerWarp, ctr, [&](QShared &mine, Counters &ct) {
+        if (cur >= 0) { // the records are the emit pass's
+            counts[cur] = head.count;
+            if (overflow) overflow[cur] = head.total > maxHits ? 1 : 0;
+        }
+        cur = atomicAdd(workCounter, 1);
+        if (cur >= n) {
+            cur = -1;
+            return false;
+        }
+        cq_capsule c = qs[cur];
+        head.count = 0, head.total = 0, head.cur = cur, head.worstRank = 0, head.worstDepth = 0.0f;
+        pool_post_overlap<COUNT>(W, wp, lane, mine, load3(c.from), c.radius, c.half_height, c.mask, ct);
+        return true;
+    }, OverlapHeapK{heads + warp * 32, out, maxHits, W.rank != nullptr});
+    pool_flush_counters(ctr, gctr, COUNT);
+}
+
+// heapsort in place: the worst entry goes to the end first, so the slots end best first — ascending rank (reference
+// order), deepest first with ties to the smaller rank (canonical order)
+__global__ void __launch_bounds__(Q_THREADS) k_overlap_wide_sort(int n, int maxHits, bool byRank, cq_overlap_hit *out,
+                                                                 const int32_t *__restrict__ counts) {
+    for (size_t q = blockIdx.x * (size_t)blockDim.x + threadIdx.x; q < (size_t)n; q += (size_t)gridDim.x * blockDim.x) {
+        const size_t base = q * maxHits;
+#pragma unroll 1
+        for (unsigned end = (unsigned)counts[q]; end > 1u; end--) {
+            const OvlEntry root = ovl_get(out, base, 0), last = ovl_get(out, base, end - 1u);
+            ovl_sift_down(out, base, end - 1u, last, byRank);
+            ovl_put(out, base, end - 1u, root);
+        }
+    }
+}
+
+// slot i = query i / maxHits, entry i % maxHits: reads its entry and writes its record from the same thread
+template <bool COUNT>
+__global__ void __launch_bounds__(Q_THREADS) k_overlap_wide_emit(WorldView W, const cq_capsule *__restrict__ qs, int n,
+                                                                 int maxHits, cq_overlap_hit *out,
+                                                                 const int32_t *__restrict__ counts, unsigned long long *gctr) {
+    Counters ctr = {0, 0, 0, 0};
+    const size_t slots = (size_t)n * maxHits;
+    for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < slots; i += (size_t)gridDim.x * blockDim.x) {
+        const size_t q = i / (size_t)maxHits;
+        const int k = (int)(i - q * (size_t)maxHits);
+        cq_overlap_hit h;
+        if (k < counts[q]) {
+            const OvlEntry e = ovl_get(out, i, 0);
+            const cq_capsule c = qs[q];
+            if (COUNT) ctr.evals++;
+            overlap_record(W, e.enc, e.gid, load3(c.from), c.radius, c.half_height, h);
+        } else {
+            write_overlap_nil(h);
+        }
+        out[i] = h;
+    }
+    pool_flush_counters(ctr, gctr, COUNT);
+}
+
 // ---------------------------------------------------------------- launchers
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 
@@ -555,8 +732,41 @@ int launch_overlap(cq_world *w, const cq_capsule *d_q, int n, cq_overlap_hit *d_
     return launch_overlap_pool<false>(w, d_q, n, 1, d_out, nullptr, d_flags, st);
 }
 
+// the wide path: the pool kernel, the sort and the emit pass, always three launches
+static int launch_overlap_wide(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
+                               uint8_t *d_overflow, cudaStream_t st) {
+    if (n <= 0) return CQ_OK;
+    CQ_TRY(await_trees(w, st));
+    const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
+    using Kernel = void (*)(WorldView, const cq_capsule *, int, int, cq_overlap_hit *, int32_t *, uint8_t *, int, uint2 *, int *,
+                            unsigned long long *);
+    static const Kernel kernels[4] = {k_capsule_overlap_wide<false, false>, k_capsule_overlap_wide<true, false>,
+                                      k_capsule_overlap_wide<false, true>, k_capsule_overlap_wide<true, true>};
+    const Kernel kernel = kernels[ci];
+    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
+    if (!resident) return CQ_ERR_CUDA;
+    int blocks = std::min(cdiv(n, 4), resident);
+    const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
+    int *work = next_work_counter(w, st);
+    if (!work) return CQ_ERR_CUDA;
+    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
+    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
+    kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, opw, ns, work, w->dCounters);
+    // grid-stride passes: a few waves of 128-thread blocks whatever n and maxHits
+    const long long wave = (long long)w->numSms * 16;
+    const int sortBlocks = (int)std::min<long long>(cdiv(n, Q_THREADS), wave);
+    k_overlap_wide_sort<<<sortBlocks, Q_THREADS, 0, st>>>(n, maxHits, w->view.rank != nullptr, d_out, d_counts);
+    const long long slots = (long long)n * maxHits;
+    const int emitBlocks = (int)std::min<long long>((slots + Q_THREADS - 1) / Q_THREADS, wave);
+    if (w->counting) k_overlap_wide_emit<true><<<emitBlocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, w->dCounters);
+    else k_overlap_wide_emit<false><<<emitBlocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, w->dCounters);
+    w->launches += 3; // the number cq.h documents
+    return finish_launch(w, st, "k_capsule_overlap_wide");
+}
+
 int launch_overlap_all(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                        uint8_t *d_overflow, cudaStream_t st) {
+    if (maxHits > CQ_OVL_WIDE_ABOVE) return launch_overlap_wide(w, d_q, n, maxHits, d_out, d_counts, d_overflow, st);
     return launch_overlap_pool<true>(w, d_q, n, maxHits, d_out, d_counts, d_overflow, st);
 }
 

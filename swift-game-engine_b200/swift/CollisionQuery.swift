@@ -94,7 +94,7 @@ public final class CollisionQuery {
 
     public func capsuleOverlapAll(from: SIMD3<Float>, radius: Float, halfHeight: Float, maxHits: Int = 8,
                                   mask: UInt32 = CollisionLayer.all) -> [CapsuleOverlapHit] {
-        let cap = min(max(1, maxHits), Int(CQ_MAX_OVERLAP_HITS))
+        let cap = max(1, maxHits) // CollisionQuery.swift:157; any larger maxHits is honoured
         var c = cq_capsule(from: (from.x, from.y, from.z), radius: radius, half_height: halfHeight, mask: mask)
         var hits = [cq_overlap_hit](repeating: cq_overlap_hit(), count: cap)
         var count: Int32 = 0
