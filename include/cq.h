@@ -326,14 +326,17 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  * ordered against them by events instead (see its ordering contract).
  *
  * CUDA-graph capture: while `stream` is being captured (cudaStreamBeginCapture, torch.cuda.graph, ...), the *_device
- * query twins, cq_move_and_slide_device(_ex), cq_world_update_transforms_device and cq_agent_separation_device_async
- * enqueue kernels, memsets, copies and (agent separation) conditional WHILE nodes only: they neither wait on nor record
- * nor create world events.  So:
+ * query twins, cq_move_and_slide_device(_ex) and cq_move_and_slide_device_platforms, cq_world_update_transforms_device,
+ * cq_world_platforms_device and cq_agent_separation_device_async enqueue kernels, memsets, copies and (agent
+ * separation) conditional WHILE nodes only: they neither wait on nor record nor create world events.  So:
  *  - a graph is ordered only by the stream it is launched on; the caller orders its replays against other work on the
  *    world, as for a synchronous call (e.g. synchronise before an uncaptured call on another stream);
  *  - kernel_launches counts the launches once, at capture; replays are not counted;
- *  - scalar arguments (n, mode, params, platforms, flags, the environment's CQ_REFIT_FULL) are recorded with the graph;
- *    device buffers are read at replay, so new models written into the same buffer move the parts of each replay;
+ *  - scalar arguments (n, mode, params, flags, n_platforms, the environment's CQ_REFIT_FULL) are recorded with the graph,
+ *    and so are the cq_platform records of the host-array calls (cq_move_and_slide_device_ex): a replay carries
+ *    characters with the records of the capture.  Device buffers are read at replay, so new models written into the
+ *    same buffer move the parts of each replay, and cq_world_platforms_device + cq_move_and_slide_device_platforms
+ *    give every replay the records of its own frame;
  *  - a call that would grow scratch, allocate, synchronise or create an event while capturing returns CQ_ERR_INVALID
  *    ("make one uncaptured call of this size first") and leaves the capture valid; so does CQ_MAS_AGENTS when its grid
  *    needs more scratch than an uncaptured call gave it;
@@ -436,6 +439,42 @@ int cq_move_and_slide_device_ex(cq_world *w, cq_character_state *d_inout, int32_
                                 const cq_controller_params *params, float dt, const float gravity[3],
                                 uint32_t flags, const cq_platform *platforms /* HOST pointer */,
                                 int32_t n_platforms, void *stream);
+
+/* Kinematic platform records from the world, on the device: d_out[i] (a cq_platform, DEVICE pointer, n records) gets
+ * the world AABB of entity d_entity_ids[i] (device, n ids) and the motion d_deltas[3i..3i+2] (device, n*3 floats,
+ * positionF - prevPositionF, which the caller owns as in the reference).  Written in stream order on `stream` (NULL = the
+ * world's stream), without synchronising, allocating or touching host memory, so a graph can rebuild the records every
+ * replay and hand them to cq_move_and_slide_device_platforms.
+ *
+ * aabb_min / aabb_max are the min / max over the world-space vertices of every part with a matching entity_id, in both
+ * sets, as left by every update queued on the world before this call: meshWorldAABB (Systems.swift:627-642) of the
+ * current model, computed with the same float32 operations as the transform update.  One difference from
+ * meshWorldAABB: parts without triangles do not contribute (updates skip them, CollisionQuery.swift:427, so their world
+ * vertices are not current); an id whose parts all lack triangles gets the empty box (min = +inf, max = -inf), which
+ * overlaps no capsule, so its record is inert.  An unknown id gets the empty box and a zero delta, inert too.  Records
+ * are independent: *d_status (a device int32, may be NULL) receives the number of unknown ids, 0 on success, in stream
+ * order, and every known id still gets its record.  NULL world, n < 0, or a NULL array with n > 0 return CQ_ERR_INVALID
+ * before any CUDA call; n == 0 returns CQ_OK and queues nothing.
+ *
+ * Ordering is that of every launcher: the call sees every update queued before it on any stream, and the next
+ * asynchronous update waits until it has read the vertices.  Launches: 1 whatever n is, one CTA per id (at most one
+ * resident wave, striding over the ids); the cost grows with the vertex count of the named entities.  May be recorded
+ * into a CUDA graph (see the capture contract below the *_device twins). */
+int cq_world_platforms_device(cq_world *w, const uint32_t *d_entity_ids, const float *d_deltas, int32_t n,
+                              cq_platform *d_out, int32_t *d_status, void *stream);
+
+/* Device-platform twin of cq_move_and_slide_device_ex: the same step, with results equal to it byte for byte for the
+ * same records (CQ_MAS_AGENTS included), except that d_platforms is a DEVICE pointer to n_platforms records that the
+ * kernels read when they execute.  A graph that recorded this call therefore uses whatever the buffer holds at replay
+ * (e.g. what cq_world_platforms_device wrote earlier in the same graph); n_platforms is a scalar recorded with the
+ * graph, like n.  Any n_platforms >= 0 is accepted (the host-array calls take at most 64, because their records travel
+ * in the kernel arguments); the cost is linear in n_platforms per character, as in the reference.  n_platforms < 0, or
+ * a NULL d_platforms with n_platforms > 0, return CQ_ERR_INVALID before any CUDA call, as do the checks of the _ex
+ * call.  Launches: the same as cq_move_and_slide_device_ex. */
+int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout, int32_t n,
+                                       const cq_controller_params *params, float dt, const float gravity[3],
+                                       uint32_t flags, const cq_platform *d_platforms, int32_t n_platforms,
+                                       void *stream);
 
 /* ---- resident crowd ------------------------------------------------------
  * The full-record calls above move 2 x 168 bytes per character per step across PCIe, which bounds them near 230 M

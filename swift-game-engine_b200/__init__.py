@@ -131,7 +131,8 @@ class Counters(C.Structure):
 
 EXPORTS = [
     "cq_world_create", "cq_world_create_ex", "cq_world_options_default", "cq_world_destroy", "cq_world_get_info", "cq_world_update_transforms",
-    "cq_world_update_transforms_async", "cq_world_update_transforms_device", "cq_world_read_soup", "cq_world_read_models",
+    "cq_world_update_transforms_async", "cq_world_update_transforms_device", "cq_world_platforms_device", "cq_world_read_soup",
+    "cq_world_read_models",
     "cq_world_triangle_material", "cq_static_mesh_load", "cq_static_mesh_free", "cq_static_mesh_part_count",
     "cq_static_mesh_part_name", "cq_static_mesh_part_transform", "cq_static_mesh_hull_count",
     "cq_static_mesh_geometry", "cq_raycast_batch", "cq_capsule_cast_batch", "cq_capsule_overlap_batch",
@@ -139,7 +140,7 @@ EXPORTS = [
     "cq_raycast_device_ex", "cq_capsule_cast_device_ex", "cq_capsule_overlap_device_ex", "cq_raycast_device", "cq_capsule_cast_device", "cq_capsule_overlap_device",
     "cq_capsule_overlap_all_device", "cq_controller_params_default", "cq_character_state_init",
     "cq_move_and_slide_batch", "cq_move_and_slide_device", "cq_move_and_slide_batch_ex",
-    "cq_move_and_slide_device_ex", "cq_agent_separation_batch", "cq_agent_separation_device",
+    "cq_move_and_slide_device_ex", "cq_move_and_slide_device_platforms", "cq_agent_separation_batch", "cq_agent_separation_device",
     "cq_agent_separation_device_async",
     "cq_world_set_counting", "cq_world_read_counters",
     "cq_crowd_create", "cq_crowd_destroy", "cq_crowd_size", "cq_crowd_step", "cq_crowd_read", "cq_crowd_write",
@@ -201,6 +202,7 @@ def lib():
         L.cq_world_update_transforms.argtypes = [vp, vp, vp, i32]
         L.cq_world_update_transforms_async.argtypes = [vp, vp, vp, i32, vp]
         L.cq_world_update_transforms_device.argtypes = [vp, vp, vp, i32, vp, vp]
+        L.cq_world_platforms_device.argtypes = [vp, vp, vp, i32, vp, vp, vp]
         L.cq_world_read_soup.argtypes = [vp, i32, vp, vp, vp, vp, vp]
         L.cq_world_read_models.argtypes = [vp, vp]
         L.cq_world_triangle_material.argtypes = [vp, i32, C.POINTER(Material)]
@@ -227,6 +229,7 @@ def lib():
         L.cq_move_and_slide_device.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp]
         L.cq_move_and_slide_batch_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32]
         L.cq_move_and_slide_device_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32, vp]
+        L.cq_move_and_slide_device_platforms.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32, vp]
         L.cq_agent_separation_batch.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32]
         L.cq_agent_separation_device.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp]
         L.cq_agent_separation_device_async.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp, vp]
@@ -460,6 +463,15 @@ class CollisionQuery:
                                                        C.c_void_p(d_status_ptr) if d_status_ptr else None,
                                                        C.c_void_p(stream) if stream else None))
 
+    def platforms_device(self, d_ids_ptr, d_deltas_ptr, n, d_out_ptr, d_status_ptr=None, stream=None):
+        """cq_world_platforms_device: n PLATFORM records (d_out_ptr, device) of the entities d_ids_ptr (n uint32, device)
+        moving by d_deltas_ptr (n*3 float32, device): the world AABB of each entity's vertices as the updates queued before
+        left them, and its delta.  Queued on `stream` without synchronising, so it can be captured in a CUDA graph.
+        Unknown ids get inert records (empty box, zero delta); d_status_ptr (a device int32, optional) receives their count."""
+        _check(lib().cq_world_platforms_device(self._h, C.c_void_p(d_ids_ptr), C.c_void_p(d_deltas_ptr), int(n),
+                                               C.c_void_p(d_out_ptr), C.c_void_p(d_status_ptr) if d_status_ptr else None,
+                                               C.c_void_p(stream) if stream else None))
+
     # raycast(origin:direction:maxDistance:mask:) (CollisionQuery.swift:85)
     def raycast(self, rays, with_flags=False):
         """with_flags: also return the per-query HIT_* flag bytes (cq_raycast_batch_ex)."""
@@ -552,6 +564,16 @@ class CollisionQuery:
         g = np.asarray(gravity, np.float32)
         _check(lib().cq_move_and_slide_device(self._h, C.c_void_p(d_states_ptr), n, _ptr(params), C.c_float(dt),
                                               _ptr(g), flags, C.c_void_p(stream) if stream else None))
+
+    def move_and_slide_device_platforms(self, d_states_ptr, n, params, d_platforms_ptr, n_platforms, dt=1.0 / 60.0,
+                                        gravity=(0.0, -98.0, 0.0), flags=MAS_APPLY_GRAVITY, stream=None):
+        """cq_move_and_slide_device_platforms: move_and_slide_device with n_platforms PLATFORM records read from device
+        memory (d_platforms_ptr) when the kernels run, so a replayed graph uses the records of its frame; any count."""
+        params = np.ascontiguousarray(params, PARAMS)
+        g = np.asarray(gravity, np.float32)
+        _check(lib().cq_move_and_slide_device_platforms(self._h, C.c_void_p(d_states_ptr), int(n), _ptr(params), C.c_float(dt),
+                                                        _ptr(g), flags, C.c_void_p(d_platforms_ptr) if d_platforms_ptr else None,
+                                                        int(n_platforms), C.c_void_p(stream) if stream else None))
 
     def capsule_overlap_all_device(self, d_q_ptr, n, max_hits, d_out_ptr, d_counts_ptr, d_overflow_ptr=None, stream=None):
         """cq_capsule_overlap_all_device: n CAPSULE records in, n * max_hits OVERLAP_HIT records, n int32 counts and

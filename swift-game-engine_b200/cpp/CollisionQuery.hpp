@@ -26,6 +26,12 @@ struct SurfaceMaterial { // Components.swift:704-716
     bool flattenGround = false;
 };
 
+// kinematic platform records in device memory (e.g. written by CollisionQuery::platformsDevice), for the device moveAndSlide
+struct DevicePlatforms {
+    const cq_platform *records;
+    int32_t count;
+};
+
 struct RaycastHit { // CollisionQuery.swift:28-34
     float distance;
     Float3 position, normal;
@@ -79,6 +85,20 @@ class CollisionQuery {
     bool updateTransformsDevice(const uint32_t *dEntities, const float *dModels16, int32_t n, int32_t *dStatus = nullptr,
                                 void *stream = nullptr) {
         return cq_world_update_transforms_device(w_, dEntities, dModels16, n, dStatus, stream) == CQ_OK;
+    }
+    // kinematic platform records on the device: dOut[i] = world AABB of entity dEntities[i] as the queued updates leave it
+    // + dDeltas[3i..3i+2]; unknown ids get inert records and are counted into *dStatus (device int32, may be null)
+    bool platformsDevice(const uint32_t *dEntities, const float *dDeltas, int32_t n, cq_platform *dOut, int32_t *dStatus = nullptr,
+                         void *stream = nullptr) {
+        return cq_world_platforms_device(w_, dEntities, dDeltas, n, dOut, dStatus, stream) == CQ_OK;
+    }
+    // move-and-slide of resident records with platforms read from device memory when the kernels run (capturable: each
+    // replay uses the records the buffer holds then); any platform count
+    bool moveAndSlide(cq_character_state *dInout, int32_t n, const cq_controller_params &p, float dt, const float gravity[3],
+                      DevicePlatforms platforms, bool agents, bool applyGravity = true, void *stream = nullptr) {
+        uint32_t flags = (applyGravity ? CQ_MAS_APPLY_GRAVITY : 0u) | (agents ? CQ_MAS_AGENTS : 0u);
+        return cq_move_and_slide_device_platforms(w_, dInout, n, &p, dt, gravity, flags, platforms.records, platforms.count,
+                                                  stream) == CQ_OK;
     }
     // agent separation of resident records, queued on `stream` without synchronising (capturable in a CUDA graph);
     // *dStatus (device int32, optional) receives CQ_SEP_STATUS_* in stream order

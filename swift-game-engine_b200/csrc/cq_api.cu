@@ -746,6 +746,16 @@ int cq_world_update_transforms_device(cq_world *w, const uint32_t *d_entity_ids,
     return refit_done(w, st);
 }
 
+int cq_world_platforms_device(cq_world *w, const uint32_t *d_entity_ids, const float *d_deltas, int32_t n, cq_platform *d_out,
+                              int32_t *d_status, void *stream) {
+    if (!w || n < 0 || (n > 0 && (!d_entity_ids || !d_deltas || !d_out))) return CQ_ERR_INVALID;
+    if (n == 0) return CQ_OK;
+    CQ_CUDA(cudaSetDevice(w->device));
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_platform_records(w, d_entity_ids, d_deltas, n, d_out, d_status, st));
+}
+
 int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, uint32_t *indices, float *tri_aabbs,
                        uint32_t *tri_layers, int32_t *tri_parts) {
     if (!w || which < 0 || which > 1) return CQ_ERR_INVALID;
@@ -899,7 +909,20 @@ int cq_move_and_slide_device_ex(cq_world *w, cq_character_state *d_inout, int32_
     if (!w || n < 0 || !params || !gravity || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, n_platforms, st));
+    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, nullptr, n_platforms, st));
+}
+int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
+                                       float dt, const float gravity[3], uint32_t flags, const cq_platform *d_platforms,
+                                       int32_t n_platforms, void *stream) {
+    if (!w || n < 0 || !params || !gravity || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
+    if (n_platforms < 0 || (n_platforms > 0 && !d_platforms)) {
+        set_error("cq_move_and_slide_device_platforms: %d platforms at %p", n_platforms, (const void *)d_platforms);
+        return CQ_ERR_INVALID;
+    }
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, nullptr,
+                                            n_platforms > 0 ? d_platforms : nullptr, n_platforms, st));
 }
 int cq_move_and_slide_device(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params, float dt,
                              const float gravity[3], uint32_t flags, void *stream) {
@@ -996,7 +1019,7 @@ int cq_move_and_slide_batch_ex(cq_world *w, cq_character_state *inout, int32_t n
     return run_batch(w, inout, sizeof(cq_character_state), inout, sizeof(cq_character_state), n,
                      [&](void *di, void *, int cnt, int, cudaStream_t st) {
                          return launch_move_and_slide(w, (cq_character_state *)di, cnt, *params, dt, gravity, flags, platforms,
-                                                      n_platforms, st);
+                                                      nullptr, n_platforms, st);
                      },
                      /*inPlace=*/true, &w->hintMas, /*singleChunk=*/(flags & CQ_MAS_AGENTS) != 0);
 }

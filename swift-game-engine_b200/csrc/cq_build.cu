@@ -1817,4 +1817,77 @@ int build_moved_device(cq_world *w, const uint32_t *dIds, const float *dModels, 
     return check_cuda(cudaGetLastError(), "transform table");
 }
 
+// ---------------------------------------------------------------- device path: kinematic platform records
+// (cq_world_platforms_device) meshWorldAABB (Systems.swift:627-642) of each named entity from the world-space vertices the
+// last update left, found through the same entity index.  One CTA per id (grid-stride over the ids): each thread takes the
+// min / max over a stride of the vertices of the entity's parts (both sets), then a warp and a block reduction.  Only parts
+// with triangles are in the index (updates skip the others, so their world vertices are not current): an id whose parts
+// all lack triangles gets the empty box (+inf, -inf), which no capsule overlaps; an unknown id gets the empty box and a
+// zero delta.  CTA 0 also counts the unknown ids into *status, so the call needs no scratch and one launch.
+#define PLAT_THREADS 256
+__global__ void __launch_bounds__(PLAT_THREADS) k_platform_records(const uint32_t *__restrict__ in, const float *__restrict__ deltas,
+                                                                   int n, const uint32_t *__restrict__ ids, int nIds,
+                                                                   const int32_t *__restrict__ off, const EntityEntry *__restrict__ entries,
+                                                                   const float4 *__restrict__ world0, const float4 *__restrict__ world1,
+                                                                   cq_platform *__restrict__ out, int32_t *status) {
+    __shared__ float part[PLAT_THREADS / 32][6];
+    __shared__ int unknown[PLAT_THREADS / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (int i = blockIdx.x; i < n; i += gridDim.x) {
+        const int e = find_entity(ids, nIds, in[i]);
+        float b[6] = {INFINITY, INFINITY, INFINITY, -INFINITY, -INFINITY, -INFINITY};
+        if (e >= 0)
+            for (int k = off[e]; k < off[e + 1]; k++) {
+                const EntityEntry x = entries[k];
+                const float4 *wp = (x.set ? world1 : world0) + x.vertLo;
+                for (int v = threadIdx.x; v < x.nVerts; v += PLAT_THREADS) {
+                    const float4 p = wp[v];
+                    b[0] = fminf(b[0], p.x), b[1] = fminf(b[1], p.y), b[2] = fminf(b[2], p.z);
+                    b[3] = fmaxf(b[3], p.x), b[4] = fmaxf(b[4], p.y), b[5] = fmaxf(b[5], p.z);
+                }
+            }
+#pragma unroll
+        for (int q = 0; q < 6; q++)
+            for (int d = 16; d > 0; d >>= 1) {
+                const float o = __shfl_xor_sync(0xffffffffu, b[q], d);
+                b[q] = q < 3 ? fminf(b[q], o) : fmaxf(b[q], o);
+            }
+        if (lane == 0)
+            for (int q = 0; q < 6; q++) part[warp][q] = b[q];
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < PLAT_THREADS / 32; w++)
+                for (int q = 0; q < 6; q++) b[q] = q < 3 ? fminf(b[q], part[w][q]) : fmaxf(b[q], part[w][q]);
+            cq_platform r;
+            for (int c = 0; c < 3; c++) {
+                r.aabb_min[c] = b[c], r.aabb_max[c] = b[3 + c];
+                r.delta[c] = e >= 0 ? deltas[3 * (size_t)i + c] : 0.0f;
+            }
+            out[i] = r;
+        }
+        __syncthreads(); // `part` is reused by the next id
+    }
+    if (status && blockIdx.x == 0) {
+        int u = 0;
+        for (int i = threadIdx.x; i < n; i += PLAT_THREADS) u += find_entity(ids, nIds, in[i]) < 0 ? 1 : 0;
+        u = __reduce_add_sync(0xffffffffu, u);
+        if (lane == 0) unknown[warp] = u;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < PLAT_THREADS / 32; w++) u += unknown[w];
+            *status = u;
+        }
+    }
+}
+
+int launch_platform_records(cq_world *w, const uint32_t *dIds, const float *dDeltas, int n, cq_platform *dOut, int32_t *dStatus,
+                            cudaStream_t st) {
+    CQ_TRY(await_trees(w, st));
+    const int grid = std::min(n, w->numSms * 8);
+    k_platform_records<<<grid, PLAT_THREADS, 0, st>>>(dIds, dDeltas, n, w->dEntityIds, w->nEntities, w->dEntityOff, w->dEntries,
+                                                      w->set[0].worldPos, w->set[1].worldPos, dOut, dStatus);
+    w->launches++;
+    return finish_launch(w, st, "k_platform_records");
+}
+
 } // namespace cq

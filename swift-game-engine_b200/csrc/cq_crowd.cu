@@ -136,7 +136,7 @@ int cq_crowd_step(cq_crowd *c, const double *velocity_in_xyz, const cq_controlle
             k_crowd_set_velocity<<<(cnt + 255) / 256, 256, 0, cs>>>(dS, c->dVelIn + 3 * (size_t)lo, cnt);
             w->launches++;
         }
-        CQ_TRY(launch_move_and_slide(w, dS, cnt, *params, dt, gravity, flags, platforms, n_platforms, cs));
+        CQ_TRY(launch_move_and_slide(w, dS, cnt, *params, dt, gravity, flags, platforms, nullptr, n_platforms, cs));
         if (pose_out) {
             k_crowd_get_pose<<<(cnt + 255) / 256, 256, 0, cs>>>(dS, c->dPose + lo, cnt);
             w->launches++;

@@ -268,6 +268,9 @@ int refit_set(cq_world *w, DeviceSet &S, const MovedPart *dTab, const RefitCount
 int refit_path(const DeviceSet &S, int moved);
 // Device path of cq_world_update_transforms_device: resolve the ids and build the table + counts on `st` (2 launches).
 int build_moved_device(cq_world *w, const uint32_t *dIds, const float *dModels, int n, int32_t *dStatus, cudaStream_t st);
+// cq_world_platforms_device: n > 0 platform records from the world-space vertices of the named entities, one launch on `st`.
+int launch_platform_records(cq_world *w, const uint32_t *dIds, const float *dDeltas, int n, cq_platform *dOut, int32_t *dStatus,
+                            cudaStream_t st);
 // a stream capture is recording `st` (cudaStreamGetCaptureInfo)
 bool stream_capturing(cudaStream_t st);
 // Calls that synchronise, allocate, create events or stage host memory: CQ_ERR_INVALID while `st` is capturing (the
@@ -301,8 +304,11 @@ int launch_overlap(cq_world *w, const cq_capsule *d_q, int n, cq_overlap_hit *d_
 int launch_overlap_all(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                        uint8_t *d_overflow, cudaStream_t st);
 // cq_mas.cu
+// Kinematic platforms come either as a host array `platforms` (at most 64, copied into the kernel arguments, so a captured
+// graph keeps them) or, when dPlatforms is non-null, as a device array the kernels read when they execute (any count).
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
-                          const float g[3], uint32_t flags, const cq_platform *platforms, int nPlatforms, cudaStream_t st);
+                          const float g[3], uint32_t flags, const cq_platform *platforms, const cq_platform *dPlatforms,
+                          int nPlatforms, cudaStream_t st);
 // cq_sep.cu
 void sep_graphs_destroy(cq_world *w);
 // Queues the whole separation on `st` without waiting for the device; the outcome goes to d_status (may be nullptr).

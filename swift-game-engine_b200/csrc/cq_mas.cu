@@ -36,7 +36,8 @@ struct MasArgs {
     float gx, gy, gz;
     uint32_t flags;
     int nPlatforms;
-    cq_platform platforms[MAS_MAX_PLATFORMS]; // kinematic platforms travel in the kernel arguments (2.3 KB at most)
+    cq_platform platforms[MAS_MAX_PLATFORMS]; // kinematic platforms travel in the kernel arguments (2.3 KB at most)...
+    const cq_platform *dPlatforms;            // ... or, when non-null, in device memory read at execution (any count)
     AgentGrid agents;                         // CQ_MAS_AGENTS: snapshot + grid of this launch
 };
 
@@ -162,7 +163,7 @@ __device__ __forceinline__ void mas_entry_motion(const cq_character_state &S, co
     }
     pos = mk3((float)S.position[0], (float)S.position[1], (float)S.position[2]);
     if (A.nPlatforms > 0) {
-        f3 platformDelta = platform_carry_delta(pos, A.p, A.platforms, A.nPlatforms);
+        f3 platformDelta = platform_carry_delta(pos, A.p, A.dPlatforms ? A.dPlatforms : A.platforms, A.nPlatforms);
         if (len2(platformDelta) > 1e-8f) pos = pos + platformDelta;
     }
     if (wasGrounded && wasGroundedNear && vel.y < 0.0) vel.y = 0.0;
@@ -799,10 +800,11 @@ __global__ void __launch_bounds__(MAS_THREADS, MAS_MIN_BLOCKS) k_move_and_slide(
 }
 
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
-                          const float g[3], uint32_t flags, const cq_platform *platforms, int nPlatforms, cudaStream_t st) {
+                          const float g[3], uint32_t flags, const cq_platform *platforms, const cq_platform *dPlatforms,
+                          int nPlatforms, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
     CQ_TRY(await_trees(w, st));
-    if (nPlatforms < 0 || nPlatforms > MAS_MAX_PLATFORMS || (nPlatforms > 0 && !platforms)) {
+    if (!dPlatforms && (nPlatforms < 0 || nPlatforms > MAS_MAX_PLATFORMS || (nPlatforms > 0 && !platforms))) {
         set_error("cq_move_and_slide: 0..%d platforms supported, got %d", MAS_MAX_PLATFORMS, nPlatforms);
         return CQ_ERR_INVALID;
     }
@@ -813,7 +815,9 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
     A.gx = g[0], A.gy = g[1], A.gz = g[2];
     A.flags = flags;
     A.nPlatforms = nPlatforms;
-    for (int k = 0; k < nPlatforms; k++) A.platforms[k] = platforms[k];
+    A.dPlatforms = dPlatforms;
+    if (!dPlatforms)
+        for (int k = 0; k < nPlatforms; k++) A.platforms[k] = platforms[k];
     const bool agents = (flags & CQ_MAS_AGENTS) != 0;
     const int staged = w->view.stagedLeaves ? 1 : 0;
     const int ci = (w->counting ? 1 : 0) + 2 * staged;

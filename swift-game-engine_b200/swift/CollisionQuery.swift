@@ -218,6 +218,36 @@ public final class CollisionQuery {
         return rc == CQ_OK
     }
 
+    /// cq_world_platforms_device: `count` kinematic platform records written to `out` (device memory) from the world-space
+    /// vertices of the entities `ids` (device) as the updates queued before left them (meshWorldAABB), with the motions
+    /// `deltas` (device, 3 Floats each: positionF - prevPositionF).  Queued on `stream` without synchronising, so it can be
+    /// recorded into a CUDA graph.  Unknown ids get inert records; `status` (a device Int32, may be nil) receives their count.
+    public func platformsDevice(ids: UnsafePointer<UInt32>, deltas: UnsafePointer<Float>, count: Int32,
+                                out: UnsafeMutablePointer<cq_platform>, status: UnsafeMutablePointer<Int32>? = nil,
+                                stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        let rc = cq_world_platforms_device(handle, ids, deltas, count, out, status, stream)
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
+    /// Move-and-slide of resident records (`states`: a device pointer) with `platformCount` platform records read from
+    /// device memory when the kernels run, so a replayed CUDA graph carries characters with the records of its frame.
+    public func moveAndSlideDevice(states: UnsafeMutablePointer<cq_character_state>, count: Int32, params: cq_controller_params,
+                                   dt: Float, gravity: SIMD3<Float> = SIMD3<Float>(0, -98, 0),
+                                   platforms: UnsafePointer<cq_platform>?, platformCount: Int32, agents: Bool,
+                                   applyGravity: Bool = true, stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        var p = params
+        var g = (gravity.x, gravity.y, gravity.z)
+        let flags = (applyGravity ? UInt32(CQ_MAS_APPLY_GRAVITY) : 0) | (agents ? UInt32(CQ_MAS_AGENTS) : 0)
+        let rc = withUnsafePointer(to: &g) { gp in
+            gp.withMemoryRebound(to: Float.self, capacity: 3) {
+                cq_move_and_slide_device_platforms(handle, states, count, &p, dt, $0, flags, platforms, platformCount, stream)
+            }
+        }
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
     /// Entities with Transform + StaticMesh (collides), ascending id (the reference iterates a Dictionary, i.e. in
     /// per-process random order — World.swift:99-118; the library fixes the order so triangle numbering is stable).
     /// Geometry is returned as plain Swift arrays; `withArrays` lends their storage to the C structs for one call.
