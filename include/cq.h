@@ -338,8 +338,8 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  *    same buffer move the parts of each replay, and cq_world_platforms_device + cq_move_and_slide_device_platforms
  *    give every replay the records of its own frame;
  *  - a call that would grow scratch, allocate, synchronise or create an event while capturing returns CQ_ERR_INVALID
- *    ("make one uncaptured call of this size first") and leaves the capture valid; so does CQ_MAS_AGENTS when its grid
- *    needs more scratch than an uncaptured call gave it;
+ *    ("make one uncaptured call of this size first") before it enqueues anything, and leaves the capture valid; so does
+ *    CQ_MAS_AGENTS when its grid needs more scratch than an uncaptured call gave it;
  *  - scratch blocks a graph recorded stay allocated when a later uncaptured call outgrows them (the call takes new
  *    blocks), so graphs stay valid until cq_world_destroy, which frees them: replay no graph after destroying its world;
  *  - cq_agent_separation_device and cq_agent_separation_batch (they synchronise to report the outcome), cq_crowd_step

@@ -37,14 +37,6 @@ int ensure_scratch(ScratchBuf &b, size_t bytes) {
     return r;
 }
 
-int grow_scratch(cq_world *w, ScratchBuf &b, size_t bytes) {
-    if (bytes > b.cap && b.captured) {
-        w->graphScratch.push_back(b.ptr);
-        b.ptr = nullptr, b.cap = 0, b.captured = false;
-    }
-    return ensure_scratch(b, bytes);
-}
-
 int resident_blocks(cq_world *w, const void *kernel, int threads, size_t dynSmem) {
     const auto it = w->residentBlocks.find(kernel);
     if (it != w->residentBlocks.end()) return it->second;
@@ -95,13 +87,6 @@ bool stream_capturing(cudaStream_t st) {
 int refuse_capture(cudaStream_t st, const char *what) {
     if (!stream_capturing(st)) return CQ_OK;
     set_error("%s cannot be captured in a CUDA graph (it synchronises or stages host memory); call it outside the capture", what);
-    return CQ_ERR_INVALID;
-}
-
-int refuse_growth(cq_world *w, const char *what) {
-    set_error("%s: the call needs more scratch than any uncaptured call gave it, and growing it cannot be captured; "
-              "make one uncaptured call of this size first", what);
-    w->captureRefused = true;
     return CQ_ERR_INVALID;
 }
 
@@ -164,23 +149,30 @@ static void destroy_scratch(ScratchBuf &b) {
     b = ScratchBuf();
 }
 
-void *pool_node_scratch(cq_world *w, size_t warps, cudaStream_t st) {
-    size_t bytes = warps * (size_t)2048 /* CQ_NSCAP */ * sizeof(uint2);
-    if (bytes > w->nodeScratch[0].cap) {
+int take_scratch(cq_world *w, ScratchBuf *ring, int nRing, int use, size_t bytes, cudaStream_t st, const char *what, void **ptr) {
+    ScratchBuf &b = ring[use];
+    if (bytes > b.cap) {
         if (w->capturing) {
-            refuse_growth(w, "node scratch");
-            return nullptr;
+            set_error("%s: the call needs more scratch than any uncaptured call gave it, and growing it cannot be captured; "
+                      "make one uncaptured call of this size first", what);
+            return CQ_ERR_INVALID;
         }
-        // grow all four regions at once (a cudaMalloc inside a timed step costs milliseconds); growing frees the
-        // old blocks, so make sure no launch still uses them
-        if (check_cuda(cudaDeviceSynchronize(), "node scratch sync") != CQ_OK) return nullptr;
-        for (int k = 0; k < 4; k++)
-            if (grow_scratch(w, w->nodeScratch[k], bytes) != CQ_OK) return nullptr;
+        // grow the whole ring at once (a cudaMalloc inside a timed step costs milliseconds); growing frees the old
+        // blocks, so make sure no launch still uses them
+        CQ_TRY(check_cuda(cudaDeviceSynchronize(), what));
+        for (int k = 0; k < nRing; k++) {
+            ScratchBuf &r = ring[k];
+            if (bytes > r.cap && r.captured) { // a graph may still use it: keep it until cq_world_destroy
+                w->graphScratch.push_back(r.ptr);
+                r.ptr = nullptr, r.cap = 0, r.captured = false;
+            }
+            CQ_TRY(ensure_scratch(r, bytes));
+        }
     }
-    ScratchBuf &b = w->nodeScratch[w->nodeSeq++ & 3];
     if (w->capturing) b.captured = true;
-    if (scratch_acquire(w, b, st) != CQ_OK) return nullptr;
-    return b.ptr;
+    CQ_TRY(scratch_acquire(w, b, st));
+    *ptr = b.ptr;
+    return CQ_OK;
 }
 
 static void make_view(cq_world *w) {
@@ -216,15 +208,11 @@ using namespace cq;
 static cudaStream_t pick_stream(cq_world *w, void *stream) { return stream ? (cudaStream_t)stream : w->stream; }
 
 // One device call being enqueued on `st`: while a stream capture records `st`, the world's helpers neither wait on nor
-// record nor create world events, and refuse to grow scratch (refuse_growth); the call then returns CQ_ERR_INVALID.
+// record nor create world events, and refuse to grow scratch (take_scratch returns CQ_ERR_INVALID).
 struct CaptureScope {
     cq_world *w;
-    CaptureScope(cq_world *world, cudaStream_t st) : w(world) {
-        w->capturing = stream_capturing(st);
-        w->captureRefused = false;
-    }
-    ~CaptureScope() { w->capturing = false, w->captureRefused = false; }
-    int result(int rc) const { return w->captureRefused ? CQ_ERR_INVALID : rc; }
+    CaptureScope(cq_world *world, cudaStream_t st) : w(world) { w->capturing = stream_capturing(st); }
+    ~CaptureScope() { w->capturing = false; }
 };
 
 // ---------------------------------------------------------------- transform updates
@@ -753,7 +741,7 @@ int cq_world_platforms_device(cq_world *w, const uint32_t *d_entity_ids, const f
     CQ_CUDA(cudaSetDevice(w->device));
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_platform_records(w, d_entity_ids, d_deltas, n, d_out, d_status, st));
+    return launch_platform_records(w, d_entity_ids, d_deltas, n, d_out, d_status, st);
 }
 
 int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, uint32_t *indices, float *tri_aabbs,
@@ -861,7 +849,7 @@ int cq_raycast_device_ex(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hi
     if (!w || n < 0 || (n > 0 && (!d_rays || !d_out))) return CQ_ERR_INVALID;
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_raycast(w, d_rays, n, d_out, d_flags, st));
+    return launch_raycast(w, d_rays, n, d_out, d_flags, st);
 }
 int cq_raycast_device(cq_world *w, const cq_ray *d_rays, int32_t n, cq_ray_hit *d_out, void *stream) {
     return cq_raycast_device_ex(w, d_rays, n, d_out, nullptr, stream);
@@ -871,7 +859,7 @@ int cq_capsule_cast_device_ex(cq_world *w, const cq_capsule_cast *d_q, int32_t n
     if (!w || n < 0 || mode < 0 || mode > 2 || (n > 0 && (!d_q || !d_out))) return CQ_ERR_INVALID;
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_cast(w, d_q, n, mode, d_out, d_flags, st));
+    return launch_cast(w, d_q, n, mode, d_out, d_flags, st);
 }
 int cq_capsule_cast_device(cq_world *w, const cq_capsule_cast *d_q, int32_t n, int32_t mode, cq_cast_hit *d_out, void *stream) {
     return cq_capsule_cast_device_ex(w, d_q, n, mode, d_out, nullptr, stream);
@@ -881,7 +869,7 @@ int cq_capsule_overlap_device_ex(cq_world *w, const cq_capsule *d_q, int32_t n, 
     if (!w || n < 0 || (n > 0 && (!d_q || !d_out))) return CQ_ERR_INVALID;
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_overlap(w, d_q, n, d_out, d_flags, st));
+    return launch_overlap(w, d_q, n, d_out, d_flags, st);
 }
 int cq_capsule_overlap_device(cq_world *w, const cq_capsule *d_q, int32_t n, cq_overlap_hit *d_out, void *stream) {
     return cq_capsule_overlap_device_ex(w, d_q, n, d_out, nullptr, stream);
@@ -901,7 +889,7 @@ int cq_capsule_overlap_all_device(cq_world *w, const cq_capsule *d_q, int32_t n,
     CQ_TRY(check_overlap_all_size(n, max_hits));
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_overlap_all(w, d_q, n, max_hits, d_out, d_counts, d_overflow, st));
+    return launch_overlap_all(w, d_q, n, max_hits, d_out, d_counts, d_overflow, st);
 }
 int cq_move_and_slide_device_ex(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
                                 float dt, const float gravity[3], uint32_t flags, const cq_platform *platforms,
@@ -909,7 +897,7 @@ int cq_move_and_slide_device_ex(cq_world *w, cq_character_state *d_inout, int32_
     if (!w || n < 0 || !params || !gravity || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, nullptr, n_platforms, st));
+    return launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, platforms, nullptr, n_platforms, st);
 }
 int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params,
                                        float dt, const float gravity[3], uint32_t flags, const cq_platform *d_platforms,
@@ -921,8 +909,8 @@ int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout,
     }
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, nullptr,
-                                            n_platforms > 0 ? d_platforms : nullptr, n_platforms, st));
+    return launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, nullptr,
+                                 n_platforms > 0 ? d_platforms : nullptr, n_platforms, st);
 }
 int cq_move_and_slide_device(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params, float dt,
                              const float gravity[3], uint32_t flags, void *stream) {
@@ -1044,8 +1032,8 @@ int cq_agent_separation_device_async(cq_world *w, cq_character_state *d_inout, i
     CQ_CUDA(cudaSetDevice(w->device));
     const cudaStream_t st = pick_stream(w, stream);
     CaptureScope cap(w, st);
-    return cap.result(launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin,
-                                              height_margin, use_query, d_status, st));
+    return launch_agent_separation(w, d_inout, n, *params, d_mass_weight, iterations, separation_margin,
+                                   height_margin, use_query, d_status, st);
 }
 
 int cq_agent_separation_batch(cq_world *w, cq_character_state *inout, int32_t n, const cq_controller_params *params,

@@ -883,8 +883,6 @@ __global__ void k_ref_refit_clear(const MovedPart *__restrict__ tab, const Refit
 }
 
 // ---------------------------------------------------------------- host orchestration
-static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
-
 // One cudaMalloc per triangle set (+ one for build temporaries): GB-scale cudaMalloc/cudaFree calls cost
 // tens to hundreds of milliseconds each on this driver, far more than the build kernels themselves.
 struct Arena {
@@ -1232,32 +1230,27 @@ __global__ void k_order_keys(const unsigned char *__restrict__ base, size_t stri
     vals[i] = (uint32_t)i;
 }
 
-const uint32_t *make_unit_order(cq_world *w, const void *dUnits, size_t stride, bool positionIsDouble, int n, cudaStream_t st) {
-    if (n < (1 << 16) || w->set[0].nTris < (1 << 18)) return nullptr; // small world / batch: everything is cache resident
-    const int tiles = cdiv(n, RS_TILE);
-    const size_t sortWords = (size_t)4 * 256 * tiles + 4 + 1024 + 1;
-    const size_t words = (size_t)4 * n + sortWords + 64;
-    ScratchBuf &b = w->orderScratch[w->orderSeq++ & 3];
-    if (words * 4 > b.cap) {
-        if (w->capturing) {
-            refuse_growth(w, "unit order scratch");
-            return nullptr;
-        }
-        if (check_cuda(cudaDeviceSynchronize(), "order scratch sync") != CQ_OK) return nullptr;
-        for (int k = 0; k < 4; k++)
-            if (grow_scratch(w, w->orderScratch[k], words * 4) != CQ_OK) return nullptr;
-    }
-    if (w->capturing) b.captured = true;
-    if (scratch_acquire(w, b, st) != CQ_OK) return nullptr;
-    uint32_t *keys = (uint32_t *)b.ptr, *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n, *scratch = valsTmp + n;
+size_t sort_scratch_words(int n) { return (size_t)4 * 256 * cdiv(n, RS_TILE) + 4 + 1024 + 1; }
+
+int take_unit_order(cq_world *w, int n, cudaStream_t st, uint32_t **scratch) {
+    *scratch = nullptr;
+    if (n < (1 << 16) || w->set[0].nTris < (1 << 18)) return CQ_OK; // small world / batch: everything is cache resident
+    const size_t words = (size_t)4 * n + sort_scratch_words(n) + 64;
+    return take_scratch(w, w->orderScratch, 4, w->orderSeq++ & 3, words * 4, st, "unit order scratch", (void **)scratch);
+}
+
+int make_unit_order(cq_world *w, uint32_t *scratch, const void *dUnits, size_t stride, bool positionIsDouble, int n,
+                    cudaStream_t st, const uint32_t **order) {
+    *order = nullptr;
+    if (!scratch) return CQ_OK;
+    uint32_t *keys = scratch, *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n, *sortScratch = valsTmp + n;
     k_order_keys<<<cdiv(n, 256), 256, 0, st>>>((const unsigned char *)dUnits, stride, positionIsDouble ? 1 : 0, n, w->set[0].hdr,
                                                keys, vals);
     w->launches++;
-    if (radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, scratch, sortWords, st, false) != CQ_OK) return nullptr;
-    return vals;
+    CQ_TRY(radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, sortScratch, sort_scratch_words(n), st, false));
+    *order = vals;
+    return CQ_OK;
 }
-
-size_t sort_scratch_words(int n) { return (size_t)4 * 256 * cdiv(n, RS_TILE) + 4 + 1024 + 1; }
 int sort_pairs_u32(cq_world *w, uint32_t *keys, uint32_t *vals, uint32_t *keysTmp, uint32_t *valsTmp, int n, uint32_t *scratch,
                    size_t scratchWords, cudaStream_t st) {
     return radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, scratch, scratchWords, st, false);
@@ -1387,33 +1380,29 @@ __global__ void k_agent_rows(const uint32_t *__restrict__ keys, const uint32_t *
     rows[2 * (size_t)orig + 1] = make_int4(se[4], se[5], ix, iz);
 }
 
-int make_agent_grid(cq_world *w, const cq_character_state *dStates, int n, float radius, float dt, const float g[3],
-                    uint32_t flags, cudaStream_t st, AgentGrid &out) {
-    const int tiles = cdiv(n, RS_TILE);
-    const size_t sortWords = (size_t)4 * 256 * tiles + 4 + 1024 + 1;
+int take_agent_grid(cq_world *w, int n, cudaStream_t st, void **scratch) {
     // [pos n][vel n][posS n][velS n] float4, [rows 2n] int4, [firstHit n] float4, [keys n][vals n][keysTmp n][valsTmp n] u32, sort scratch,
     // bounds, params
-    const size_t bytes = (size_t)n * 112 + ((size_t)4 * n + sortWords + 64) * 4;
-    if (bytes > w->agentScratch.cap) {
-        if (w->capturing) return refuse_growth(w, "CQ_MAS_AGENTS grid scratch");
-        CQ_CUDA(cudaDeviceSynchronize());
-        CQ_TRY(grow_scratch(w, w->agentScratch, bytes));
-    }
-    if (w->capturing) w->agentScratch.captured = true;
-    CQ_TRY(scratch_acquire(w, w->agentScratch, st));
-    float4 *pos = (float4 *)w->agentScratch.ptr, *vel = pos + n, *posS = vel + n, *velS = posS + n;
+    const size_t bytes = (size_t)n * 112 + ((size_t)4 * n + sort_scratch_words(n) + 64) * 4;
+    return take_scratch(w, &w->agentScratch, 1, 0, bytes, st, "CQ_MAS_AGENTS grid scratch", scratch);
+}
+
+int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, int n, float radius, float dt,
+                    const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out) {
+    const size_t sortWords = sort_scratch_words(n);
+    float4 *pos = (float4 *)scratch, *vel = pos + n, *posS = vel + n, *velS = posS + n;
     int4 *rows = (int4 *)(velS + n);
     float4 *firstHit = (float4 *)(rows + 2 * (size_t)n);
     uint32_t *keys = (uint32_t *)(firstHit + n), *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n;
-    uint32_t *scratch = valsTmp + n;
-    int *bounds = (int *)(scratch + sortWords);
+    uint32_t *sortScratch = valsTmp + n;
+    int *bounds = (int *)(sortScratch + sortWords);
     AgentGridParams *gp = (AgentGridParams *)(bounds + 8);
     k_agent_bounds_init<<<1, 32, 0, st>>>(bounds);
     k_agent_snapshot<<<cdiv(n, 256), 256, 0, st>>>(dStates, n, dt, g[0], g[1], g[2], flags, pos, vel, bounds);
     k_agent_grid_params<<<1, 1, 0, st>>>(bounds, radius, dt, gp);
     k_agent_keys<<<cdiv(n, 256), 256, 0, st>>>(pos, n, gp, keys, vals);
     w->launches += 4;
-    CQ_TRY(radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, scratch, sortWords, st, false));
+    CQ_TRY(radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, sortScratch, sortWords, st, false));
     k_agent_gather<<<cdiv(n, 256), 256, 0, st>>>(vals, n, pos, vel, posS, velS);
     k_agent_rows<<<cdiv(n, 256), 256, 0, st>>>(keys, vals, n, gp, rows);
     w->launches += 2;

@@ -73,7 +73,7 @@ struct ScratchBuf {
     cudaEvent_t ev = nullptr;
     cudaStream_t last = nullptr;
     bool recorded = false;
-    bool captured = false; // a stream capture recorded this block's address: on growth it is kept, not freed (grow_scratch)
+    bool captured = false; // a stream capture recorded this block's address: on growth it is kept, not freed (take_scratch)
 };
 
 // One row of the part table a transform update stages (cq_api.cu: update_transforms_on): a moved part of one set, its
@@ -191,9 +191,8 @@ struct cq_world {
     cq::MovedPart *dDevTable = nullptr;     // static set's rows at [0, devRows0), dynamic set's after
     int nEntities = 0, devRows0 = 0;
     // a device call is being recorded into a stream capture (CaptureScope, cq_api.cu): no world event is waited on,
-    // recorded or created, and scratch must not grow (captureRefused then makes the call return CQ_ERR_INVALID)
+    // recorded or created, and scratch must not grow (take_scratch refuses)
     bool capturing = false;
-    bool captureRefused = false;
     std::vector<void *> graphScratch; // outgrown scratch blocks that captured graphs may still use: freed by cq_world_destroy
     std::vector<void *> retiredDev, retiredHost; // outgrown table buffers a queued update may still use (cq_api.cu: free_retired)
     // Ordering of stream-ordered refits against every other launch on the world (await_trees / note_reader):
@@ -204,6 +203,7 @@ struct cq_world {
 };
 
 namespace cq {
+inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 void set_error(const char *fmt, ...);
 int check_cuda(cudaError_t e, const char *what);
 #define CQ_CUDA(x)                                        \
@@ -219,9 +219,6 @@ int check_cuda(cudaError_t e, const char *what);
     } while (0)
 
 int ensure_scratch(ScratchBuf &b, size_t bytes);
-// ensure_scratch for the blocks a captured call may use (node, unit-order and agent scratch): a block whose address a
-// graph recorded (ScratchBuf::captured) is moved to w->graphScratch instead of being freed, so replays stay valid
-int grow_scratch(cq_world *w, ScratchBuf &b, size_t bytes);
 // CTAs of `kernel` (`threads` per CTA, `dynSmem` bytes of dynamic shared memory) that fit on the device at once: SMs x
 // resident CTAs per SM (at least one per SM), cached per world.  dynSmem > 0 also raises the kernel's dynamic shared-memory
 // limit to dynSmem.  0 on CUDA error.
@@ -238,6 +235,13 @@ int check_status(cq_world *w, const char *what);
 // release_held(w, st) once everything that touches its blocks is enqueued (records the completion events).
 int scratch_acquire(cq_world *w, ScratchBuf &b, cudaStream_t st);
 int release_held(cq_world *w, cudaStream_t st);
+// The only code that grows the scratch a launch uses: takes ring[use] of the nRing blocks of `ring` (one block, or a ring
+// of four used round-robin so that up to four launches on different streams run concurrently; a fifth waits for the
+// first) for a launch on `st` and returns its address in *ptr.  A block smaller than `bytes` is refused under capture (CQ_ERR_INVALID, naming `what`;
+// nothing is enqueued and the capture stays valid); uncaptured, all nRing blocks grow together after one device
+// synchronisation, and a block whose address a graph recorded (ScratchBuf::captured) is moved to w->graphScratch instead
+// of being freed, so replays stay valid.  Under capture the block is marked captured; then it is acquired for `st`.
+int take_scratch(cq_world *w, ScratchBuf *ring, int nRing, int use, size_t bytes, cudaStream_t st, const char *what, void **ptr);
 // First call of every launcher: a launch on `st` must see the trees the latest asynchronous refit writes, so `st` waits
 // for that refit when it was queued on another stream.
 int await_trees(const cq_world *w, cudaStream_t st);
@@ -247,10 +251,6 @@ int finish_launch(cq_world *w, cudaStream_t st, const char *what);
 #define CQ_WORK_RING 256
 // zeroed work counter for the next persistent-kernel launch on `st` (nullptr on CUDA error)
 int *next_work_counter(cq_world *w, cudaStream_t st);
-// node-stack scratch for one persistent-kernel launch with `warps` warps (CQ_NSCAP uint2 entries per warp);
-// four regions are used round-robin so that up to four launches on different streams run concurrently (a fifth
-// waits for the first, see scratch_acquire).  nullptr on CUDA error.
-void *pool_node_scratch(cq_world *w, size_t warps, cudaStream_t st);
 
 // cq_build.cu
 int build_set(cq_world *w, DeviceSet &S, const SetPlan &in /* upload plan of the set, cq_assemble.h */,
@@ -277,19 +277,21 @@ bool stream_capturing(cudaStream_t st);
 // capture stays valid), else CQ_OK.
 int refuse_capture(cudaStream_t st, const char *what);
 #define CQ_NO_CAPTURE(st, what) CQ_TRY(cq::refuse_capture((st), (what)))
-// Under capture: the call needs more scratch than any uncaptured call gave it, which would take a synchronisation and an
-// allocation.  Sets the error and w->captureRefused, returns CQ_ERR_INVALID.  captureRefused is only ever true between a
-// CaptureScope's construction and its destruction (cq_api.cu), so uncaptured calls never see it set.
-int refuse_growth(cq_world *w, const char *what);
 // reference order: rebuild the reference's tree on the host from the set's triangle boxes, upload rank + tree (cq_reftree.h)
 int attach_ref_order(cq_world *w);
 void free_set(DeviceSet &S);
 // Morton-sorted processing order of n work units whose position (3 floats or 3 doubles) sits at the start of each
-// `stride`-byte record; nullptr when ordering is not worthwhile (small world / batch) or on error
-// CQ_MAS_AGENTS pre-pass: snapshot (after the gravity rule), XZ grid, sort by cell.  Stream-ordered on `st`.
-int make_agent_grid(cq_world *w, const cq_character_state *dStates, int n, float radius, float dt, const float g[3],
-                    uint32_t flags, cudaStream_t st, AgentGrid &out);
-const uint32_t *make_unit_order(cq_world *w, const void *dUnits, size_t stride, bool positionIsDouble, int n, cudaStream_t st);
+// `stride`-byte record.  take_unit_order takes the order's scratch for `st` (take_scratch); *scratch = nullptr when
+// ordering is not worthwhile (small world / batch).  make_unit_order enqueues the keys and the sort into that scratch on
+// `st` and returns the order in *order (nullptr when scratch is).
+int take_unit_order(cq_world *w, int n, cudaStream_t st, uint32_t **scratch);
+int make_unit_order(cq_world *w, uint32_t *scratch, const void *dUnits, size_t stride, bool positionIsDouble, int n,
+                    cudaStream_t st, const uint32_t **order);
+// CQ_MAS_AGENTS pre-pass of n agents: take_agent_grid takes its scratch for `st` (take_scratch); make_agent_grid enqueues
+// the snapshot (after the gravity rule), XZ grid and sort by cell into that scratch on `st`.
+int take_agent_grid(cq_world *w, int n, cudaStream_t st, void **scratch);
+int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, int n, float radius, float dt,
+                    const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out);
 
 // 32-bit key / value LSD radix sort (onesweep); `scratch` holds sort_scratch_words(n) words.  Result in (keys, vals).
 size_t sort_scratch_words(int n);
@@ -297,6 +299,21 @@ int sort_pairs_u32(cq_world *w, uint32_t *keys, uint32_t *vals, uint32_t *keysTm
                    size_t scratchWords, cudaStream_t st);
 
 // cq_query.cu
+// What pool_launch_setup gives one launch of a persistent pair-pool kernel.
+struct PoolLaunch {
+    int blocks = 0;                  // CTAs: one resident wave at most
+    int ownersPerWarp = 0;           // pool_owners_per_warp
+    uint2 *nodeScratch = nullptr;    // CQ_NSCAP node-stack entries per warp
+    int *work = nullptr;             // the zeroed dynamic-fetch counter
+    const uint32_t *order = nullptr; // unit order, nullptr = the units' own order
+};
+// The prologue of every pool-kernel launch of n units on `st`: await_trees; blocks = min(cdiv(n, unitsPerCta), one
+// resident wave of `kernel` at `threads` threads and `smem` bytes of dynamic shared memory); owners per warp over
+// blocks * threads / 32 warps.  It first takes every scratch block the launch needs (node stacks when `nodeScratch`, the
+// unit order's when `units` is non-null: records of `stride` bytes, see make_unit_order), so a refused call enqueues
+// nothing, and only then enqueues the work-counter memset and the unit order's keys and sort.
+int pool_launch_setup(cq_world *w, const void *kernel, int threads, size_t smem, int unitsPerCta, int n, bool nodeScratch,
+                      const void *units, size_t stride, bool positionIsDouble, cudaStream_t st, PoolLaunch &out);
 // d_flags (may be nullptr): one CQ_HIT_* byte per query
 int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, uint8_t *d_flags, cudaStream_t st);
 int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cast_hit *d_out, uint8_t *d_flags, cudaStream_t st);

@@ -803,7 +803,6 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
                           const float g[3], uint32_t flags, const cq_platform *platforms, const cq_platform *dPlatforms,
                           int nPlatforms, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
-    CQ_TRY(await_trees(w, st));
     if (!dPlatforms && (nPlatforms < 0 || nPlatforms > MAS_MAX_PLATFORMS || (nPlatforms > 0 && !platforms))) {
         set_error("cq_move_and_slide: 0..%d platforms supported, got %d", MAS_MAX_PLATFORMS, nPlatforms);
         return CQ_ERR_INVALID;
@@ -828,26 +827,20 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
                                          {k_move_and_slide<false, true, false>, k_move_and_slide<true, true, false>,
                                           k_move_and_slide<false, true, true>, k_move_and_slide<true, true, true>}};
     const Kernel kernel = kernels[agents ? 1 : 0][ci];
-    const int resident = resident_blocks(w, (const void *)kernel, MAS_THREADS, MAS_SMEM_BYTES);
-    if (!resident) return CQ_ERR_CUDA;
-    int *work = next_work_counter(w, st);
-    if (!work) return CQ_ERR_CUDA;
+    void *agentScratch = nullptr;
+    if (agents) CQ_TRY(take_agent_grid(w, n, st, &agentScratch));
     // persistent lanes: one resident wave of CTAs, lanes stride over characters; small batches still fill the machine
     // (>= 4 units per CTA)
-    const int blocks = std::min((n + 3) / 4, resident);
-    const int opw = pool_owners_per_warp(n, (long long)blocks * MAS_WARPS);
-    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * MAS_WARPS, st);
-    if (!ns) return CQ_ERR_CUDA;
-    const uint32_t *order = make_unit_order(w, d_inout, sizeof(cq_character_state), true, n, st);
-    // refused under capture: the kernels are not enqueued; the work-counter memset (and, for CQ_MAS_AGENTS, the unit
-    // order's keys and sort) already are, and only write scratch
-    if (w->captureRefused) return CQ_ERR_INVALID;
-    if (flags & CQ_MAS_AGENTS) {
-        CQ_TRY(make_agent_grid(w, d_inout, n, p.radius, dt, g, flags, st, A.agents));
+    PoolLaunch L;
+    CQ_TRY(pool_launch_setup(w, (const void *)kernel, MAS_THREADS, MAS_SMEM_BYTES, 4, n, true, d_inout, sizeof(cq_character_state),
+                             true, st, L));
+    if (agents) {
+        CQ_TRY(make_agent_grid(w, agentScratch, d_inout, n, p.radius, dt, g, flags, st, A.agents));
         k_agent_first_hit<<<(n + 255) / 256, 256, 0, st>>>(d_inout, n, A);
         w->launches++;
     }
-    kernel<<<blocks, MAS_THREADS, MAS_SMEM_BYTES, st>>>(w->view, d_inout, n, A, opw, ns, work, order, w->dCounters);
+    kernel<<<L.blocks, MAS_THREADS, MAS_SMEM_BYTES, st>>>(w->view, d_inout, n, A, L.ownersPerWarp, L.nodeScratch, L.work, L.order,
+                                                          w->dCounters);
     w->launches++;
     return finish_launch(w, st, "k_move_and_slide");
 }

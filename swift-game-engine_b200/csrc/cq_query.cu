@@ -657,49 +657,52 @@ __global__ void __launch_bounds__(Q_THREADS) k_overlap_wide_emit(WorldView W, co
 }
 
 // ---------------------------------------------------------------- launchers
-static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
+int pool_launch_setup(cq_world *w, const void *kernel, int threads, size_t smem, int unitsPerCta, int n, bool nodeScratch,
+                      const void *units, size_t stride, bool positionIsDouble, cudaStream_t st, PoolLaunch &out) {
+    CQ_TRY(await_trees(w, st));
+    const int resident = resident_blocks(w, kernel, threads, smem);
+    if (!resident) return CQ_ERR_CUDA;
+    const int warps = threads / 32;
+    out.blocks = std::min(cdiv(n, unitsPerCta), resident); // one resident wave of persistent lanes
+    out.ownersPerWarp = pool_owners_per_warp(n, (long long)out.blocks * warps);
+    const size_t nodeBytes = (size_t)out.blocks * warps * CQ_NSCAP * sizeof(uint2);
+    void *ns = nullptr;
+    uint32_t *orderScratch = nullptr;
+    if (nodeScratch) CQ_TRY(take_scratch(w, w->nodeScratch, 4, w->nodeSeq++ & 3, nodeBytes, st, "node scratch", &ns));
+    if (units) CQ_TRY(take_unit_order(w, n, st, &orderScratch));
+    out.nodeScratch = (uint2 *)ns;
+    out.work = next_work_counter(w, st);
+    if (!out.work) return CQ_ERR_CUDA;
+    return make_unit_order(w, orderScratch, units, stride, positionIsDouble, n, st, &out.order);
+}
 
 int launch_raycast(cq_world *w, const cq_ray *d_rays, int n, cq_ray_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
-    CQ_TRY(await_trees(w, st));
     const bool ref = w->order == CQ_ORDER_REFERENCE; // the reference's own walk over the reference's own tree
     const int ci = (w->counting ? 1 : 0) + (ref ? 2 : 0);
     using Kernel = void (*)(WorldView, const cq_ray *, int, cq_ray_hit *, uint8_t *, int *, const uint32_t *, unsigned long long *);
     static const Kernel kernels[4] = {k_raycast_phased<false, false>, k_raycast_phased<true, false>, k_raycast_phased<false, true>,
                                       k_raycast_phased<true, true>};
     const Kernel kernel = kernels[ci];
-    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
-    if (!resident) return CQ_ERR_CUDA;
-    int blocks = std::min(cdiv(n, Q_THREADS), resident); // one resident wave of persistent lanes
-    int *work = next_work_counter(w, st);
-    if (!work) return CQ_ERR_CUDA;
-    const uint32_t *order = make_unit_order(w, d_rays, sizeof(cq_ray), false, n, st);
-    if (w->captureRefused) return CQ_ERR_INVALID; // the query kernel is not enqueued (the work counter memset already is)
-    kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_rays, n, d_out, d_flags, work, order, w->dCounters);
+    PoolLaunch L;
+    CQ_TRY(pool_launch_setup(w, (const void *)kernel, Q_THREADS, 0, Q_THREADS, n, false, d_rays, sizeof(cq_ray), false, st, L));
+    kernel<<<L.blocks, Q_THREADS, 0, st>>>(w->view, d_rays, n, d_out, d_flags, L.work, L.order, w->dCounters);
     w->launches++;
     return finish_launch(w, st, ref ? "k_raycast_ref" : "k_raycast");
 }
 
 int launch_cast(cq_world *w, const cq_capsule_cast *d_q, int n, int mode, cq_cast_hit *d_out, uint8_t *d_flags, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
-    CQ_TRY(await_trees(w, st));
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     using Kernel = void (*)(WorldView, const cq_capsule_cast *, int, int, cq_cast_hit *, uint8_t *, int, uint2 *, int *,
                             const uint32_t *, unsigned long long *);
     static const Kernel kernels[4] = {k_capsule_cast<false, false>, k_capsule_cast<true, false>, k_capsule_cast<false, true>,
                                       k_capsule_cast<true, true>};
     const Kernel kernel = kernels[ci];
-    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
-    if (!resident) return CQ_ERR_CUDA;
-    int blocks = std::min(cdiv(n, 4), resident); // one resident wave of persistent lanes
-    const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
-    int *work = next_work_counter(w, st);
-    if (!work) return CQ_ERR_CUDA;
-    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
-    if (!ns) return CQ_ERR_CUDA;
-    const uint32_t *order = make_unit_order(w, d_q, sizeof(cq_capsule_cast), false, n, st);
-    if (w->captureRefused) return CQ_ERR_INVALID; // the query kernel is not enqueued (the work counter memset already is)
-    kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, mode, d_out, d_flags, opw, ns, work, order, w->dCounters);
+    PoolLaunch L;
+    CQ_TRY(pool_launch_setup(w, (const void *)kernel, Q_THREADS, 0, 4, n, true, d_q, sizeof(cq_capsule_cast), false, st, L));
+    kernel<<<L.blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, mode, d_out, d_flags, L.ownersPerWarp, L.nodeScratch, L.work, L.order,
+                                           w->dCounters);
     w->launches++;
     return finish_launch(w, st, "k_capsule_cast");
 }
@@ -708,22 +711,16 @@ template <bool ALL>
 static int launch_overlap_pool(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                                uint8_t *d_overflow, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
-    CQ_TRY(await_trees(w, st));
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     using Kernel = void (*)(WorldView, const cq_capsule *, int, int, cq_overlap_hit *, int32_t *, uint8_t *, int, uint2 *, int *,
                             unsigned long long *);
     static const Kernel kernels[4] = {k_capsule_overlap_pool<false, ALL, false>, k_capsule_overlap_pool<true, ALL, false>,
                                       k_capsule_overlap_pool<false, ALL, true>, k_capsule_overlap_pool<true, ALL, true>};
     const Kernel kernel = kernels[ci];
-    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
-    if (!resident) return CQ_ERR_CUDA;
-    int blocks = std::min(cdiv(n, 4), resident);
-    const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
-    int *work = next_work_counter(w, st);
-    if (!work) return CQ_ERR_CUDA;
-    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
-    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
-    kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, opw, ns, work, w->dCounters);
+    PoolLaunch L;
+    CQ_TRY(pool_launch_setup(w, (const void *)kernel, Q_THREADS, 0, 4, n, true, nullptr, 0, false, st, L));
+    kernel<<<L.blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, L.ownersPerWarp, L.nodeScratch,
+                                           L.work, w->dCounters);
     w->launches++;
     return finish_launch(w, st, "k_capsule_overlap_pool");
 }
@@ -736,22 +733,16 @@ int launch_overlap(cq_world *w, const cq_capsule *d_q, int n, cq_overlap_hit *d_
 static int launch_overlap_wide(cq_world *w, const cq_capsule *d_q, int n, int maxHits, cq_overlap_hit *d_out, int32_t *d_counts,
                                uint8_t *d_overflow, cudaStream_t st) {
     if (n <= 0) return CQ_OK;
-    CQ_TRY(await_trees(w, st));
     const int ci = (w->counting ? 1 : 0) + 2 * (w->view.stagedLeaves ? 1 : 0);
     using Kernel = void (*)(WorldView, const cq_capsule *, int, int, cq_overlap_hit *, int32_t *, uint8_t *, int, uint2 *, int *,
                             unsigned long long *);
     static const Kernel kernels[4] = {k_capsule_overlap_wide<false, false>, k_capsule_overlap_wide<true, false>,
                                       k_capsule_overlap_wide<false, true>, k_capsule_overlap_wide<true, true>};
     const Kernel kernel = kernels[ci];
-    const int resident = resident_blocks(w, (const void *)kernel, Q_THREADS, 0);
-    if (!resident) return CQ_ERR_CUDA;
-    int blocks = std::min(cdiv(n, 4), resident);
-    const int opw = pool_owners_per_warp(n, (long long)blocks * CAST_WARPS);
-    int *work = next_work_counter(w, st);
-    if (!work) return CQ_ERR_CUDA;
-    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)blocks * CAST_WARPS, st);
-    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
-    kernel<<<blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, opw, ns, work, w->dCounters);
+    PoolLaunch L;
+    CQ_TRY(pool_launch_setup(w, (const void *)kernel, Q_THREADS, 0, 4, n, true, nullptr, 0, false, st, L));
+    kernel<<<L.blocks, Q_THREADS, 0, st>>>(w->view, d_q, n, maxHits, d_out, d_counts, d_overflow, L.ownersPerWarp, L.nodeScratch,
+                                           L.work, w->dCounters);
     // grid-stride passes: a few waves of 128-thread blocks whatever n and maxHits
     const long long wave = (long long)w->numSms * 16;
     const int sortBlocks = (int)std::min<long long>(cdiv(n, Q_THREADS), wave);

@@ -27,7 +27,6 @@
 namespace cq {
 
 #define SEP_THREADS 128
-static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 #define SEP_WARPS (SEP_THREADS / 32)
 
 struct SepGridParams {
@@ -857,20 +856,15 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     // float4 x5 (pos vel orig posSave velSave), int4 x2 (rows), int2 x2 (cellRaw cell0), int x3 (cnt queueA queueB),
     // u32 x4 (sort), scratch
     const size_t bytes = (size_t)n * (7 * 16 + 2 * 8 + 3 * 4 + 4 * 4) + sortWords * 4 + 256;
-    if (bytes > w->sepScratch.cap) {
-        if (w->capturing) return refuse_growth(w, "agent separation scratch");
-        CQ_CUDA(cudaDeviceSynchronize());
-        CQ_TRY(grow_scratch(w, w->sepScratch, bytes));
-    }
-    if (w->capturing) w->sepScratch.captured = true;
-    CQ_TRY(scratch_acquire(w, w->sepScratch, st));
-    float4 *pos = (float4 *)w->sepScratch.ptr, *vel = pos + n, *orig = vel + n, *posSave = orig + n, *velSave = posSave + n;
+    void *sepScratch = nullptr;
+    CQ_TRY(take_scratch(w, &w->sepScratch, 1, 0, bytes, st, "agent separation scratch", &sepScratch));
+    float4 *pos = (float4 *)sepScratch, *vel = pos + n, *orig = vel + n, *posSave = orig + n, *velSave = posSave + n;
     int4 *rows = (int4 *)(velSave + n);
     int2 *cellRaw = (int2 *)(rows + 2 * (size_t)n), *cell0 = cellRaw + n;
     int *cnt = (int *)(cell0 + n), *queueA = cnt + n, *queueB = queueA + n;
     uint32_t *keys = (uint32_t *)(queueB + n), *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n;
     uint32_t *scratch = valsTmp + n;
-    int *small = sep_small(w->sepScratch.ptr, n);
+    int *small = sep_small(sepScratch, n);
     int *bounds = small, *flags = small + 4, *qcount = small + 12, *work = small + 14;
     SepGridParams *gp = (SepGridParams *)(small + 16);
     SepState *state = (SepState *)(small + 24);
@@ -883,8 +877,10 @@ int launch_agent_separation(cq_world *w, cq_character_state *d_inout, int n, con
     const int postBlocksMax = resident_blocks(w, postKernel, SEP_THREADS, postSmem);
     if (!turnBlocksMax || !postBlocksMax) return CQ_ERR_CUDA;
     const int turnBlocks = std::min(cdiv(n, 4), turnBlocksMax), postBlocks = std::min(cdiv(n, 4), postBlocksMax);
-    uint2 *ns = (uint2 *)pool_node_scratch(w, (size_t)std::max(turnBlocks, postBlocks) * SEP_WARPS, st);
-    if (!ns) return w->captureRefused ? CQ_ERR_INVALID : CQ_ERR_CUDA;
+    const size_t nodeBytes = (size_t)std::max(turnBlocks, postBlocks) * SEP_WARPS * CQ_NSCAP * sizeof(uint2);
+    void *nodeScratch = nullptr;
+    CQ_TRY(take_scratch(w, w->nodeScratch, 4, w->nodeSeq++ & 3, nodeBytes, st, "node scratch", &nodeScratch));
+    uint2 *ns = (uint2 *)nodeScratch;
 
     const float cellSize = sep_cell_size(p, sepMargin);
     CQ_CUDA(cudaMemsetAsync(state, 0, sizeof(SepState), st));
