@@ -85,7 +85,7 @@ typedef struct cq_world_info {
     float build_ms;              /* device time of upload+filter+Morton+sort+tree+fit */
     float refit_ms;              /* device time of the last cq_world_update_transforms (the async call leaves it unchanged) */
     int32_t order;               /* CQ_ORDER_* the world was created with */
-    float ref_order_ms;          /* host time of the reference-order build (0 in canonical order) */
+    float ref_order_ms;          /* wall time of the reference-order build (0 in canonical order) */
     int32_t n_ref_nodes;         /* nodes of the reference's own tree, both sets (0 in canonical order) */
     int32_t _reserved;
 } cq_world_info;
@@ -99,12 +99,12 @@ typedef struct cq_world_info {
  * cache is keyed by triangle index (Systems.swift:1169-1204), so the choice is visible.
  *
  *  CQ_ORDER_REFERENCE (default): the library derives every triangle's visiting rank from the reference's own tree
- *      (rebuilt on the host at world creation: swift-game-engine_b200/csrc/cq_reftree.h) and resolves ties / keeps the
+ *      (cut on the device at world creation: attach_ref_order in csrc/cq_build.cu) and resolves ties / keeps the
  *      first maxHits overlaps by that rank; raycasts walk that tree with the reference's own slab test, so even the
  *      grazing hits its non-conservative test culls (:933, :1603-1631) come out the same.  Results equal the reference's
- *      for the same entity order.  Costs host time at creation (about 2 s per 10 M triangles), none per query.
+ *      for the same entity order.  Costs a device build at creation (DESIGN.md §2.1), none per query.
  *  CQ_ORDER_CANONICAL: tree-independent rule — ties go to the smallest triangle index, capsuleOverlapAll keeps the
- *      maxHits deepest (deepest first), a raycast returns the nearest triangle over ALL triangles.  No host build. */
+ *      maxHits deepest (deepest first), a raycast returns the nearest triangle over ALL triangles.  No reference tree. */
 #define CQ_ORDER_REFERENCE 0
 #define CQ_ORDER_CANONICAL 1
 
@@ -205,6 +205,26 @@ int cq_world_read_soup(const cq_world *w, int32_t which,
                        float *tri_aabbs /* n_triangles*6: min xyz, max xyz */,
                        uint32_t *tri_layers /* n_triangles */,
                        int32_t *tri_parts /* n_triangles: index into the parts array */);
+
+/* Rebuild the world in place from a new parts array: afterwards every query, move-and-slide, separation, read and device
+ * update answers exactly as a fresh cq_world_create_ex(parts, n_parts, options) would (the entity index of the device
+ * updates included).  The new geometry is built aside and swapped in only on success: on any error (bad arguments, an
+ * index out of range, a reference tree too deep, a CUDA error) the world keeps answering exactly as before, and
+ * cq_last_error says why.  Before the swap it waits for every launch already queued on the world, on any stream, that may
+ * read the old geometry (those launches see the old geometry), then releases it.  The device, streams, events, pinned
+ * staging and launch scratch are kept.  Crowds created on the world stay valid with their records unchanged; triangle
+ * indices already in them (contact caches) keep the old numbering, as the reference's controllers keep theirs across a
+ * rebuild.  CUDA graphs recorded before a rebuild hold the old geometry's addresses and must not be replayed after it.
+ * Synchronous: refused (CQ_ERR_INVALID, nothing enqueued) while the world's stream or a stream that launched work on the
+ * world is being captured. */
+int cq_world_rebuild(cq_world *w, const cq_mesh_part *parts, int32_t n_parts, const cq_world_options *options);
+
+/* The reference's own tree of one set (which: 0 = static, 1 = dynamic), as the world built it on the device at creation:
+ * order[p] = the set-local triangle at position p of the reference's triOrder, rank[t] = the position of set-local
+ * triangle t in the reference's depth-first visiting order (0 = visited first).  Exact ties and capsuleOverlapAll's
+ * maxHits cut follow this rank.  Either pointer may be NULL; each takes n_triangles of the set.  CQ_ERR_INVALID in
+ * canonical order.  Not capturable. */
+int cq_world_read_ref_order(const cq_world *w, int32_t which, int32_t *order, int32_t *rank);
 
 /* The model matrix of every part (n_parts * 16 floats, column-major, in the order of the parts array given to
  * cq_world_create), as the last completed update left it.  Waits for queued updates like cq_world_read_soup. */
@@ -342,6 +362,8 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  *    CQ_MAS_AGENTS when its grid needs more scratch than an uncaptured call gave it;
  *  - scratch blocks a graph recorded stay allocated when a later uncaptured call outgrows them (the call takes new
  *    blocks), so graphs stay valid until cq_world_destroy, which frees them: replay no graph after destroying its world;
+ *  - cq_world_rebuild replaces the geometry whose addresses a graph recorded: replay no graph recorded before a rebuild
+ *    after it (record it again);
  *  - cq_agent_separation_device and cq_agent_separation_batch (they synchronise to report the outcome), cq_crowd_step
  *    and the host-pointer calls (checked on the world's stream, or on `stream` where they take one) refuse a capture the
  *    same way.

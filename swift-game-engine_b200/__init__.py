@@ -132,6 +132,7 @@ class Counters(C.Structure):
 EXPORTS = [
     "cq_world_create", "cq_world_create_ex", "cq_world_options_default", "cq_world_destroy", "cq_world_get_info", "cq_world_update_transforms",
     "cq_world_update_transforms_async", "cq_world_update_transforms_device", "cq_world_platforms_device", "cq_world_read_soup",
+    "cq_world_read_ref_order", "cq_world_rebuild",
     "cq_world_read_models",
     "cq_world_triangle_material", "cq_static_mesh_load", "cq_static_mesh_free", "cq_static_mesh_part_count",
     "cq_static_mesh_part_name", "cq_static_mesh_part_transform", "cq_static_mesh_hull_count",
@@ -204,6 +205,8 @@ def lib():
         L.cq_world_update_transforms_device.argtypes = [vp, vp, vp, i32, vp, vp]
         L.cq_world_platforms_device.argtypes = [vp, vp, vp, i32, vp, vp, vp]
         L.cq_world_read_soup.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+        L.cq_world_read_ref_order.argtypes = [vp, i32, vp, vp]
+        L.cq_world_rebuild.argtypes = [vp, vp, i32, vp]
         L.cq_world_read_models.argtypes = [vp, vp]
         L.cq_world_triangle_material.argtypes = [vp, i32, C.POINTER(Material)]
         L.cq_static_mesh_load.argtypes = [C.c_char_p, C.POINTER(vp)]
@@ -366,13 +369,20 @@ class CollisionQuery:
     def __init__(self, parts, order=ORDER_REFERENCE):
         """order: ORDER_REFERENCE (default: exact ties and overlap-all overflow resolved in the reference's own visiting
         order, raycasts walk the reference's own tree) or ORDER_CANONICAL (tree-independent rule); include/cq.h."""
-        self._keep = []
+        h = C.c_void_p()
+        keep = []
+        arr, opt = self._parts_args(parts, order, keep)
+        _check(lib().cq_world_create_ex(C.byref(arr), len(parts), C.byref(opt), C.byref(h)))
         self.order = order
+        self._h = h
+
+    @staticmethod
+    def _parts_args(parts, order, keep):
         arr = (MeshPart * max(len(parts), 1))()
         for i, p in enumerate(parts):
             pos = np.ascontiguousarray(p["positions"], np.float32).reshape(-1, 3)
             idx = np.ascontiguousarray(p["indices"], np.uint32).reshape(-1)
-            self._keep += [pos, idx]
+            keep += [pos, idx]
             arr[i].positions_xyz = pos.ctypes.data
             arr[i].indices = idx.ctypes.data
             arr[i].n_verts = pos.shape[0]
@@ -386,11 +396,17 @@ class CollisionQuery:
             arr[i].flatten_ground = int(bool(p.get("flatten_ground", False)))
             arr[i].is_dynamic = int(bool(p.get("is_dynamic", False)))
             arr[i].entity_id = int(p.get("entity_id", i))
-        h = C.c_void_p()
-        opt = _world_options(parts, order, self._keep)
-        _check(lib().cq_world_create_ex(C.byref(arr), len(parts), C.byref(opt), C.byref(h)))
-        self._h = h
-        self._keep = []
+        return arr, _world_options(parts, order, keep)
+
+    def rebuild(self, parts, order=None):
+        """cq_world_rebuild: the world in place from new parts, as a fresh CollisionQuery(parts, order) would be (order
+        None keeps the world's).  On failure CQError is raised and the world answers exactly as before.  Crowds made on
+        the world stay valid; CUDA graphs recorded before the rebuild must not be replayed after it."""
+        order = self.order if order is None else order
+        keep = []
+        arr, opt = self._parts_args(parts, order, keep)
+        _check(lib().cq_world_rebuild(self._h, C.byref(arr), len(parts), C.byref(opt)))
+        self.order = order
 
     def close(self):
         if getattr(self, "_h", None):
@@ -423,6 +439,14 @@ class CollisionQuery:
         par = np.zeros(nt, np.int32)
         _check(lib().cq_world_read_soup(self._h, which, _ptr(pos), _ptr(idx), _ptr(aabb), _ptr(lay), _ptr(par)))
         return {"positions": pos, "indices": idx, "aabbs": aabb, "layers": lay, "parts": par}
+
+    def read_ref_order(self, which=0):
+        """cq_world_read_ref_order: (order, rank) of the reference's tree of one set, set-local triangle numbering."""
+        inf = self.info()
+        nt = inf["n_dynamic_triangles"] if which else inf["n_static_triangles"]
+        order, rank = np.zeros(nt, np.int32), np.zeros(nt, np.int32)
+        _check(lib().cq_world_read_ref_order(self._h, which, _ptr(order), _ptr(rank)))
+        return order, rank
 
     def read_models(self):
         """cq_world_read_models: every part's current model matrix, (n_parts, 16) column-major, in parts order."""

@@ -69,6 +69,18 @@ class CollisionQuery {
             throw std::runtime_error(std::string("cq_world_create: ") + cq_last_error());
     }
     ~CollisionQuery() { cq_world_destroy(w_); }
+    // cq_world_rebuild: the same world from new parts, as a fresh CollisionQuery(parts, ...) would be.  On failure it
+    // throws and the world answers exactly as before.  Crowds stay valid; graphs recorded before must not be replayed.
+    void rebuild(const std::vector<cq_mesh_part> &parts, bool referenceOrder = true,
+                 const std::vector<cq_triangle_materials> &triangleMaterials = {}) {
+        cq_world_options opt;
+        cq_world_options_default(&opt);
+        opt.order = referenceOrder ? CQ_ORDER_REFERENCE : CQ_ORDER_CANONICAL;
+        opt.n_triangle_materials = (int32_t)triangleMaterials.size();
+        opt.triangle_materials = triangleMaterials.empty() ? nullptr : triangleMaterials.data();
+        if (cq_world_rebuild(w_, parts.data(), (int32_t)parts.size(), &opt) != CQ_OK)
+            throw std::runtime_error(std::string("cq_world_rebuild: ") + cq_last_error());
+    }
     CollisionQuery(const CollisionQuery &) = delete;
     CollisionQuery &operator=(const CollisionQuery &) = delete;
 

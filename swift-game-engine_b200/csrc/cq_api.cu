@@ -488,6 +488,134 @@ void cq_world_options_default(cq_world_options *o) {
     o->order = CQ_ORDER_REFERENCE;
 }
 
+// The geometry of a world, everything cq_world_rebuild replaces: the part table, models and materials, both triangle sets
+// with their LBVHs, the reference order and the entity index of the device updates.  Built into `w` on w->stream, the
+// only world resource it uses (with w->view.status for the sort's overflow flag).  Shared by cq_world_create_ex and
+// cq_world_rebuild; on failure the caller frees what was built (free_geometry).
+static int build_geometry(cq_world *w, const cq_mesh_part *parts, int32_t n_parts, const cq_world_options &opt) {
+    int rc = CQ_OK;
+    // host-side assembly of the two sets' input arrays (partitionEntities, CollisionQuery.swift:886-900): cq_assemble.h
+    SetPlan input[2];
+    std::vector<PartPlacement> place;
+    const PlanError bad = plan_upload(parts, n_parts, input, place);
+    if (bad.code != CQ_OK) {
+        if (bad.kind == 3)
+            set_error("cq_world_create: more than 2^31 vertices or indices in one triangle set (at part %d)", bad.part);
+        else
+            set_error("cq_world_create: part %d has invalid arrays", bad.part);
+        return bad.code;
+    }
+    std::vector<float> models((size_t)n_parts * 16);
+    std::vector<float4> materials(n_parts);
+    // per-triangle materials (options->triangle_materials): rows appended to the table after the parts' own rows; a part
+    // whose array does not have exactly one entry per triangle keeps its own material (CollisionQuery.swift:365-369)
+    std::vector<int32_t> matIn[2];
+    if (opt.n_triangle_materials > 0) {
+        if (!opt.triangle_materials) {
+            set_error("cq_world_create_ex: n_triangle_materials = %d without an array", opt.n_triangle_materials);
+            return CQ_ERR_INVALID;
+        }
+        for (int k = 0; k < opt.n_triangle_materials; k++) {
+            const cq_triangle_materials &tm = opt.triangle_materials[k];
+            for (int s = 0; s < 2; s++)
+                for (const PartRow &row : input[s].rows) {
+                    if (parts[row.part].entity_id != tm.entity_id || tm.n != row.nTris || row.nTris == 0) continue;
+                    if (!tm.materials) {
+                        set_error("cq_world_create_ex: triangle_materials[%d] has no array", k);
+                        return CQ_ERR_INVALID;
+                    }
+                    if (matIn[s].empty()) { // default: every input triangle points at its part's row
+                        matIn[s].resize(input[s].nTris);
+                        for (const PartRow &r : input[s].rows) std::fill_n(matIn[s].begin() + r.triStart, r.nTris, r.part);
+                    }
+                    const int32_t base = (int32_t)materials.size();
+                    for (int t = 0; t < row.nTris; t++) {
+                        const cq_surface_material &m = tm.materials[t];
+                        materials.push_back(make_float4(m.mu_s, m.mu_k, m.flatten_ground ? 1.0f : 0.0f, 0.0f));
+                        matIn[s][(size_t)row.triStart + t] = base + t;
+                    }
+                }
+        }
+    }
+    w->parts.resize(n_parts);
+    for (int p = 0; p < n_parts; p++) {
+        const cq_mesh_part &mp = parts[p];
+        PartInfo &pi = w->parts[p];
+        pi.entityId = mp.entity_id;
+        pi.set = place[p].set;
+        pi.vertLo = place[p].vertLo, pi.vertHi = place[p].vertHi;
+        pi.material = {mp.mu_s, mp.mu_k, mp.flatten_ground ? 1 : 0};
+        pi.layer = mp.layer;
+        memcpy(&models[(size_t)p * 16], mp.model, sizeof(float) * 16);
+        materials[p] = make_float4(mp.mu_s, mp.mu_k, mp.flatten_ground ? 1.0f : 0.0f, 0.0f);
+        w->partsOfEntity[mp.entity_id].push_back(p);
+    }
+    w->movedSlot.assign(n_parts, -1);
+
+    if ((rc = check_cuda(cudaMalloc((void **)&w->dModels, sizeof(float) * 16 * (size_t)std::max(n_parts, 1)), "models")) != CQ_OK)
+        return rc;
+    if ((rc = check_cuda(cudaMalloc((void **)&w->dMaterials, sizeof(float4) * std::max(materials.size(), (size_t)1)), "materials")) != CQ_OK)
+        return rc;
+    w->hMaterials.resize(materials.size());
+    for (size_t k = 0; k < materials.size(); k++) w->hMaterials[k] = {materials[k].x, materials[k].y, materials[k].z != 0.0f ? 1 : 0};
+    if (n_parts) {
+        cudaMemcpyAsync(w->dModels, models.data(), sizeof(float) * 16 * (size_t)n_parts, cudaMemcpyHostToDevice, w->stream);
+        cudaMemcpyAsync(w->dMaterials, materials.data(), sizeof(float4) * materials.size(), cudaMemcpyHostToDevice, w->stream);
+    }
+    w->buildMs = 0.0f; // accumulated by build_set: device time of the build kernels only
+    for (int s = 0; s < 2; s++) {
+        std::vector<int> &partTriStart = input[s].partTriStart; // in: before the degenerate filter; out: after
+        int badTri = -1;
+        rc = build_set(w, w->set[s], input[s], partTriStart, &badTri, matIn[s].empty() ? nullptr : matIn[s].data());
+        if (rc != CQ_OK && badTri >= 0) { // name the part and the first offending index of that triangle
+            const PartRow &row = input[s].rows[part_row_of(input[s].rows.data(), (int)input[s].rows.size(), badTri, true)];
+            const uint32_t *tri = parts[row.part].indices + 3 * (size_t)(badTri - row.triStart);
+            uint32_t li = tri[0];
+            for (int k = 2; k >= 0; k--)
+                if (tri[k] >= (uint32_t)row.nVerts) li = tri[k];
+            set_error("cq_world_create: part %d index %u out of range (%d vertices)", row.part, li, row.nVerts);
+        }
+        if (rc != CQ_OK) return rc;
+        for (size_t k = 0; k < input[s].partOfSet.size(); k++) {
+            PartInfo &pi = w->parts[input[s].partOfSet[k]];
+            pi.triLo = partTriStart[k];
+            pi.triHi = partTriStart[k + 1];
+        }
+    }
+    if ((rc = check_cuda(cudaStreamSynchronize(w->stream), "build")) != CQ_OK) return rc;
+    for (int s = 0; s < 2; s++)
+        if (w->set[s].triMat && w->set[s].nTris > 0) { // host copy for cq_world_triangle_material
+            w->hTriMat[s].resize((size_t)w->set[s].nTris);
+            if ((rc = check_cuda(cudaMemcpy(w->hTriMat[s].data(), w->set[s].triMat, sizeof(int32_t) * (size_t)w->set[s].nTris,
+                                            cudaMemcpyDeviceToHost), "triangle materials")) != CQ_OK)
+                return rc;
+        }
+    if (w->order == CQ_ORDER_REFERENCE && (rc = attach_ref_order(w)) != CQ_OK) return rc;
+    if ((rc = upload_entity_index(w)) != CQ_OK) return rc;
+    return CQ_OK;
+}
+
+// The device memory build_geometry allocates.
+static void free_geometry(cq_world *w) {
+    for (int s = 0; s < 2; s++) free_set(w->set[s]);
+    cudaFree(w->dModels), cudaFree(w->dMaterials), cudaFree(w->dRank), cudaFree(w->dEncOfRank), cudaFree(w->devArena);
+    w->dModels = nullptr, w->dMaterials = nullptr, w->dRank = nullptr, w->dEncOfRank = nullptr, w->devArena = nullptr;
+}
+
+// Exchange what build_geometry built between two worlds (everything else stays with its world).
+static void swap_geometry(cq_world *a, cq_world *b) {
+    using std::swap;
+    swap(a->order, b->order);
+    swap(a->set[0], b->set[0]), swap(a->set[1], b->set[1]);
+    swap(a->parts, b->parts), swap(a->dModels, b->dModels), swap(a->dMaterials, b->dMaterials);
+    swap(a->hMaterials, b->hMaterials), swap(a->hTriMat[0], b->hTriMat[0]), swap(a->hTriMat[1], b->hTriMat[1]);
+    swap(a->dRank, b->dRank), swap(a->dEncOfRank, b->dEncOfRank), swap(a->refBuildMs, b->refBuildMs), swap(a->buildMs, b->buildMs);
+    swap(a->partsOfEntity, b->partsOfEntity), swap(a->movedSlot, b->movedSlot);
+    swap(a->devArena, b->devArena), swap(a->dEntityIds, b->dEntityIds), swap(a->dEntityOff, b->dEntityOff);
+    swap(a->dEntries, b->dEntries), swap(a->dLastWriter, b->dLastWriter), swap(a->dDevHdr, b->dDevHdr);
+    swap(a->dDevTable, b->dDevTable), swap(a->nEntities, b->nEntities), swap(a->devRows0, b->devRows0);
+}
+
 int cq_world_create(const cq_mesh_part *parts, int32_t n_parts, cq_world **out) {
     return cq_world_create_ex(parts, n_parts, nullptr, out);
 }
@@ -531,70 +659,6 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
     if ((rc = check_cuda(cudaEventCreate(&w->evB), "event")) != CQ_OK) return fail(rc);
     if ((rc = check_cuda(cudaEventCreateWithFlags(&w->evTrees, cudaEventDisableTiming), "event")) != CQ_OK) return fail(rc);
 
-    // host-side assembly of the two sets' input arrays (partitionEntities, CollisionQuery.swift:886-900): cq_assemble.h
-    SetPlan input[2];
-    std::vector<PartPlacement> place;
-    const PlanError bad = plan_upload(parts, n_parts, input, place);
-    if (bad.code != CQ_OK) {
-        if (bad.kind == 3)
-            set_error("cq_world_create: more than 2^31 vertices or indices in one triangle set (at part %d)", bad.part);
-        else
-            set_error("cq_world_create: part %d has invalid arrays", bad.part);
-        return fail(bad.code);
-    }
-    std::vector<float> models((size_t)n_parts * 16);
-    std::vector<float4> materials(n_parts);
-    // per-triangle materials (options->triangle_materials): rows appended to the table after the parts' own rows; a part
-    // whose array does not have exactly one entry per triangle keeps its own material (CollisionQuery.swift:365-369)
-    std::vector<int32_t> matIn[2];
-    if (opt.n_triangle_materials > 0) {
-        if (!opt.triangle_materials) {
-            set_error("cq_world_create_ex: n_triangle_materials = %d without an array", opt.n_triangle_materials);
-            return fail(CQ_ERR_INVALID);
-        }
-        for (int k = 0; k < opt.n_triangle_materials; k++) {
-            const cq_triangle_materials &tm = opt.triangle_materials[k];
-            for (int s = 0; s < 2; s++)
-                for (const PartRow &row : input[s].rows) {
-                    if (parts[row.part].entity_id != tm.entity_id || tm.n != row.nTris || row.nTris == 0) continue;
-                    if (!tm.materials) {
-                        set_error("cq_world_create_ex: triangle_materials[%d] has no array", k);
-                        return fail(CQ_ERR_INVALID);
-                    }
-                    if (matIn[s].empty()) { // default: every input triangle points at its part's row
-                        matIn[s].resize(input[s].nTris);
-                        for (const PartRow &r : input[s].rows) std::fill_n(matIn[s].begin() + r.triStart, r.nTris, r.part);
-                    }
-                    const int32_t base = (int32_t)materials.size();
-                    for (int t = 0; t < row.nTris; t++) {
-                        const cq_surface_material &m = tm.materials[t];
-                        materials.push_back(make_float4(m.mu_s, m.mu_k, m.flatten_ground ? 1.0f : 0.0f, 0.0f));
-                        matIn[s][(size_t)row.triStart + t] = base + t;
-                    }
-                }
-        }
-    }
-    w->parts.resize(n_parts);
-    for (int p = 0; p < n_parts; p++) {
-        const cq_mesh_part &mp = parts[p];
-        PartInfo &pi = w->parts[p];
-        pi.entityId = mp.entity_id;
-        pi.set = place[p].set;
-        pi.vertLo = place[p].vertLo, pi.vertHi = place[p].vertHi;
-        pi.material = {mp.mu_s, mp.mu_k, mp.flatten_ground ? 1 : 0};
-        pi.layer = mp.layer;
-        memcpy(&models[(size_t)p * 16], mp.model, sizeof(float) * 16);
-        materials[p] = make_float4(mp.mu_s, mp.mu_k, mp.flatten_ground ? 1.0f : 0.0f, 0.0f);
-        w->partsOfEntity[mp.entity_id].push_back(p);
-    }
-    w->movedSlot.assign(n_parts, -1);
-
-    if ((rc = check_cuda(cudaMalloc((void **)&w->dModels, sizeof(float) * 16 * (size_t)std::max(n_parts, 1)), "models")) != CQ_OK)
-        return fail(rc);
-    if ((rc = check_cuda(cudaMalloc((void **)&w->dMaterials, sizeof(float4) * std::max(materials.size(), (size_t)1)), "materials")) != CQ_OK)
-        return fail(rc);
-    w->hMaterials.resize(materials.size());
-    for (size_t k = 0; k < materials.size(); k++) w->hMaterials[k] = {materials[k].x, materials[k].y, materials[k].z != 0.0f ? 1 : 0};
     if ((rc = check_cuda(cudaMalloc((void **)&w->dCounters, sizeof(unsigned long long) * 4), "counters")) != CQ_OK) return fail(rc);
     cudaMemsetAsync(w->dCounters, 0, sizeof(unsigned long long) * 4, w->stream);
     if ((rc = check_cuda(cudaMalloc((void **)&w->dWork, sizeof(int) * CQ_WORK_RING), "work counters")) != CQ_OK) return fail(rc);
@@ -602,51 +666,61 @@ int cq_world_create_ex(const cq_mesh_part *parts, int32_t n_parts, const cq_worl
         return fail(rc);
     *w->hStatus = 0;
     cudaHostGetDevicePointer((void **)&w->view.status, w->hStatus, 0);
-    if (n_parts) {
-        cudaMemcpyAsync(w->dModels, models.data(), sizeof(float) * 16 * (size_t)n_parts, cudaMemcpyHostToDevice, w->stream);
-        cudaMemcpyAsync(w->dMaterials, materials.data(), sizeof(float4) * materials.size(), cudaMemcpyHostToDevice, w->stream);
-    }
-    w->buildMs = 0.0f; // accumulated by build_set: device time of the build kernels only
-    for (int s = 0; s < 2; s++) {
-        std::vector<int> &partTriStart = input[s].partTriStart; // in: before the degenerate filter; out: after
-        int badTri = -1;
-        rc = build_set(w, w->set[s], input[s], partTriStart, &badTri, matIn[s].empty() ? nullptr : matIn[s].data());
-        if (rc != CQ_OK && badTri >= 0) { // name the part and the first offending index of that triangle
-            const PartRow &row = input[s].rows[part_row_of(input[s].rows.data(), (int)input[s].rows.size(), badTri, true)];
-            const uint32_t *tri = parts[row.part].indices + 3 * (size_t)(badTri - row.triStart);
-            uint32_t li = tri[0];
-            for (int k = 2; k >= 0; k--)
-                if (tri[k] >= (uint32_t)row.nVerts) li = tri[k];
-            set_error("cq_world_create: part %d index %u out of range (%d vertices)", row.part, li, row.nVerts);
-        }
-        if (rc != CQ_OK) return fail(rc);
-        for (size_t k = 0; k < input[s].partOfSet.size(); k++) {
-            PartInfo &pi = w->parts[input[s].partOfSet[k]];
-            pi.triLo = partTriStart[k];
-            pi.triHi = partTriStart[k + 1];
-        }
-    }
-    if ((rc = check_cuda(cudaStreamSynchronize(w->stream), "build")) != CQ_OK) return fail(rc);
-    for (int s = 0; s < 2; s++)
-        if (w->set[s].triMat && w->set[s].nTris > 0) { // host copy for cq_world_triangle_material
-            w->hTriMat[s].resize((size_t)w->set[s].nTris);
-            if ((rc = check_cuda(cudaMemcpy(w->hTriMat[s].data(), w->set[s].triMat, sizeof(int32_t) * (size_t)w->set[s].nTris,
-                                            cudaMemcpyDeviceToHost), "triangle materials")) != CQ_OK)
-                return fail(rc);
-        }
-    if (w->order == CQ_ORDER_REFERENCE && (rc = attach_ref_order(w)) != CQ_OK) return fail(rc);
-    if ((rc = upload_entity_index(w)) != CQ_OK) return fail(rc);
+    if ((rc = build_geometry(w, parts, n_parts, opt)) != CQ_OK) return fail(rc);
     make_view(w);
     *out = w;
     return CQ_OK;
+}
+
+int cq_world_rebuild(cq_world *w, const cq_mesh_part *parts, int32_t n_parts, const cq_world_options *options) {
+    if (!w || n_parts < 0 || (n_parts > 0 && !parts)) {
+        set_error("cq_world_rebuild: invalid arguments");
+        return CQ_ERR_INVALID;
+    }
+    cq_world_options opt;
+    cq_world_options_default(&opt);
+    if (options) opt = *options;
+    if (opt.order != CQ_ORDER_REFERENCE && opt.order != CQ_ORDER_CANONICAL) {
+        set_error("cq_world_rebuild: unknown order %d", opt.order);
+        return CQ_ERR_INVALID;
+    }
+    CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_rebuild");
+    for (const ReaderEvent &e : w->readers) CQ_NO_CAPTURE(e.st, "cq_world_rebuild"); // a graph being recorded on the world
+    // the new geometry is built aside, into a staging world that borrows this world's stream and status word; the
+    // world keeps answering from its old geometry until the swap
+    cq_world *g = new cq_world();
+    g->device = w->device, g->numSms = w->numSms, g->order = opt.order, g->stream = w->stream, g->view.status = w->view.status;
+    int rc = build_geometry(g, parts, n_parts, opt);
+    if (rc == CQ_OK) {
+        // launches already queued on any stream may still read the old trees (every launch records its stream's reader
+        // event, every stream-ordered refit records evTrees): wait for them, not for the whole device
+        for (ReaderEvent &e : w->readers)
+            if (rc == CQ_OK) rc = check_cuda(cudaEventSynchronize(e.ev), "cq_world_rebuild");
+        if (rc == CQ_OK) rc = check_cuda(cudaEventSynchronize(w->evTrees), "cq_world_rebuild");
+    }
+    if (rc == CQ_OK) {
+        for (ReaderEvent &e : w->readers) e.pending = false;
+        w->treesPending = false;
+        swap_geometry(w, g);
+        w->movedRows[0].clear(), w->movedRows[1].clear();
+        sep_graphs_destroy(w); // its instantiated graphs hold the old geometry's addresses
+        make_view(w);
+        w->launches += g->launches;
+    }
+    cudaStreamSynchronize(w->stream); // on failure, the staging build's copies may still be queued
+    free_geometry(g);                 // the old geometry after a swap, the new one after a failure
+    g->stream = nullptr;
+    delete g;
+    return rc;
 }
 
 void cq_world_destroy(cq_world *w) {
     if (!w) return;
     cudaSetDevice(w->device);
     cudaDeviceSynchronize(); // *_device launches may still be in flight on the caller's streams
-    for (int s = 0; s < 2; s++) free_set(w->set[s]);
-    cudaFree(w->dModels), cudaFree(w->dMaterials), cudaFree(w->dCounters), cudaFree(w->dWork), cudaFree(w->dRank), cudaFree(w->dEncOfRank);
+    free_geometry(w);
+    cudaFree(w->dCounters), cudaFree(w->dWork);
     if (w->hStatus) cudaFreeHost(w->hStatus);
     destroy_scratch(w->in), destroy_scratch(w->out), destroy_scratch(w->aux), destroy_scratch(w->aux2);
     for (int k = 0; k < 4; k++) destroy_scratch(w->nodeScratch[k]), destroy_scratch(w->orderScratch[k]);
@@ -654,7 +728,6 @@ void cq_world_destroy(cq_world *w) {
     sep_graphs_destroy(w);
     destroy_scratch(w->sepScratch);
     destroy_scratch(w->dTable);
-    cudaFree(w->devArena);
     for (void *p : w->graphScratch) cudaFree(p);
     free_retired(w);
     for (StageSlot &s : w->stage) {
@@ -779,6 +852,31 @@ int cq_world_read_soup(const cq_world *w, int32_t which, float *positions_xyz, u
         CQ_CUDA(cudaMemcpy(tri_layers, S.triLayer, sizeof(uint32_t) * (size_t)S.nTris, cudaMemcpyDeviceToHost));
     if (tri_parts && S.nTris)
         CQ_CUDA(cudaMemcpy(tri_parts, S.triPart, sizeof(int32_t) * (size_t)S.nTris, cudaMemcpyDeviceToHost));
+    return CQ_OK;
+}
+
+int cq_world_read_ref_order(const cq_world *w, int32_t which, int32_t *order, int32_t *rank) {
+    if (!w || which < 0 || which > 1) return CQ_ERR_INVALID;
+    if (w->order != CQ_ORDER_REFERENCE) {
+        set_error("cq_world_read_ref_order: the world was created in canonical order");
+        return CQ_ERR_INVALID;
+    }
+    CQ_CUDA(cudaSetDevice(w->device));
+    CQ_NO_CAPTURE(w->stream, "cq_world_read_ref_order");
+    const DeviceSet &S = w->set[which];
+    const int n = S.nTris, off = which ? w->set[0].nTris : 0;
+    if (n <= 0) return CQ_OK;
+    CQ_CUDA(cudaStreamSynchronize(w->stream));
+    if (order) { // triOrder position -> sorted slot -> soup triangle
+        std::vector<uint32_t> slot(n), sorted(n);
+        CQ_CUDA(cudaMemcpy(slot.data(), S.refSlot, sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToHost));
+        CQ_CUDA(cudaMemcpy(sorted.data(), S.sortedTri, sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToHost));
+        for (int p = 0; p < n; p++) order[p] = (int32_t)sorted[slot[p]];
+    }
+    if (rank) {
+        CQ_CUDA(cudaMemcpy(rank, w->dRank + off, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost));
+        for (int t = 0; t < n; t++) rank[t] -= off;
+    }
     return CQ_OK;
 }
 

@@ -14,7 +14,6 @@
 #include <cstring>
 
 #include "cq_internal.h"
-#include "cq_reftree.h"
 
 namespace cq {
 
@@ -1410,7 +1409,7 @@ int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dState
     return check_cuda(cudaGetLastError(), "agent grid");
 }
 
-// ---------------------------------------------------------------- reference order (cq_reftree.h)
+// ---------------------------------------------------------------- reference order
 // Boxes of the reference's tree, bottom-up: one thread per leaf computes boundsForRange (CollisionQuery.swift:662-677)
 // from the leaf's triangles, writes it into its parent's child slot and climbs while it is the second child to arrive
 // (merge = component-wise min / max, :700-702 — exact, so the arrival order does not matter).  Arrival counters are
@@ -1473,82 +1472,521 @@ static int ref_fit(cq_world *w, DeviceSet &S, cudaStream_t st, const RefitCounts
     return check_cuda(cudaGetLastError(), "k_ref_fit");
 }
 
-static inline float int_bits_as_float(int v) {
-    float f;
-    memcpy(&f, &v, sizeof(f));
-    return f;
+// The reference's own tree (CollisionQuery.swift:577-670), cut on the device.  The split rule is the reference's: centroid
+// bounds of the range (:679-694), longest axis with x beating y beating z on ties (:602-610), spatial-median pivot
+// (:612-617), the swap-with-tail partition (:617-634), the stable sort by the centroid on that axis cut at count / 2 when
+// everything lands on one side (:637-653), leaves of at most 4 triangles (:473).  tests/hostmath/reftree.cpp compiles the
+// host restatement (cq_reftree.h) that the tests compare this build with.
+//
+// The swap-with-tail loop examines a merge of two streams: the range read forwards from its start and backwards from its
+// end.  After a `< pivot` element the next one comes from the forward stream, after a `>=` one from the backward stream,
+// and exactly `count` elements are examined; `<` elements fill the front and `>=` ones the back, both in examination
+// order.  So run k of the forward stream ends at its k-th `>=` element and run k of the backward stream at its k-th `<`,
+// and every destination follows from prefix counts (k_lv_less, k_lv_scatter; the numpy model is in tests/test_ref_tree_device.py).
+//
+// Shape: ranges above RT_SMALL triangles are cut level by level, in tiles of RT_THREADS positions with one CTA per tile
+// and one per range for the plane, the scan of the tiles' counts and the fallback (the host reads one count per level;
+// the number of levels is the depth of the tree's top, which the refusal below bounds); ranges of at most RT_SMALL
+// triangles are finished depth-first by one thread each, with the reference's loop itself.  No node gets an id while the
+// tree is cut: the leaves partition [0, n), so a leaf is named by its start and an internal node by its cut (the start
+// of its right child), which is the start of exactly one leaf.  Records are written at those positions, and one scan
+// over the leaf starts numbers both kinds (leaf id = leaf starts before it; internal id = leaf id of its cut - 1).
+//
+// Centroids with a NaN component follow the host's sequential bounds (a NaN first element makes that bound NaN, later
+// NaNs are ignored) and its comparisons (NaN is never `< pivot`).  Both tiers' median fallback orders keys by their bits
+// with -0 and +0 as one key and NaN above +inf (below -inf with the sign bit set).  std::stable_sort leaves NaN keys
+// unordered, so a range whose fallback sorts a NaN key is deterministic here but need not match the host builder.  A NaN
+// vertex is NaN in all three world coordinates (the model matrix multiplies it by zero too), so a NaN triangle that comes
+// first in a range makes the pivot NaN and sends that range to the fallback.  An infinite vertex coordinate passes the
+// degenerate filter too and gives an infinite centroid (with NaN in the other two coordinates): infinities are ordinary
+// values here (an extent inf - inf is NaN and loses every `>=` of the axis choice, the fallback's key orders +-inf as `<`
+// does), so such trees equal the host builder's.
+#define RT_THREADS 256
+#define RT_SMALL 32 // ranges of at most this many triangles: one thread each
+
+struct RtSeg {
+    int32_t start, count, pw, depth; // pw: (cut of the parent << 1) | right child, -1 for the root
+};
+
+struct RtLevel {
+    int32_t axis, totL; // totL: elements < pivot in the range
+    float pivot;
+};
+
+struct RtBuf {
+    float4 *items, *tmp;      // (centroid xyz, bits(soup triangle)), in triOrder positions once cut
+    int32_t *less;            // per position: 2 * (elements < pivot before it in its range) + (it is < pivot)
+    int32_t *lenF, *lenB;     // per range: element count of the first k runs of each stream, at start + k - 1
+    int32_t *leafCnt, *leafPar; // at a leaf's start: its count (0 = no leaf starts here), its parent as pw
+    int32_t *intPar;          // at an internal node's cut: pw + 2 (0 = no node)
+    RtSeg *segA, *segB, *small;
+    int32_t *ctr;             // [0] ranges of the next level, [1] small ranges, [2] deepest leaf
+    uint32_t *flag, *leafId, *tileSums, *total;
+    // one level of ranges above RT_SMALL: per range its first tile and split; per tile its range, bounds, `<` count
+    uint32_t *segTile, *nTiles;
+    struct RtLevel *lvl;
+    int32_t *tileSeg;
+    float4 *tileLo, *tileHi;
+    uint32_t *tileLess;
+};
+
+__host__ __device__ __forceinline__ int rt_tiles(int count) { return (count + RT_THREADS - 1) / RT_THREADS; }
+__device__ __forceinline__ float rt_axis(const float4 &c, int a) { return a == 0 ? c.x : (a == 1 ? c.y : c.z); }
+// std::stable_sort's `<` on a float as an unsigned order: -0 and +0 are one key
+__device__ __forceinline__ uint32_t rt_sort_key(float v) {
+    const uint32_t u = __float_as_uint(v == 0.0f ? 0.0f : v);
+    return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ void rt_plane(const float lo[3], const float hi[3], int &axis, float &pivot) {
+    const float ex = hi[0] - lo[0], ey = hi[1] - lo[1], ez = hi[2] - lo[2];
+    axis = (ex >= ey && ex >= ez) ? 0 : (ey >= ez ? 1 : 2);
+    pivot = (lo[axis] + hi[axis]) * 0.5f;
 }
 
-// Reference order: download the sets' triangle boxes, rebuild the reference's tree on the host (cq_reftree.h), upload
-// the visiting ranks (one global array, static set first like the reference's own merge of its two sets,
-// CollisionQuery.swift:990-1008) and the tree itself for the ray walk.
+// a child range: a leaf is recorded at once, a larger range queued for the next level (`next`) or for the small pass
+__device__ void rt_child(const RtBuf &B, RtSeg *next, int32_t start, int32_t count, int32_t pw, int32_t depth) {
+    if (count <= 4) {
+        B.leafCnt[start] = count, B.leafPar[start] = pw;
+        atomicMax(&B.ctr[2], depth);
+    } else if (count <= RT_SMALL) {
+        B.small[atomicAdd(&B.ctr[1], 1)] = RtSeg{start, count, pw, depth};
+    } else {
+        next[atomicAdd(&B.ctr[0], 1)] = RtSeg{start, count, pw, depth};
+    }
+}
+
+__global__ void k_rt_items(const float4 *__restrict__ boxLo, const float4 *__restrict__ boxHi, const uint32_t *__restrict__ sortedTri,
+                           int n, RtBuf B) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const float4 l = boxLo[n - 1 + k], h = boxHi[n - 1 + k]; // leaf boxes of the sorted order
+    const uint32_t t = sortedTri[k];
+    B.items[t] = make_float4((l.x + h.x) * 0.5f, (l.y + h.y) * 0.5f, (l.z + h.z) * 0.5f, __uint_as_float(t));
+}
+
+__global__ void k_rt_root(int n, RtBuf B) {
+    B.ctr[0] = B.ctr[1] = B.ctr[2] = 0;
+    rt_child(B, B.segA, 0, n, -1, 0);
+}
+
+__device__ __forceinline__ void rt_block_bounds(float lo[3], float hi[3], float (*sm)[RT_THREADS / 32]) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+#pragma unroll
+        for (int o = 16; o; o >>= 1) {
+            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+        }
+        if (lane == 0) sm[a][warp] = lo[a], sm[3 + a][warp] = hi[a];
+    }
+    __syncthreads();
+#pragma unroll
+    for (int a = 0; a < 3; a++) {
+        lo[a] = sm[a][0], hi[a] = sm[3 + a][0];
+        for (int k = 1; k < RT_THREADS / 32; k++) lo[a] = fminf(lo[a], sm[a][k]), hi[a] = fmaxf(hi[a], sm[3 + a][k]);
+    }
+    __syncthreads();
+}
+
+// ---- one level of ranges above RT_SMALL triangles: tiles of RT_THREADS positions, one CTA per tile (a tile belongs to
+// one range), and one CTA per range for the steps that need the whole range
+__global__ void k_lv_tile_counts(const RtSeg *__restrict__ segs, int nSeg, uint32_t *__restrict__ tiles) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < nSeg) tiles[i] = (uint32_t)rt_tiles(segs[i].count);
+}
+
+__global__ void k_lv_map(const RtSeg *__restrict__ segs, RtBuf B) {
+    const int n = rt_tiles(segs[blockIdx.x].count), off = (int)B.segTile[blockIdx.x];
+    for (int t = threadIdx.x; t < n; t += blockDim.x) B.tileSeg[off + t] = blockIdx.x;
+}
+
+// this CTA's tile: its range and the position of this thread (valid = inside the range); false past the last tile
+__device__ __forceinline__ bool rt_tile(const RtSeg *__restrict__ segs, const RtBuf &B, int &si, RtSeg &g, int &p, bool &valid) {
+    if (blockIdx.x >= *B.nTiles) return false;
+    si = B.tileSeg[blockIdx.x];
+    g = segs[si];
+    p = g.start + ((int)blockIdx.x - (int)B.segTile[si]) * RT_THREADS + (int)threadIdx.x;
+    valid = p < g.start + g.count;
+    return true;
+}
+
+__global__ void __launch_bounds__(RT_THREADS) k_lv_bounds(const RtSeg *__restrict__ segs, RtBuf B) {
+    __shared__ float sb[6][RT_THREADS / 32];
+    int si, p;
+    RtSeg g;
+    bool valid;
+    if (!rt_tile(segs, B, si, g, p, valid)) return;
+    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    if (valid) {
+        const float4 v = B.items[p];
+        lo[0] = hi[0] = v.x, lo[1] = hi[1] = v.y, lo[2] = hi[2] = v.z;
+    }
+    rt_block_bounds(lo, hi, sb);
+    if (threadIdx.x == 0) {
+        B.tileLo[blockIdx.x] = make_float4(lo[0], lo[1], lo[2], 0.0f);
+        B.tileHi[blockIdx.x] = make_float4(hi[0], hi[1], hi[2], 0.0f);
+    }
+}
+
+// Bounds of a range from its tiles: an ordinary min / max, except that the host's sequential `v < lo ? v : lo` seeded
+// with the first element keeps a NaN first element and ignores every later NaN (fminf / fmaxf ignore NaN).
+__global__ void __launch_bounds__(RT_THREADS) k_lv_plane(const RtSeg *__restrict__ segs, RtBuf B) {
+    __shared__ float sb[6][RT_THREADS / 32];
+    const RtSeg g = segs[blockIdx.x];
+    const int off = (int)B.segTile[blockIdx.x], nT = rt_tiles(g.count);
+    float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+    for (int t = threadIdx.x; t < nT; t += RT_THREADS) {
+        const float4 l = B.tileLo[off + t], h = B.tileHi[off + t];
+        lo[0] = fminf(lo[0], l.x), lo[1] = fminf(lo[1], l.y), lo[2] = fminf(lo[2], l.z);
+        hi[0] = fmaxf(hi[0], h.x), hi[1] = fmaxf(hi[1], h.y), hi[2] = fmaxf(hi[2], h.z);
+    }
+    rt_block_bounds(lo, hi, sb);
+    if (threadIdx.x) return;
+    const float4 first = B.items[g.start];
+    if (isnan(first.x)) lo[0] = hi[0] = first.x;
+    if (isnan(first.y)) lo[1] = hi[1] = first.y;
+    if (isnan(first.z)) lo[2] = hi[2] = first.z;
+    RtLevel L;
+    rt_plane(lo, hi, L.axis, L.pivot);
+    L.totL = 0;
+    B.lvl[blockIdx.x] = L;
+}
+
+__global__ void __launch_bounds__(RT_THREADS) k_lv_count(const RtSeg *__restrict__ segs, RtBuf B) {
+    int si, p;
+    RtSeg g;
+    bool valid;
+    if (!rt_tile(segs, B, si, g, p, valid)) return;
+    const RtLevel L = B.lvl[si];
+    const int c = __syncthreads_count(valid && rt_axis(B.items[p], L.axis) < L.pivot);
+    if (threadIdx.x == 0) B.tileLess[blockIdx.x] = (uint32_t)c;
+}
+
+// per range: exclusive scan of its tiles' `< pivot` counts, in place; the range's total
+__global__ void __launch_bounds__(RT_THREADS) k_lv_scan(const RtSeg *__restrict__ segs, RtBuf B) {
+    __shared__ uint32_t sw[33];
+    const int off = (int)B.segTile[blockIdx.x], nT = rt_tiles(segs[blockIdx.x].count);
+    uint32_t run = 0;
+    for (int base = 0; base < nT; base += RT_THREADS) {
+        const int t = base + (int)threadIdx.x;
+        const uint32_t v = t < nT ? B.tileLess[off + t] : 0u;
+        uint32_t tot;
+        const uint32_t ex = block_exclusive_scan(v, sw, tot);
+        if (t < nT) B.tileLess[off + t] = run + ex;
+        run += tot;
+    }
+    if (threadIdx.x == 0) B.lvl[blockIdx.x].totL = (int)run;
+}
+
+// per position: `< pivot` before it in its range; run lengths: the k-th >= of the forward stream ends its run k, the
+// k-th < of the backward stream ends its run k
+__global__ void __launch_bounds__(RT_THREADS) k_lv_less(const RtSeg *__restrict__ segs, RtBuf B) {
+    __shared__ uint32_t sw[33];
+    int si, p;
+    RtSeg g;
+    bool valid;
+    if (!rt_tile(segs, B, si, g, p, valid)) return;
+    const RtLevel L = B.lvl[si];
+    const uint32_t lt = valid && rt_axis(B.items[p], L.axis) < L.pivot ? 1u : 0u;
+    uint32_t tot;
+    const int less = (int)(B.tileLess[blockIdx.x] + block_exclusive_scan(lt, sw, tot));
+    if (!valid) return;
+    const int s = g.start, e = s + g.count, i = p - s;
+    B.less[p] = 2 * less + (int)lt;
+    if (lt) B.lenB[s + (L.totL - less - 1)] = e - p;
+    else B.lenF[s + (i - less)] = i + 1;
+}
+
+// the destination of every position under the swap-with-tail loop, from the prefix counts and run lengths
+__global__ void __launch_bounds__(RT_THREADS) k_lv_scatter(const RtSeg *__restrict__ segs, RtBuf B) {
+    int si, p;
+    RtSeg g;
+    bool valid;
+    if (!rt_tile(segs, B, si, g, p, valid) || !valid) return;
+    const int totL = B.lvl[si].totL, s = g.start, c = g.count;
+    const int w = B.less[p], less = w >> 1, lt = w & 1, i = p - s, geF = i - less;
+    const int lenBv = geF == 0 ? 0 : (geF <= totL ? B.lenB[s + geF - 1] : c);
+    int d;
+    if (i + lenBv < c) { // examined from the front
+        d = lt ? i : c - 1 - lenBv;
+    } else { // examined from the back
+        const int lessB = totL - less - lt, m = lessB + 1;
+        const int lenFv = m <= c - totL ? B.lenF[s + m - 1] : c;
+        d = lt ? lessB + lenFv - m : i - 1;
+    }
+    B.tmp[s + d] = B.items[p];
+}
+
+// per range: the median fallback when one side is empty (a stable sort by the axis key in this CTA, as LSD binary splits
+// over the bits that vary, leaving the result in tmp), the node's record and its children
+__global__ void __launch_bounds__(RT_THREADS) k_lv_finish(const RtSeg *__restrict__ segs, RtSeg *next, RtBuf B) {
+    __shared__ uint32_t sw[33];
+    __shared__ uint32_t sOr;
+    const RtSeg g = segs[blockIdx.x];
+    const RtLevel L = B.lvl[blockIdx.x];
+    const int s = g.start, c = g.count, e = s + c, tid = threadIdx.x;
+    int mid = s + L.totL;
+    if (L.totL == 0 || L.totL == c) {
+        float4 *src = B.tmp, *dst = B.items;
+        if (tid == 0) sOr = 0;
+        __syncthreads();
+        const uint32_t k0 = rt_sort_key(rt_axis(src[s], L.axis));
+        uint32_t diff = 0;
+        for (int p = s + tid; p < e; p += RT_THREADS) diff |= rt_sort_key(rt_axis(src[p], L.axis)) ^ k0;
+        atomicOr(&sOr, diff);
+        __syncthreads();
+        const uint32_t vary = sOr;
+        for (int b = 0; b < 32; b++) {
+            if (!((vary >> b) & 1u)) continue;
+            int zeros = 0;
+            for (int base = s; base < e; base += RT_THREADS) {
+                const int p = base + tid;
+                zeros += __syncthreads_count(p < e && !((rt_sort_key(rt_axis(src[p], L.axis)) >> b) & 1u));
+            }
+            int run0 = 0, run1 = zeros;
+            for (int base = s; base < e; base += RT_THREADS) {
+                const int p = base + tid;
+                const bool valid = p < e;
+                const float4 v = valid ? src[p] : make_float4(0, 0, 0, 0);
+                const uint32_t z = valid && !((rt_sort_key(rt_axis(v, L.axis)) >> b) & 1u) ? 1u : 0u;
+                uint32_t tot;
+                const uint32_t ex = block_exclusive_scan(z, sw, tot);
+                if (valid) dst[s + (z ? run0 + (int)ex : run1 + (tid - (int)ex))] = v;
+                run0 += (int)tot, run1 += min(RT_THREADS, e - base) - (int)tot;
+            }
+            __syncthreads();
+            float4 *t = src;
+            src = dst, dst = t;
+        }
+        if (src != B.tmp)
+            for (int p = s + tid; p < e; p += RT_THREADS) B.tmp[p] = src[p];
+        mid = s + c / 2;
+    }
+    if (tid == 0) {
+        B.intPar[mid] = g.pw + 2;
+        rt_child(B, next, s, mid - s, mid << 1, g.depth + 1);
+        rt_child(B, next, mid, e - mid, (mid << 1) | 1, g.depth + 1);
+    }
+}
+
+__global__ void __launch_bounds__(RT_THREADS) k_lv_copy(const RtSeg *__restrict__ segs, RtBuf B) {
+    int si, p;
+    RtSeg g;
+    bool valid;
+    if (rt_tile(segs, B, si, g, p, valid) && valid) B.items[p] = B.tmp[p];
+}
+
+// One thread finishes one range of at most RT_SMALL triangles depth-first, with the reference's loop itself.
+__global__ void k_rt_small(int nSeg, RtBuf B) {
+    const int t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= nSeg) return;
+    RtSeg stack[RT_SMALL]; // a cut takes at least one triangle off each side: depth < RT_SMALL
+    int sp = 0;
+    stack[sp++] = B.small[t];
+    float4 *it = B.items;
+    while (sp) {
+        const RtSeg g = stack[--sp];
+        const int s = g.start, c = g.count, e = s + c;
+        // the host's `v < lo ? v : lo` seeded with the first element, spelled out: the compiler may turn that select
+        // into a min instruction, which ignores a NaN first element instead of keeping it
+        const float4 first = it[s];
+        float lo[3] = {first.x, first.y, first.z}, hi[3] = {lo[0], lo[1], lo[2]};
+        for (int i = s + 1; i < e; i++) {
+            const float4 v = it[i];
+            lo[0] = fminf(lo[0], v.x), lo[1] = fminf(lo[1], v.y), lo[2] = fminf(lo[2], v.z);
+            hi[0] = fmaxf(hi[0], v.x), hi[1] = fmaxf(hi[1], v.y), hi[2] = fmaxf(hi[2], v.z);
+        }
+        if (isnan(first.x)) lo[0] = hi[0] = first.x;
+        if (isnan(first.y)) lo[1] = hi[1] = first.y;
+        if (isnan(first.z)) lo[2] = hi[2] = first.z;
+        int axis;
+        float pivot;
+        rt_plane(lo, hi, axis, pivot);
+        int i = s, j = e - 1;
+        while (i <= j) {
+            const float4 a = it[i], b = it[j];
+            const bool lt = rt_axis(a, axis) < pivot;
+            it[i] = lt ? a : b;
+            it[j] = lt ? b : a;
+            i += lt ? 1 : 0;
+            j -= lt ? 0 : 1;
+        }
+        if (i == s || i == e) { // stable insertion sort on the same key as k_lv_finish
+            for (int q = s + 1; q < e; q++) {
+                const float4 x = it[q];
+                const uint32_t kx = rt_sort_key(rt_axis(x, axis));
+                int r = q - 1;
+                while (r >= s && kx < rt_sort_key(rt_axis(it[r], axis))) it[r + 1] = it[r], r--;
+                it[r + 1] = x;
+            }
+            i = s + c / 2;
+        }
+        B.intPar[i] = g.pw + 2;
+        const RtSeg kids[2] = {{s, i - s, i << 1, g.depth + 1}, {i, e - i, (i << 1) | 1, g.depth + 1}};
+        for (int k = 0; k < 2; k++) {
+            if (kids[k].count <= 4) {
+                B.leafCnt[kids[k].start] = kids[k].count, B.leafPar[kids[k].start] = kids[k].pw;
+                atomicMax(&B.ctr[2], kids[k].depth);
+            } else {
+                stack[sp++] = kids[k];
+            }
+        }
+    }
+}
+
+__global__ void k_rt_leaf_flags(int n, const int32_t *__restrict__ leafCnt, uint32_t *__restrict__ flag) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n) flag[p] = leafCnt[p] > 0 ? 1u : 0u;
+}
+
+// the device form: a parent's child slot holds the child's ref (internal id, or ~((start << 2) | (count - 1)) for a leaf)
+__device__ __forceinline__ void rt_set_child(Node *nodes, int32_t parent, int side, int32_t ref) {
+    reinterpret_cast<float *>(nodes + parent)[side ? 7 : 3] = __int_as_float(ref);
+}
+
+// per leaf: range, parent, its slot in the parent, and for its triangles refSlot, leafOfTri, rank and encOfRank
+__global__ void k_rt_leaves(int n, int set, int off, RtBuf B, const uint32_t *__restrict__ slotOfTri, Node *refNodes,
+                            int32_t *refLeafParent, int32_t *refLeafRange, uint32_t *refSlot, int32_t *refLeafOfTri,
+                            SetHeader *refHdr, int32_t *rank, uint32_t *encOfRank) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= n) return;
+    const int cnt = B.leafCnt[p];
+    if (!cnt) return;
+    const int id = (int)B.leafId[p], pw = B.leafPar[p], ref = ~((p << 2) | (cnt - 1));
+    refLeafRange[id] = (p << 2) | (cnt - 1);
+    if (pw < 0) {
+        refLeafParent[id] = -1;
+        refHdr->rootRef = ref;
+    } else {
+        const int parent = (int)B.leafId[pw >> 1] - 1;
+        refLeafParent[id] = (parent << 1) | (pw & 1);
+        rt_set_child(refNodes, parent, pw & 1, ref);
+    }
+    // the walk pops the right child first: a triangle at position q of the leaf [p, p + cnt) is visited after the
+    // n - (p + cnt) triangles of the leaves to its right
+    for (int q = p; q < p + cnt; q++) {
+        const uint32_t tri = __float_as_uint(B.items[q].w), slot = slotOfTri[tri];
+        const int r = n - (p + cnt) + (q - p);
+        refSlot[q] = slot;
+        refLeafOfTri[tri] = id;
+        rank[off + tri] = off + r;
+        encOfRank[off + r] = ((uint32_t)set << 26) | slot;
+    }
+}
+
+__global__ void k_rt_internal(int n, RtBuf B, Node *refNodes, int32_t *refNodeParent, SetHeader *refHdr) {
+    const int m = blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= n) return;
+    const int v = B.intPar[m];
+    if (!v) return;
+    const int id = (int)B.leafId[m] - 1, pw = v - 2;
+    if (pw < 0) {
+        refNodeParent[id] = -1;
+        refHdr->rootRef = id;
+    } else {
+        const int parent = (int)B.leafId[pw >> 1] - 1;
+        refNodeParent[id] = (parent << 1) | (pw & 1);
+        rt_set_child(refNodes, parent, pw & 1, id);
+    }
+}
+
+static RtBuf rt_carve(Arena &a, int n) {
+    RtBuf B;
+    const int nBig = n / (RT_SMALL + 1) + 1, nSmall = n / 5 + 1;
+    B.items = a.take<float4>(n), B.tmp = a.take<float4>(n);
+    B.less = a.take<int32_t>(n), B.lenF = a.take<int32_t>(n), B.lenB = a.take<int32_t>(n);
+    B.leafCnt = a.take<int32_t>(n), B.leafPar = a.take<int32_t>(n), B.intPar = a.take<int32_t>(n);
+    B.segA = a.take<RtSeg>(nBig), B.segB = a.take<RtSeg>(nBig), B.small = a.take<RtSeg>(nSmall);
+    B.ctr = a.take<int32_t>(4);
+    B.flag = a.take<uint32_t>(n), B.leafId = a.take<uint32_t>(n), B.tileSums = a.take<uint32_t>(cdiv(n, SCAN_TILE) + 1);
+    B.total = a.take<uint32_t>(1);
+    const int nTileMax = n / RT_THREADS + nBig + 1; // a range of count c has cdiv(c, RT_THREADS) tiles
+    B.segTile = a.take<uint32_t>(nBig), B.nTiles = a.take<uint32_t>(1), B.lvl = a.take<RtLevel>(nBig);
+    B.tileSeg = a.take<int32_t>(nTileMax), B.tileLo = a.take<float4>(nTileMax), B.tileHi = a.take<float4>(nTileMax);
+    B.tileLess = a.take<uint32_t>(nTileMax);
+    return B;
+}
+
+// Cut the set's tree into B (triOrder in B.items, the records, B.leafId); returns the leaf count and the depth.
+static int rt_cut(cq_world *w, const DeviceSet &S, RtBuf &B, int &nLeaves, int &depthMax) {
+    cudaStream_t st = w->stream;
+    const int n = S.nTris;
+    CQ_CUDA(cudaMemsetAsync(B.leafCnt, 0, sizeof(int32_t) * (size_t)n, st));
+    CQ_CUDA(cudaMemsetAsync(B.intPar, 0, sizeof(int32_t) * (size_t)n, st));
+    k_rt_items<<<cdiv(n, 256), 256, 0, st>>>(S.boxLo, S.boxHi, S.sortedTri, n, B);
+    k_rt_root<<<1, 1, 0, st>>>(n, B);
+    w->launches += 2;
+    int32_t ctr[3];
+    RtSeg *cur = B.segA, *nxt = B.segB;
+    for (;;) {
+        CQ_CUDA(cudaMemcpyAsync(ctr, B.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, st));
+        CQ_CUDA(cudaStreamSynchronize(st));
+        if (ctr[0] == 0) break;
+        const int nSeg = ctr[0], nTile = n / RT_THREADS + nSeg + 1; // an upper bound: CTAs past *B.nTiles exit
+        CQ_CUDA(cudaMemsetAsync(B.ctr, 0, sizeof(int32_t), st));
+        k_lv_tile_counts<<<cdiv(nSeg, 256), 256, 0, st>>>(cur, nSeg, B.flag);
+        w->launches++;
+        CQ_TRY(exclusive_scan_u32(w, B.flag, nSeg, B.segTile, B.tileSums, B.nTiles));
+        k_lv_map<<<nSeg, 256, 0, st>>>(cur, B);
+        k_lv_bounds<<<nTile, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_plane<<<nSeg, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_count<<<nTile, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_scan<<<nSeg, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_less<<<nTile, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_scatter<<<nTile, RT_THREADS, 0, st>>>(cur, B);
+        k_lv_finish<<<nSeg, RT_THREADS, 0, st>>>(cur, nxt, B);
+        k_lv_copy<<<nTile, RT_THREADS, 0, st>>>(cur, B);
+        w->launches += 9;
+        CQ_CUDA(cudaGetLastError());
+        std::swap(cur, nxt);
+    }
+    if (ctr[1] > 0) {
+        k_rt_small<<<cdiv(ctr[1], 128), 128, 0, st>>>(ctr[1], B);
+        w->launches++;
+    }
+    k_rt_leaf_flags<<<cdiv(n, 256), 256, 0, st>>>(n, B.leafCnt, B.flag);
+    w->launches++;
+    CQ_TRY(exclusive_scan_u32(w, B.flag, n, B.leafId, B.tileSums, B.total));
+    uint32_t total;
+    CQ_CUDA(cudaMemcpyAsync(&total, B.total, sizeof(total), cudaMemcpyDeviceToHost, st));
+    CQ_CUDA(cudaMemcpyAsync(ctr, B.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, st));
+    CQ_CUDA(cudaStreamSynchronize(st));
+    nLeaves = (int)total, depthMax = ctr[2];
+    return check_cuda(cudaGetLastError(), "reference tree");
+}
+
+// Reference order: cut the reference's tree of each set on the device from the triangle boxes the LBVH build computed,
+// write the visiting ranks (one global array, static set first like the reference's own merge of its two sets,
+// CollisionQuery.swift:990-1008) and the tree itself for the ray walk, then fit its boxes.
 int attach_ref_order(cq_world *w) {
     const auto t0 = std::chrono::steady_clock::now();
     cudaStream_t st = w->stream;
-    const int nS = w->set[0].nTris, nD = w->set[1].nTris;
-    std::vector<int32_t> rankAll((size_t)nS + nD);
-    std::vector<uint32_t> encOfRank((size_t)nS + nD);
-    for (int s = 0; s < 2; s++) {
+    const int nS = w->set[0].nTris, nD = w->set[1].nTris, nMax = std::max(nS, nD);
+    if (nS + nD <= 0) {
+        w->refBuildMs = 0.0f;
+        return CQ_OK;
+    }
+    CQ_CUDA(cudaMalloc((void **)&w->dRank, sizeof(int32_t) * (size_t)(nS + nD)));
+    CQ_CUDA(cudaMalloc((void **)&w->dEncOfRank, sizeof(uint32_t) * (size_t)(nS + nD)));
+    Arena tmp;
+    tmp.cap = arena_layout([&](Arena &a) { rt_carve(a, nMax); });
+    CQ_CUDA(cudaMalloc((void **)&tmp.base, tmp.cap));
+    RtBuf B = rt_carve(tmp, nMax);
+    int rc = CQ_OK;
+    for (int s = 0; s < 2 && rc == CQ_OK; s++) {
         DeviceSet &S = w->set[s];
         const int n = S.nTris;
         if (n <= 0) continue;
-        // triangle boxes as the device computed them (leaf boxes of the sorted order) back in the soup's numbering
-        std::vector<float4> sLo(n), sHi(n), lo(n), hi(n);
-        std::vector<uint32_t> sorted(n), slotOf(n);
-        CQ_CUDA(cudaMemcpyAsync(sLo.data(), S.boxLo + (n - 1), sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CQ_CUDA(cudaMemcpyAsync(sHi.data(), S.boxHi + (n - 1), sizeof(float4) * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CQ_CUDA(cudaMemcpyAsync(sorted.data(), S.sortedTri, sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToHost, st));
-        CQ_CUDA(cudaStreamSynchronize(st));
-        for (int k = 0; k < n; k++) lo[sorted[k]] = sLo[k], hi[sorted[k]] = sHi[k], slotOf[sorted[k]] = (uint32_t)k;
-        RefTree T;
-        build_ref_tree(&lo[0].x, &hi[0].x, 4, n, T);
-        const int off = s == 0 ? 0 : nS;
-        for (int t = 0; t < n; t++) {
-            rankAll[(size_t)off + t] = off + T.rank[t];
-            encOfRank[(size_t)off + T.rank[t]] = ((uint32_t)s << 26) | slotOf[t];
-        }
-        // device form: internal nodes and leaves numbered separately
-        const int nNodes = (int)T.nodes.size();
-        std::vector<int32_t> idOf(nNodes);
-        int nInt = 0, nLeaf = 0;
-        for (int k = 0; k < nNodes; k++) idOf[k] = T.nodes[k].left >= 0 ? nInt++ : nLeaf++;
-        std::vector<Node> nodes(std::max(nInt, 1));
-        std::vector<int32_t> nodeParent(std::max(nInt, 1), -1), leafParent(std::max(nLeaf, 1), -1), leafRange(std::max(nLeaf, 1), 0);
-        std::vector<uint32_t> refSlot(n);
-        for (int p = 0; p < n; p++) refSlot[p] = slotOf[T.order[p]];
-        std::vector<int32_t> leafOfTri(n);
-        auto ref_of = [&](int k) { // reference to node k as a parent stores it
-            const RefNode &nd = T.nodes[k];
-            return nd.left >= 0 ? idOf[k] : ~((nd.start << 2) | (nd.count - 1));
-        };
-        int depthMax = 0; // the ray walk keeps one stack entry per level
-        for (int k = 0; k < nNodes; k++) {
-            if (T.nodes[k].left >= 0) continue;
-            int d = 0;
-            for (int q = T.nodes[k].parent; q >= 0; q = T.nodes[q].parent) d++;
-            depthMax = std::max(depthMax, d);
-        }
-        for (int k = 0; k < nNodes; k++) {
-            const RefNode &nd = T.nodes[k];
-            int pw = -1;
-            if (nd.parent >= 0) pw = (idOf[nd.parent] << 1) | (T.nodes[nd.parent].right == k ? 1 : 0);
-            if (nd.left >= 0) {
-                Node &o = nodes[idOf[k]];
-                o.n0 = make_float4(0, 0, 0, int_bits_as_float(ref_of(nd.left)));
-                o.n1 = make_float4(0, 0, 0, int_bits_as_float(ref_of(nd.right)));
-                o.n2 = make_float4(0, 0, 0, 0), o.n3 = make_float4(0, 0, 0, 0);
-                nodeParent[idOf[k]] = pw;
-            } else {
-                leafParent[idOf[k]] = pw;
-                leafRange[idOf[k]] = (nd.start << 2) | (nd.count - 1);
-                for (int q = nd.start; q < nd.start + nd.count; q++) leafOfTri[T.order[q]] = idOf[k];
-            }
-        }
-        if (depthMax + 2 > CQ_STACK) {
+        int nLeaf = 0, depthMax = 0;
+        if ((rc = rt_cut(w, S, B, nLeaf, depthMax)) != CQ_OK) break;
+        if (depthMax + 2 > CQ_STACK) { // the ray walk keeps one stack entry per level
             set_error("cq_world_create: the reference tree of set %d is %d levels deep (limit %d); use CQ_ORDER_CANONICAL", s, depthMax,
                       CQ_STACK - 2);
-            return CQ_ERR_INVALID;
+            rc = CQ_ERR_INVALID;
+            break;
         }
+        const int nInt = nLeaf - 1;
         auto carve = [&](Arena &a) {
             S.refNodes = a.take<Node>(nInt);
             S.refSlot = a.take<uint32_t>(n);
@@ -1563,33 +2001,32 @@ int attach_ref_order(cq_world *w) {
         };
         Arena arena;
         arena.cap = arena_layout(carve);
-        CQ_CUDA(cudaMalloc((void **)&arena.base, arena.cap));
+        if ((rc = check_cuda(cudaMalloc((void **)&arena.base, arena.cap), "reference tree")) != CQ_OK) break;
         S.refArena = arena.base;
         carve(arena);
         S.nRefInternal = nInt, S.nRefLeaves = nLeaf, S.refDepth = depthMax;
-        SetHeader h;
+        SetHeader h; // rootRef is written by k_rt_leaves / k_rt_internal
         h.nTris = n;
-        h.rootRef = ref_of(0);
+        h.rootRef = 0;
         h.lo[0] = h.lo[1] = h.lo[2] = 0.0f, h.hi[0] = h.hi[1] = h.hi[2] = 0.0f;
-        CQ_CUDA(cudaMemcpyAsync(S.refNodes, nodes.data(), sizeof(Node) * (size_t)std::max(nInt, 1), cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemcpyAsync(S.refSlot, refSlot.data(), sizeof(uint32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemcpyAsync(S.refNodeParent, nodeParent.data(), sizeof(int32_t) * (size_t)std::max(nInt, 1), cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemcpyAsync(S.refLeafParent, leafParent.data(), sizeof(int32_t) * (size_t)std::max(nLeaf, 1), cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemcpyAsync(S.refLeafRange, leafRange.data(), sizeof(int32_t) * (size_t)std::max(nLeaf, 1), cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemsetAsync(S.refVisit, 0, sizeof(int32_t) * (size_t)std::max(nInt, 1), st));
-        CQ_CUDA(cudaMemsetAsync(S.refExpect, 0, sizeof(int32_t) * (size_t)std::max(nInt, 1), st));
-        CQ_CUDA(cudaMemsetAsync(S.refLeafMark, 0, sizeof(int32_t) * (size_t)std::max(nLeaf, 1), st));
-        CQ_CUDA(cudaMemcpyAsync(S.refLeafOfTri, leafOfTri.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, st));
-        CQ_CUDA(cudaMemcpyAsync(S.refHdr, &h, sizeof(h), cudaMemcpyHostToDevice, st));
-        CQ_TRY(ref_fit(w, S, st));
-        CQ_CUDA(cudaStreamSynchronize(st)); // the host vectors above are the copies' sources
+        const size_t intBytes = sizeof(int32_t) * (size_t)std::max(nInt, 1);
+        if ((rc = check_cuda(cudaMemsetAsync(S.refNodes, 0, sizeof(Node) * (size_t)std::max(nInt, 1), st), "reference tree")) != CQ_OK ||
+            (rc = check_cuda(cudaMemsetAsync(S.refVisit, 0, intBytes, st), "reference tree")) != CQ_OK ||
+            (rc = check_cuda(cudaMemsetAsync(S.refExpect, 0, intBytes, st), "reference tree")) != CQ_OK ||
+            (rc = check_cuda(cudaMemsetAsync(S.refLeafMark, 0, sizeof(int32_t) * (size_t)nLeaf, st), "reference tree")) != CQ_OK ||
+            (rc = check_cuda(cudaMemcpyAsync(S.refHdr, &h, sizeof(h), cudaMemcpyHostToDevice, st), "reference tree")) != CQ_OK)
+            break;
+        const int off = s == 0 ? 0 : nS;
+        k_rt_leaves<<<cdiv(n, 256), 256, 0, st>>>(n, s, off, B, S.slotOfTri, S.refNodes, S.refLeafParent, S.refLeafRange, S.refSlot,
+                                                  S.refLeafOfTri, S.refHdr, w->dRank, w->dEncOfRank);
+        k_rt_internal<<<cdiv(n, 256), 256, 0, st>>>(n, B, S.refNodes, S.refNodeParent, S.refHdr);
+        w->launches += 2;
+        if ((rc = check_cuda(cudaGetLastError(), "reference tree")) != CQ_OK || (rc = ref_fit(w, S, st)) != CQ_OK) break;
+        if ((rc = check_cuda(cudaStreamSynchronize(st), "reference tree")) != CQ_OK) break; // &h is the header copy's source
     }
-    if (nS + nD > 0) {
-        CQ_CUDA(cudaMalloc((void **)&w->dRank, sizeof(int32_t) * (size_t)(nS + nD)));
-        CQ_CUDA(cudaMemcpy(w->dRank, rankAll.data(), sizeof(int32_t) * (size_t)(nS + nD), cudaMemcpyHostToDevice));
-        CQ_CUDA(cudaMalloc((void **)&w->dEncOfRank, sizeof(uint32_t) * (size_t)(nS + nD)));
-        CQ_CUDA(cudaMemcpy(w->dEncOfRank, encOfRank.data(), sizeof(uint32_t) * (size_t)(nS + nD), cudaMemcpyHostToDevice));
-    }
+    cudaStreamSynchronize(st);
+    cudaFree(tmp.base);
+    if (rc != CQ_OK) return rc;
     // the ranks travel in tv2.w: rewrite the sorted SoA now that they are known (it was gathered with rank = index)
     for (int s = 0; s < 2; s++) {
         DeviceSet &S = w->set[s];

@@ -51,7 +51,7 @@ struct DeviceSet {
     int32_t *expect = nullptr;   // dirty-subtree refit: dirty children per internal node (zero between refits)
     uint32_t *slotOfTri = nullptr; // soup triangle id -> slot of the sorted SoA
     SetHeader *hdr = nullptr;
-    // reference order (cq_reftree.h -> attach_ref_order): the reference's own tree, for the ray walk and its refit
+    // reference order (attach_ref_order): the reference's own tree, for the ray walk and its refit
     void *refArena = nullptr;
     int nRefInternal = 0, nRefLeaves = 0, refDepth = 0;
     Node *refNodes = nullptr;          // internal nodes
@@ -277,7 +277,7 @@ bool stream_capturing(cudaStream_t st);
 // capture stays valid), else CQ_OK.
 int refuse_capture(cudaStream_t st, const char *what);
 #define CQ_NO_CAPTURE(st, what) CQ_TRY(cq::refuse_capture((st), (what)))
-// reference order: rebuild the reference's tree on the host from the set's triangle boxes, upload rank + tree (cq_reftree.h)
+// reference order: cut the reference's tree of each set on the device from its triangle boxes; ranks + tree (cq_build.cu)
 int attach_ref_order(cq_world *w);
 void free_set(DeviceSet &S);
 // Morton-sorted processing order of n work units whose position (3 floats or 3 doubles) sits at the start of each

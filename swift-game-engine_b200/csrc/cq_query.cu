@@ -44,8 +44,8 @@ __device__ __forceinline__ bool ref_ray_aabb(f3 o, f3 inv, f3 lo, f3 hi, float &
 // One kernel, both order rules (REF):
 //   canonical  the triangle with the smallest t over ALL triangles (ties -> smallest index); boxes only skip work and the
 //              box test is conservative (see ray_box).
-//   reference  the reference's walk itself (CollisionQuery.swift:916-978) over the reference's own tree (cq_reftree.h,
-//              uploaded by attach_ref_order): per set, closestT starts at maxDistance; pop a node, cull it when rayAABB
+//   reference  the reference's walk itself (CollisionQuery.swift:916-978) over the reference's own tree (cut on the device
+//              by attach_ref_order): per set, closestT starts at maxDistance; pop a node, cull it when rayAABB
 //              (ref_ray_aabb) misses or starts beyond closestT, test a leaf's triangles in triOrder with strict
 //              `t < closestT`, push left then right.  The slab test of a child is evaluated when its parent is visited (a
 //              miss never depends on closestT) and its tmin travels with the stack entry, so the `tmin > closestT` test

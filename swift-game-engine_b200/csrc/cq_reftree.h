@@ -1,4 +1,4 @@
-// cq_reftree.h — the reference's own BVH (Game/CollisionQuery.swift:496-707), rebuilt on the host, for ONE purpose:
+// cq_reftree.h — the reference's own BVH (Game/CollisionQuery.swift:496-707), restated on the host, for ONE purpose:
 // the ORDER in which the reference visits triangles.
 //
 // Why it exists.  Every query of the reference is a depth-first walk of its median-split tree that pushes the left
@@ -9,8 +9,9 @@
 // same `maxHits` overlaps, it needs the reference's visiting rank of every triangle.  That rank is a property of the
 // tree alone: subtrees are only ever skipped, never reordered.  Raycasts additionally cull by `tmin > closestT` with a
 // slab test that is not conservative in floating point (:933, :1603-1631), so their answers can depend on the tree's
-// boxes themselves; in reference order the ray kernel therefore walks THIS tree (uploaded as 64-byte nodes,
-// cq_build.cu: upload_ref_tree) with the reference's own slab test.
+// boxes themselves; in reference order the ray kernel therefore walks THIS tree (as 64-byte nodes) with the reference's
+// own slab test.  The library cuts the same tree on the device (cq_build.cu: attach_ref_order); this restatement is the
+// reference the tests compare that build with.
 //
 // The split rule is restated from the Swift (spatial median of the centroid bounds along their longest axis, the
 // swap-with-tail partition of :617-634, the sorted-median fallback of :637-653, leaves of <= 4 triangles); the

@@ -51,7 +51,7 @@ struct SetView {
     const int32_t *triPart; // per triangle of the set (soup numbering): index of the part (entity) it came from -> material
     const int32_t *triMat;  // per triangle: row of the material table, or nullptr = the part's own row (no per-triangle materials)
     int triOffset; // added to triangle ids of this set (dynamic set: static count, CollisionQuery.swift:782)
-    // Reference order only (cq_reftree.h): the reference's own median-split tree as 64-byte nodes (child 0 = left,
+    // Reference order only (attach_ref_order): the reference's own median-split tree as 64-byte nodes (child 0 = left,
     // child 1 = right; a leaf reference ~((start << 2) | (count - 1)) names positions of refSlot), walked by the ray
     // kernel exactly as CollisionQuery.swift:916-978 walks it.  refSlot: triOrder position -> slot of the sorted SoA.
     const Node *refNodes;

@@ -49,6 +49,38 @@ public final class CollisionQuery {
         }
     }
 
+    /// cq_world_rebuild: the same world from new entities, as a fresh init would build it (the reference rebuilds its
+    /// query when the active chunk set or a body type changes).  Returns false and keeps the old world on failure
+    /// (lastError says why).  Not compiled: no Swift toolchain was available when this was written.
+    @discardableResult
+    public func rebuild(world: World, activeEntityIDs: Set<UInt32>? = nil, referenceOrder: Bool = true) -> Bool {
+        guard let h = handle else { return false }
+        let built = CollisionQuery.makeParts(world: world, activeEntityIDs: activeEntityIDs)
+        var parts = built.parts
+        var options = cq_world_options()
+        cq_world_options_default(&options)
+        options.order = referenceOrder ? Int32(CQ_ORDER_REFERENCE) : Int32(CQ_ORDER_CANONICAL)
+        var perTri: [cq_triangle_materials] = []
+        let rc: Int32 = CollisionQuery.withMaterialArrays(built.triangleMaterials, &perTri) {
+            perTri.withUnsafeBufferPointer { tm in
+                options.n_triangle_materials = Int32(tm.count)
+                options.triangle_materials = tm.baseAddress
+                return CollisionQuery.withArrays(built.positions, built.indices, &parts) {
+                    cq_world_rebuild(h, &parts, Int32(parts.count), &options)
+                }
+            }
+        }
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        if rc != CQ_OK { return false }
+        knownIDs.removeAll()
+        dynamicIDs.removeAll()
+        for p in built.parts {
+            knownIDs.insert(p.entity_id)
+            if p.is_dynamic != 0 { dynamicIDs.insert(p.entity_id) }
+        }
+        return true
+    }
+
     deinit { cq_world_destroy(handle) }
 
     public func updateStaticTransforms(world: World, entities: [Entity], activeEntityIDs: Set<UInt32>? = nil) {
