@@ -346,8 +346,9 @@ int cq_capsule_overlap_all_batch(cq_world *w, const cq_capsule *q, int32_t n, in
  * ordered against them by events instead (see its ordering contract).
  *
  * CUDA-graph capture: while `stream` is being captured (cudaStreamBeginCapture, torch.cuda.graph, ...), the *_device
- * query twins, cq_move_and_slide_device(_ex) and cq_move_and_slide_device_platforms, cq_world_update_transforms_device,
- * cq_world_platforms_device and cq_agent_separation_device_async enqueue kernels, memsets, copies and (agent
+ * query twins, cq_move_and_slide_device(_ex) and cq_move_and_slide_device_platforms, cq_agent_snapshot_device and
+ * cq_move_and_slide_device_agents, cq_world_update_transforms_device, cq_world_platforms_device and
+ * cq_agent_separation_device_async enqueue kernels, memsets, copies and (agent
  * separation) conditional WHILE nodes only: they neither wait on nor record nor create world events.  So:
  *  - a graph is ordered only by the stream it is launched on; the caller orders its replays against other work on the
  *    world, as for a synchronous call (e.g. synchronise before an uncaptured call on another stream);
@@ -498,6 +499,42 @@ int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout,
                                        uint32_t flags, const cq_platform *d_platforms, int32_t n_platforms,
                                        void *stream);
 
+/* ---- a crowd moved in slices ------------------------------------------------
+ * CQ_MAS_AGENTS in two stages, so that the slices of one crowd can move on different GPUs (or in different calls) and
+ * still see each other: every slice first writes the snapshot records of its own characters into its range of one
+ * crowd-wide snapshot array, the array is made whole (cq_group_gather_records / cq_group_gather_records_local, 32-byte
+ * records), then every slice moves its characters against the whole snapshot.  An agent's identity is its position in
+ * the snapshot array. */
+typedef struct cq_agent_snapshot {   /* collectAgentStates (Systems.swift:1592-1611), one per character */
+    float position[3]; float _reserved0;   /* positionF */
+    float velocity[3]; float _reserved1;   /* post-gravity linearVelocity as Float */
+} cq_agent_snapshot;                      /* 32 bytes */
+
+/* d_out[i] (DEVICE, n records) = the snapshot of d_states[i] (DEVICE, n records) that a CQ_MAS_AGENTS step with the same
+ * dt, gravity and flags takes: the gravity rule of CQ_MAS_APPLY_GRAVITY, then position and velocity converted to float;
+ * the reserved words are written as zero.  One launch on `stream` (NULL = the world's stream), no scratch, no
+ * synchronisation, no allocation.  NULL world, n < 0, or a NULL array with n > 0 return CQ_ERR_INVALID before any CUDA
+ * call; n == 0 returns CQ_OK and queues nothing. */
+int cq_agent_snapshot_device(cq_world *w, const cq_character_state *d_states, int32_t n, float dt, const float gravity[3],
+                             uint32_t flags, cq_agent_snapshot *d_out, void *stream);
+
+/* One CQ_MAS_AGENTS step of the characters d_inout[0..n) (DEVICE), which are agents first_agent .. first_agent + n - 1
+ * of the crowd whose snapshot is d_agents[0..n_agents) (DEVICE).  Each slice builds the crowd's whole agent grid from
+ * the snapshot and moves only its own characters.  When every slice of a crowd is snapshotted first
+ * (cq_agent_snapshot_device) and then moved with the same dt, gravity, flags and platforms, the records equal one
+ * cq_move_and_slide_device_platforms(..., CQ_MAS_AGENTS) call on the whole crowd, byte for byte.  Platforms are a
+ * DEVICE array read when the kernels run, as in cq_move_and_slide_device_platforms.
+ * CQ_ERR_INVALID before any CUDA call: flags without CQ_MAS_AGENTS; n, n_agents or first_agent below 0;
+ * first_agent + n > n_agents; a NULL array with a count above 0; any check of cq_move_and_slide_device_platforms.
+ * n == 0 returns CQ_OK and queues nothing.  Stream-ordered with the other CQ_MAS_AGENTS calls on the world (they share
+ * the grid scratch); may be recorded into a CUDA graph (see the capture contract above).
+ * Launches: 14, plus 7 for the processing order when n >= 65,536 on a world of >= 262,144 static triangles (the
+ * launches of cq_move_and_slide_device_platforms with CQ_MAS_AGENTS on n characters), whatever n_agents is. */
+int cq_move_and_slide_device_agents(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_agent_snapshot *d_agents,
+                                    int32_t n_agents, int32_t first_agent, const cq_controller_params *params, float dt,
+                                    const float gravity[3], uint32_t flags, const cq_platform *d_platforms,
+                                    int32_t n_platforms, void *stream);
+
 /* ---- resident crowd ------------------------------------------------------
  * The full-record calls above move 2 x 168 bytes per character per step across PCIe, which bounds them near 230 M
  * characters/s per GPU whatever the kernel does.  A crowd keeps the records in HBM between steps — they are private to
@@ -627,9 +664,18 @@ cq_world *cq_multi_world_replica(cq_multi_world *mw, int32_t i); /* for the *_de
 int cq_multi_update_transforms(cq_multi_world *mw, const uint32_t *entity_ids, const float *models, int32_t n);
 int cq_multi_raycast_batch(cq_multi_world *mw, const cq_ray *rays, int32_t n, cq_ray_hit *out);
 int cq_multi_capsule_cast_batch(cq_multi_world *mw, const cq_capsule_cast *q, int32_t n, int32_t mode, cq_cast_hit *out);
-/* CQ_MAS_AGENTS is refused: the batch is the crowd, agents of different shards would not see each other. */
+/* CQ_MAS_AGENTS is refused here (use cq_multi_move_and_slide_batch_ex). */
 int cq_multi_move_and_slide_batch(cq_multi_world *mw, cq_character_state *inout, int32_t n,
                                   const cq_controller_params *params, float dt, const float gravity[3], uint32_t flags);
+/* The step of cq_move_and_slide_batch_ex (0..64 host platforms) sharded over the replicas, CQ_MAS_AGENTS included: the
+ * batch is one crowd.  With agents, each replica snapshots its shard (cq_agent_snapshot_device) into its range of a
+ * crowd-sized snapshot buffer, one NCCL all-gather of the 32-byte records makes the snapshot whole on every replica, and
+ * each replica moves its shard against it (cq_move_and_slide_device_agents).  Records equal cq_move_and_slide_batch_ex
+ * on one GPU, byte for byte.  The multi world keeps the per-replica buffers (grown on demand, freed by
+ * cq_multi_world_destroy).  Without agents: cq_multi_move_and_slide_batch plus platforms. */
+int cq_multi_move_and_slide_batch_ex(cq_multi_world *mw, cq_character_state *inout, int32_t n,
+                                     const cq_controller_params *params, float dt, const float gravity[3], uint32_t flags,
+                                     const cq_platform *platforms, int32_t n_platforms);
 
 /* ---- instrumentation ------------------------------------------------------
  * Work counters of the last device/batch call, accumulated on the device when

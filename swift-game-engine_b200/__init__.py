@@ -50,6 +50,9 @@ CROWD_POSE = np.dtype([("position", "<f8", 3), ("velocity", "<f8", 3), ("ground_
                        ("grounded_near", "u1"), ("ground_sliding", "u1"), ("_pad", "u1")])
 assert CROWD_POSE.itemsize == 56
 PLATFORM = np.dtype([("aabb_min", "<f4", 3), ("aabb_max", "<f4", 3), ("delta", "<f4", 3)])
+# cq_agent_snapshot: one agent of a crowd as every character's sweeps see it (positionF, post-gravity velocity)
+AGENT_SNAPSHOT = np.dtype([("position", "<f4", 3), ("_reserved0", "<f4"), ("velocity", "<f4", 3), ("_reserved1", "<f4")])
+assert AGENT_SNAPSHOT.itemsize == 32
 CAST_ALL, CAST_BLOCKING, CAST_GROUND = 0, 1, 2
 MAS_APPLY_GRAVITY = 1
 MAS_AGENTS = 2  # characters of the batch collide with each other (capsule-capsule CCD)
@@ -141,7 +144,8 @@ EXPORTS = [
     "cq_raycast_device_ex", "cq_capsule_cast_device_ex", "cq_capsule_overlap_device_ex", "cq_raycast_device", "cq_capsule_cast_device", "cq_capsule_overlap_device",
     "cq_capsule_overlap_all_device", "cq_controller_params_default", "cq_character_state_init",
     "cq_move_and_slide_batch", "cq_move_and_slide_device", "cq_move_and_slide_batch_ex",
-    "cq_move_and_slide_device_ex", "cq_move_and_slide_device_platforms", "cq_agent_separation_batch", "cq_agent_separation_device",
+    "cq_move_and_slide_device_ex", "cq_move_and_slide_device_platforms", "cq_agent_snapshot_device",
+    "cq_move_and_slide_device_agents", "cq_agent_separation_batch", "cq_agent_separation_device",
     "cq_agent_separation_device_async",
     "cq_world_set_counting", "cq_world_read_counters",
     "cq_crowd_create", "cq_crowd_destroy", "cq_crowd_size", "cq_crowd_step", "cq_crowd_read", "cq_crowd_write",
@@ -150,7 +154,7 @@ EXPORTS = [
     "cq_group_size", "cq_group_rank", "cq_group_device", "cq_group_gather_records", "cq_group_gather_records_local",
     "cq_group_synchronize", "cq_world_create_multi", "cq_multi_world_destroy", "cq_multi_world_size",
     "cq_multi_world_replica", "cq_multi_update_transforms", "cq_multi_raycast_batch", "cq_multi_capsule_cast_batch",
-    "cq_multi_move_and_slide_batch",
+    "cq_multi_move_and_slide_batch", "cq_multi_move_and_slide_batch_ex",
     "cq_host_alloc", "cq_host_free", "cq_last_error", "cq_version",
 ]
 GROUP_ID_BYTES = 128
@@ -233,6 +237,8 @@ def lib():
         L.cq_move_and_slide_batch_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32]
         L.cq_move_and_slide_device_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32, vp]
         L.cq_move_and_slide_device_platforms.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32, vp]
+        L.cq_agent_snapshot_device.argtypes = [vp, vp, i32, f32, vp, u32, vp, vp]
+        L.cq_move_and_slide_device_agents.argtypes = [vp, vp, i32, vp, i32, i32, vp, f32, vp, u32, vp, i32, vp]
         L.cq_agent_separation_batch.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32]
         L.cq_agent_separation_device.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp]
         L.cq_agent_separation_device_async.argtypes = [vp, vp, i32, vp, vp, i32, f32, f32, i32, vp, vp]
@@ -268,6 +274,7 @@ def lib():
         L.cq_multi_raycast_batch.argtypes = [vp, vp, i32, vp]
         L.cq_multi_capsule_cast_batch.argtypes = [vp, vp, i32, i32, vp]
         L.cq_multi_move_and_slide_batch.argtypes = [vp, vp, i32, vp, f32, vp, u32]
+        L.cq_multi_move_and_slide_batch_ex.argtypes = [vp, vp, i32, vp, f32, vp, u32, vp, i32]
         L.cq_world_set_counting.argtypes = [vp, i32]
         L.cq_world_read_counters.argtypes = [vp, C.POINTER(Counters), i32]
         _lib = L
@@ -599,6 +606,28 @@ class CollisionQuery:
                                                         _ptr(g), flags, C.c_void_p(d_platforms_ptr) if d_platforms_ptr else None,
                                                         int(n_platforms), C.c_void_p(stream) if stream else None))
 
+    def agent_snapshot_device(self, d_states_ptr, n, d_out_ptr, dt=1.0 / 60.0, gravity=(0.0, -98.0, 0.0),
+                              flags=MAS_APPLY_GRAVITY | MAS_AGENTS, stream=None):
+        """cq_agent_snapshot_device: n AGENT_SNAPSHOT records (device, d_out_ptr, 16-byte aligned) of n STATE records
+        (device), as a CQ_MAS_AGENTS step with the same dt, gravity and flags takes them.  One launch, capturable."""
+        g = np.asarray(gravity, np.float32)
+        _check(lib().cq_agent_snapshot_device(self._h, C.c_void_p(d_states_ptr), int(n), C.c_float(dt), _ptr(g), flags,
+                                              C.c_void_p(d_out_ptr), C.c_void_p(stream) if stream else None))
+
+    def move_and_slide_device_agents(self, d_states_ptr, n, d_agents_ptr, n_agents, first_agent, params, dt=1.0 / 60.0,
+                                     gravity=(0.0, -98.0, 0.0), flags=MAS_APPLY_GRAVITY | MAS_AGENTS, d_platforms_ptr=None,
+                                     n_platforms=0, stream=None):
+        """cq_move_and_slide_device_agents: one CQ_MAS_AGENTS step of the n STATE records at d_states_ptr, which are agents
+        first_agent .. first_agent + n - 1 of the crowd whose n_agents AGENT_SNAPSHOT records are at d_agents_ptr.  Every
+        slice snapshotted first, then each moved: the records of one whole-crowd call, byte for byte."""
+        params = np.ascontiguousarray(params, PARAMS)
+        g = np.asarray(gravity, np.float32)
+        _check(lib().cq_move_and_slide_device_agents(self._h, C.c_void_p(d_states_ptr), int(n),
+                                                     C.c_void_p(d_agents_ptr) if d_agents_ptr else None, int(n_agents),
+                                                     int(first_agent), _ptr(params), C.c_float(dt), _ptr(g), flags,
+                                                     C.c_void_p(d_platforms_ptr) if d_platforms_ptr else None,
+                                                     int(n_platforms), C.c_void_p(stream) if stream else None))
+
     def capsule_overlap_all_device(self, d_q_ptr, n, max_hits, d_out_ptr, d_counts_ptr, d_overflow_ptr=None, stream=None):
         """cq_capsule_overlap_all_device: n CAPSULE records in, n * max_hits OVERLAP_HIT records, n int32 counts and
         (optional) n overflow bytes out, all device pointers, enqueued on `stream` without synchronising."""
@@ -770,6 +799,19 @@ class MultiWorld:
         params = np.ascontiguousarray(params, PARAMS)
         g = np.asarray(gravity, np.float32)
         _check(lib().cq_multi_move_and_slide_batch(self._h, _ptr(states), len(states), _ptr(params), C.c_float(dt), _ptr(g), flags))
+        return states
+
+    def move_and_slide_ex(self, states, params, dt=1.0 / 60.0, gravity=(0.0, -98.0, 0.0), flags=MAS_APPLY_GRAVITY,
+                          platforms=None):
+        """cq_multi_move_and_slide_batch_ex: the batch is one crowd, CQ_MAS_AGENTS included (snapshot per shard, NCCL
+        all-gather of the snapshot, move per shard); platforms: up to 64 PLATFORM records.  Equals
+        CollisionQuery.move_and_slide byte for byte."""
+        assert states.dtype == STATE and states.flags["C_CONTIGUOUS"]
+        params = np.ascontiguousarray(params, PARAMS)
+        g = np.asarray(gravity, np.float32)
+        pl = np.ascontiguousarray(platforms if platforms is not None else np.zeros(0, PLATFORM), PLATFORM)
+        _check(lib().cq_multi_move_and_slide_batch_ex(self._h, _ptr(states), len(states), _ptr(params), C.c_float(dt), _ptr(g),
+                                                      flags, _ptr(pl) if len(pl) else None, len(pl)))
         return states
 
 

@@ -112,6 +112,22 @@ class CollisionQuery {
         return cq_move_and_slide_device_platforms(w_, dInout, n, &p, dt, gravity, flags, platforms.records, platforms.count,
                                                   stream) == CQ_OK;
     }
+    // a crowd moved in slices (on several GPUs, or in several calls): every slice writes the snapshot of its n characters
+    // into its range of one crowd-wide snapshot array (dOut, device, 16-byte aligned) ...
+    bool agentSnapshotDevice(const cq_character_state *dStates, int32_t n, float dt, const float gravity[3], cq_agent_snapshot *dOut,
+                             bool applyGravity = true, void *stream = nullptr) {
+        uint32_t flags = (applyGravity ? CQ_MAS_APPLY_GRAVITY : 0u) | CQ_MAS_AGENTS;
+        return cq_agent_snapshot_device(w_, dStates, n, dt, gravity, flags, dOut, stream) == CQ_OK;
+    }
+    // ... and once the array is whole, moves its characters, agents firstAgent .. firstAgent + n - 1 of the nAgents in
+    // dAgents: together the slices equal one agents moveAndSlide of the whole crowd, byte for byte
+    bool moveAndSlideAgents(cq_character_state *dInout, int32_t n, const cq_agent_snapshot *dAgents, int32_t nAgents,
+                            int32_t firstAgent, const cq_controller_params &p, float dt, const float gravity[3],
+                            DevicePlatforms platforms = {nullptr, 0}, bool applyGravity = true, void *stream = nullptr) {
+        uint32_t flags = (applyGravity ? CQ_MAS_APPLY_GRAVITY : 0u) | CQ_MAS_AGENTS;
+        return cq_move_and_slide_device_agents(w_, dInout, n, dAgents, nAgents, firstAgent, &p, dt, gravity, flags, platforms.records,
+                                               platforms.count, stream) == CQ_OK;
+    }
     // agent separation of resident records, queued on `stream` without synchronising (capturable in a CUDA graph);
     // *dStatus (device int32, optional) receives CQ_SEP_STATUS_* in stream order
     bool agentSeparationDeviceAsync(cq_character_state *dInout, int32_t n, const cq_controller_params &p,

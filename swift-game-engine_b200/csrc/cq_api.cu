@@ -1010,6 +1010,43 @@ int cq_move_and_slide_device_platforms(cq_world *w, cq_character_state *d_inout,
     return launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, nullptr,
                                  n_platforms > 0 ? d_platforms : nullptr, n_platforms, st);
 }
+// the snapshot is read as float4 pairs
+static bool snapshot_aligned(const void *p) { return ((uintptr_t)p & 15) == 0; }
+
+int cq_agent_snapshot_device(cq_world *w, const cq_character_state *d_states, int32_t n, float dt, const float gravity[3],
+                             uint32_t flags, cq_agent_snapshot *d_out, void *stream) {
+    if (!w || n < 0 || (n > 0 && (!d_states || !d_out || !gravity))) return CQ_ERR_INVALID;
+    if (!snapshot_aligned(d_out)) {
+        set_error("cq_agent_snapshot_device: the snapshot array must be 16-byte aligned");
+        return CQ_ERR_INVALID;
+    }
+    if (n == 0) return CQ_OK;
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return launch_agent_snapshot(w, d_states, n, dt, gravity, flags, d_out, st);
+}
+int cq_move_and_slide_device_agents(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_agent_snapshot *d_agents,
+                                    int32_t n_agents, int32_t first_agent, const cq_controller_params *params, float dt,
+                                    const float gravity[3], uint32_t flags, const cq_platform *d_platforms, int32_t n_platforms,
+                                    void *stream) {
+    if (!w || n < 0 || !params || !gravity || (n > 0 && !d_inout)) return CQ_ERR_INVALID;
+    if (!(flags & CQ_MAS_AGENTS) || n_agents < 0 || first_agent < 0 || (int64_t)first_agent + n > (int64_t)n_agents ||
+        (n_agents > 0 && !d_agents) || !snapshot_aligned(d_agents)) {
+        set_error("cq_move_and_slide_device_agents: characters %d..%lld of a %d-agent snapshot at %p (flags 0x%x: needs "
+                  "CQ_MAS_AGENTS, a 16-byte aligned snapshot)", first_agent, (long long)first_agent + n, n_agents,
+                  (const void *)d_agents, flags);
+        return CQ_ERR_INVALID;
+    }
+    if (n_platforms < 0 || (n_platforms > 0 && !d_platforms)) {
+        set_error("cq_move_and_slide_device_agents: %d platforms at %p", n_platforms, (const void *)d_platforms);
+        return CQ_ERR_INVALID;
+    }
+    if (n == 0) return CQ_OK;
+    const cudaStream_t st = pick_stream(w, stream);
+    CaptureScope cap(w, st);
+    return launch_move_and_slide(w, d_inout, n, *params, dt, gravity, flags, nullptr, n_platforms > 0 ? d_platforms : nullptr,
+                                 n_platforms, st, d_agents, n_agents, first_agent);
+}
 int cq_move_and_slide_device(cq_world *w, cq_character_state *d_inout, int32_t n, const cq_controller_params *params, float dt,
                              const float gravity[3], uint32_t flags, void *stream) {
     return cq_move_and_slide_device_ex(w, d_inout, n, params, dt, gravity, flags, nullptr, 0, stream);

@@ -1256,6 +1256,7 @@ int sort_pairs_u32(cq_world *w, uint32_t *keys, uint32_t *vals, uint32_t *keysTm
 }
 
 // ---------------------------------------------------------------- agent snapshot + grid (CQ_MAS_AGENTS)
+// Snapshot records are cq_agent_snapshot, read as two float4: (position, 0), (velocity, 0).
 // bounds: [0..1] min x,z  [2..3] max x,z  [4] max |v|  (ordered ints)
 __global__ void k_agent_bounds_init(int *bounds) {
     if (threadIdx.x < 5) {
@@ -1263,23 +1264,13 @@ __global__ void k_agent_bounds_init(int *bounds) {
         bounds[threadIdx.x] = float_to_ordered(init);
     }
 }
-__global__ void k_agent_snapshot(const cq_character_state *__restrict__ states, int n, float dt, float gx, float gy, float gz,
-                                 uint32_t flags, float4 *__restrict__ pos, float4 *__restrict__ vel, int *bounds) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    float v[5] = {FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, 0.0f};
-    if (i < n) {
-        const cq_character_state &S = states[i];
-        d3 vd = {S.velocity[0], S.velocity[1], S.velocity[2]};
-        // collectAgentStates runs after GravitySystem (system #3), so the snapshot carries the post-gravity velocity
-        if ((flags & CQ_MAS_APPLY_GRAVITY) && !(S.grounded != 0 && S.grounded_near != 0))
-            vd = vd + to_d3(mk3(gx, gy, gz)) * (double)dt;
-        f3 p = {(float)S.position[0], (float)S.position[1], (float)S.position[2]};
-        f3 vf = to_f3(vd);
-        pos[i] = make_float4(p.x, p.y, p.z, __int_as_float(i));
-        vel[i] = make_float4(vf.x, vf.y, vf.z, 0.0f);
-        v[0] = p.x, v[1] = p.z, v[2] = p.x, v[3] = p.z;
-        v[4] = sqrtf(vf.x * vf.x + vf.y * vf.y + vf.z * vf.z);
-    }
+// the snapshot's contribution to the bounds: position and velocity of one agent (none: the identities of min / max)
+__device__ __forceinline__ void agent_bounds_values(float4 p, float4 vf, float (&v)[5]) {
+    v[0] = p.x, v[1] = p.z, v[2] = p.x, v[3] = p.z;
+    v[4] = sqrtf(vf.x * vf.x + vf.y * vf.y + vf.z * vf.z);
+}
+// block-wide min / max of the values of every thread, folded into `bounds` with one atomic per value
+__device__ __forceinline__ void agent_bounds_reduce(const float (&v)[5], int *bounds) {
     __shared__ float red[5][8];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
@@ -1299,6 +1290,34 @@ __global__ void k_agent_snapshot(const cq_character_state *__restrict__ states, 
         if (k < 2) atomicMin(bounds + k, float_to_ordered(x));
         else atomicMax(bounds + k, float_to_ordered(x));
     }
+}
+// BOUNDS: the single-batch step, which also reduces the bounds of its own snapshot in the same pass
+template <bool BOUNDS>
+__global__ void k_agent_snapshot(const cq_character_state *__restrict__ states, int n, float dt, float gx, float gy, float gz,
+                                 uint32_t flags, float4 *__restrict__ snap, int *bounds) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    float v[5] = {FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, 0.0f};
+    if (i < n) {
+        const cq_character_state &S = states[i];
+        d3 vd = {S.velocity[0], S.velocity[1], S.velocity[2]};
+        // collectAgentStates runs after GravitySystem (system #3), so the snapshot carries the post-gravity velocity
+        if ((flags & CQ_MAS_APPLY_GRAVITY) && !(S.grounded != 0 && S.grounded_near != 0))
+            vd = vd + to_d3(mk3(gx, gy, gz)) * (double)dt;
+        const f3 vf = to_f3(vd);
+        const float4 p = make_float4((float)S.position[0], (float)S.position[1], (float)S.position[2], 0.0f);
+        const float4 q = make_float4(vf.x, vf.y, vf.z, 0.0f);
+        snap[2 * (size_t)i] = p;
+        snap[2 * (size_t)i + 1] = q;
+        if (BOUNDS) agent_bounds_values(p, q, v);
+    }
+    if (BOUNDS) agent_bounds_reduce(v, bounds);
+}
+// the bounds of a snapshot someone else took (a crowd moved in slices)
+__global__ void k_agent_bounds(const float4 *__restrict__ snap, int n, int *bounds) {
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    float v[5] = {FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, 0.0f};
+    if (i < n) agent_bounds_values(snap[2 * (size_t)i], snap[2 * (size_t)i + 1], v);
+    agent_bounds_reduce(v, bounds);
 }
 
 // cell = the farthest two agents can be apart (XZ) and still touch within one step, so a sweep looks at 3x3 cells;
@@ -1322,49 +1341,56 @@ __global__ void k_agent_grid_params(const int *bounds, float radius, float dt, A
     out->_pad = 0.0f;
 }
 
-__global__ void k_agent_keys(const float4 *__restrict__ pos, int n, const AgentGridParams *__restrict__ gp, uint32_t *keys,
+__device__ __forceinline__ uint32_t agent_key(float4 p, const AgentGridParams &G) {
+    return (uint32_t)agent_cell(p.z, G.originZ, G.invCell, G.dimZ) * (uint32_t)G.dimX +
+           (uint32_t)agent_cell(p.x, G.originX, G.invCell, G.dimX);
+}
+
+__global__ void k_agent_keys(const float4 *__restrict__ snap, int n, const AgentGridParams *__restrict__ gp, uint32_t *keys,
                              uint32_t *vals) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const AgentGridParams G = *gp;
-    float4 p = pos[i];
-    keys[i] = (uint32_t)agent_cell(p.z, G.originZ, G.invCell, G.dimZ) * (uint32_t)G.dimX +
-              (uint32_t)agent_cell(p.x, G.originX, G.invCell, G.dimX);
+    keys[i] = agent_key(snap[2 * (size_t)i], G);
     vals[i] = (uint32_t)i;
 }
 
-__global__ void k_agent_gather(const uint32_t *__restrict__ vals, int n, const float4 *__restrict__ pos,
-                               const float4 *__restrict__ vel, float4 *__restrict__ posS, float4 *__restrict__ velS) {
+// the sorted arrays: position with w = agent index (bits), velocity
+__global__ void k_agent_gather(const uint32_t *__restrict__ vals, int n, const float4 *__restrict__ snap,
+                               float4 *__restrict__ posS, float4 *__restrict__ velS) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     uint32_t j = vals[i];
-    posS[i] = pos[j];
-    velS[i] = vel[j];
+    const float4 p = snap[2 * (size_t)j];
+    posS[i] = make_float4(p.x, p.y, p.z, __int_as_float((int)j));
+    velS[i] = snap[2 * (size_t)j + 1];
 }
 
-// one thread per agent: the three sorted-array ranges its 3x3 cell neighbourhood occupies (binary searches done here,
-// at full occupancy, instead of by a lone lane inside the move-and-slide kernel)
-__global__ void k_agent_rows(const uint32_t *__restrict__ keys, const uint32_t *__restrict__ vals, int n,
+// one thread per character of the launch: the three sorted-array ranges its 3x3 cell neighbourhood occupies (binary
+// searches done here, at full occupancy, instead of by a lone lane inside the move-and-slide kernel).  The cell comes
+// from the character's own snapshot record, so only the launch's n characters are visited, whatever the crowd's size.
+__global__ void k_agent_rows(const float4 *__restrict__ snap, int first, int n, const uint32_t *__restrict__ keys, int nAgents,
                              const AgentGridParams *__restrict__ gp, int4 *__restrict__ rows) {
-    int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
-    const int dimX = gp->dimX, dimZ = gp->dimZ;
-    const uint32_t key = keys[j];
-    const int iz = (int)(key / (uint32_t)dimX), ix = (int)(key % (uint32_t)dimX);
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const AgentGridParams G = *gp;
+    const float4 p = snap[2 * ((size_t)first + i)];
+    const int dimX = G.dimX, dimZ = G.dimZ;
+    const int iz = agent_cell(p.z, G.originZ, G.invCell, dimZ), ix = agent_cell(p.x, G.originX, G.invCell, dimX);
     int se[6];
     for (int dz = -1; dz <= 1; dz++) {
         int row = iz + dz, start = 0, end = 0;
         if (row >= 0 && row < dimZ) {
             const uint32_t keyLo = (uint32_t)row * (uint32_t)dimX + (uint32_t)max(ix - 1, 0);
             const uint32_t keyHi = (uint32_t)row * (uint32_t)dimX + (uint32_t)min(ix + 1, dimX - 1);
-            int lo = 0, hi = n;
+            int lo = 0, hi = nAgents;
             while (lo < hi) { // lower_bound(keyLo)
                 int mid = (lo + hi) >> 1;
                 if (keys[mid] < keyLo) lo = mid + 1;
                 else hi = mid;
             }
             start = lo;
-            hi = n;
+            hi = nAgents;
             while (lo < hi) { // upper_bound(keyHi)
                 int mid = (lo + hi) >> 1;
                 if (keys[mid] <= keyHi) lo = mid + 1;
@@ -1374,38 +1400,51 @@ __global__ void k_agent_rows(const uint32_t *__restrict__ keys, const uint32_t *
         }
         se[2 * (dz + 1)] = start, se[2 * (dz + 1) + 1] = end;
     }
-    const uint32_t orig = vals[j];
-    rows[2 * (size_t)orig] = make_int4(se[0], se[1], se[2], se[3]);
-    rows[2 * (size_t)orig + 1] = make_int4(se[4], se[5], ix, iz);
+    rows[2 * (size_t)i] = make_int4(se[0], se[1], se[2], se[3]);
+    rows[2 * (size_t)i + 1] = make_int4(se[4], se[5], ix, iz);
 }
 
-int take_agent_grid(cq_world *w, int n, cudaStream_t st, void **scratch) {
-    // [pos n][vel n][posS n][velS n] float4, [rows 2n] int4, [firstHit n] float4, [keys n][vals n][keysTmp n][valsTmp n] u32, sort scratch,
-    // bounds, params
-    const size_t bytes = (size_t)n * 112 + ((size_t)4 * n + sort_scratch_words(n) + 64) * 4;
-    return take_scratch(w, &w->agentScratch, 1, 0, bytes, st, "CQ_MAS_AGENTS grid scratch", scratch);
+// [snap 2 nAgents float4, when the launch takes its own snapshot][posS nAgents][velS nAgents] float4, [rows 2n] int4,
+// [firstHit n] float4, [keys][vals][keysTmp][valsTmp] nAgents u32 each, sort scratch, bounds, params
+static size_t agent_grid_bytes(int nAgents, int n, bool ownSnapshot) {
+    return (size_t)nAgents * (ownSnapshot ? 64 : 32) + (size_t)n * 48 + ((size_t)4 * nAgents + sort_scratch_words(nAgents) + 64) * 4;
 }
 
-int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, int n, float radius, float dt,
-                    const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out) {
-    const size_t sortWords = sort_scratch_words(n);
-    float4 *pos = (float4 *)scratch, *vel = pos + n, *posS = vel + n, *velS = posS + n;
-    int4 *rows = (int4 *)(velS + n);
+int take_agent_grid(cq_world *w, int nAgents, int n, bool ownSnapshot, cudaStream_t st, void **scratch) {
+    return take_scratch(w, &w->agentScratch, 1, 0, agent_grid_bytes(nAgents, n, ownSnapshot), st, "CQ_MAS_AGENTS grid scratch",
+                        scratch);
+}
+
+int launch_agent_snapshot(cq_world *w, const cq_character_state *dStates, int n, float dt, const float g[3], uint32_t flags,
+                          cq_agent_snapshot *dOut, cudaStream_t st) {
+    k_agent_snapshot<false><<<cdiv(n, 256), 256, 0, st>>>(dStates, n, dt, g[0], g[1], g[2], flags, (float4 *)dOut, nullptr);
+    w->launches++;
+    return check_cuda(cudaGetLastError(), "agent snapshot");
+}
+
+int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, const cq_agent_snapshot *dAgents, int nAgents,
+                    int first, int n, float radius, float dt, const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out) {
+    const size_t sortWords = sort_scratch_words(nAgents);
+    float4 *own = (float4 *)scratch, *posS = dAgents ? own : own + 2 * (size_t)nAgents, *velS = posS + nAgents;
+    int4 *rows = (int4 *)(velS + nAgents);
     float4 *firstHit = (float4 *)(rows + 2 * (size_t)n);
-    uint32_t *keys = (uint32_t *)(firstHit + n), *vals = keys + n, *keysTmp = vals + n, *valsTmp = keysTmp + n;
-    uint32_t *sortScratch = valsTmp + n;
+    uint32_t *keys = (uint32_t *)(firstHit + n), *vals = keys + nAgents, *keysTmp = vals + nAgents, *valsTmp = keysTmp + nAgents;
+    uint32_t *sortScratch = valsTmp + nAgents;
     int *bounds = (int *)(sortScratch + sortWords);
     AgentGridParams *gp = (AgentGridParams *)(bounds + 8);
+    const float4 *snap = dAgents ? (const float4 *)dAgents : own;
     k_agent_bounds_init<<<1, 32, 0, st>>>(bounds);
-    k_agent_snapshot<<<cdiv(n, 256), 256, 0, st>>>(dStates, n, dt, g[0], g[1], g[2], flags, pos, vel, bounds);
+    if (dAgents) k_agent_bounds<<<cdiv(nAgents, 256), 256, 0, st>>>(snap, nAgents, bounds);
+    else k_agent_snapshot<true><<<cdiv(n, 256), 256, 0, st>>>(dStates, n, dt, g[0], g[1], g[2], flags, own, bounds);
     k_agent_grid_params<<<1, 1, 0, st>>>(bounds, radius, dt, gp);
-    k_agent_keys<<<cdiv(n, 256), 256, 0, st>>>(pos, n, gp, keys, vals);
+    k_agent_keys<<<cdiv(nAgents, 256), 256, 0, st>>>(snap, nAgents, gp, keys, vals);
     w->launches += 4;
-    CQ_TRY(radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, n, sortScratch, sortWords, st, false));
-    k_agent_gather<<<cdiv(n, 256), 256, 0, st>>>(vals, n, pos, vel, posS, velS);
-    k_agent_rows<<<cdiv(n, 256), 256, 0, st>>>(keys, vals, n, gp, rows);
+    CQ_TRY(radix_sort_pairs_onesweep(w, keys, vals, keysTmp, valsTmp, nAgents, sortScratch, sortWords, st, false));
+    k_agent_gather<<<cdiv(nAgents, 256), 256, 0, st>>>(vals, nAgents, snap, posS, velS);
+    k_agent_rows<<<cdiv(n, 256), 256, 0, st>>>(snap, first, n, keys, nAgents, gp, rows);
     w->launches += 2;
-    out.pos = posS, out.vel = velS, out.keys = keys, out.params = gp, out.rows = rows, out.firstHit = firstHit, out.n = n;
+    out.pos = posS, out.vel = velS, out.keys = keys, out.params = gp, out.rows = rows, out.firstHit = firstHit;
+    out.n = nAgents, out.first = first;
     return check_cuda(cudaGetLastError(), "agent grid");
 }
 

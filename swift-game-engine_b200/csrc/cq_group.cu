@@ -158,9 +158,18 @@ struct cq_group {
     std::vector<cudaStream_t> streams; // local groups: a stream per device for the collective calls
 };
 
+// One replica's buffers of cq_multi_move_and_slide_batch_ex with CQ_MAS_AGENTS, grown on demand.
+struct MultiAgentBuffers {
+    cq_character_state *states = nullptr; // the replica's shard
+    cq_agent_snapshot *snap = nullptr;    // the whole crowd's snapshot
+    cq_platform *platforms = nullptr;     // MAS_MAX_PLATFORMS records
+    size_t capStates = 0, capSnap = 0;
+};
+
 struct cq_multi_world {
     cq_group *group = nullptr;
     std::vector<cq_world *> replicas;
+    std::vector<MultiAgentBuffers> agentBufs; // one per replica
 };
 
 // every worker runs fn(i); the first failure (lowest device index) is reported in the caller's thread
@@ -193,6 +202,17 @@ template <class Fn> static int sharded(cq_multi_world *mw, int64_t n, Fn fn) { /
         cq_shard_range(n, ranks, i, &lo, &hi);
         return hi > lo ? fn(mw->replicas[i], lo, (int32_t)(hi - lo)) : CQ_OK;
     });
+}
+
+// a device buffer of at least `count` records of T on the current device; a larger one frees the old (the replica's
+// stream is idle between calls: every call ends with its synchronisation)
+template <class T> static int grow(T *&p, size_t &cap, size_t count, const char *what) {
+    if (count <= cap) return CQ_OK;
+    cudaFree(p);
+    p = nullptr, cap = 0;
+    CQ_TRY(check_cuda(cudaMalloc((void **)&p, count * sizeof(T)), what));
+    cap = count;
+    return CQ_OK;
 }
 
 extern "C" {
@@ -396,6 +416,11 @@ void cq_multi_world_destroy(cq_multi_world *mw) {
     if (!mw) return;
     int prev = 0;
     cudaGetDevice(&prev);
+    for (size_t i = 0; i < mw->agentBufs.size(); i++) {
+        MultiAgentBuffers &b = mw->agentBufs[i];
+        cudaSetDevice(mw->group->devices[i]);
+        cudaFree(b.states), cudaFree(b.snap), cudaFree(b.platforms);
+    }
     for (cq_world *w : mw->replicas)
         if (w) cq_world_destroy(w);
     cudaSetDevice(prev);
@@ -426,11 +451,72 @@ int cq_multi_move_and_slide_batch(cq_multi_world *mw, cq_character_state *inout,
                                   float dt, const float gravity[3], uint32_t flags) {
     if (n > 0 && !inout) return CQ_ERR_INVALID;
     if (flags & CQ_MAS_AGENTS) { // the batch is the crowd: agents of different shards would not see each other
-        set_error("cq_multi_move_and_slide_batch: CQ_MAS_AGENTS couples the characters of a batch; shard agent crowds by region");
+        set_error("cq_multi_move_and_slide_batch: CQ_MAS_AGENTS couples the characters of a batch; use cq_multi_move_and_slide_batch_ex");
         return CQ_ERR_INVALID;
     }
     return sharded(mw, n, [&](cq_world *w, int64_t lo, int32_t cnt) {
         return cq_move_and_slide_batch(w, inout + lo, cnt, params, dt, gravity, flags);
+    });
+}
+
+int cq_multi_move_and_slide_batch_ex(cq_multi_world *mw, cq_character_state *inout, int32_t n, const cq_controller_params *params,
+                                     float dt, const float gravity[3], uint32_t flags, const cq_platform *platforms,
+                                     int32_t n_platforms) {
+    if (!mw || n < 0 || !params || !gravity || (n > 0 && !inout) || n_platforms < 0 || n_platforms > 64 ||
+        (n_platforms > 0 && !platforms)) {
+        set_error("cq_multi_move_and_slide_batch_ex: invalid arguments (0..64 host platforms)");
+        return CQ_ERR_INVALID;
+    }
+    if (!(flags & CQ_MAS_AGENTS))
+        return sharded(mw, n, [&](cq_world *w, int64_t lo, int32_t cnt) {
+            return cq_move_and_slide_batch_ex(w, inout + lo, cnt, params, dt, gravity, flags, platforms, n_platforms);
+        });
+    if (n == 0) return CQ_OK;
+    const int ranks = (int)mw->replicas.size();
+    mw->agentBufs.resize(ranks);
+    // 1. every replica uploads its shard and snapshots it into its range of a crowd-sized snapshot
+    CQ_TRY(on_every_device(mw->group, [&](int i) {
+        cq_world *w = mw->replicas[i];
+        MultiAgentBuffers &b = mw->agentBufs[i];
+        int64_t lo, hi;
+        cq_shard_range(n, ranks, i, &lo, &hi);
+        const int32_t cnt = (int32_t)(hi - lo);
+        CQ_TRY(grow(b.states, b.capStates, (size_t)std::max(cnt, 1), "multi agents: shard"));
+        CQ_TRY(grow(b.snap, b.capSnap, (size_t)n, "multi agents: snapshot"));
+        if (!b.platforms) CQ_CUDA(cudaMalloc((void **)&b.platforms, 64 * sizeof(cq_platform)));
+        CQ_NO_CAPTURE(w->stream, "cq_multi_move_and_slide_batch_ex");
+        if (cnt == 0) return CQ_OK;
+        CQ_CUDA(cudaMemcpyAsync(b.states, inout + lo, sizeof(cq_character_state) * (size_t)cnt, cudaMemcpyHostToDevice, w->stream));
+        return cq_agent_snapshot_device(w, b.states, cnt, dt, gravity, flags, b.snap + lo, w->stream);
+    }));
+    // 2. one all-gather of the 32-byte records, in place, on the replicas' streams (ordered after the snapshots)
+    std::vector<const void *> local(ranks);
+    std::vector<void *> all(ranks), streams(ranks);
+    for (int i = 0; i < ranks; i++) {
+        int64_t lo, hi;
+        cq_shard_range(n, ranks, i, &lo, &hi);
+        local[i] = mw->agentBufs[i].snap + lo;
+        all[i] = mw->agentBufs[i].snap;
+        streams[i] = (void *)mw->replicas[i]->stream;
+    }
+    CQ_TRY(cq_group_gather_records_local(mw->group, local.data(), n, sizeof(cq_agent_snapshot), all.data(), streams.data()));
+    // 3. every replica moves its shard against the whole snapshot and downloads it
+    return on_every_device(mw->group, [&](int i) {
+        cq_world *w = mw->replicas[i];
+        MultiAgentBuffers &b = mw->agentBufs[i];
+        int64_t lo, hi;
+        cq_shard_range(n, ranks, i, &lo, &hi);
+        const int32_t cnt = (int32_t)(hi - lo);
+        if (n_platforms > 0)
+            CQ_CUDA(cudaMemcpyAsync(b.platforms, platforms, sizeof(cq_platform) * (size_t)n_platforms, cudaMemcpyHostToDevice,
+                                    w->stream));
+        if (cnt > 0) {
+            CQ_TRY(cq_move_and_slide_device_agents(w, b.states, cnt, b.snap, n, (int32_t)lo, params, dt, gravity, flags, b.platforms,
+                                                   n_platforms, w->stream));
+            CQ_CUDA(cudaMemcpyAsync(inout + lo, b.states, sizeof(cq_character_state) * (size_t)cnt, cudaMemcpyDeviceToHost, w->stream));
+        }
+        CQ_CUDA(cudaStreamSynchronize(w->stream));
+        return check_status(w, "cq_multi_move_and_slide_batch_ex");
     });
 }
 

@@ -287,11 +287,18 @@ void free_set(DeviceSet &S);
 int take_unit_order(cq_world *w, int n, cudaStream_t st, uint32_t **scratch);
 int make_unit_order(cq_world *w, uint32_t *scratch, const void *dUnits, size_t stride, bool positionIsDouble, int n,
                     cudaStream_t st, const uint32_t **order);
-// CQ_MAS_AGENTS pre-pass of n agents: take_agent_grid takes its scratch for `st` (take_scratch); make_agent_grid enqueues
-// the snapshot (after the gravity rule), XZ grid and sort by cell into that scratch on `st`.
-int take_agent_grid(cq_world *w, int n, cudaStream_t st, void **scratch);
-int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, int n, float radius, float dt,
-                    const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out);
+// CQ_MAS_AGENTS pre-pass of a launch that moves n characters, agents first .. first + n - 1 of a crowd of nAgents.
+// take_agent_grid takes the grid's scratch for `st` (take_scratch): sort side nAgents-sized, per-character rows n-sized,
+// plus room for the snapshot when the launch takes its own (ownSnapshot: the single-batch step, first = 0, nAgents = n).
+// make_agent_grid enqueues on `st`: the snapshot of dStates (after the gravity rule) into that scratch when dAgents is
+// nullptr, else the bounds of the snapshot dAgents; then the XZ grid and sort by cell over all nAgents, and the cell
+// ranges of the n moving characters.
+int take_agent_grid(cq_world *w, int nAgents, int n, bool ownSnapshot, cudaStream_t st, void **scratch);
+int make_agent_grid(cq_world *w, void *scratch, const cq_character_state *dStates, const cq_agent_snapshot *dAgents, int nAgents,
+                    int first, int n, float radius, float dt, const float g[3], uint32_t flags, cudaStream_t st, AgentGrid &out);
+// cq_agent_snapshot_device: n > 0 snapshot records of dStates into dOut, one launch on `st`
+int launch_agent_snapshot(cq_world *w, const cq_character_state *dStates, int n, float dt, const float g[3], uint32_t flags,
+                          cq_agent_snapshot *dOut, cudaStream_t st);
 
 // 32-bit key / value LSD radix sort (onesweep); `scratch` holds sort_scratch_words(n) words.  Result in (keys, vals).
 size_t sort_scratch_words(int n);
@@ -323,9 +330,12 @@ int launch_overlap_all(cq_world *w, const cq_capsule *d_q, int n, int maxHits, c
 // cq_mas.cu
 // Kinematic platforms come either as a host array `platforms` (at most 64, copied into the kernel arguments, so a captured
 // graph keeps them) or, when dPlatforms is non-null, as a device array the kernels read when they execute (any count).
+// CQ_MAS_AGENTS: dAgents = nullptr makes the batch the crowd; otherwise the batch is agents first .. first + n - 1 of
+// the nAgents-record snapshot dAgents.
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
                           const float g[3], uint32_t flags, const cq_platform *platforms, const cq_platform *dPlatforms,
-                          int nPlatforms, cudaStream_t st);
+                          int nPlatforms, cudaStream_t st, const cq_agent_snapshot *dAgents = nullptr, int nAgents = 0,
+                          int first = 0);
 // cq_sep.cu
 void sep_graphs_destroy(cq_world *w);
 // Queues the whole separation on `st` without waiting for the device; the outcome goes to d_status (may be nullptr).

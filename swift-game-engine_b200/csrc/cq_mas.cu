@@ -95,7 +95,7 @@ __device__ __noinline__ f3 platform_carry_delta(f3 position, const cq_controller
 
 // AgentSweepSolver.bestHit (SYS:1053-1091) over the grid cells the sweep can reach instead of every agent.  Exact:
 // an agent outside the reach box cannot produce a hit, and ties keep the smallest index, which is what the
-// reference's strict `<` over its index-ordered loop keeps.
+// reference's strict `<` over its index-ordered loop keeps.  selfIndex: the character's index in the launch (agent G.first + selfIndex).
 __device__ __noinline__ bool agent_best_hit(const AgentGrid &G, f3 position, f3 remaining, float remainingLen, float baseMoveLen,
                                             float dt, int selfIndex, float radius, float halfHeight, AgentHit &best) {
     const AgentGridParams gp = *G.params;
@@ -133,7 +133,7 @@ __device__ __noinline__ bool agent_best_hit(const AgentGrid &G, f3 position, f3 
         for (; j < end; j++) {
             const float4 op = __ldg(G.pos + j);
             const int other = __float_as_int(op.w);
-            if (other == selfIndex) continue;
+            if (other - G.first == selfIndex) continue;
             // cheap exact reject: farther apart in XZ than the reach -> the sweep cannot hit
             const float dx = op.x - position.x, dz = op.z - position.z;
             if (dx * dx + dz * dz > reach * reach) continue;
@@ -801,7 +801,7 @@ __global__ void __launch_bounds__(MAS_THREADS, MAS_MIN_BLOCKS) k_move_and_slide(
 
 int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const cq_controller_params &p, float dt,
                           const float g[3], uint32_t flags, const cq_platform *platforms, const cq_platform *dPlatforms,
-                          int nPlatforms, cudaStream_t st) {
+                          int nPlatforms, cudaStream_t st, const cq_agent_snapshot *dAgents, int nAgents, int first) {
     if (n <= 0) return CQ_OK;
     if (!dPlatforms && (nPlatforms < 0 || nPlatforms > MAS_MAX_PLATFORMS || (nPlatforms > 0 && !platforms))) {
         set_error("cq_move_and_slide: 0..%d platforms supported, got %d", MAS_MAX_PLATFORMS, nPlatforms);
@@ -828,14 +828,15 @@ int launch_move_and_slide(cq_world *w, cq_character_state *d_inout, int n, const
                                           k_move_and_slide<false, true, true>, k_move_and_slide<true, true, true>}};
     const Kernel kernel = kernels[agents ? 1 : 0][ci];
     void *agentScratch = nullptr;
-    if (agents) CQ_TRY(take_agent_grid(w, n, st, &agentScratch));
+    if (!dAgents) nAgents = n, first = 0;
+    if (agents) CQ_TRY(take_agent_grid(w, nAgents, n, dAgents == nullptr, st, &agentScratch));
     // persistent lanes: one resident wave of CTAs, lanes stride over characters; small batches still fill the machine
     // (>= 4 units per CTA)
     PoolLaunch L;
     CQ_TRY(pool_launch_setup(w, (const void *)kernel, MAS_THREADS, MAS_SMEM_BYTES, 4, n, true, d_inout, sizeof(cq_character_state),
                              true, st, L));
     if (agents) {
-        CQ_TRY(make_agent_grid(w, agentScratch, d_inout, n, p.radius, dt, g, flags, st, A.agents));
+        CQ_TRY(make_agent_grid(w, agentScratch, d_inout, dAgents, nAgents, first, n, p.radius, dt, g, flags, st, A.agents));
         k_agent_first_hit<<<(n + 255) / 256, 256, 0, st>>>(d_inout, n, A);
         w->launches++;
     }

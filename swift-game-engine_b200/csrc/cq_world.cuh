@@ -77,8 +77,10 @@ struct WorldView {
                       // (worlds that do not fit L1); the tiny-world variant keeps the shorter per-lane loop
 };
 
-// Snapshot of every agent of a move-and-slide batch, taken before any character of the step moves
-// (collectAgentStates, Systems.swift:1592-1611), binned into a uniform XZ grid and sorted by cell key.
+// Snapshot of every agent of a crowd, taken before any character of the step moves (collectAgentStates,
+// Systems.swift:1592-1611; one cq_agent_snapshot per agent), binned into a uniform XZ grid and sorted by cell key.  The
+// launch moves characters 0..n) of its batch, which are agents first .. first + n - 1 of the crowd: the whole crowd when
+// first = 0 and the grid holds n agents, one slice of it otherwise.
 struct AgentGridParams { // written by k_agent_grid_params, read by the move-and-slide kernel
     float originX, originZ, invCell, cell;
     int dimX, dimZ;
@@ -90,11 +92,12 @@ struct AgentGrid {
     const float4 *vel;  // same order
     const uint32_t *keys; // sorted cell keys: iz * dimX + ix
     const AgentGridParams *params;
-    const int4 *rows; // per ORIGINAL index, 2 x int4: (start,end) in the sorted arrays of the cells ix-1..ix+1 of the rows
-                      // iz-1, iz, iz+1 around the agent's snapshot cell, then (ix, iz) -- found once, in parallel
-    float4 *firstHit; // per ORIGINAL index: (normal, toi) of the agent hit of the FIRST slide iteration, computed by a
-                      // pre-pass under the assumption that depenetration does not move the character; toi -1 = none
-    int n;
+    const int4 *rows; // per character of the launch, 2 x int4: (start,end) in the sorted arrays of the cells ix-1..ix+1 of
+                      // the rows iz-1, iz, iz+1 around its snapshot cell, then (ix, iz) -- found once, in parallel
+    float4 *firstHit; // per character of the launch: (normal, toi) of the agent hit of the FIRST slide iteration, computed
+                      // by a pre-pass under the assumption that depenetration does not move the character; toi -1 = none
+    int n;            // agents in the grid
+    int first;        // agent index of the launch's character 0
 };
 __device__ __forceinline__ int agent_cell(float x, float origin, float invCell, int dim) { // monotonic in x
     float c = floorf((x - origin) * invCell);

@@ -280,6 +280,44 @@ public final class CollisionQuery {
         return rc == CQ_OK
     }
 
+    /// cq_agent_snapshot_device: the agent snapshot of `count` resident records (device) written to `out` (device, 16-byte
+    /// aligned), as an agents step with the same dt, gravity and flags takes it.  A crowd moved in slices writes every
+    /// slice's snapshot into its range of one crowd-wide array, makes the array whole, then calls moveAndSlideAgents.
+    public func agentSnapshotDevice(states: UnsafePointer<cq_character_state>, count: Int32, dt: Float,
+                                    gravity: SIMD3<Float> = SIMD3<Float>(0, -98, 0), out: UnsafeMutablePointer<cq_agent_snapshot>,
+                                    applyGravity: Bool = true, stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        var g = (gravity.x, gravity.y, gravity.z)
+        let flags = (applyGravity ? UInt32(CQ_MAS_APPLY_GRAVITY) : 0) | UInt32(CQ_MAS_AGENTS)
+        let rc = withUnsafePointer(to: &g) { gp in
+            gp.withMemoryRebound(to: Float.self, capacity: 3) {
+                cq_agent_snapshot_device(handle, states, count, dt, $0, flags, out, stream)
+            }
+        }
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
+    /// cq_move_and_slide_device_agents: one agents step of `count` resident records, which are agents
+    /// firstAgent ..< firstAgent + count of the crowd snapshot `agents` (device, agentCount records).  Every slice of a crowd
+    /// snapshotted, then each moved: the records of one agents moveAndSlideDevice call on the whole crowd, byte for byte.
+    public func moveAndSlideAgents(states: UnsafeMutablePointer<cq_character_state>, count: Int32,
+                                   agents: UnsafePointer<cq_agent_snapshot>, agentCount: Int32, firstAgent: Int32,
+                                   params: cq_controller_params, dt: Float, gravity: SIMD3<Float> = SIMD3<Float>(0, -98, 0),
+                                   platforms: UnsafePointer<cq_platform>? = nil, platformCount: Int32 = 0,
+                                   applyGravity: Bool = true, stream: UnsafeMutableRawPointer? = nil) -> Bool {
+        var p = params
+        var g = (gravity.x, gravity.y, gravity.z)
+        let flags = (applyGravity ? UInt32(CQ_MAS_APPLY_GRAVITY) : 0) | UInt32(CQ_MAS_AGENTS)
+        let rc = withUnsafePointer(to: &g) { gp in
+            gp.withMemoryRebound(to: Float.self, capacity: 3) {
+                cq_move_and_slide_device_agents(handle, states, count, agents, agentCount, firstAgent, &p, dt, $0, flags,
+                                                platforms, platformCount, stream)
+            }
+        }
+        lastError = rc == CQ_OK ? nil : String(cString: cq_last_error())
+        return rc == CQ_OK
+    }
+
     /// Entities with Transform + StaticMesh (collides), ascending id (the reference iterates a Dictionary, i.e. in
     /// per-process random order — World.swift:99-118; the library fixes the order so triangle numbering is stable).
     /// Geometry is returned as plain Swift arrays; `withArrays` lends their storage to the C structs for one call.
